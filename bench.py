@@ -4,6 +4,7 @@
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
   python bench.py --impl reference [--gpus N] ...               # CPU oracle port, host cores, same config
   torchrun ... bench.py --gpus N ...                            # one rank per GPU (N > 1)
+  python bench.py ... --dump-outputs DIR                        # + the last timed frame's outputs as DIR/<name>.npy
 
 Headline workload (config.workload = "C3", BASELINE.json configs[2], the north_star frame and the largest
 single-GPU configuration): HDL-64E-shaped 120 000-ray scans, 10 000 keypoints per frame, frame-to-frame:
@@ -24,6 +25,11 @@ whole path.  The detector / normals run in the only mode there is: the reference
  * extra objects at N = 1: "c2" (BASELINE.json configs[1]: HDL-32E sequence, K = 2 048, per-frame p50 / p99 over
            500 distinct frames), "c3_radius_sweep" (extraction throughput over the SHOT radius, FULL normals).
  * --impl reference: the oracle port of the reference's CPU path on all host cores, same config / frames / metric.
+ * --dump-outputs DIR: what the last timed step of the headline path computed, as a caller of bshot_process_frame_dev
+           receives it (bshot_fetch_frame), in float arrays so that two builds can be compared output for output: kp_idx
+           (K), descriptor_bits (K x 352, one 0 / 1 per bit) and pairs (P x 2, query / target keypoint ordinals).  The
+           frames are seeded, so the same arguments give the same inputs on every run.
+The benchmark writes nothing into the source tree (no bytecode either): that tree may be read-only.
 """
 import argparse
 import json
@@ -35,6 +41,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 from conftest import load_bshot, load_oracle, load_sharded, load_synth  # noqa: E402  (loaders only, no pytest needed)
 
@@ -45,6 +52,7 @@ WORKLOADS = {  # name: (sensor, rays per frame, keypoints per frame, distinct fr
     "C2": ("hdl32e", 69440, 2048, 12),
 }
 METRIC, UNIT = "bshot_frontend_descriptors_per_s", "descriptors/s"
+DUMP_LIMIT_BYTES = 64 << 20
 
 
 def peaks():
@@ -152,23 +160,17 @@ def run_reference(args, rank):
     oracle, synth = load_oracle(), load_synth()
     cores = os.cpu_count() or 1
     frames = make_frames(synth, args.workload)
-    W, K = max(args.warmup, 3), max(args.steps, 1)
+    W, K = max(args.warmup, 3), args.steps
     prev = None
-    t_first, prev = cpu_front_end(oracle, frames[:1], args.top_k, cores)
-    # bound the run: a few minutes at most (the driver's default K = 20 takes well under one)
-    budget_frames = max(2, int(150.0 / max(t_first, 1e-3)))
-    k_timed = min(K, budget_frames)
-    for i in range(1, min(W, 2)):
+    for i in range(W):
         _, prev = cpu_front_end(oracle, [frames[i % len(frames)]], args.top_k, cores, prev=prev)
     per = []
-    for s in range(k_timed):
+    for s in range(K):
         t, prev = cpu_front_end(oracle, [frames[(W + s) % len(frames)]], args.top_k, cores, prev=prev)
         per.append(t)
     sec = float(np.mean(per))
     val = args.top_k / sec
-    sample = f"{k_timed} whole frames of this workload (detector + top-K + normals + SHOT + B-SHOT + match), OpenMP over {cores} threads"
-    if k_timed < K:
-        sample += f"; the remaining {K - k_timed} steps are the same frames again and were extrapolated from this mean"
+    sample = f"{K} whole frames of this workload (detector + top-K + normals + SHOT + B-SHOT + match), OpenMP over {cores} threads"
     line = {
         "impl": "reference", "metric": METRIC, "value": val, "unit": UNIT, "n_gpus": args.gpus, "steps": K, "warmup": W,
         "ms_per_step": sec * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32/f64+u32",
@@ -177,6 +179,22 @@ def run_reference(args, rank):
         "e2e": {"value": val, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }
     print(json.dumps(line))
+
+
+def dump_outputs(out_dir, synth, frame):
+    """one frame's outputs (Context.fetch_frame) as DIR/<name>.npy in float32 / float64; above DUMP_LIMIT_BYTES in all,
+    descriptor_bits keeps a seeded sample of its rows and descriptor_rows says which"""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"kp_idx": frame["kp_idx"].astype(np.float64), "pairs": frame["pairs"].astype(np.float64)}
+    bits = synth.unpack_bits(frame["bits"]).astype(np.float32)
+    room = DUMP_LIMIT_BYTES - sum(a.nbytes for a in arrays.values())
+    if bits.nbytes > room:
+        rows = np.sort(np.random.default_rng(0).choice(len(bits), room // (bits.shape[1] * 4 + 8), replace=False))
+        arrays["descriptor_rows"] = rows.astype(np.float64)
+        bits = bits[rows]
+    arrays["descriptor_bits"] = bits
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def percentile_summary(x):
@@ -200,7 +218,10 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the C2 sequence and the C3 SHOT-radius sweep objects")
     ap.add_argument("--map-only", action="store_true", help="debug: print only the map_match object")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed frame's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.top_k is None:
         args.top_k = WORKLOADS[args.workload][2]
 
@@ -208,6 +229,8 @@ def main():
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs: the outputs are those of the CUDA path (--impl ours)")
         run_reference(args, rank)
         return
 
@@ -221,7 +244,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     bs, synth = load_bshot(), load_synth()
     W = max(args.warmup, 3)
-    K = max(args.steps, 1)
+    K = args.steps
     hbm_peak, peak_src = peaks()
 
     def barrier():
@@ -294,6 +317,8 @@ def main():
     if sampler:
         sampler.active = False
     launches = ctx.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, synth, ctx.fetch_frame(args.top_k))
     per_step = [a.elapsed_time(b) for a, b in ev]
     ms_total = max_over_ranks(sum(per_step))
     ms_step = ms_total / K

@@ -5,12 +5,15 @@ CPU: it compiles/links and fails loudly without a GPU.  GPU: the reference's cal
 import os
 import struct
 import subprocess
+import sys
 
 import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "b-shot-slam_b200")
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+from snapshots import ExpectedPreprocessing, Snapshots  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -31,7 +34,7 @@ def test_shims_compile_and_fail_loudly_without_gpu(shim_binary):
 
 
 @pytest.mark.gpu
-def test_reference_call_order_two_frames(shim_binary, tmp_path, oracle, synth):
+def test_reference_call_order_two_frames(shim_binary, tmp_path, oracle, synth, gpu_ctx):
     scans = [synth.make_scan("hdl32e", f)[::2].copy() for f in (0, 1)]
     paths = []
     for i, s in enumerate(scans):
@@ -45,10 +48,13 @@ def test_reference_call_order_two_frames(shim_binary, tmp_path, oracle, synth):
         fh.write(L["azimuth"].tobytes() + L["vertical"].tobytes() + L["distance"].tobytes())
     r = subprocess.run([shim_binary, paths[0], paths[1], outp, lasers, pre_out], capture_output=True, text=True)
     assert r.returncode == 0, r.stdout + r.stderr
-    # myslam::Preprocessor shim == the reference's preprocess.cpp compiled unchanged
-    if oracle.ref_lib() is not None:
-        got = np.fromfile(pre_out, np.float32).reshape(-1, 3)
-        assert np.array_equal(got, oracle.ref_preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"]))
+    # myslam::Preprocessor shim == the reference's preprocess.cpp compiled unchanged where it is built, and everywhere
+    # the regression snapshot of the device preprocessor (tests/golden/snapshots.py)
+    got = np.fromfile(pre_out, np.float32).reshape(-1, 3)
+    snapshots = Snapshots()
+    want = ExpectedPreprocessing(snapshots, oracle, gpu_ctx).preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"])
+    snapshots.save()
+    want.check(got, "preprocessed points")
     raw = open(outp, "rb").read()
     off, frames, rest = 0, [], []
     for _ in range(2):

@@ -1,8 +1,9 @@
 """Scan preprocessor (SURVEY 8f #4): bshot_preprocess against myslam::Preprocessor::run of the reference
 (src/preprocess.cpp:213-223).  The checker is the reference's OWN source compiled unchanged (oracle/_ref/libbshot_ref.so,
-built by oracle/Makefile `ref`; it travels to the GPU box) plus golden vectors made by it (tests/golden/preprocess_pin.npz,
-tests/golden/make_preprocess_pin.py), which hold on any machine.  Bar: same number of points, the same coordinates bit for
-bit, in the same order."""
+built by oracle/Makefile `ref` where the reference sources are at hand).  Golden vectors made by it
+(tests/golden/preprocess_pin.npz, tests/golden/make_preprocess_pin.py) hold on any machine.  The other device cases below
+compare live with that library where it is built, and everywhere with a regression snapshot of the device output
+(tests/golden/snapshots.py).  Bar: same number of points, the same coordinates bit for bit, in the same order."""
 import os
 import sys
 import zlib
@@ -13,6 +14,7 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, "golden"))
 from make_preprocess_pin import CASES, lasers_crc  # noqa: E402
+from snapshots import ExpectedPreprocessing, Snapshots  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -23,11 +25,22 @@ def pin():
 @pytest.fixture(scope="module")
 def ref(oracle):
     if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref/libbshot_ref.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libbshot_ref.so not built (needs the reference sources at build time)")
     return oracle
 
 
+@pytest.fixture(scope="module")
+def expected(oracle, gpu_ctx):
+    """what the device tests below must return (tests/golden/snapshots.py)"""
+    snapshots = Snapshots()
+    yield ExpectedPreprocessing(snapshots, oracle, gpu_ctx)
+    snapshots.save()
+
+
 def same_points(a, b):
+    if hasattr(b, "check"):        # an expectation of tests/golden/snapshots.py
+        b.check(a, "points")
+        return
     assert a.shape == b.shape, f"{a.shape[0]} points, expected {b.shape[0]}"
     diff = (a.view(np.uint32) != b.view(np.uint32)).any(axis=1)
     assert not diff.any(), f"{int(diff.sum())} of {len(a)} points differ, first at {int(np.argmax(diff))}: {a[np.argmax(diff)]} vs {b[np.argmax(diff)]}"
@@ -93,9 +106,9 @@ def test_gpu_matches_reference_made_vectors(gpu_ctx, synth, pin, name):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("sensor,frame", [("hdl32e", 0), ("hdl32e", 5), ("hdl64e", 1)])
-def test_gpu_matches_reference_on_a_full_rotation(gpu_ctx, ref, synth, sensor, frame):
+def test_gpu_matches_reference_on_a_full_rotation(gpu_ctx, expected, synth, sensor, frame):
     L = synth.make_lasers(sensor, frame)
-    want = ref.ref_preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"])
+    want = expected.preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"])
     assert 0.2 * L["distance"].size < len(want) < 0.9 * L["distance"].size   # the ground is a large part of the scan
     same_points(gpu_ctx.preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"]), want)
     # the same rotation sorted the way `capture.retrieve(lasers, true)` sorts it: nothing changes
@@ -104,21 +117,21 @@ def test_gpu_matches_reference_on_a_full_rotation(gpu_ctx, ref, synth, sensor, f
 
 
 @pytest.mark.gpu
-def test_gpu_other_thresholds(gpu_ctx, ref, synth):
+def test_gpu_other_thresholds(gpu_ctx, expected, synth):
     L = synth.make_lasers("hdl32e", 3)
     for vert_init, lowpt in ((-0.6, -1700.0), (-0.55, -2200.0), (-0.7, -1950.0)):
-        want = ref.ref_preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"], vert_init, lowpt)
+        want = expected.preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"], vert_init, lowpt)
         same_points(gpu_ctx.preprocess(L["azimuth"], L["vertical"], L["distance"], L["ring_deg"], vert_init, lowpt), want)
 
 
 @pytest.mark.gpu
-def test_gpu_edge_cases(gpu_ctx, ref, bshot):
+def test_gpu_edge_cases(gpu_ctx, expected, bshot):
     rng = np.random.default_rng(5)
     empty = gpu_ctx.preprocess(np.zeros(0), np.zeros(0), np.zeros(0, np.uint16), RING)
     assert empty.shape == (0, 3)
 
     def both(L, ring=RING):
-        want = ref.ref_preprocess(L["azimuth"], L["vertical"], L["distance"], ring)
+        want = expected.preprocess(L["azimuth"], L["vertical"], L["distance"], ring)
         same_points(gpu_ctx.preprocess(L["azimuth"], L["vertical"], L["distance"], ring), want)
         return want
 
@@ -153,7 +166,7 @@ def test_gpu_edge_cases(gpu_ctx, ref, bshot):
     assert len(w) < 60 * 6
     # no ring table: the occlusion pass has nothing to walk
     L = cat(cols)
-    same_points(gpu_ctx.preprocess(L["azimuth"], L["vertical"], L["distance"], np.zeros(0)), ref.ref_preprocess(L["azimuth"], L["vertical"], L["distance"], np.zeros(0)))
+    same_points(gpu_ctx.preprocess(L["azimuth"], L["vertical"], L["distance"], np.zeros(0)), expected.preprocess(L["azimuth"], L["vertical"], L["distance"], np.zeros(0)))
     # random soup: arbitrary double azimuths incl. negative and -0.0 / +0.0 as one key
     n = 5000
     az = rng.choice(np.concatenate([rng.uniform(-5.0, 5.0, 300), [0.0, -0.0]]), n)
@@ -162,22 +175,22 @@ def test_gpu_edge_cases(gpu_ctx, ref, bshot):
 
 
 @pytest.mark.gpu
-def test_gpu_point_selection(gpu_ctx, ref, synth):
+def test_gpu_point_selection(gpu_ctx, expected, synth):
     """setSelectedPoints / haveSelectList / saveSelectPoints (test/odometry_test.cpp:144-160): selected returns only, or
     everything but them; an unsorted list with a duplicate (the cursor of readFrame stops advancing at it)"""
     L = synth.make_lasers("hdl32e", 1, firings=400, start_deg=200.0)
     n = L["azimuth"].size
     rng = np.random.default_rng(2)
     args = (L["azimuth"], L["vertical"], L["distance"], L["ring_deg"])
-    everything = ref.ref_preprocess(*args)
+    everything = expected.preprocess(*args)
     for sel in (np.arange(0, n, 3), rng.permutation(n)[: n // 2], np.array([5, 900, 900, 4000, 7000]), np.zeros(0, np.int32), np.array([n + 5, -3, 10])):
         for save in (True, False):
-            want = ref.ref_preprocess(*args, select=sel, save_selected=save)
+            want = expected.preprocess(*args, select=sel, save_selected=save)
             same_points(gpu_ctx.preprocess(*args, select=sel, save_selected=save), want)
-        kept = len(ref.ref_preprocess(*args, select=sel, save_selected=True)) + len(ref.ref_preprocess(*args, select=sel, save_selected=False))
+        kept = len(expected.preprocess(*args, select=sel, save_selected=True)) + len(expected.preprocess(*args, select=sel, save_selected=False))
         assert kept == len(everything)
     # no list but "save the unselected": nothing is written
-    assert len(gpu_ctx.preprocess(*args, save_selected=False)) == len(ref.ref_preprocess(*args, save_selected=False)) == 0
+    assert len(gpu_ctx.preprocess(*args, save_selected=False)) == len(expected.preprocess(*args, save_selected=False)) == 0
 
 
 @pytest.mark.gpu

@@ -1,18 +1,21 @@
-"""Pins the oracle and the CUDA path to REFERENCE-COMPILED code: oracle/_ref/libbshot_ref.so is
-/root/reference/include/bshot_bits.h compiled unchanged (oracle/ref_shim.cpp; PCL names -> oracle/pcl_stub).
+"""Pins the oracle and the CUDA path to REFERENCE-COMPILED code: oracle/_ref/libbshot_ref.so is the reference's
+include/bshot_bits.h compiled unchanged (oracle/ref_shim.cpp; PCL names -> oracle/pcl_stub).
  * golden vectors produced by that library (tests/golden/ref_pin.npz, made by tests/golden/make_ref_pin.py) are
    checked on every machine, CPU (oracle) and GPU (-m gpu, through the C ABI);
- * where the library itself is present (build container, and the GPU box -- the .so travels), larger random cases
-   are compared live.
+ * larger random cases are compared live with that library where it is built, and everywhere with a regression
+   snapshot of the oracle's output (tests/golden/snapshots.py); minVect is checked where the library is built.
 Pinned outright (reference arithmetic end to end): compute_bshot_from_SHOT (include/bshot_bits.h:144-278), minVect
 (:6-20) and the std::bitset<352> record.  Pinned as control flow + data placement around the oracle's PCL
 restatement: calculate_normals (:43-94, keypoint-ordinal placement, persistent cloud1_normals) and calculate_SHOT."""
 import os
+import sys
 
 import numpy as np
 import pytest
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+sys.path.insert(0, os.path.join(HERE, "golden"))
+from snapshots import Snapshots  # noqa: E402
 
 
 @pytest.fixture(scope="module")
@@ -23,8 +26,37 @@ def pin():
 @pytest.fixture(scope="module")
 def ref(oracle):
     if oracle.ref_lib() is None:
-        pytest.skip("oracle/_ref/libbshot_ref.so not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/libbshot_ref.so not built (needs the reference sources at build time)")
     return oracle
+
+
+class ExpectedReference:
+    """expected output of bshot::compute_bshot_from_SHOT and of the featureMatching loops: snapshot of the oracle's output,
+    plus the reference-compiled library's (oracle/_ref) where it is built"""
+
+    def __init__(self, snapshots, oracle):
+        self.snapshots, self.oracle = snapshots, oracle
+        self.built = oracle.ref_lib() is not None
+
+    def _oracle_matching(self, q, t):
+        m = self.oracle.match(q, t)
+        return dict(left_idx=m["left_idx"], right_idx=m["right_idx"], pairs=self.oracle.mutual(m["left_idx"], m["right_idx"]))
+
+    def bshot(self, shot):
+        return self.snapshots.expect("bshot_from_shot", (np.ascontiguousarray(shot, dtype=np.float32),), self.oracle.bshot, "oracle",
+                                     self.oracle.ref_bshot if self.built else None)
+
+    def feature_matching(self, q, t):
+        args = (np.ascontiguousarray(q, dtype=np.uint64), np.ascontiguousarray(t, dtype=np.uint64))
+        return self.snapshots.expect("feature_matching", args, self._oracle_matching, "oracle",
+                                     self.oracle.ref_feature_matching if self.built else None)
+
+
+@pytest.fixture(scope="module")
+def expected(oracle):
+    snapshots = Snapshots()
+    yield ExpectedReference(snapshots, oracle)
+    snapshots.save()
 
 
 def flow_frames(synth, pin):
@@ -63,13 +95,13 @@ def test_orc_descriptor_flow_matches_reference_vectors(oracle, synth, pin):
     assert np.array_equal(oracle.bshot(shot), pin["flow_bits1"])
 
 
-# ---- live comparison with the reference-compiled library ------------------------------------------------------
-def test_live_bshot_random(ref):
+# ---- live comparison with the reference-compiled library where it is built, snapshots everywhere -------------
+def test_live_bshot_random(oracle, expected):
     rng = np.random.default_rng(5)
     s = (rng.random((4000, 352)) ** 8).astype(np.float32)
     s[rng.random(s.shape) < 0.6] = 0
     s[rng.random(s.shape) < 0.001] = np.nan
-    assert np.array_equal(ref.ref_bshot(s), ref.bshot(s))
+    expected.bshot(s).check(oracle.bshot(s), "B-SHOT bits")
 
 
 def test_live_minvect_first_minimum(ref):
@@ -79,14 +111,15 @@ def test_live_minvect_first_minimum(ref):
 
 
 @pytest.mark.parametrize("nq,nt,seed", [(1, 1, 0), (7, 300, 1), (300, 7, 2), (257, 511, 3)])
-def test_live_feature_matching(ref, synth, nq, nt, seed):
+def test_live_feature_matching(oracle, expected, synth, nq, nt, seed):
     q = synth.random_descriptors(nq, seed=100 + seed, density=30)
     t = synth.random_descriptors(nt, seed=200 + seed, density=30)
     t[nt // 2:] = t[: nt - nt // 2]                     # duplicated targets: ties everywhere
-    r = ref.ref_feature_matching(q, t)
-    m = ref.match(q, t)
-    assert np.array_equal(m["left_idx"], r["left_idx"]) and np.array_equal(m["right_idx"], r["right_idx"])
-    assert np.array_equal(ref.mutual(m["left_idx"], m["right_idx"]), r["pairs"])
+    r = expected.feature_matching(q, t)
+    m = oracle.match(q, t)
+    r["left_idx"].check(m["left_idx"], "left_idx")
+    r["right_idx"].check(m["right_idx"], "right_idx")
+    r["pairs"].check(oracle.mutual(m["left_idx"], m["right_idx"]), "pairs")
 
 
 # ---- the CUDA path vs the same reference-made vectors --------------------------------------------------------
