@@ -36,6 +36,7 @@ EXPORTS = [
     "bshot_match_map_sharded", "bshot_gmap_create", "bshot_gmap_reset", "bshot_gmap_size", "bshot_gmap_add",
     "bshot_gmap_update_from_frame", "bshot_gmap_get_keypoints", "bshot_extract_frame", "bshot_match_frame_to_map", "bshot_frame_commit", "bshot_ransac",
     "bshot_preprocess", "bshot_preprocess_select", "bshot_extract_scan", "bshot_icp", "bshot_evaluate_estimation", "bshot_set_matcher",
+    "bshot_iss_params_default", "bshot_detect_iss", "bshot_kp_repeatability",
 ]
 
 
@@ -44,6 +45,13 @@ class Params(C.Structure):
                 ("top_k", C.c_int), ("normal_radius", C.c_float), ("normal_max_nn", C.c_int),
                 ("normals_mode", C.c_int), ("shot_radius", C.c_float)]
 
+
+class IssParams(C.Structure):
+    _fields_ = [("salient_radius", C.c_float), ("non_max_radius", C.c_float), ("gamma_21", C.c_double),
+                ("gamma_32", C.c_double), ("min_neighbors", C.c_int)]
+
+
+E_CAPACITY = -2
 
 CAND_DTYPE = np.dtype([("k1", "<u8"), ("k2", "<u8"), ("rq", "<u4"), ("pad", "<u4")])
 NONE_KEY = np.uint64(0xFFFFFFFFFFFFFFFF)
@@ -141,6 +149,10 @@ def lib():
         L.bshot_popc_peak.argtypes = [vp, C.POINTER(C.c_double)]
         L.bshot_set_matcher.argtypes = [vp, ci]
         L.bshot_debug_counters.argtypes = [vp, C.POINTER(C.c_ulonglong * 8)]
+        L.bshot_iss_params_default.argtypes = [C.POINTER(IssParams)]
+        L.bshot_iss_params_default.restype = None
+        L.bshot_detect_iss.argtypes = [vp, C.POINTER(IssParams), vp, vp, sz, C.POINTER(sz), vp]
+        L.bshot_kp_repeatability.argtypes = [vp, vp, sz, vp, vp, sz, vp, cf, vp, vp, C.POINTER(sz)]
         _LIB = L
     return _LIB
 
@@ -162,6 +174,27 @@ def default_params(**kw):
             raise AttributeError(k)
         setattr(p, k, v)
     return p
+
+
+def iss_default_params(**kw):
+    """ISS parameters of issKpDetection (src/lidar_odometry.cpp:447-461); keyword arguments override fields"""
+    p = IssParams()
+    lib().bshot_iss_params_default(C.byref(p))
+    for k, v in kw.items():
+        if not hasattr(p, k):
+            raise AttributeError(k)
+        setattr(p, k, v)
+    return p
+
+
+def _pose12(pose):
+    """None, a row-major [R|T] (12 values) or a 4 x 4 matrix -> 12 contiguous float32 (None stays None)"""
+    if pose is None:
+        return None
+    m = np.asarray(pose, dtype=np.float32)
+    if m.size == 16:
+        m = m.reshape(4, 4)[:3]
+    return np.ascontiguousarray(m.reshape(12))
 
 
 def unpack_cands(cand):
@@ -347,6 +380,7 @@ class Context:
     def process_frame_dev(self, d_xyz_ptr, n, stride_bytes, params):
         """device-resident cloud (raw device pointer), asynchronous on the context stream"""
         _chk(lib().bshot_process_frame_dev(self.h, C.byref(params), d_xyz_ptr, n, stride_bytes))
+        self.n_points = n
 
     def fetch_frame(self, top_k):
         kp_idx = np.empty(top_k, np.int32)
@@ -509,6 +543,41 @@ class Context:
 
     def frame_commit(self):
         _chk(lib().bshot_frame_commit(self.h))
+
+    # ISS keypoints + repeatability (the reference's kp_test evaluation)
+    def detect_iss(self, params=None, want_eigs=False):
+        """ISS keypoints of the cloud the context holds: dict(idx, xyz) in ascending point index, plus eigs (N x 3,
+        lambda1..3) when want_eigs"""
+        params = iss_default_params() if params is None else params
+        cap = min(self.n_points, 8192)
+        cnt = C.c_size_t()
+        eigs = np.empty((self.n_points, 3), np.float64) if want_eigs else None
+        while True:
+            idx = np.empty(max(cap, 1), np.int32)
+            xyz = np.empty((max(cap, 1), 3), np.float32)
+            rc = lib().bshot_detect_iss(self.h, C.byref(params), _p(idx), _p(xyz), cap, C.byref(cnt), _p(eigs))
+            if rc == E_CAPACITY and cnt.value > cap:
+                cap = cnt.value
+                continue
+            _chk(rc)
+            break
+        k = cnt.value
+        out = dict(idx=idx[:k].copy(), xyz=xyz[:k].copy())
+        if want_eigs:
+            out["eigs"] = eigs
+        return out
+
+    def kp_repeatability(self, a, b, pose_a=None, pose_b=None, radius=30.0):
+        """nearest point of B for every point of A (both moved by their 3x4 poses): dict(nn_idx, nn_dist, hits, rate)"""
+        a = np.ascontiguousarray(a, dtype=np.float32).reshape(-1, 3)
+        b = np.ascontiguousarray(b, dtype=np.float32).reshape(-1, 3)
+        pa, pb = _pose12(pose_a), _pose12(pose_b)
+        na = a.shape[0]
+        idx = np.empty(max(na, 1), np.int32)
+        dist = np.empty(max(na, 1), np.float32)
+        hits = C.c_size_t()
+        _chk(lib().bshot_kp_repeatability(self.h, _p(a), na, _p(pa), _p(b), b.shape[0], _p(pb), radius, _p(idx), _p(dist), C.byref(hits)))
+        return dict(nn_idx=idx[:na].copy(), nn_dist=dist[:na].copy(), hits=hits.value, rate=hits.value / na if na else 0.0)
 
     # multi-rank exchange behind the C ABI (CUDA IPC peer memory)
     def comm_create(self, rank, nranks, max_queries):

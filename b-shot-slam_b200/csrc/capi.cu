@@ -3,6 +3,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <cmath>
 #include <new>
 #include <vector>
 
@@ -233,6 +234,7 @@ void bshot_ctx_destroy(bshot_ctx* c) {
     if (c->stream) cudaStreamSynchronize(c->stream);
     comm_free(c);
     gmap_free(c);
+    iss_free(c);
     void* ptrs[] = {c->d_raw, c->d_pts, c->d_sorted, c->d_cell_of, c->d_cell_start, c->d_cell_cursor, c->d_block_sums,
                     c->d_grid, c->d_bbox, c->d_lvl, c->d_sorted_pos, c->d_kp_flag, c->d_blocks, c->d_blk_area, c->d_nblocks, c->d_ovf, c->d_rho_hint, c->d_shot_order, c->d_qsums, c->d_fb_list, c->d_ratio, c->d_keys, c->d_kp_idx, c->d_kp_ratio, c->d_kp, c->d_kp_count,
                     c->d_tk_hist, c->d_tk_state, c->d_tk_sure, c->d_tk_tie, c->d_normals, c->d_qnormals, c->d_shot, c->d_rf, c->d_nn, c->d_sum_nn, c->d_bits, c->d_prev_bits, c->d_prev_kp,
@@ -975,6 +977,57 @@ int bshot_preprocess_select(bshot_ctx* ctx, const double* azimuth_deg, const dou
 int bshot_preprocess(bshot_ctx* ctx, const double* azimuth_deg, const double* vertical_deg, const unsigned short* distance, size_t n, const double* ring_deg,
                      size_t nv, double vert_init_rad, double lowpt_th, float* xyz_out, size_t cap, size_t* n_out) {
     return bshot_preprocess_select(ctx, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, vert_init_rad, lowpt_th, nullptr, 0, 0, 1, xyz_out, cap, n_out);
+}
+
+// ---- ISS keypoints + keypoint repeatability (kp_test evaluation, src/lidar_odometry.cpp:392-461) -----------------------
+void bshot_iss_params_default(bshot_iss_params* p) {
+    if (!p) return;
+    p->salient_radius = 60.0f;
+    p->non_max_radius = 40.0f;
+    p->gamma_21 = 0.975;
+    p->gamma_32 = 0.975;
+    p->min_neighbors = 5;
+}
+
+int bshot_detect_iss(bshot_ctx* ctx, const bshot_iss_params* p, int* idx_out, float* kp_xyz_out, size_t cap, size_t* count_out,
+                     double* eig_out) {
+    CHECK_CTX(ctx);
+    bshot_iss_params dp;
+    if (!p) { bshot_iss_params_default(&dp); p = &dp; }
+    if (!(p->salient_radius > 0.0f) || !(p->non_max_radius > 0.0f) || !std::isfinite(p->salient_radius) || !std::isfinite(p->non_max_radius) ||
+        p->min_neighbors < 1 || !std::isfinite(p->gamma_21) || !std::isfinite(p->gamma_32)) {
+        set_error("bshot_detect_iss: radii must be finite and > 0, min_neighbors >= 1, thresholds finite");
+        return BSHOT_E_INVALID;
+    }
+    if (!ctx->have_cloud) { set_error("bshot_detect_iss: no cloud"); return BSHOT_E_STATE; }
+    size_t count = 0;
+    BSHOT_TRY(iss_detect(ctx, p->salient_radius, p->non_max_radius, p->gamma_21, p->gamma_32, p->min_neighbors, cap, eig_out != nullptr, &count));
+    if (count_out) *count_out = count;
+    const size_t m = std::min(count, cap);
+    const int4* rec = ctx->iss.h_rec + 1;
+    for (size_t i = 0; i < m; ++i) {
+        if (idx_out) idx_out[i] = rec[i].x;
+        if (kp_xyz_out) {
+            memcpy(&kp_xyz_out[3 * i], &rec[i].y, sizeof(float));
+            memcpy(&kp_xyz_out[3 * i + 1], &rec[i].z, sizeof(float));
+            memcpy(&kp_xyz_out[3 * i + 2], &rec[i].w, sizeof(float));
+        }
+    }
+    if (eig_out) {
+        BSHOT_TRY(d2h(ctx, eig_out, ctx->iss.d_eig, sizeof(double) * 3 * ctx->n_points));
+        BSHOT_TRY(sync(ctx));
+    }
+    if (count > cap) { set_error("bshot_detect_iss: %zu keypoints > capacity %zu", count, cap); return BSHOT_E_CAPACITY; }
+    return BSHOT_OK;
+}
+
+int bshot_kp_repeatability(bshot_ctx* ctx, const float* a_xyz, size_t na, const float* a_pose3x4, const float* b_xyz, size_t nb,
+                           const float* b_pose3x4, float radius, int* nn_idx_out, float* nn_dist_out, size_t* hits_out) {
+    CHECK_CTX(ctx);
+    if ((!a_xyz && na) || (!b_xyz && nb)) { set_error("bshot_kp_repeatability: null point set"); return BSHOT_E_INVALID; }
+    if (!(radius > 0.0f) || !std::isfinite(radius)) { set_error("bshot_kp_repeatability: radius must be finite and > 0"); return BSHOT_E_INVALID; }
+    if (na > 0x7FFFFFFull || nb > 0x7FFFFFFull) { set_error("bshot_kp_repeatability: too many points"); return BSHOT_E_CAPACITY; }
+    return kp_repeatability(ctx, a_xyz, na, a_pose3x4, b_xyz, nb, b_pose3x4, radius, nn_idx_out, nn_dist_out, hits_out);
 }
 
 // ---- multi-rank exchange behind the C ABI (no Python / torch needed) -------------------------------------------

@@ -96,6 +96,16 @@ struct Gmap {
     size_t entries_upper = 0;           // host-side upper bound of the number of entries (sizes the match grid without a sync)
 };
 
+// ISS keypoints (iss.cu): max_points-sized buffers, allocated by the first bshot_detect_iss of the context
+struct Iss {
+    double* d_l3 = nullptr;             // per cell-sorted position: third_eigen_value (0 = not salient)
+    double* d_eig = nullptr;            // per original index: lambda1..3
+    unsigned char* d_flag = nullptr;    // per original index: keypoint
+    unsigned* d_tile_sums = nullptr;    // keypoints per compaction tile
+    int4* d_rec = nullptr;              // [0].x = count, then {index, x, y, z} records in ascending index
+    int4* h_rec = nullptr;              // pinned staging of d_rec
+};
+
 // query blocks are listed by weight class (class c: kBlockClasses regions of max_points entries in d_blocks / d_blk_area)
 constexpr int kBlockClasses = 8;
 
@@ -196,6 +206,7 @@ struct Ctx {
 
     Comm comm;
     Gmap gmap;
+    Iss iss;
     float4* d_prev_kp = nullptr;        // K: keypoint positions of the previous frame (reference frame of the map match)
     void* d_pre[3] = {nullptr, nullptr, nullptr};  // scratch grown on demand: preprocessor per-return / per-column, ICP
     size_t pre_bytes[3] = {0, 0, 0};

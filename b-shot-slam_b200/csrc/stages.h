@@ -80,6 +80,13 @@ int preprocess_run(Ctx* c, const double* az_deg, const double* vert_deg, const u
                    double vert_init, double lowpt_th, const unsigned char* sel, int save_sel, float* xyz_out, size_t cap, size_t* n_out,
                    const float** d_xyz_out = nullptr);
 
+// ISS keypoints on the resident cloud and keypoint repeatability (iss.cu).  iss_detect leaves the count and the first
+// min(cap, n) records {index, x, y, z} in c->iss.h_rec[1..] (synchronous); the eigenvalues stay in c->iss.d_eig
+int iss_detect(Ctx* c, float rs, float rnm, double g21, double g32, int min_nn, size_t cap, bool want_eig, size_t* count_out);
+void iss_free(Ctx* c);
+int kp_repeatability(Ctx* c, const float* a_xyz, size_t na, const float* a_pose, const float* b_xyz, size_t nb, const float* b_pose, float radius,
+                     int* nn_idx_out, float* nn_dist_out, size_t* hits_out);
+
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);
 int frame_commit(Ctx* c, size_t k);

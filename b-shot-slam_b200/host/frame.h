@@ -22,6 +22,7 @@ public:
     PCPtr pointcloud_;                       // pre-processed scan
     PCPtr keypoints_;                        // ascending seg-ratio, as extractKeypoints leaves them
     DCPPtr descriptors_;                     // one record per keypoint
+    PCPtr iss_keypoints_;                    // ISS keypoints (LidarOdometry::issKpDetection), ascending point index
     bool is_key_frame_ = false;
 
     Frame() = default;
@@ -49,6 +50,8 @@ public:
     PCPtr getKeypoints() { return keypoints_; }
     void setDescriptors(DCPPtr dcpts) { descriptors_ = std::move(dcpts); }
     DCPPtr getDescriptors() { return descriptors_; }
+    void setISSKeypoints(PCPtr kps) { iss_keypoints_ = std::move(kps); }
+    PCPtr getISSKeypoints() { return iss_keypoints_; }
     unsigned long getID() { return id_; }
     bool isKeyframe() { return is_key_frame_; }
 

@@ -1,7 +1,8 @@
 // lidar_odometry.h -- the per-frame stage methods of the reference's LidarOdometry (include/lidar_odometry.h:22-31,
 // src/lidar_odometry.cpp:51-376) over the B200 C ABI: extractKeypoints, computeDescriptors, featureMatching (mutual
 // Hamming matching + RANSAC rejection), evaluateEstimation (gate + ICP), poseEstimation, updateMap -- the call order of
-// test/odometry_test.cpp:174-192.  The viewer, the ISS evaluation path and the printing are not carried over.
+// test/odometry_test.cpp:174-192 -- and the keypoint evaluation of the kp_test driver: issKpDetection and kpEvaluation.
+// The viewer and the printing are not carried over.
 #ifndef BSHOT_B200_HOST_LIDAR_ODOMETRY_H
 #define BSHOT_B200_HOST_LIDAR_ODOMETRY_H
 
@@ -30,7 +31,9 @@ public:
     void setTopK(int k) { top_k_ = k; }
     void setRun() { status_ = RUN; }
 
-    void extractKeypoints() {  // :51-162 (ISS detection :164-170 is evaluation only and not part of the path)
+    // :51-162.  The reference also runs ISS detection from here (:164-170); that is issKpDetection() below, called
+    // separately, so that the odometry path does not pay for an evaluation-only detector.
+    void extractKeypoints() {
         bshot_ctx* ctx = cb.context();
         const int sr = sr_type_ == "CVS" ? BSHOT_SR_CVS : (sr_type_ == "CVSN" ? BSHOT_SR_CVSN : BSHOT_SR_CV);
         cb.cloud1 = src_pcl_;
@@ -135,6 +138,46 @@ public:
         }
         status_ = RUN;
     }
+    // :447-461: pcl::ISSKeypoint3D (salient radius 60, non-max radius 40, thresholds 0.975 / 0.975) on the source cloud
+    // -> the source frame's ISS keypoints.  Runs on the cloud extractKeypoints() left in the context (call it after that).
+    void issKpDetection() {
+        bshot_ctx* ctx = cb.context();
+        bshot_iss_params prm;
+        bshot_iss_params_default(&prm);
+        size_t n = 0;
+        std::vector<int> idx(4096);
+        std::vector<float> xyz(3 * idx.size());
+        last_status_ = bshot_detect_iss(ctx, &prm, idx.data(), xyz.data(), idx.size(), &n, nullptr);
+        if (last_status_ == BSHOT_E_CAPACITY) {
+            idx.resize(n);
+            xyz.resize(3 * n);
+            last_status_ = bshot_detect_iss(ctx, &prm, idx.data(), xyz.data(), n, &n, nullptr);
+        }
+        auto kps = std::make_shared<std::vector<Vector3f>>();
+        if (last_status_ == BSHOT_OK)
+            for (size_t i = 0; i < n; ++i) kps->push_back(Vector3f(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]));
+        src_->setISSKeypoints(kps);
+    }
+
+    // :392-445: repeat rates of the source frame's seg-ratio and ISS keypoints against the reference frame's, each set
+    // moved by its frame's pose: the share of source keypoints whose nearest reference keypoint lies within 30 mm
+    // (bshot_kp_repeatability; the port's definition, the reference prints its own "Repeat rate").  Kept, not printed.
+    void kpEvaluation() {
+        float Ts[16], Tr[16];
+        to_row_major(src_->getPose(), Ts);
+        to_row_major(ref_->getPose(), Tr);
+        auto rate = [&](const Frame::PCPtr& a, const Frame::PCPtr& b, double& out) {
+            out = 0.0;
+            const size_t na = a ? a->size() : 0, nb = b ? b->size() : 0;
+            size_t hits = 0;
+            last_status_ = bshot_kp_repeatability(cb.context(), na ? &(*a)[0][0] : nullptr, na, Ts, nb ? &(*b)[0][0] : nullptr, nb, Tr, 30.0f,
+                                                  nullptr, nullptr, &hits);
+            if (last_status_ == BSHOT_OK && na) out = (double)hits / (double)na;
+            return last_status_ == BSHOT_OK;
+        };
+        if (rate(src_->getKeypoints(), ref_->getKeypoints(), sr_repeat_rate_)) rate(src_->getISSKeypoints(), ref_->getISSKeypoints(), iss_repeat_rate_);
+    }
+
     void setRunICP(bool run_icp) { run_icp_ = run_icp; }
     Matrix4f getBestTransformation() const { return T_best_; }
     Matrix4f getRansacTransformation() const { return T_ransac_; }
@@ -170,6 +213,7 @@ public:
     float h_diff_ = 0, t_diff_ = 0;
     int icp_iterations_ = 0;
     std::vector<float> seg_ratios_;
+    double sr_repeat_rate_ = 0.0, iss_repeat_rate_ = 0.0;  // kpEvaluation
 
 private:
     Frame::Ptr ref_, src_;

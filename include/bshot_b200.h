@@ -255,6 +255,37 @@ int bshot_extract_scan(bshot_ctx* ctx, const bshot_params* p, const double* azim
                        double lowpt_th, float* cloud_xyz_out, size_t cloud_cap, size_t* n_points_out, int* kp_idx_out,
                        float* kp_xyz_out, float* seg_ratio_out, uint64_t* bits_out, int* n_kp_out);
 
+/* ---- ISS keypoints and keypoint repeatability (the reference's kp_test evaluation) ------------ */
+/* issKpDetection (src/lidar_odometry.cpp:447-461): pcl::ISSKeypoint3D (PCL 1.8, border radius 0) on the cloud the context
+ * holds (after bshot_set_cloud / bshot_extract_frame / bshot_process_frame[_dev] / bshot_extract_scan), on its voxel table.
+ * Every finite point p: neighbours = points with fp32 squared distance < salient_radius^2 (p included); with fewer than
+ * min_neighbors the scatter matrix is zero, else sum (n - p)(n - p)^T in double; eigenvalues l1 >= l2 >= l3; p is salient
+ * when all are finite, l3 >= 0 (PCL leaves both cases to stale memory; here they are "not salient"), l2/l1 < gamma_21 and
+ * l3/l2 < gamma_32, and then third_eigen_value(p) = l3, else 0.  Keypoints: third_eigen_value > 0, at least min_neighbors
+ * points within non_max_radius (p included) and none of them with a strictly larger third_eigen_value.
+ * The call reads no frame state and changes none (keypoints, normals, previous frame, map stay as they were); its
+ * max_points-sized buffers are allocated by the first call on a context. */
+typedef struct bshot_iss_params {
+    float salient_radius;   /* 60     setSalientRadius  src/lidar_odometry.cpp:447-461 */
+    float non_max_radius;   /* 40     setNonMaxRadius */
+    double gamma_21;        /* 0.975  setThreshold21 */
+    double gamma_32;        /* 0.975  setThreshold32 */
+    int min_neighbors;      /* 5      PCL's default */
+} bshot_iss_params;
+void bshot_iss_params_default(bshot_iss_params* p);
+/* idx_out / kp_xyz_out: up to cap records, ascending point index. eig_out (N x 3 doubles, lambda1..3; zeros where
+ * skipped) may be NULL. count > cap: the first cap are written and BSHOT_E_CAPACITY is returned. */
+int bshot_detect_iss(bshot_ctx* ctx, const bshot_iss_params* p, int* idx_out, float* kp_xyz_out, size_t cap,
+                     size_t* count_out, double* eig_out);
+/* kpEvaluation (src/lidar_odometry.cpp:392-445), the port's own definition: set A (na x 3 floats) moved by a_pose3x4 and
+ * set B moved by b_pose3x4 (row-major [R|T], NULL = identity, R * p + T in fp32 as updateMap does); for every point of A
+ * the nearest point of B by fp32 squared distance (no FMA contraction, lowest index on ties) -> nn_idx_out[i] (-1 when B
+ * is empty) and nn_dist_out[i] (Euclidean, mm); a point is a hit when its squared distance is < radius^2.  The repeat
+ * rate is *hits_out / na.  Outputs may be NULL. */
+int bshot_kp_repeatability(bshot_ctx* ctx, const float* a_xyz, size_t na, const float* a_pose3x4, const float* b_xyz,
+                           size_t nb, const float* b_pose3x4, float radius, int* nn_idx_out, float* nn_dist_out,
+                           size_t* hits_out);
+
 /* ---- sharded map matching (north_star multi-GPU piece) -------------------------------------- */
 /* The accumulated map descriptors (Map::getKeypoints output, include/mymap.h:34-38) are split
  * across ranks; each rank keeps its shard resident.  global_base = index of the shard's first
