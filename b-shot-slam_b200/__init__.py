@@ -36,7 +36,7 @@ EXPORTS = [
     "bshot_match_map_sharded", "bshot_gmap_create", "bshot_gmap_reset", "bshot_gmap_size", "bshot_gmap_add",
     "bshot_gmap_update_from_frame", "bshot_gmap_get_keypoints", "bshot_extract_frame", "bshot_match_frame_to_map", "bshot_frame_commit", "bshot_ransac",
     "bshot_preprocess", "bshot_preprocess_select", "bshot_extract_scan", "bshot_icp", "bshot_evaluate_estimation", "bshot_set_matcher",
-    "bshot_iss_params_default", "bshot_detect_iss", "bshot_kp_repeatability",
+    "bshot_iss_params_default", "bshot_detect_iss", "bshot_kp_repeatability", "bshot_voxel_grid",
 ]
 
 
@@ -153,6 +153,7 @@ def lib():
         L.bshot_iss_params_default.restype = None
         L.bshot_detect_iss.argtypes = [vp, C.POINTER(IssParams), vp, vp, sz, C.POINTER(sz), vp]
         L.bshot_kp_repeatability.argtypes = [vp, vp, sz, vp, vp, sz, vp, cf, vp, vp, C.POINTER(sz)]
+        L.bshot_voxel_grid.argtypes = [vp, vp, sz, sz, cf, cf, cf, vp, sz, C.POINTER(sz)]
         _LIB = L
     return _LIB
 
@@ -578,6 +579,25 @@ class Context:
         hits = C.c_size_t()
         _chk(lib().bshot_kp_repeatability(self.h, _p(a), na, _p(pa), _p(b), b.shape[0], _p(pb), radius, _p(idx), _p(dist), C.byref(hits)))
         return dict(nn_idx=idx[:na].copy(), nn_dist=dist[:na].copy(), hits=hits.value, rate=hits.value / na if na else 0.0)
+
+    # voxel-grid downsampling (the reference's bshot::calculate_voxel_grid_keypoints)
+    def voxel_grid(self, xyz, leaf):
+        """pcl::VoxelGrid centroids of a host cloud ((N, 3) or (N, 4) float32; not the context's cloud, which stays as it
+        was) with leaf sizes `leaf` (a scalar or a 3-sequence, mm) -> (M, 3) float32 in ascending voxel index"""
+        xyz = np.ascontiguousarray(xyz, dtype=np.float32)
+        assert xyz.ndim == 2 and xyz.shape[1] in (3, 4)
+        lx, ly, lz = (float(v) for v in np.broadcast_to(np.asarray(leaf, dtype=np.float32), (3,)))
+        cap = min(xyz.shape[0], 16384)
+        cnt = C.c_size_t()
+        while True:
+            out = np.empty((max(cap, 1), 3), np.float32)
+            rc = lib().bshot_voxel_grid(self.h, _p(xyz), xyz.shape[0], xyz.shape[1] * 4, lx, ly, lz, _p(out), cap, C.byref(cnt))
+            if rc == E_CAPACITY and cnt.value > cap:
+                cap = cnt.value
+                continue
+            _chk(rc)
+            break
+        return out[:cnt.value].copy()
 
     # multi-rank exchange behind the C ABI (CUDA IPC peer memory)
     def comm_create(self, rank, nranks, max_queries):

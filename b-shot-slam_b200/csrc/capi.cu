@@ -235,6 +235,7 @@ void bshot_ctx_destroy(bshot_ctx* c) {
     comm_free(c);
     gmap_free(c);
     iss_free(c);
+    vg_free(c);
     void* ptrs[] = {c->d_raw, c->d_pts, c->d_sorted, c->d_cell_of, c->d_cell_start, c->d_cell_cursor, c->d_block_sums,
                     c->d_grid, c->d_bbox, c->d_lvl, c->d_sorted_pos, c->d_kp_flag, c->d_blocks, c->d_blk_area, c->d_nblocks, c->d_ovf, c->d_rho_hint, c->d_shot_order, c->d_qsums, c->d_fb_list, c->d_ratio, c->d_keys, c->d_kp_idx, c->d_kp_ratio, c->d_kp, c->d_kp_count,
                     c->d_tk_hist, c->d_tk_state, c->d_tk_sure, c->d_tk_tie, c->d_normals, c->d_qnormals, c->d_shot, c->d_rf, c->d_nn, c->d_sum_nn, c->d_bits, c->d_prev_bits, c->d_prev_kp,
@@ -1028,6 +1029,30 @@ int bshot_kp_repeatability(bshot_ctx* ctx, const float* a_xyz, size_t na, const 
     if (!(radius > 0.0f) || !std::isfinite(radius)) { set_error("bshot_kp_repeatability: radius must be finite and > 0"); return BSHOT_E_INVALID; }
     if (na > 0x7FFFFFFull || nb > 0x7FFFFFFull) { set_error("bshot_kp_repeatability: too many points"); return BSHOT_E_CAPACITY; }
     return kp_repeatability(ctx, a_xyz, na, a_pose3x4, b_xyz, nb, b_pose3x4, radius, nn_idx_out, nn_dist_out, hits_out);
+}
+
+// ---- voxel-grid downsampling (bshot::calculate_voxel_grid_keypoints, pcl::VoxelGrid) ------------------------------------
+int bshot_voxel_grid(bshot_ctx* ctx, const float* xyz, size_t n, size_t stride_bytes, float leaf_x, float leaf_y, float leaf_z,
+                     float* xyz_out, size_t cap, size_t* count_out) {
+    CHECK_CTX(ctx);
+    if (!xyz && n) { set_error("bshot_voxel_grid: null cloud"); return BSHOT_E_INVALID; }
+    if (stride_bytes != 12 && stride_bytes != 16) { set_error("bshot_voxel_grid: stride must be 12 or 16 bytes"); return BSHOT_E_INVALID; }
+    const float leaf[3] = {leaf_x, leaf_y, leaf_z};
+    float inv[3];
+    for (int a = 0; a < 3; ++a) {
+        inv[a] = 1.0f / leaf[a];  // PCL: inverse_leaf_size_ = Array4f::Ones () / leaf_size_
+        if (!(leaf[a] > 0.0f) || !std::isfinite(leaf[a]) || !std::isfinite(inv[a])) {
+            set_error("bshot_voxel_grid: leaf sizes must be finite and > 0 with a finite reciprocal");
+            return BSHOT_E_INVALID;
+        }
+    }
+    if (n > ctx->max_points) { set_error("bshot_voxel_grid: %zu points > capacity %zu", n, ctx->max_points); return BSHOT_E_CAPACITY; }
+    size_t count = 0;
+    BSHOT_TRY(voxel_grid(ctx, xyz, n, (int)(stride_bytes / 4), inv, cap, &count));
+    if (count_out) *count_out = count;
+    if (xyz_out) memcpy(xyz_out, ctx->vg.h_out + 4, sizeof(float) * 3 * std::min(count, cap));
+    if (count > cap) { set_error("bshot_voxel_grid: %zu voxels > capacity %zu", count, cap); return BSHOT_E_CAPACITY; }
+    return BSHOT_OK;
 }
 
 // ---- multi-rank exchange behind the C ABI (no Python / torch needed) -------------------------------------------

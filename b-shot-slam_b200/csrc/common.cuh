@@ -106,6 +106,19 @@ struct Iss {
     int4* h_rec = nullptr;              // pinned staging of d_rec
 };
 
+// voxel-grid downsampling (voxel_grid.cu): max_points-sized buffers, allocated by the first bshot_voxel_grid of the context
+struct Vg {
+    float* d_in = nullptr;              // staging of the caller's cloud (stride 12 or 16)
+    unsigned* d_ctl = nullptr;          // VgParams + bbox + ticket (voxel_grid.cu)
+    unsigned* d_tile = nullptr;         // per compaction tile: finite points, then voxel heads
+    unsigned* d_keys[2] = {nullptr, nullptr};  // voxel index per finite point, radix ping-pong
+    unsigned* d_vals[2] = {nullptr, nullptr};  // point index per finite point, radix ping-pong
+    unsigned* d_hist = nullptr;         // per radix tile: 256 digit counts
+    unsigned* d_seg = nullptr;          // first sorted position of every voxel, then the finite count
+    float* d_out = nullptr;             // [0] = count (as unsigned), [1..3] unused, then {x, y, z} records
+    float* h_out = nullptr;             // pinned staging of d_out
+};
+
 // query blocks are listed by weight class (class c: kBlockClasses regions of max_points entries in d_blocks / d_blk_area)
 constexpr int kBlockClasses = 8;
 
@@ -207,6 +220,7 @@ struct Ctx {
     Comm comm;
     Gmap gmap;
     Iss iss;
+    Vg vg;
     float4* d_prev_kp = nullptr;        // K: keypoint positions of the previous frame (reference frame of the map match)
     void* d_pre[3] = {nullptr, nullptr, nullptr};  // scratch grown on demand: preprocessor per-return / per-column, ICP
     size_t pre_bytes[3] = {0, 0, 0};
@@ -260,6 +274,21 @@ __device__ __forceinline__ int warp_sum(int v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
+}
+
+// float min / max through the integer atomics, for non-NaN values.  v >= 0 takes the signed path, where the order of the
+// bit patterns is the order of the floats; v < 0 takes the unsigned path, where it is the reverse.  -0.0 compares
+// >= 0 but its bit pattern is INT_MIN, so it is first turned into +0.0 (-0 + +0 = +0; every other v is unchanged); the
+// stored extreme is then +0.0 where the floats' extreme is a zero of either sign.
+__device__ __forceinline__ void atomic_min_float(float* a, float v) {
+    v = __fadd_rn(v, 0.0f);
+    if (v >= 0.0f) atomicMin(reinterpret_cast<int*>(a), __float_as_int(v));
+    else atomicMax(reinterpret_cast<unsigned*>(a), __float_as_uint(v));
+}
+__device__ __forceinline__ void atomic_max_float(float* a, float v) {
+    v = __fadd_rn(v, 0.0f);
+    if (v >= 0.0f) atomicMax(reinterpret_cast<int*>(a), __float_as_int(v));
+    else atomicMin(reinterpret_cast<unsigned*>(a), __float_as_uint(v));
 }
 
 // FLANN L2_Simple in fp32 without FMA contraction (SURVEY Appendix A.1)

@@ -22,15 +22,6 @@ constexpr int SCAN_THREADS = 1024;
 constexpr int SCAN_ITEMS = 8;                        // cells per thread
 constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS; // 8192 cells per block
 
-__device__ __forceinline__ void atomic_min_float(float* a, float v) {
-    if (v >= 0.0f) atomicMin(reinterpret_cast<int*>(a), __float_as_int(v));
-    else atomicMax(reinterpret_cast<unsigned*>(a), __float_as_uint(v));
-}
-__device__ __forceinline__ void atomic_max_float(float* a, float v) {
-    if (v >= 0.0f) atomicMax(reinterpret_cast<int*>(a), __float_as_int(v));
-    else atomicMin(reinterpret_cast<unsigned*>(a), __float_as_uint(v));
-}
-
 __device__ void grid_params_from_bbox(float* bbox, unsigned n, float cell0, float yz_mul, unsigned max_cells, GridParams* g) {
     GridParams p;
     float mn[3] = {bbox[0], bbox[1], bbox[2]}, mx[3] = {bbox[3], bbox[4], bbox[5]};

@@ -87,6 +87,11 @@ void iss_free(Ctx* c);
 int kp_repeatability(Ctx* c, const float* a_xyz, size_t na, const float* a_pose, const float* b_xyz, size_t nb, const float* b_pose, float radius,
                      int* nn_idx_out, float* nn_dist_out, size_t* hits_out);
 
+// voxel-grid downsampling of a host cloud (voxel_grid.cu): inv = 1 / leaf per axis.  Leaves the count and the first
+// min(cap, n) records {x, y, z} in c->vg.h_out[4..] (synchronous)
+int voxel_grid(Ctx* c, const float* xyz, size_t n, int stride_floats, const float inv[3], size_t cap, size_t* count_out);
+void vg_free(Ctx* c);
+
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);
 int frame_commit(Ctx* c, size_t k);

@@ -7,11 +7,14 @@
 //   minVect<T>            :6-20                   identical semantics (first minimum), header-only
 //   bshot_descriptor      :23-27                  std::bitset<352> bits  (48 B, passed to the GPU as is)
 //   calculate_normals(r)  :43-94                  bshot_set_cloud + bshot_set_keypoints + bshot_compute_normals
+//   calculate_voxel_grid_keypoints(leaf) :97-110  bshot_voxel_grid on cloud1 and on cloud2
 //   calculate_SHOT(r)     :113-135                bshot_compute_shot (fills cloud1_shot incl. rf[9])
 //   compute_bshot()       :138-142                bits of the same call (already on the device)
 //   compute_bshot_from_SHOT(cloud, out) :144-278  bshot_binarize
 #ifndef BSHOT_B200_HOST_BSHOT_BITS_H
 #define BSHOT_B200_HOST_BSHOT_BITS_H
+
+#include <algorithm>
 
 #include "bshot_headers_bits.h"
 #include "../../include/bshot_b200.h"
@@ -99,6 +102,21 @@ public:
         bits_valid_ = true;
     }
 
+    // pcl::VoxelGrid (cubic leaf) of cloud1 into cloud1_keypoints, then of cloud2 into cloud2_keypoints.  The body was
+    // restated from the upstream B-SHOT header that `class bshot` comes from, not read from :97-110.  Output clouds as
+    // PCL leaves them: width = count, height 1, is_dense; when the grid would overflow PCL copies the input cloud, and
+    // the copy keeps the input's width, height and is_dense.  On failure status_ is set and both clouds are empty.
+    // The next calculate_normals / calculate_SHOT upload the new keypoints (content fingerprint).
+    void calculate_voxel_grid_keypoints(float leaf_size) {
+        cloud1_keypoints.clear();
+        cloud2_keypoints.clear();
+        if (!ctx_) { status_ = BSHOT_E_CUDA; return; }
+        if (!voxel_grid(cloud1, leaf_size, cloud1_keypoints) || !voxel_grid(cloud2, leaf_size, cloud2_keypoints)) {
+            cloud1_keypoints.clear();
+            cloud2_keypoints.clear();
+        }
+    }
+
     void compute_bshot() {
         if (bits_valid_ && pending_bits_.size() == cloud1_shot.size()) cloud1_bshot = pending_bits_;  // fused on the device
         else compute_bshot_from_SHOT(cloud1_shot, cloud1_bshot);
@@ -141,6 +159,44 @@ private:
         for (size_t i = 0; i < n; i += step) mix(i);
         mix(n - 1);
         return h;
+    }
+
+    bool voxel_grid(const pcl::PointCloud<pcl::PointXYZ>& in, float leaf, pcl::PointCloud<pcl::PointXYZ>& out) {
+        const size_t n = in.size();
+        std::vector<float> xyz(3 * n);
+        size_t count = 0;
+        status_ = bshot_voxel_grid(ctx_, n ? in.points[0].data : nullptr, n, sizeof(pcl::PointXYZ), leaf, leaf, leaf, xyz.data(), n,
+                                   &count);
+        if (status_ != BSHOT_OK) return false;
+        out.points.resize(count);
+        for (size_t i = 0; i < count; ++i) out.points[i] = pcl::PointXYZ(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2]);
+        out.width = (uint32_t)count; out.height = 1; out.is_dense = true;
+        // PCL's overflow branch is `output = *input_`: the input's layout too.  Only a result of n points can be that
+        // copy; every voxel holding one point also gives n points, so the test itself decides.
+        if (count == n && grid_overflows(in, leaf)) { out.width = in.width; out.height = in.height; out.is_dense = in.is_dense; }
+        return true;
+    }
+
+    // PCL 1.8 VoxelGrid::applyFilter's overflow test with a cubic leaf, in the fp32 arithmetic bshot_voxel_grid uses:
+    // over the finite points, (int64)((max - min) * (1 / leaf)) + 1 cells per axis, more than INT32_MAX cells in all
+    static bool grid_overflows(const pcl::PointCloud<pcl::PointXYZ>& in, float leaf) {
+        const float inv = 1.0f / leaf;
+        float mn[3] = {INFINITY, INFINITY, INFINITY}, mx[3] = {-INFINITY, -INFINITY, -INFINITY};
+        bool any = false;
+        for (const auto& p : in.points) {
+            if (!std::isfinite(p.x) || !std::isfinite(p.y) || !std::isfinite(p.z)) continue;
+            for (int a = 0; a < 3; ++a) { mn[a] = std::min(mn[a], p.data[a]); mx[a] = std::max(mx[a], p.data[a]); }
+            any = true;
+        }
+        if (!any) return false;
+        int64_t cells = 1;
+        for (int a = 0; a < 3; ++a) {
+            const float f = (mx[a] - mn[a]) * inv;
+            if (!(f < 2147483648.0f)) return true;
+            cells *= (int64_t)f + 1;
+            if (cells > (int64_t)INT32_MAX) return true;
+        }
+        return false;
     }
 
     bool upload() {

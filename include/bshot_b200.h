@@ -286,6 +286,22 @@ int bshot_kp_repeatability(bshot_ctx* ctx, const float* a_xyz, size_t na, const 
                            size_t nb, const float* b_pose3x4, float radius, int* nn_idx_out, float* nn_dist_out,
                            size_t* hits_out);
 
+/* ---- voxel-grid downsampling (the reference's bshot::calculate_voxel_grid_keypoints) --------- */
+/* pcl::VoxelGrid<PointXYZ>::applyFilter of PCL 1.8 with its defaults (all fields averaged, no filter field, no minimum
+ * point count) on a host cloud of n points (stride 12 or 16 bytes; not the context's cloud).  inv = 1 / leaf per axis in
+ * fp32; non-finite points are skipped; bbox = fp32 min / max of the finite points.  If the grid of
+ * (int64)((max - min) * inv) + 1 cells per axis has more than INT32_MAX cells, the output is the input cloud unchanged
+ * (every point in order, non-finite ones included).  Otherwise min_b = (int)floor(min * inv), div_b = max_b - min_b + 1,
+ * and every finite point goes to voxel idx = ijk . (1, div_b.x, div_b.x * div_b.y) modulo 2^32 with
+ * ijk = (int)(floor(p * inv) - (float)min_b) (fp32 products).  One point per occupied voxel in ascending idx: the fp32
+ * running sum of its points in ascending point index, divided by the (float) count.
+ * xyz_out: up to cap records {x, y, z}; count > cap: the first cap are written, *count_out is the full count and
+ * BSHOT_E_CAPACITY is returned.  Leaves that are not finite and > 0, or whose reciprocal is not finite: BSHOT_E_INVALID;
+ * n > max_points: BSHOT_E_CAPACITY.  The call reads no frame state and changes none (cloud, voxel table, keypoints,
+ * normals, previous frame, map); its max_points-sized buffers are allocated by the first call on a context. */
+int bshot_voxel_grid(bshot_ctx* ctx, const float* xyz, size_t n, size_t stride_bytes, float leaf_x, float leaf_y,
+                     float leaf_z, float* xyz_out, size_t cap, size_t* count_out);
+
 /* ---- sharded map matching (north_star multi-GPU piece) -------------------------------------- */
 /* The accumulated map descriptors (Map::getKeypoints output, include/mymap.h:34-38) are split
  * across ranks; each rank keeps its shard resident.  global_base = index of the shard's first
