@@ -37,6 +37,7 @@ EXPORTS = [
     "bshot_gmap_update_from_frame", "bshot_gmap_get_keypoints", "bshot_extract_frame", "bshot_match_frame_to_map", "bshot_frame_commit", "bshot_ransac",
     "bshot_preprocess", "bshot_preprocess_select", "bshot_extract_scan", "bshot_icp", "bshot_evaluate_estimation", "bshot_set_matcher",
     "bshot_iss_params_default", "bshot_detect_iss", "bshot_kp_repeatability", "bshot_voxel_grid",
+    "bshot_odom_params_default", "bshot_odometry_step", "bshot_odometry_step_cloud", "bshot_odometry_reset", "bshot_ransac_dev",
 ]
 
 
@@ -51,14 +52,28 @@ class IssParams(C.Structure):
                 ("gamma_32", C.c_double), ("min_neighbors", C.c_int)]
 
 
-E_CAPACITY = -2
+class OdomParams(C.Structure):
+    _fields_ = [("front", Params), ("vert_init_rad", C.c_double), ("lowpt_th", C.c_double), ("map_range", C.c_float),
+                ("ransac_iterations", C.c_int), ("inlier_threshold", C.c_float), ("run_icp", C.c_int)]
+
+
+class OdomReport(C.Structure):
+    _fields_ = [("pose", C.c_float * 16), ("T_ransac", C.c_float * 16), ("n_points", C.c_size_t), ("n_targets", C.c_size_t),
+                ("n_keypoints", C.c_int), ("n_pairs", C.c_int), ("n_inliers", C.c_int), ("ransac_iterations", C.c_int),
+                ("icp_iterations", C.c_int), ("should_update_map", C.c_int), ("was_initial", C.c_int),
+                ("h_diff_rad", C.c_float), ("t_diff_mm", C.c_float)]
+
+
+E_INVALID, E_CAPACITY, E_CUDA, E_STATE = -1, -2, -3, -4
 
 CAND_DTYPE = np.dtype([("k1", "<u8"), ("k2", "<u8"), ("rq", "<u4"), ("pad", "<u4")])
 NONE_KEY = np.uint64(0xFFFFFFFFFFFFFFFF)
 
 
 class BshotError(RuntimeError):
-    pass
+    def __init__(self, msg, code=None):
+        super().__init__(msg)
+        self.code = code
 
 
 def build(verbose=False):
@@ -154,13 +169,19 @@ def lib():
         L.bshot_detect_iss.argtypes = [vp, C.POINTER(IssParams), vp, vp, sz, C.POINTER(sz), vp]
         L.bshot_kp_repeatability.argtypes = [vp, vp, sz, vp, vp, sz, vp, cf, vp, vp, C.POINTER(sz)]
         L.bshot_voxel_grid.argtypes = [vp, vp, sz, sz, cf, cf, cf, vp, sz, C.POINTER(sz)]
+        L.bshot_odom_params_default.argtypes = [C.POINTER(OdomParams)]
+        L.bshot_odom_params_default.restype = None
+        L.bshot_odometry_step.argtypes = [vp, C.POINTER(OdomParams), vp, vp, vp, sz, vp, sz, C.POINTER(OdomReport)]
+        L.bshot_odometry_step_cloud.argtypes = [vp, C.POINTER(OdomParams), vp, sz, sz, C.POINTER(OdomReport)]
+        L.bshot_odometry_reset.argtypes = [vp]
+        L.bshot_ransac_dev.argtypes = [vp, vp, vp, vp, vp, sz, ci, cf, vp, vp, vp, vp]
         _LIB = L
     return _LIB
 
 
 def _chk(rc):
     if rc != 0:
-        raise BshotError(f"bshot error {rc}: {lib().bshot_last_error().decode()}")
+        raise BshotError(f"bshot error {rc}: {lib().bshot_last_error().decode()}", rc)
 
 
 def _p(a):
@@ -186,6 +207,28 @@ def iss_default_params(**kw):
             raise AttributeError(k)
         setattr(p, k, v)
     return p
+
+
+def odom_default_params(**kw):
+    """parameters of the odometry step (test/odometry_test.cpp:32-33, src/lidar_odometry.cpp:6,198,255,258); keyword
+    arguments override fields, and the extraction fields (kp_radius, top_k, ...) reach `front`"""
+    p = OdomParams()
+    lib().bshot_odom_params_default(C.byref(p))
+    for k, v in kw.items():
+        if hasattr(p, k):
+            setattr(p, k, v)
+        elif hasattr(p.front, k):
+            setattr(p.front, k, v)
+        else:
+            raise AttributeError(k)
+    return p
+
+
+def _report(r):
+    out = {name: getattr(r, name) for name, _ in OdomReport._fields_ if name not in ("pose", "T_ransac")}
+    out["pose"] = np.ctypeslib.as_array(r.pose).reshape(4, 4).copy()
+    out["T_ransac"] = np.ctypeslib.as_array(r.T_ransac).reshape(4, 4).copy()
+    return out
 
 
 def _pose12(pose):
@@ -544,6 +587,55 @@ class Context:
 
     def frame_commit(self):
         _chk(lib().bshot_frame_commit(self.h))
+
+    # the per-scan odometry step (lasers or a preprocessed cloud -> pose in one call)
+    def odometry_step(self, azimuth_deg, vertical_deg, distance, ring_deg, params=None):
+        """Preprocessor::run -> extraction -> matching -> RANSAC -> gate + ICP -> pose -> map update -> reference frame, on
+        the device.  Returns the report as a dict; "pose" (4 x 4 float32, row-major) is T_best.  Needs gmap_create first."""
+        params = odom_default_params() if params is None else params
+        az = np.ascontiguousarray(azimuth_deg, dtype=np.float64)
+        ve = np.ascontiguousarray(vertical_deg, dtype=np.float64)
+        di = np.ascontiguousarray(distance, dtype=np.uint16)
+        ring = np.ascontiguousarray(ring_deg, dtype=np.float64)
+        assert az.shape == ve.shape == di.shape
+        r = OdomReport()
+        _chk(lib().bshot_odometry_step(self.h, C.byref(params), _p(az), _p(ve), _p(di), az.size, _p(ring), ring.size, C.byref(r)))
+        self.n_points, self.n_kp = r.n_points, r.n_keypoints
+        return _report(r)
+
+    def odometry_step_cloud(self, xyz, params=None):
+        """the same on an already-preprocessed (N, 3) or (N, 4) float32 cloud"""
+        params = odom_default_params() if params is None else params
+        xyz = np.ascontiguousarray(xyz, dtype=np.float32)
+        assert xyz.ndim == 2 and xyz.shape[1] in (3, 4)
+        r = OdomReport()
+        _chk(lib().bshot_odometry_step_cloud(self.h, C.byref(params), _p(xyz), xyz.shape[0], xyz.shape[1] * 4, C.byref(r)))
+        self.n_points, self.n_kp = r.n_points, r.n_keypoints
+        return _report(r)
+
+    def odometry_reset(self):
+        """INITIAL status, identity pose, empty map, no reference frame"""
+        _chk(lib().bshot_odometry_reset(self.h))
+
+    def ransac_dev(self, src4, tgt4, pairs, n_pairs, max_iterations=2000, threshold=1500.0):
+        """bshot_ransac on CUDA tensors: src4 / tgt4 (N, 4) float32, pairs (P, 2) int32, n_pairs (1,) int32 (the valid
+        prefix of pairs).  Returns dict(pairs, n_inliers, transform, iterations) of CUDA tensors; the call is complete
+        on return."""
+        import torch
+        for t, dt in ((src4, torch.float32), (tgt4, torch.float32), (pairs, torch.int32), (n_pairs, torch.int32)):
+            if not (t.is_cuda and t.dtype == dt and t.is_contiguous()):
+                raise BshotError("ransac_dev: contiguous CUDA tensors of float32 (points) and int32 (pairs, count) expected", E_INVALID)
+        cap = pairs.shape[0]
+        dev = pairs.device
+        out_pairs = torch.zeros((max(cap, 1), 2), dtype=torch.int32, device=dev)
+        n_out = torch.zeros(1, dtype=torch.int32, device=dev)
+        T = torch.zeros((4, 4), dtype=torch.float32, device=dev)
+        it = torch.zeros(1, dtype=torch.int32, device=dev)
+        torch.cuda.synchronize(dev)   # the inputs are complete before the context's stream reads them
+        _chk(lib().bshot_ransac_dev(self.h, src4.data_ptr(), tgt4.data_ptr(), pairs.data_ptr(), n_pairs.data_ptr(), cap, max_iterations, threshold,
+                                    out_pairs.data_ptr(), n_out.data_ptr(), T.data_ptr(), it.data_ptr()))
+        self.sync()
+        return dict(pairs=out_pairs, n_inliers=n_out, transform=T, iterations=it)
 
     # ISS keypoints + repeatability (the reference's kp_test evaluation)
     def detect_iss(self, params=None, want_eigs=False):

@@ -10,6 +10,7 @@
 #include "common.cuh"
 #include <stdlib.h>
 
+#include "odom_math.cuh"
 #include "stages.h"
 
 namespace bshot {
@@ -236,6 +237,7 @@ void bshot_ctx_destroy(bshot_ctx* c) {
     gmap_free(c);
     iss_free(c);
     vg_free(c);
+    odom_free(c);
     void* ptrs[] = {c->d_raw, c->d_pts, c->d_sorted, c->d_cell_of, c->d_cell_start, c->d_cell_cursor, c->d_block_sums,
                     c->d_grid, c->d_bbox, c->d_lvl, c->d_sorted_pos, c->d_kp_flag, c->d_blocks, c->d_blk_area, c->d_nblocks, c->d_ovf, c->d_rho_hint, c->d_shot_order, c->d_qsums, c->d_fb_list, c->d_ratio, c->d_keys, c->d_kp_idx, c->d_kp_ratio, c->d_kp, c->d_kp_count,
                     c->d_tk_hist, c->d_tk_state, c->d_tk_sure, c->d_tk_tie, c->d_normals, c->d_qnormals, c->d_shot, c->d_rf, c->d_nn, c->d_sum_nn, c->d_bits, c->d_prev_bits, c->d_prev_kp,
@@ -891,48 +893,13 @@ int bshot_icp(bshot_ctx* ctx, const float* src_xyz, size_t n_src, const float* t
     return icp_run(ctx, src_xyz, n_src, tgt_xyz, n_tgt, pre4x4, max_iterations, final4x4_out, iterations_out, state_out, mse_out);
 }
 
-// general 4x4 inverse by cofactors in float (Matrix4f::inverse(), src/lidar_odometry.cpp:269)
-static void inverse4x4(const float* m, float* o) {
-    float inv[16];
-    inv[0] = m[5] * m[10] * m[15] - m[5] * m[11] * m[14] - m[9] * m[6] * m[15] + m[9] * m[7] * m[14] + m[13] * m[6] * m[11] - m[13] * m[7] * m[10];
-    inv[4] = -m[4] * m[10] * m[15] + m[4] * m[11] * m[14] + m[8] * m[6] * m[15] - m[8] * m[7] * m[14] - m[12] * m[6] * m[11] + m[12] * m[7] * m[10];
-    inv[8] = m[4] * m[9] * m[15] - m[4] * m[11] * m[13] - m[8] * m[5] * m[15] + m[8] * m[7] * m[13] + m[12] * m[5] * m[11] - m[12] * m[7] * m[9];
-    inv[12] = -m[4] * m[9] * m[14] + m[4] * m[10] * m[13] + m[8] * m[5] * m[14] - m[8] * m[6] * m[13] - m[12] * m[5] * m[10] + m[12] * m[6] * m[9];
-    inv[1] = -m[1] * m[10] * m[15] + m[1] * m[11] * m[14] + m[9] * m[2] * m[15] - m[9] * m[3] * m[14] - m[13] * m[2] * m[11] + m[13] * m[3] * m[10];
-    inv[5] = m[0] * m[10] * m[15] - m[0] * m[11] * m[14] - m[8] * m[2] * m[15] + m[8] * m[3] * m[14] + m[12] * m[2] * m[11] - m[12] * m[3] * m[10];
-    inv[9] = -m[0] * m[9] * m[15] + m[0] * m[11] * m[13] + m[8] * m[1] * m[15] - m[8] * m[3] * m[13] - m[12] * m[1] * m[11] + m[12] * m[3] * m[9];
-    inv[13] = m[0] * m[9] * m[14] - m[0] * m[10] * m[13] - m[8] * m[1] * m[14] + m[8] * m[2] * m[13] + m[12] * m[1] * m[10] - m[12] * m[2] * m[9];
-    inv[2] = m[1] * m[6] * m[15] - m[1] * m[7] * m[14] - m[5] * m[2] * m[15] + m[5] * m[3] * m[14] + m[13] * m[2] * m[7] - m[13] * m[3] * m[6];
-    inv[6] = -m[0] * m[6] * m[15] + m[0] * m[7] * m[14] + m[4] * m[2] * m[15] - m[4] * m[3] * m[14] - m[12] * m[2] * m[7] + m[12] * m[3] * m[6];
-    inv[10] = m[0] * m[5] * m[15] - m[0] * m[7] * m[13] - m[4] * m[1] * m[15] + m[4] * m[3] * m[13] + m[12] * m[1] * m[7] - m[12] * m[3] * m[5];
-    inv[14] = -m[0] * m[5] * m[14] + m[0] * m[6] * m[13] + m[4] * m[1] * m[14] - m[4] * m[2] * m[13] - m[12] * m[1] * m[6] + m[12] * m[2] * m[5];
-    inv[3] = -m[1] * m[6] * m[11] + m[1] * m[7] * m[10] + m[5] * m[2] * m[11] - m[5] * m[3] * m[10] - m[9] * m[2] * m[7] + m[9] * m[3] * m[6];
-    inv[7] = m[0] * m[6] * m[11] - m[0] * m[7] * m[10] - m[4] * m[2] * m[11] + m[4] * m[3] * m[10] + m[8] * m[2] * m[7] - m[8] * m[3] * m[6];
-    inv[11] = -m[0] * m[5] * m[11] + m[0] * m[7] * m[9] + m[4] * m[1] * m[11] - m[4] * m[3] * m[9] - m[8] * m[1] * m[7] + m[8] * m[3] * m[5];
-    inv[15] = m[0] * m[5] * m[10] - m[0] * m[6] * m[9] - m[4] * m[1] * m[10] + m[4] * m[2] * m[9] + m[8] * m[1] * m[6] - m[8] * m[2] * m[5];
-    const float det = m[0] * inv[0] + m[1] * inv[4] + m[2] * inv[8] + m[3] * inv[12];
-    const float id = 1.0f / det;
-    for (int e = 0; e < 16; ++e) o[e] = inv[e] * id;
-}
-
-static void mul4x4(const float* a, const float* b, float* o) {
-    float r[16];
-    for (int i = 0; i < 4; ++i)
-        for (int j = 0; j < 4; ++j) r[4 * i + j] = ((a[4 * i] * b[j] + a[4 * i + 1] * b[4 + j]) + a[4 * i + 2] * b[8 + j]) + a[4 * i + 3] * b[12 + j];
-    for (int e = 0; e < 16; ++e) o[e] = r[e];
-}
-
 int bshot_evaluate_estimation(bshot_ctx* ctx, const float* T_ransac, const float* T_ref, int n_correspondences, const float* src_kp, size_t n_src,
                               const float* tgt_kp, size_t n_tgt, int run_icp, float* T_best_out, int* should_update_map_out, float* h_diff_out,
                               float* t_diff_out, int* icp_iterations_out) {
     CHECK_CTX(ctx);
     if (!T_ransac || !T_ref || !T_best_out) { set_error("bshot_evaluate_estimation: null matrix"); return BSHOT_E_INVALID; }
-    float Ti_inv[16], Tij[16];
-    inverse4x4(T_ref, Ti_inv);
-    mul4x4(Ti_inv, T_ransac, Tij);                                   // T_ij = T_i.inverse() * T_j (:269)
-    const float h_diff = acosf(Tij[5]);                              // heading (0,1,0): heading^T R heading = R(1,1) (:271-272)
-    const float t_diff = sqrtf((Tij[3] * Tij[3] + Tij[7] * Tij[7]) + Tij[11] * Tij[11]);
-    const bool reject = (double)(h_diff * 180) / M_PI > 10 || t_diff > 1200 || n_correspondences < 15;   // :281
+    float h_diff, t_diff;
+    const bool reject = estimation_gate(T_ransac, T_ref, n_correspondences, &h_diff, &t_diff);   // :269-281 (odom_math.cuh)
     const float* T_est = reject ? T_ref : T_ransac;
     if (should_update_map_out) *should_update_map_out = reject ? 0 : 1;
     if (h_diff_out) *h_diff_out = h_diff;
@@ -978,6 +945,74 @@ int bshot_preprocess_select(bshot_ctx* ctx, const double* azimuth_deg, const dou
 int bshot_preprocess(bshot_ctx* ctx, const double* azimuth_deg, const double* vertical_deg, const unsigned short* distance, size_t n, const double* ring_deg,
                      size_t nv, double vert_init_rad, double lowpt_th, float* xyz_out, size_t cap, size_t* n_out) {
     return bshot_preprocess_select(ctx, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, vert_init_rad, lowpt_th, nullptr, 0, 0, 1, xyz_out, cap, n_out);
+}
+
+// ---- the per-scan odometry step (test/odometry_test.cpp:143-184, odometry.cu) ---------------------------------------
+void bshot_odom_params_default(bshot_odom_params* p) {
+    if (!p) return;
+    bshot_params_default(&p->front);
+    p->vert_init_rad = -0.6;
+    p->lowpt_th = -1950.0;
+    p->map_range = 100000.0f;
+    p->ransac_iterations = 2000;
+    p->inlier_threshold = 1500.0f;
+    p->run_icp = 1;
+}
+
+static int odom_args_ok(bshot_ctx* ctx, const bshot_odom_params* p, const char* who) {
+    if (p->ransac_iterations < 1 || p->ransac_iterations > 100000) { set_error("%s: ransac_iterations %d outside [1, 100000]", who, p->ransac_iterations); return BSHOT_E_INVALID; }
+    if (!(p->inlier_threshold > 0.0f) || !std::isfinite(p->inlier_threshold)) { set_error("%s: inlier_threshold must be finite and > 0", who); return BSHOT_E_INVALID; }
+    if (!(p->map_range >= 0.0f) || !std::isfinite(p->map_range)) { set_error("%s: map_range must be finite and >= 0", who); return BSHOT_E_INVALID; }
+    if (!ctx->gmap.d_tab) { set_error("%s: needs a map (bshot_gmap_create)", who); return BSHOT_E_STATE; }
+    return BSHOT_OK;
+}
+
+int bshot_odometry_step(bshot_ctx* ctx, const bshot_odom_params* p, const double* azimuth_deg, const double* vertical_deg, const unsigned short* distance,
+                        size_t n, const double* ring_deg, size_t nv, bshot_odom_report* out) {
+    CHECK_CTX(ctx);
+    bshot_odom_params dp;
+    if (!p) { bshot_odom_params_default(&dp); p = &dp; }
+    if (n && (!azimuth_deg || !vertical_deg || !distance)) { set_error("bshot_odometry_step: null input"); return BSHOT_E_INVALID; }
+    if (nv && !ring_deg) { set_error("bshot_odometry_step: null ring table"); return BSHOT_E_INVALID; }
+    if (n > 0xFFFFFFFFull) { set_error("bshot_odometry_step: too many returns"); return BSHOT_E_CAPACITY; }
+    BSHOT_TRY(odom_args_ok(ctx, p, "bshot_odometry_step"));
+    // Preprocessor::run; its two count read-backs size the front end's grids, the cloud stays on the device
+    size_t kept = 0;
+    const float* d_cloud = nullptr;
+    BSHOT_TRY(preprocess_run(ctx, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, p->vert_init_rad, p->lowpt_th, nullptr, 1, nullptr, std::max<size_t>(n, 1),
+                             &kept, &d_cloud));
+    BSHOT_TRY(frame_args_ok(ctx, &p->front, kept, 12, "bshot_odometry_step"));
+    return odometry_run(ctx, p, d_cloud, kept, 3, out);
+}
+
+int bshot_odometry_step_cloud(bshot_ctx* ctx, const bshot_odom_params* p, const float* xyz, size_t n, size_t stride_bytes, bshot_odom_report* out) {
+    CHECK_CTX(ctx);
+    bshot_odom_params dp;
+    if (!p) { bshot_odom_params_default(&dp); p = &dp; }
+    if (!xyz && n) { set_error("bshot_odometry_step_cloud: null cloud"); return BSHOT_E_INVALID; }
+    BSHOT_TRY(odom_args_ok(ctx, p, "bshot_odometry_step_cloud"));
+    BSHOT_TRY(frame_args_ok(ctx, &p->front, n, stride_bytes, "bshot_odometry_step_cloud"));
+    BSHOT_TRY(h2d(ctx, ctx->d_raw, xyz, n * stride_bytes));
+    return odometry_run(ctx, p, ctx->d_raw, n, (int)(stride_bytes / 4), out);
+}
+
+int bshot_odometry_reset(bshot_ctx* ctx) {
+    CHECK_CTX(ctx);
+    if (!ctx->gmap.d_tab) { set_error("bshot_odometry_reset: needs a map (bshot_gmap_create)"); return BSHOT_E_STATE; }
+    return odometry_reset(ctx);
+}
+
+int bshot_ransac_dev(bshot_ctx* ctx, const void* d_src4, const void* d_tgt4, const void* d_pairs, const void* d_n_pairs, size_t n_pairs_cap,
+                     int max_iterations, float inlier_threshold, void* d_inlier_pairs_out, void* d_n_inliers_out, void* d_transform_out,
+                     void* d_iterations_out) {
+    CHECK_CTX(ctx);
+    if (!d_n_pairs || !d_n_inliers_out || !d_transform_out || !d_iterations_out || (n_pairs_cap && (!d_src4 || !d_tgt4 || !d_pairs || !d_inlier_pairs_out))) {
+        set_error("bshot_ransac_dev: null device pointer");
+        return BSHOT_E_INVALID;
+    }
+    return ransac_run_dev(ctx, reinterpret_cast<const float4*>(d_src4), reinterpret_cast<const float4*>(d_tgt4), reinterpret_cast<const int*>(d_pairs), 2,
+                          reinterpret_cast<const int*>(d_n_pairs), n_pairs_cap, max_iterations, (double)inlier_threshold, reinterpret_cast<int*>(d_inlier_pairs_out),
+                          reinterpret_cast<int*>(d_n_inliers_out), reinterpret_cast<float*>(d_transform_out), reinterpret_cast<int*>(d_iterations_out), nullptr);
 }
 
 // ---- ISS keypoints + keypoint repeatability (kp_test evaluation, src/lidar_odometry.cpp:392-461) -----------------------

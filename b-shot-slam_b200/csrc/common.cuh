@@ -77,6 +77,8 @@ struct SumGate {
     int top_k;
 };
 
+struct IcpState;   // icp.cu / stages.h
+
 // GPU-resident global keypoint map (gmap.cu)
 struct Gmap {
     void* d_tab = nullptr;              // block hash table (GmapBlock[tab_cap])
@@ -117,6 +119,19 @@ struct Vg {
     unsigned* d_seg = nullptr;          // first sorted position of every voxel, then the finite count
     float* d_out = nullptr;             // [0] = count (as unsigned), [1..3] unused, then {x, y, z} records
     float* h_out = nullptr;             // pinned staging of d_out
+};
+
+// per-scan odometry step (odometry.cu): allocated by the first bshot_odometry_step / bshot_ransac_dev of the context
+struct OdomDev;
+struct Odom {
+    OdomDev* d = nullptr;               // report, error flag, pose, gate matrices, RANSAC outputs (odometry.cu)
+    int* d_inlier_pairs = nullptr;      // max_kp x 2: the pairs RANSAC keeps
+    float4* d_icp_cur = nullptr;        // max_kp: ICP sources (moved)
+    unsigned long long* d_icp_keys = nullptr;  // max_kp
+    float4* d_icp_tgt = nullptr;        // max_targets: ICP targets, NaN past the true count
+    IcpState* d_icp_state = nullptr;
+    void* h_out = nullptr;              // pinned staging of the report
+    bool run = false;                   // RUN status: a step has succeeded since creation / bshot_odometry_reset
 };
 
 // query blocks are listed by weight class (class c: kBlockClasses regions of max_points entries in d_blocks / d_blk_area)
@@ -221,6 +236,7 @@ struct Ctx {
     Gmap gmap;
     Iss iss;
     Vg vg;
+    Odom odom;
     float4* d_prev_kp = nullptr;        // K: keypoint positions of the previous frame (reference frame of the map match)
     void* d_pre[3] = {nullptr, nullptr, nullptr};  // scratch grown on demand: preprocessor per-return / per-column, ICP
     size_t pre_bytes[3] = {0, 0, 0};

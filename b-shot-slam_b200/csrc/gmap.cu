@@ -16,6 +16,8 @@
 // table slot {key, count, first chunk, last chunk} plus a chain of 32-index chunks, so a warp reads a block 32 entries
 // at a time.  Admission is sequential per block (the rule is order dependent) and parallel across blocks: one warp per
 // block touched by the frame walks the frame's keypoints in order.
+#include <cmath>
+
 #include "common.cuh"
 #include "stages.h"
 
@@ -171,11 +173,15 @@ __host__ __device__ inline GmapCube gm_cube(float px, float py, float pz, float 
 
 // one CTA: counts of the probed blocks in loop order (x outermost, z innermost), exclusive scan -> offsets
 __global__ void __launch_bounds__(1024)
-gm_probe_kernel(const GmapBlock* __restrict__ tab, unsigned mask, GmapCube cube, unsigned* __restrict__ probe_slot,
-                unsigned* __restrict__ probe_off, unsigned* __restrict__ ctl, unsigned max_probe) {
+gm_probe_kernel(const GmapBlock* __restrict__ tab, unsigned mask, GmapCube cube, const float* __restrict__ dev_pose, float range,
+                unsigned* __restrict__ probe_slot, unsigned* __restrict__ probe_off, unsigned* __restrict__ ctl, unsigned max_probe) {
     __shared__ unsigned ws[32];
     __shared__ unsigned carry;
     const unsigned tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    if (dev_pose) {   // position = translation of the row-major [R|T]; a non-finite pose probes nothing
+        cube = gm_cube(dev_pose[3], dev_pose[7], dev_pose[11], range);
+        if (cube.nx <= 0 || cube.ny <= 0 || cube.nz <= 0) cube.nx = cube.ny = cube.nz = 0;
+    }
     const unsigned np = min((unsigned)(cube.nx * cube.ny * cube.nz), max_probe);
     if (tid == 0) carry = 0;
     __syncthreads();
@@ -305,12 +311,12 @@ int gmap_reset(Ctx* c) {
 }
 
 // ctl: [0] entries, [1] touched blocks of the current update, [2] chunks, [3] dropped (capacity), [4] gathered map entries, [5] probes
-int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t* d_bits, const int* d_count, size_t n_cap, const float* pose12) {
+int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t* d_bits, const int* d_count, size_t n_cap, const float* pose12, bool pose_on_device) {
     Gmap& g = c->gmap;
     if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
     if (n_cap == 0) return BSHOT_OK;
     if (n_cap > c->max_kp) { set_error("map update: %zu keypoints > capacity %zu", n_cap, c->max_kp); return BSHOT_E_CAPACITY; }
-    if (pose12) BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_pose, pose12, sizeof(float) * 12, cudaMemcpyHostToDevice, c->stream));
+    if (pose12) BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_pose, pose12, sizeof(float) * 12, pose_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, c->stream));
     BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_ctl + 1, 0, sizeof(unsigned), c->stream));
     ++g.epoch;
     const unsigned n = (unsigned)n_cap;
@@ -326,13 +332,23 @@ int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t
 // target set of featureMatching in RUN status: map keypoints within `range` of `pos`, then the reference frame
 // (d_ref_* may be null).  Descriptors -> d_t_out (the matcher's target buffer), positions -> g.d_tpos; *d_total = count.
 int gmap_gather(Ctx* c, const float pos[3], float range, const float4* d_ref_kp, const uint64_t* d_ref_bits, const int* d_ref_count,
-                size_t ref_cap, const float* ref_pose12, uint64_t* d_t_out, size_t out_cap, unsigned* d_total) {
+                size_t ref_cap, const float* ref_pose12, uint64_t* d_t_out, size_t out_cap, unsigned* d_total, bool pose_on_device) {
     Gmap& g = c->gmap;
     if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
-    const GmapCube cube = gm_cube(pos[0], pos[1], pos[2], range);
-    if ((long long)cube.nx * cube.ny * cube.nz > (long long)g.max_probe) { set_error("map gather: range %.0f probes more than %u blocks", range, g.max_probe); return BSHOT_E_CAPACITY; }
-    if (ref_pose12) BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_pose + 12, ref_pose12, sizeof(float) * 12, cudaMemcpyHostToDevice, c->stream));
-    gm_probe_kernel<<<1, 1024, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.tab_cap - 1, cube, g.d_probe_slot, g.d_probe_off, g.d_ctl, g.max_probe);
+    GmapCube cube = {0, 0, 0, 0, 0, 0};
+    if (pose_on_device) {
+        // position = translation of the device-side pose: the cube is computed by the probe kernel.  Its edge is at most
+        // round((p + r) / 10 m) - round((p - r) / 10 m) + 1 <= 2 r / 10 m + 3 blocks (rounding included), whatever p is
+        const double edge = std::floor(2.0 * (double)range / (double)GM_PREC) + 3.0;
+        if (!ref_pose12 || edge * edge * edge > (double)g.max_probe) { set_error("map gather: range %.0f probes more than %u blocks", range, g.max_probe); return BSHOT_E_CAPACITY; }
+    } else {
+        cube = gm_cube(pos[0], pos[1], pos[2], range);
+        if ((long long)cube.nx * cube.ny * cube.nz > (long long)g.max_probe) { set_error("map gather: range %.0f probes more than %u blocks", range, g.max_probe); return BSHOT_E_CAPACITY; }
+    }
+    if (ref_pose12)
+        BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_pose + 12, ref_pose12, sizeof(float) * 12, pose_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, c->stream));
+    gm_probe_kernel<<<1, 1024, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.tab_cap - 1, cube, pose_on_device ? g.d_pose + 12 : nullptr, range,
+                                               g.d_probe_slot, g.d_probe_off, g.d_ctl, g.max_probe);
     gm_collect_kernel<<<(unsigned)c->sm_count * 2u, 128, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.d_probe_slot, g.d_probe_off, g.d_ctl, g.d_chunks,
                                                                         g.d_epos, g.d_edesc, g.d_tpos, d_t_out, (unsigned)out_cap);
     const unsigned nref = d_ref_bits ? (unsigned)ref_cap : 0u;

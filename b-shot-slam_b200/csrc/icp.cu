@@ -29,12 +29,6 @@ constexpr int ICP_TGT = 2048;     // targets per CTA of the search kernel
 
 enum { ICP_NOT_CONVERGED = 0, ICP_ITERATIONS = 1, ICP_TRANSFORM = 2, ICP_ABS_MSE = 3, ICP_REL_MSE = 4, ICP_NO_CORRESPONDENCES = 5 };
 
-struct IcpState {
-    float final_T[16];
-    double prev_mse, mse;
-    int iterations, state, done, pad;
-};
-
 // nearest target of every source point: CTA = 128 sources x a slice of the targets staged through shared memory,
 // the slices meet in a packed atomicMin (squared distance bits << 32 | index: lowest index wins ties)
 __global__ void __launch_bounds__(ICP_SRC)
@@ -240,6 +234,58 @@ int icp_run(Ctx* c, const float* src_xyz, size_t n_src, const float* tgt_xyz, si
     if (state_out) *state_out = h.state;
     if (mse_out) *mse_out = h.mse;
     return BSHOT_OK;
+}
+
+// ---- device inputs (the odometry step) -----------------------------------------------------------------------------------
+// Sources: the frame's keypoints (float4) moved by the device-side pre-transform; targets: any float4 array.  Both counts
+// stay on the device: the kernels above run on the host-known capacities, and the slots past the true counts hold NaN,
+// which never becomes a correspondence (icp_nn_kernel tests d == d), so icp_fit_kernel's 256 strided partial sums -- and
+// hence every bit of the result -- depend only on the true points.  A set *d_skip makes every launch a no-op.
+__global__ void icp_init_dev_kernel(const float4* __restrict__ src, const int* __restrict__ d_ns, unsigned ns_cap, const float4* __restrict__ tgt,
+                                    const unsigned* __restrict__ d_nt, unsigned nt_cap, const float* __restrict__ pre, const int* __restrict__ skip,
+                                    float4* __restrict__ cur, float4* __restrict__ tgt_out, unsigned long long* __restrict__ keys, IcpState* __restrict__ st) {
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned ns = min((unsigned)max(*d_ns, 0), ns_cap), nt = min(*d_nt, nt_cap);
+    const float nan = __int_as_float(0x7fc00000);
+    if (i < ns_cap) {
+        float4 o = make_float4(nan, nan, nan, 0.f);
+        if (i < ns) {
+            const float4 p = src[i];
+            const float x = p.x, y = p.y, z = p.z;
+            o.x = ((pre[0] * x + pre[1] * y) + pre[2] * z) + pre[3];
+            o.y = ((pre[4] * x + pre[5] * y) + pre[6] * z) + pre[7];
+            o.z = ((pre[8] * x + pre[9] * y) + pre[10] * z) + pre[11];
+        }
+        cur[i] = o;
+        keys[i] = ~0ull;
+    }
+    if (i < nt_cap) {
+        const float4 q = (i < nt) ? tgt[i] : make_float4(nan, nan, nan, 0.f);
+        tgt_out[i] = make_float4(q.x, q.y, q.z, 0.f);
+    }
+    if (i == 0) {
+        for (int e = 0; e < 16; ++e) st->final_T[e] = (e % 5 == 0) ? 1.0f : 0.0f;
+        st->prev_mse = 1.7976931348623157e308;
+        st->mse = 0.0; st->iterations = 0; st->state = ICP_NOT_CONVERGED; st->pad = 0;
+        st->done = (skip && *skip) ? 1 : 0;
+        if (ns == 0 || nt == 0) { st->state = ICP_NO_CORRESPONDENCES; st->done = 1; }
+    }
+}
+
+int icp_run_dev(Ctx* c, const float4* d_src, const int* d_ns, size_t ns_cap, const float4* d_tgt, const unsigned* d_nt, size_t nt_cap, const float* d_pre,
+                int max_iterations, const int* d_skip, float4* d_cur, float4* d_tgt_buf, unsigned long long* d_keys, IcpState* d_st) {
+    const unsigned ns = (unsigned)ns_cap, nt = (unsigned)nt_cap, nmax = std::max(std::max(ns, nt), 1u);
+    icp_init_dev_kernel<<<(nmax + 255) / 256, 256, 0, c->stream>>>(d_src, d_ns, ns, d_tgt, d_nt, nt, d_pre, d_skip, d_cur, d_tgt_buf, d_keys, d_st);
+    count_launch(c);
+    if (ns && nt) {
+        const dim3 grid((ns + ICP_SRC - 1) / ICP_SRC, (nt + ICP_TGT - 1) / ICP_TGT);
+        for (int it = 0; it < max_iterations; ++it) {
+            icp_nn_kernel<<<grid, ICP_SRC, 0, c->stream>>>(d_cur, ns, d_tgt_buf, nt, d_keys, d_st);
+            icp_fit_kernel<<<1, ICP_T, 0, c->stream>>>(d_cur, ns, d_tgt_buf, d_keys, d_st, max_iterations);
+        }
+        count_launch(c, 2 * max_iterations);
+    }
+    return check_launch("device ICP kernels");
 }
 
 }  // namespace bshot

@@ -1,0 +1,202 @@
+// odometry.cu -- the per-scan odometry step on the device (test/odometry_test.cpp:143-184 in one call).
+//
+// The stages are the existing ones; what changes is that their inputs stay on the device:
+//   extract (frame_extract) -> first scan: the frame's descriptors against themselves, later scans: the map keypoints in
+//   range of the stored pose ++ the reference frame moved by it (gmap_gather with the pose on the device) -> mutual nearest
+//   neighbours (device-side counts) -> RANSAC on the device (ransac_run_dev) -> the gate of evaluateEstimation
+//   (odom_math.cuh, the host's code) -> ICP on the device (icp_run_dev) -> T_best -> updateMap (gmap_update with the pose on
+//   the device) -> the frame becomes the reference frame.
+// The only host round trip after the preprocessor is the copy of the report at the end.  A target set larger than
+// max_targets is detected on the device (the host call's test, on device counts): the flag makes RANSAC and ICP no-ops and
+// keeps the pose, the map and the reference frame as they were.  Compiled with -fmad=false: the gate and the composition
+// T_best = F * T_est give the host's bits.
+#include <cmath>
+
+#include "common.cuh"
+#include "odom_math.cuh"
+#include "stages.h"
+
+namespace bshot {
+
+struct OdomDev {
+    bshot_odom_report rep;   // copied to the host at the end of a step, together with err
+    int err;                 // BSHOT_E_* raised on the device during the step (0 = none)
+    int eff_count;           // keypoints the map update takes: the frame's count, 0 after an error
+    float pose[16];          // pose of the last successful step, row-major (identity after a reset)
+    float T_est[16];
+    float T_ransac[16];
+    int n_inliers, ransac_iterations;
+};
+
+__global__ void odom_reset_kernel(OdomDev* d) {
+    if (threadIdx.x < 16) d->pose[threadIdx.x] = (threadIdx.x % 5 == 0) ? 1.0f : 0.0f;
+    if (threadIdx.x == 0) d->err = 0;
+}
+
+// bshot_match_frame_to_map's capacity test on device counts: ctl[4] map entries in range, ctl[6] targets assembled
+__global__ void odom_check_kernel(const unsigned* __restrict__ ctl, unsigned long long n_prev, unsigned long long max_targets, OdomDev* d) {
+    if ((unsigned long long)ctl[4] + n_prev > max_targets && (unsigned long long)ctl[6] == max_targets) d->err = BSHOT_E_CAPACITY;
+}
+
+// evaluateEstimation's gate (src/lidar_odometry.cpp:267-281): T_est = T_ref when rejected, else T_ransac
+__global__ void odom_gate_kernel(OdomDev* d) {
+    float h, t;
+    const bool reject = estimation_gate(d->T_ransac, d->pose, d->n_inliers, &h, &t);
+    for (int e = 0; e < 16; ++e) d->T_est[e] = reject ? d->pose[e] : d->T_ransac[e];
+    d->rep.h_diff_rad = h;
+    d->rep.t_diff_mm = t;
+    d->rep.should_update_map = reject ? 0 : 1;
+}
+
+// T_best (:293 / :295), the report, and -- without an error -- the new pose and the map update's count
+__global__ void odom_final_kernel(OdomDev* d, const IcpState* __restrict__ icp, int run_icp, const int* __restrict__ kp_count,
+                                  const int* __restrict__ pair_count, const unsigned* __restrict__ d_total, int k, unsigned long long n_points,
+                                  int was_initial) {
+    float T_best[16];
+    if (run_icp) mul4x4(icp->final_T, d->T_est, T_best);
+    else for (int e = 0; e < 16; ++e) T_best[e] = d->T_ransac[e];
+    bshot_odom_report& r = d->rep;
+    for (int e = 0; e < 16; ++e) { r.pose[e] = T_best[e]; r.T_ransac[e] = d->T_ransac[e]; }
+    const int nk = min(max(*kp_count, 0), k);
+    r.n_points = (size_t)n_points;
+    r.n_targets = was_initial ? (size_t)nk : (size_t)*d_total;
+    r.n_keypoints = nk;
+    r.n_pairs = min(max(*pair_count, 0), k);
+    r.n_inliers = d->n_inliers;
+    r.ransac_iterations = d->ransac_iterations;
+    r.icp_iterations = run_icp ? icp->iterations : 0;
+    r.was_initial = was_initial;
+    if (d->err == 0) {
+        for (int e = 0; e < 16; ++e) d->pose[e] = T_best[e];
+        d->eff_count = *kp_count;
+    } else {
+        d->eff_count = 0;
+    }
+}
+
+// frame_commit's copy, skipped after an error (the reference frame stays)
+__global__ void odom_commit_kernel(const uint64_t* __restrict__ bits, const float4* __restrict__ kp, const int* __restrict__ count, unsigned cap,
+                                   const OdomDev* __restrict__ d, uint64_t* __restrict__ prev, float4* __restrict__ prev_kp, int* __restrict__ prev_count) {
+    if (d->err) return;
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    const int k = *count;
+    if (i < cap * 6 && (int)(i / 6) < k) prev[i] = bits[i];
+    if (i < cap && (int)i < k) prev_kp[i] = kp[i];
+    if (i == 0) *prev_count = k;
+}
+
+int odom_ensure(Ctx* c) {
+    Odom& o = c->odom;
+    if (o.d) return BSHOT_OK;
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d, sizeof(OdomDev)));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_inlier_pairs, sizeof(int) * 2 * c->max_kp));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_icp_cur, sizeof(float4) * c->max_kp));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_icp_keys, sizeof(unsigned long long) * c->max_kp));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_icp_tgt, sizeof(float4) * c->max_targets));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_icp_state, sizeof(IcpState)));
+    BSHOT_CUDA_TRY(cudaMallocHost(&o.h_out, sizeof(OdomDev)));
+    BSHOT_CUDA_TRY(cudaMemsetAsync(o.d, 0, sizeof(OdomDev), c->stream));
+    odom_reset_kernel<<<1, 32, 0, c->stream>>>(o.d);
+    count_launch(c);
+    o.run = false;
+    return check_launch("odom_reset_kernel");
+}
+
+void odom_free(Ctx* c) {
+    Odom& o = c->odom;
+    void* ptrs[] = {o.d, o.d_inlier_pairs, o.d_icp_cur, o.d_icp_keys, o.d_icp_tgt, o.d_icp_state};
+    for (void* p : ptrs) if (p) cudaFree(p);
+    if (o.h_out) cudaFreeHost(o.h_out);
+    o = Odom();
+}
+
+int odometry_reset(Ctx* c) {
+    BSHOT_TRY(odom_ensure(c));
+    odom_reset_kernel<<<1, 32, 0, c->stream>>>(c->odom.d);
+    count_launch(c);
+    BSHOT_TRY(check_launch("odom_reset_kernel"));
+    c->odom.run = false;
+    BSHOT_TRY(gmap_reset(c));
+    c->gmap.entries_upper = 0;
+    // no reference frame, and the cross-frame state of the front end as a new context has it
+    BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_prev_count, 0, sizeof(int), c->stream));
+    BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_normals, 0, sizeof(float4) * c->max_points, c->stream));
+    c->n_prev = 0;
+    c->normals_valid = 0;
+    c->have_normals = false;
+    c->gate_top_k = 0;
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    return BSHOT_OK;
+}
+
+// everything after the cloud is on the device (d_cloud: n points, stride_floats 3 or 4); n_points is reported as is
+int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_t n, int stride_floats, bshot_odom_report* out) {
+    BSHOT_TRY(odom_ensure(c));
+    Odom& o = c->odom;
+    Gmap& g = c->gmap;
+    OdomDev* d = o.d;
+    BSHOT_TRY(frame_extract(c, &p->front, d_cloud, n, stride_floats));
+    const size_t k = (size_t)p->front.top_k;
+    const bool initial = !o.run;
+    BSHOT_CUDA_TRY(cudaMemsetAsync(&d->err, 0, sizeof(int), c->stream));
+    const unsigned* d_nq = reinterpret_cast<const unsigned*>(c->d_kp_count);
+    const float4* tgt_pos;
+    const unsigned* d_nt;
+    size_t nt_cap;
+    if (initial) {   // src/lidar_odometry.cpp:187-194: the target is the frame itself
+        BSHOT_TRY(hamming_match_rq(c, c->d_bits, k, c->d_bits, k, 0, c->d_cand, d_nq, d_nq));
+        BSHOT_TRY(hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq));
+        tgt_pos = c->d_kp;
+        d_nt = d_nq;
+        nt_cap = k;
+    } else {         // :197-206: map keypoints in range of the last pose ++ the reference frame moved by that pose
+        unsigned* d_total = g.d_ctl + 6;
+        BSHOT_TRY(gmap_gather(c, nullptr, p->map_range, c->d_prev_kp, c->d_prev_bits, c->d_prev_count, c->n_prev, d->pose, c->d_t, c->max_targets, d_total,
+                              /*pose_on_device=*/true));
+        odom_check_kernel<<<1, 1, 0, c->stream>>>(g.d_ctl, (unsigned long long)c->n_prev, (unsigned long long)c->max_targets, d);
+        count_launch(c);
+        nt_cap = std::min(c->max_targets, g.entries_upper + c->n_prev);
+        if (nt_cap == 0) {
+            BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_pair_count, 0, sizeof(int), c->stream));
+        } else {
+            BSHOT_TRY(hamming_match_rq(c, c->d_bits, k, c->d_t, nt_cap, 0, c->d_cand, d_nq, d_total));
+            BSHOT_TRY(hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq));
+        }
+        tgt_pos = g.d_tpos;
+        d_nt = d_total;
+    }
+    // featureMatching's RANSAC (:251-261) on the pairs (query, match, distance) the matcher left on the device
+    BSHOT_TRY(ransac_run_dev(c, c->d_kp, tgt_pos, c->d_pairs, 3, c->d_pair_count, k, p->ransac_iterations, (double)p->inlier_threshold, o.d_inlier_pairs,
+                             &d->n_inliers, d->T_ransac, &d->ransac_iterations, &d->err));
+    odom_gate_kernel<<<1, 1, 0, c->stream>>>(d);
+    count_launch(c);
+    if (p->run_icp) {   // :283-293 on the frame's keypoints and the target set
+        BSHOT_TRY(icp_run_dev(c, c->d_kp, c->d_kp_count, k, tgt_pos, d_nt, nt_cap, d->T_est, 10, &d->err, o.d_icp_cur, o.d_icp_tgt, o.d_icp_keys,
+                              o.d_icp_state));
+    }
+    odom_final_kernel<<<1, 1, 0, c->stream>>>(d, o.d_icp_state, p->run_icp ? 1 : 0, c->d_kp_count, c->d_pair_count, initial ? nullptr : g.d_ctl + 6, (int)k,
+                                              (unsigned long long)n, initial ? 1 : 0);
+    count_launch(c);
+    BSHOT_TRY(check_launch("odometry step kernels"));
+    // updateMap (:343-358) with T_best, whatever the gate said; after an error the count is 0 and the map stays
+    BSHOT_TRY(gmap_update(c, c->d_kp, c->d_kp_ratio, c->d_bits, &d->eff_count, c->last_top_k, d->pose, /*pose_on_device=*/true));
+    odom_commit_kernel<<<(unsigned)((k * 6 + 255) / 256), 256, 0, c->stream>>>(c->d_bits, c->d_kp, c->d_kp_count, (unsigned)k, d, c->d_prev_bits,
+                                                                                c->d_prev_kp, c->d_prev_count);
+    count_launch(c);
+    BSHOT_TRY(check_launch("odom_commit_kernel"));
+    OdomDev* h = reinterpret_cast<OdomDev*>(o.h_out);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(h, d, offsetof(OdomDev, err) + sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    c->n_kp = (size_t)h->rep.n_keypoints;
+    if (h->err) {
+        set_error("bshot_odometry_step: target set exceeds max_targets %zu", c->max_targets);
+        return h->err;
+    }
+    g.entries_upper += c->last_top_k;
+    c->n_prev = k;
+    o.run = true;
+    if (out) *out = h->rep;
+    return BSHOT_OK;
+}
+
+}  // namespace bshot

@@ -64,11 +64,8 @@ __host__ __device__ inline float transfer_sqd(const float T[16], float sx, float
 }
 
 // one warp per hypothesis: model from its three pairs, inlier count over all correspondences
-__global__ void __launch_bounds__(128)
-ransac_score_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, unsigned n, const int* __restrict__ samples, unsigned n_hyp,
-                    double thresh2, float* __restrict__ models, int* __restrict__ counts) {
-    const unsigned lane = threadIdx.x & 31, h = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (h >= n_hyp) return;
+__device__ __forceinline__ void ransac_score_one(const float4* __restrict__ src, const float4* __restrict__ tgt, unsigned n, const int* __restrict__ samples,
+                                                 unsigned h, unsigned lane, double thresh2, float* __restrict__ models, int* __restrict__ counts) {
     float T[16];
     {
         double s[3][3], d[3][3];
@@ -90,15 +87,26 @@ ransac_score_kernel(const float4* __restrict__ src, const float4* __restrict__ t
     if (lane < 16) models[16 * h + lane] = T[lane];
 }
 
+__global__ void __launch_bounds__(128)
+ransac_score_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, unsigned n, const int* __restrict__ samples, unsigned n_hyp,
+                    double thresh2, float* __restrict__ models, int* __restrict__ counts) {
+    const unsigned lane = threadIdx.x & 31, h = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (h >= n_hyp) return;
+    ransac_score_one(src, tgt, n, samples, h, lane, thresh2, models, counts);
+}
+
+__device__ __forceinline__ unsigned char ransac_is_inlier(const float* __restrict__ model, const float4 a, const float4 b, double thresh2) {
+    float T[16];
+#pragma unroll
+    for (int k = 0; k < 16; ++k) T[k] = model[k];
+    return ((double)transfer_sqd(T, a.x, a.y, a.z, b.x, b.y, b.z) < thresh2) ? 1 : 0;
+}
+
 __global__ void ransac_select_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, unsigned n, const float* __restrict__ model,
                                      double thresh2, unsigned char* __restrict__ inlier) {
     const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
-    float T[16];
-#pragma unroll
-    for (int k = 0; k < 16; ++k) T[k] = model[k];
-    const float4 a = src[i], b = tgt[i];
-    inlier[i] = ((double)transfer_sqd(T, a.x, a.y, a.z, b.x, b.y, b.z) < thresh2) ? 1 : 0;
+    inlier[i] = ransac_is_inlier(model, src[i], tgt[i], thresh2);
 }
 
 // ---- host: PCL's sample sequence ------------------------------------------------------------------------------------------
@@ -125,13 +133,21 @@ struct Mt19937 {  // boost::mt19937 / std::mt19937 recurrence
     }
 };
 
-// pcl::eigen33 eigenvalues of a symmetric 3x3 in float are only needed for sample_dist_thresh; computed here in double
-// by Jacobi and rounded (the threshold only steers which samples are retried)
-void sym_eigenvalues(const double m_in[9], double w[3]) {
-    double U[9], V[9];
-    svd3_hestenes(m_in, U, w, V);  // symmetric positive semi-definite: singular values = eigenvalues
-}
 }  // namespace
+
+// sample_dist_thresh from the float sums {xx, xy, xz, yy, yz, zz, x, y, z} of n sources (host and device share it)
+__host__ __device__ inline double sample_dist_from_sums(float a[9], size_t n) {
+    const float fn = (float)n;
+    for (int k = 0; k < 9; ++k) a[k] /= fn;
+    const double cov[9] = {(double)(a[0] - a[6] * a[6]), (double)(a[1] - a[6] * a[7]), (double)(a[2] - a[6] * a[8]),
+                           (double)(a[1] - a[6] * a[7]), (double)(a[3] - a[7] * a[7]), (double)(a[4] - a[7] * a[8]),
+                           (double)(a[2] - a[6] * a[8]), (double)(a[4] - a[7] * a[8]), (double)(a[5] - a[8] * a[8])};
+    double U[9], w[3], V[9];
+    svd3_hestenes(cov, U, w, V);  // symmetric positive semi-definite: singular values = eigenvalues
+    const float e0 = (float)w[0], e1 = (float)w[1], e2 = (float)w[2];
+    double t = (double)((sqrtf(fmaxf(e0, 0.0f)) + sqrtf(fmaxf(e1, 0.0f))) + sqrtf(fmaxf(e2, 0.0f))) / 3.0;
+    return t * t;
+}
 
 // sample_dist_thresh of SampleConsensusModelRegistration::computeSampleDistanceThreshold over the correspondence sources
 static double sample_dist_threshold(const float* src4, size_t n) {
@@ -141,16 +157,7 @@ static double sample_dist_threshold(const float* src4, size_t n) {
         const float x = src4[4 * i], y = src4[4 * i + 1], z = src4[4 * i + 2];
         a[0] += x * x; a[1] += x * y; a[2] += x * z; a[3] += y * y; a[4] += y * z; a[5] += z * z; a[6] += x; a[7] += y; a[8] += z;
     }
-    const float fn = (float)n;
-    for (int k = 0; k < 9; ++k) a[k] /= fn;
-    const double cov[9] = {(double)(a[0] - a[6] * a[6]), (double)(a[1] - a[6] * a[7]), (double)(a[2] - a[6] * a[8]),
-                           (double)(a[1] - a[6] * a[7]), (double)(a[3] - a[7] * a[7]), (double)(a[4] - a[7] * a[8]),
-                           (double)(a[2] - a[6] * a[8]), (double)(a[4] - a[7] * a[8]), (double)(a[5] - a[8] * a[8])};
-    double w[3];
-    sym_eigenvalues(cov, w);
-    const float e0 = (float)w[0], e1 = (float)w[1], e2 = (float)w[2];
-    double t = (double)((sqrtf(fmaxf(e0, 0.0f)) + sqrtf(fmaxf(e1, 0.0f))) + sqrtf(fmaxf(e2, 0.0f))) / 3.0;
-    return t * t;
+    return sample_dist_from_sums(a, n);
 }
 
 int ransac_run(Ctx* c, const float* src_xyz, const float* tgt_xyz, const int* pairs, size_t n_pairs, int max_iterations, double threshold,
@@ -255,6 +262,274 @@ int ransac_run(Ctx* c, const float* src_xyz, const float* tgt_xyz, const int* pa
     if (transform_out) memcpy(transform_out, model, sizeof(model));
     if (iterations_out) *iterations_out = iterations;
     return BSHOT_OK;
+}
+
+// ---- device inputs: the whole of ransac_run without a host round trip (bshot_ransac_dev, the odometry step) ----------------
+// The correspondence count stays on the device.  PCL's sample sequence is produced on the device in batches of 208 tries
+// (= 624 draws, one mt19937 twist): the twist, the tempering and the moduli (mt() >> 1) % (n - j % 3) run in parallel, the
+// swap chain (the only sequential part: draw j always swaps position j % 3) runs on one thread with positions 0..2 in
+// registers, the distance tests of the 208 triples run in parallel, and one thread walks the test results in order, which
+// makes a try a hypothesis, counts the tries of the current hypothesis and gives up after 1000 -- exactly the host loop, for
+// any number of tries.  Scores, selection and the adaptive-stop replay are the host's, fed by device-side counts.
+struct RansacDevState {
+    double sdt;
+    int n, n_valid, best, iterations;
+};
+
+constexpr int RS_TRIES = 208;           // tries per batch: 3 x 208 = 624 draws = one twist
+constexpr int RS_THREADS = 256;
+
+__global__ void ransac_gather_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const int* __restrict__ pairs, int stride,
+                                     const int* __restrict__ d_n, unsigned cap, const int* __restrict__ skip, float4* __restrict__ s_out,
+                                     float4* __restrict__ t_out, RansacDevState* __restrict__ st) {
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned n = (skip && *skip) ? 0u : min((unsigned)max(*d_n, 0), cap);
+    if (i == 0) { st->n = (int)n; st->n_valid = 0; st->best = -1; st->iterations = 0; }
+    if (i >= n) return;
+    const float4 a = src[pairs[(size_t)stride * i]], b = tgt[pairs[(size_t)stride * i + 1]];
+    s_out[i] = make_float4(a.x, a.y, a.z, 1.0f);
+    t_out[i] = make_float4(b.x, b.y, b.z, 1.0f);
+}
+
+__device__ __forceinline__ double rs_d2(const float4* __restrict__ s, int a, int b) {
+    const float4 p = s[a], q = s[b];
+    const float dx = q.x - p.x, dy = q.y - p.y, dz = q.z - p.z;
+    return (double)(dx * dx + dy * dy + dz * dz);
+}
+
+// one CTA: sample_dist_thresh, then the sample sequence -> samples[3 * h ..], st->n_valid.  shuffled: n ints (shared memory
+// when it fits, else global scratch)
+__global__ void __launch_bounds__(RS_THREADS)
+ransac_sample_kernel(const float4* __restrict__ s4, RansacDevState* __restrict__ st, unsigned n_hyp, int* __restrict__ samples, int* g_shuffled) {
+    extern __shared__ int dyn_shuffled[];
+    __shared__ uint32_t mt[624];
+    __shared__ uint32_t mod[624];
+    __shared__ int trip[RS_TRIES * 3];
+    __shared__ unsigned char good[RS_TRIES];
+    __shared__ double s_sdt;
+    __shared__ int s_done;
+    const int tid = threadIdx.x;
+    const unsigned n = (unsigned)st->n;
+    if (n < 3) return;   // everything is kept (finish kernel)
+    int* sh = g_shuffled ? g_shuffled : dyn_shuffled;
+    // computeMeanAndCovarianceMatrix: float sums in index order.  Warp 0 gathers 32 sources at a time and every lane replays
+    // them in order, so the sequential chain never waits on a global load
+    if (tid < 32) {
+        float a[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
+        for (unsigned base = 0; base < n; base += 32) {
+            const float4 p = (base + tid < n) ? s4[base + tid] : make_float4(0.f, 0.f, 0.f, 0.f);
+            const unsigned m = min(32u, n - base);
+            for (unsigned j = 0; j < m; ++j) {
+                const float x = __shfl_sync(0xffffffffu, p.x, j), y = __shfl_sync(0xffffffffu, p.y, j), z = __shfl_sync(0xffffffffu, p.z, j);
+                a[0] += x * x; a[1] += x * y; a[2] += x * z; a[3] += y * y; a[4] += y * z; a[5] += z * z; a[6] += x; a[7] += y; a[8] += z;
+            }
+        }
+        if (tid == 0) {
+            s_sdt = sample_dist_from_sums(a, n);
+            st->sdt = s_sdt;
+        }
+    }
+    // mt19937 seeded 12345
+    if (tid == 0) {
+        mt[0] = 12345u;
+        for (int i = 1; i < 624; ++i) mt[i] = 1812433253u * (mt[i - 1] ^ (mt[i - 1] >> 30)) + (uint32_t)i;
+        s_done = 0;
+    }
+    for (unsigned i = tid; i < n; i += RS_THREADS) sh[i] = (int)i;
+    __syncthreads();
+    const double sdt = s_sdt;
+    int a0 = 0, a1 = 0, a2 = 0;                      // positions 0..2 of the shuffled list (thread 0)
+    if (tid == 0) { a0 = sh[0]; a1 = sh[1]; a2 = sh[2]; }
+    unsigned h = 0, tries = 0;                        // hypotheses found, tries of the current one (thread 0)
+    while (true) {
+        // twist in three dependency phases: [0, 227) reads old words only, [227, 454) reads the new [0, 227),
+        // [454, 624) reads the new [227, 397) and (i = 623) the new word 0
+        const int lo[3] = {0, 227, 454}, hi[3] = {227, 454, 624};
+        for (int ph = 0; ph < 3; ++ph) {
+            const int i = lo[ph] + tid;
+            uint32_t v = 0;
+            if (i < hi[ph]) {
+                const uint32_t y = (mt[i] & 0x80000000u) | (mt[(i + 1) % 624] & 0x7FFFFFFFu);
+                v = mt[(i + 397) % 624] ^ (y >> 1) ^ ((y & 1u) ? 0x9908B0DFu : 0u);
+            }
+            __syncthreads();
+            if (i < hi[ph]) mt[i] = v;
+            __syncthreads();
+        }
+        for (int j = tid; j < 624; j += RS_THREADS) {
+            uint32_t y = mt[j];
+            y ^= y >> 11; y ^= (y << 7) & 0x9D2C5680u; y ^= (y << 15) & 0xEFC60000u; y ^= y >> 18;
+            mod[j] = (y >> 1) % (n - (unsigned)(j % 3));
+        }
+        __syncthreads();
+        if (tid == 0) {   // the swap chain: std::swap(shuffled[p], shuffled[p + r]) for p = 0, 1, 2
+            for (int t = 0; t < RS_TRIES; ++t) {
+                const unsigned q0 = mod[3 * t], q1 = 1u + mod[3 * t + 1], q2 = 2u + mod[3 * t + 2];
+                int x;
+                if (q0 == 1u) { x = a0; a0 = a1; a1 = x; }
+                else if (q0 == 2u) { x = a0; a0 = a2; a2 = x; }
+                else if (q0 > 2u) { x = sh[q0]; sh[q0] = a0; a0 = x; }
+                if (q1 == 2u) { x = a1; a1 = a2; a2 = x; }
+                else if (q1 > 2u) { x = sh[q1]; sh[q1] = a1; a1 = x; }
+                if (q2 > 2u) { x = sh[q2]; sh[q2] = a2; a2 = x; }
+                trip[3 * t] = a0; trip[3 * t + 1] = a1; trip[3 * t + 2] = a2;
+            }
+        }
+        __syncthreads();
+        if (tid < RS_TRIES) {
+            const int i0 = trip[3 * tid], i1 = trip[3 * tid + 1], i2 = trip[3 * tid + 2];
+            good[tid] = (rs_d2(s4, i0, i1) > sdt && rs_d2(s4, i0, i2) > sdt && rs_d2(s4, i1, i2) > sdt) ? 1 : 0;
+        }
+        __syncthreads();
+        if (tid == 0) {   // the host loop over the tries of this batch
+            for (int t = 0; t < RS_TRIES; ++t) {
+                ++tries;
+                if (good[t]) {
+                    samples[3 * h] = trip[3 * t]; samples[3 * h + 1] = trip[3 * t + 1]; samples[3 * h + 2] = trip[3 * t + 2];
+                    ++h;
+                    tries = 0;
+                    if (h == n_hyp) { s_done = 1; break; }
+                } else if (tries == 1000u) {   // max_sample_checks_: "Could not select sample points", PCL stops here
+                    s_done = 1;
+                    break;
+                }
+            }
+            if (s_done) st->n_valid = (int)h;
+        }
+        __syncthreads();
+        if (s_done) break;
+    }
+}
+
+__global__ void __launch_bounds__(128)
+ransac_score_dev_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const RansacDevState* __restrict__ st, const int* __restrict__ samples,
+                        double thresh2, float* __restrict__ models, int* __restrict__ counts) {
+    const unsigned lane = threadIdx.x & 31, h = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (st->n < 3 || h >= (unsigned)st->n_valid) return;
+    ransac_score_one(src, tgt, (unsigned)st->n, samples, h, lane, thresh2, models, counts);
+}
+
+// RandomSampleConsensus::computeModel replayed over the scores (one thread; the host loop verbatim)
+__global__ void ransac_replay_kernel(RansacDevState* __restrict__ st, const int* __restrict__ counts, int max_iterations) {
+    if (threadIdx.x != 0 || blockIdx.x != 0) return;
+    const int n = st->n, n_valid = st->n_valid;
+    if (n < 3) return;
+    int iterations = 0, best = -1, n_best = -2147483647;
+    double k = 1.0;
+    const double log_probability = log(1.0 - 0.99), one_over_indices = 1.0 / (double)n;
+    while ((double)iterations < k) {
+        if (iterations >= n_valid) break;
+        const int cnt = counts[iterations];
+        if (cnt > n_best) {
+            n_best = cnt;
+            best = iterations;
+            const double w = (double)n_best * one_over_indices;
+            double p_no_outliers = 1.0 - pow(w, 3.0);
+            p_no_outliers = fmax(2.220446049250313e-16, p_no_outliers);
+            p_no_outliers = fmin(1.0 - 2.220446049250313e-16, p_no_outliers);
+            k = log_probability / log(p_no_outliers);
+        }
+        ++iterations;
+        if (iterations > max_iterations) break;
+    }
+    st->best = best;
+    st->iterations = iterations;
+}
+
+__global__ void ransac_select_dev_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const RansacDevState* __restrict__ st,
+                                         const float* __restrict__ models, double thresh2, unsigned char* __restrict__ inlier) {
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (st->best < 0 || i >= (unsigned)st->n) return;
+    inlier[i] = ransac_is_inlier(models + 16 * (size_t)st->best, src[i], tgt[i], thresh2);
+}
+
+// one CTA: the inliers of the best model in their original order, or (fewer than 3 correspondences / no hypothesis / fewer
+// than 3 inliers) every correspondence with the identity -- PCL's behaviour, as ransac_run's keep_all
+__global__ void __launch_bounds__(1024)
+ransac_finish_kernel(const RansacDevState* __restrict__ st, const int* __restrict__ pairs, int stride, const unsigned char* __restrict__ inlier,
+                     const float* __restrict__ models, int* __restrict__ pairs_out, int* __restrict__ n_out, float* __restrict__ T_out,
+                     int* __restrict__ iterations_out) {
+    __shared__ unsigned ws[32];
+    __shared__ unsigned carry;
+    const unsigned tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const unsigned n = (unsigned)max(st->n, 0);
+    const int best = st->best;
+    bool keep_all = n < 3 || best < 0;
+    if (tid == 0) carry = 0;
+    __syncthreads();
+    if (!keep_all) {
+        unsigned c = 0;
+        for (unsigned i = tid; i < n; i += 1024) c += inlier[i];
+        for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+        if (lane == 0) atomicAdd(&carry, c);
+        __syncthreads();
+        keep_all = carry < 3;
+        __syncthreads();
+        if (tid == 0) carry = 0;
+        __syncthreads();
+    }
+    for (unsigned base = 0; base < n; base += 1024) {
+        const unsigned i = base + tid;
+        const unsigned f = (i < n) ? (keep_all ? 1u : (unsigned)inlier[i]) : 0u;
+        unsigned inc = f;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned up = __shfl_up_sync(0xffffffffu, inc, o);
+            if (lane >= (unsigned)o) inc += up;
+        }
+        if (lane == 31) ws[wid] = inc;
+        __syncthreads();
+        if (wid == 0) {
+            const unsigned v = ws[lane];
+            unsigned winc = v;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned up = __shfl_up_sync(0xffffffffu, winc, o);
+                if (lane >= (unsigned)o) winc += up;
+            }
+            ws[lane] = winc - v;
+        }
+        __syncthreads();
+        const unsigned excl = carry + ws[wid] + inc - f;
+        if (f) { pairs_out[2 * excl] = pairs[(size_t)stride * i]; pairs_out[2 * excl + 1] = pairs[(size_t)stride * i + 1]; }
+        __syncthreads();
+        if (tid == 1023) carry = excl + f;
+        __syncthreads();
+    }
+    if (tid < 16) T_out[tid] = keep_all ? ((tid % 5 == 0) ? 1.0f : 0.0f) : models[16 * (size_t)best + tid];
+    if (tid == 0) { *n_out = (int)carry; *iterations_out = keep_all ? 0 : st->iterations; }
+}
+
+int ransac_run_dev(Ctx* c, const float4* d_src, const float4* d_tgt, const int* d_pairs, int pair_stride, const int* d_n_pairs, size_t n_cap,
+                   int max_iterations, double threshold, int* d_pairs_out, int* d_n_out, float* d_T_out, int* d_iterations_out, const int* d_skip) {
+    if (n_cap > c->max_kp) { set_error("bshot_ransac_dev: %zu correspondences > max_keypoints %zu", n_cap, c->max_kp); return BSHOT_E_CAPACITY; }
+    if (max_iterations < 1 || max_iterations > 100000) { set_error("bshot_ransac_dev: bad max_iterations"); return BSHOT_E_INVALID; }
+    const size_t n_hyp = (size_t)max_iterations + 1, cap = std::max<size_t>(n_cap, 1);
+    // scratch: correspondence sources | targets in d_gather; state, samples, models, counts, inlier flags (+ the shuffled
+    // list when it does not fit in shared memory) in d_partial
+    float4* s4 = reinterpret_cast<float4*>(c->d_gather);
+    float4* t4 = s4 + cap;
+    char* base = reinterpret_cast<char*>(c->d_partial);
+    RansacDevState* st = reinterpret_cast<RansacDevState*>(base);
+    int* samples = reinterpret_cast<int*>(base + 64);
+    float* models = reinterpret_cast<float*>(samples + 3 * n_hyp);
+    int* counts = reinterpret_cast<int*>(models + 16 * n_hyp);
+    unsigned char* inlier = reinterpret_cast<unsigned char*>(counts + n_hyp);
+    int* g_shuffled = reinterpret_cast<int*>(base + ((64 + (3 + 16 + 1) * n_hyp * 4 + cap + 15) & ~(size_t)15));
+    const size_t smem = 4 * cap;
+    const bool in_smem = smem <= 160 * 1024;
+    const size_t need = (size_t)(reinterpret_cast<char*>(g_shuffled) - base) + (in_smem ? 0 : 4 * cap);
+    if (need > c->partial_cap * 8) { set_error("bshot_ransac_dev: scratch too small for %d iterations", max_iterations); return BSHOT_E_CAPACITY; }
+    const double thresh2 = threshold * threshold;
+    ransac_gather_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, c->stream>>>(d_src, d_tgt, d_pairs, pair_stride, d_n_pairs, (unsigned)n_cap, d_skip, s4, t4, st);
+    if (in_smem && smem > 48 * 1024) BSHOT_CUDA_TRY(cudaFuncSetAttribute(ransac_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    ransac_sample_kernel<<<1, RS_THREADS, in_smem ? smem : 0, c->stream>>>(s4, st, (unsigned)n_hyp, samples, in_smem ? nullptr : g_shuffled);
+    ransac_score_dev_kernel<<<(unsigned)((n_hyp * 32 + 127) / 128), 128, 0, c->stream>>>(s4, t4, st, samples, thresh2, models, counts);
+    ransac_replay_kernel<<<1, 32, 0, c->stream>>>(st, counts, max_iterations);
+    ransac_select_dev_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, c->stream>>>(s4, t4, st, models, thresh2, inlier);
+    ransac_finish_kernel<<<1, 1024, 0, c->stream>>>(st, d_pairs, pair_stride, inlier, models, d_pairs_out, d_n_out, d_T_out, d_iterations_out);
+    count_launch(c, 6);
+    return check_launch("device RANSAC kernels");
 }
 
 }  // namespace bshot

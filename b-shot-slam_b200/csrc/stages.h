@@ -62,17 +62,32 @@ int hamming_tc2_partials(Ctx* c, const void* d_q, size_t nq, const void* d_t, si
 int gmap_create(Ctx* c, size_t max_entries, size_t max_blocks);
 void gmap_free(Ctx* c);
 int gmap_reset(Ctx* c);
-int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t* d_bits, const int* d_count, size_t n_cap, const float* pose12);
+// pose_on_device: pose12 / ref_pose12 are device pointers (the odometry step); gmap_gather then takes the position from the
+// translation of ref_pose12 on the device (pos unused)
+int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t* d_bits, const int* d_count, size_t n_cap, const float* pose12,
+                bool pose_on_device = false);
 int gmap_gather(Ctx* c, const float pos[3], float range, const float4* d_ref_kp, const uint64_t* d_ref_bits, const int* d_ref_count,
-                size_t ref_cap, const float* ref_pose12, uint64_t* d_t_out, size_t out_cap, unsigned* d_total);
+                size_t ref_cap, const float* ref_pose12, uint64_t* d_t_out, size_t out_cap, unsigned* d_total, bool pose_on_device = false);
 
 // RANSAC correspondence rejection (ransac.cu)
 int ransac_run(Ctx* c, const float* src_xyz, const float* tgt_xyz, const int* pairs, size_t n_pairs, int max_iterations, double threshold,
                int* inlier_pairs_out, int* n_inliers_out, float* transform_out, int* iterations_out);
+// the same on device inputs: d_pairs = n_cap records of pair_stride ints (query, match, ...), *d_n_pairs of them valid;
+// outputs in device memory.  A set *d_skip (may be null) treats the input as empty.  Asynchronous
+int ransac_run_dev(Ctx* c, const float4* d_src, const float4* d_tgt, const int* d_pairs, int pair_stride, const int* d_n_pairs, size_t n_cap,
+                   int max_iterations, double threshold, int* d_pairs_out, int* d_n_out, float* d_T_out, int* d_iterations_out, const int* d_skip);
 
 // ICP refinement (icp.cu)
+struct IcpState {
+    float final_T[16];
+    double prev_mse, mse;
+    int iterations, state, done, pad;
+};
 int icp_run(Ctx* c, const float* src_xyz, size_t n_src, const float* tgt_xyz, size_t n_tgt, const float* pre4x4, int max_iterations,
             float* final4x4_out, int* iterations_out, int* state_out, double* mse_out);
+// the same on device inputs with device-side counts (see icp.cu); the result stays in *d_st
+int icp_run_dev(Ctx* c, const float4* d_src, const int* d_ns, size_t ns_cap, const float4* d_tgt, const unsigned* d_nt, size_t nt_cap, const float* d_pre,
+                int max_iterations, const int* d_skip, float4* d_cur, float4* d_tgt_buf, unsigned long long* d_keys, IcpState* d_st);
 
 // scan preprocessor (preprocess.cu); scratch_reserve grows one of the context's on-demand scratch buffers
 int scratch_reserve(Ctx* c, int which, size_t bytes);
@@ -91,6 +106,13 @@ int kp_repeatability(Ctx* c, const float* a_xyz, size_t na, const float* a_pose,
 // min(cap, n) records {x, y, z} in c->vg.h_out[4..] (synchronous)
 int voxel_grid(Ctx* c, const float* xyz, size_t n, int stride_floats, const float inv[3], size_t cap, size_t* count_out);
 void vg_free(Ctx* c);
+
+// per-scan odometry step (odometry.cu): odometry_run takes the cloud already on the device and ends with one
+// synchronisation (the report); odometry_reset is synchronous
+int odom_ensure(Ctx* c);
+void odom_free(Ctx* c);
+int odometry_reset(Ctx* c);
+int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_t n, int stride_floats, bshot_odom_report* out);
 
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);

@@ -1,0 +1,72 @@
+// device_odometry.h -- the body of odometry_test.cpp's per-scan loop (test/odometry_test.cpp:143-184) as one call: the
+// rotation's velodyne::Laser records go to bshot_odometry_step, which runs the preprocessor, extraction, matching against
+// the map, RANSAC, the gate + ICP, the map update and the reference-frame hand-over on the device and returns the pose.
+// LidarOdometry and its reference-named stage methods stay available for callers that want the stages one by one.
+#ifndef BSHOT_B200_HOST_DEVICE_ODOMETRY_H
+#define BSHOT_B200_HOST_DEVICE_ODOMETRY_H
+
+#include <vector>
+
+#include "../../include/bshot_b200.h"
+#include "bshot_headers_bits.h"
+#include "preprocess.h"
+
+namespace myslam {
+
+class DeviceOdometry {
+public:
+    // a context sized for one rotation (max_points returns kept), the map of the reference driver (max_map entries)
+    explicit DeviceOdometry(int device = 0, size_t max_points = 131072, size_t max_keypoints = 1024, size_t max_targets = 1u << 16,
+                            size_t max_map = 1u << 16, size_t max_blocks = 4096) {
+        bshot_odom_params_default(&params_);
+        status_ = bshot_ctx_create(&ctx_, device, max_points, max_keypoints, max_targets);
+        if (status_ == BSHOT_OK) status_ = bshot_gmap_create(ctx_, max_map, max_blocks);
+    }
+    ~DeviceOdometry() { if (ctx_) bshot_ctx_destroy(ctx_); }
+    DeviceOdometry(const DeviceOdometry&) = delete;
+    DeviceOdometry& operator=(const DeviceOdometry&) = delete;
+
+    bshot_odom_params& params() { return params_; }
+
+    // one rotation -> T_best (the pose poseEstimation sets); on an error the pose of the last good step is returned and
+    // last_status() / bshot_last_error() say why
+    Matrix4f step(const std::vector<velodyne::Laser>& lasers, const std::vector<double>& ring_deg) {
+        const size_t n = lasers.size();
+        az_.resize(n); vert_.resize(n); dist_.resize(n);
+        for (size_t i = 0; i < n; ++i) { az_[i] = lasers[i].azimuth; vert_[i] = lasers[i].vertical; dist_[i] = lasers[i].distance; }
+        if (ctx_) {
+            bshot_odom_report r;
+            status_ = bshot_odometry_step(ctx_, &params_, az_.data(), vert_.data(), dist_.data(), n, ring_deg.data(), ring_deg.size(), &r);
+            if (status_ == BSHOT_OK) {
+                report_ = r;
+                for (int row = 0; row < 4; ++row) for (int col = 0; col < 4; ++col) pose_(row, col) = r.pose[4 * row + col];
+            }
+        }
+        return pose_;
+    }
+
+    const bshot_odom_report& report() const { return report_; }
+
+    // INITIAL status, identity pose, empty map, no reference frame
+    int reset() {
+        if (ctx_) status_ = bshot_odometry_reset(ctx_);
+        pose_ = Matrix4f::Identity();
+        report_ = bshot_odom_report();
+        return status_;
+    }
+
+    int last_status() const { return status_; }
+    bshot_ctx* context() { return ctx_; }
+
+private:
+    bshot_ctx* ctx_ = nullptr;
+    bshot_odom_params params_;
+    bshot_odom_report report_ = bshot_odom_report();
+    Matrix4f pose_ = Matrix4f::Identity();
+    int status_ = BSHOT_OK;
+    std::vector<double> az_, vert_;
+    std::vector<unsigned short> dist_;
+};
+
+}  // namespace myslam
+#endif

@@ -255,6 +255,54 @@ int bshot_extract_scan(bshot_ctx* ctx, const bshot_params* p, const double* azim
                        double lowpt_th, float* cloud_xyz_out, size_t cloud_cap, size_t* n_points_out, int* kp_idx_out,
                        float* kp_xyz_out, float* seg_ratio_out, uint64_t* bits_out, int* n_kp_out);
 
+/* ---- the per-scan odometry step on the device (test/odometry_test.cpp:143-184 in one call) ----------------------------
+ * One rotation in, one pose out: Preprocessor::run -> extractKeypoints -> computeDescriptors -> featureMatching (first
+ * scan: the frame against itself; later scans: map keypoints within map_range of the last pose ++ the reference frame
+ * moved by that pose, mutual nearest neighbours) -> RANSAC -> evaluateEstimation (gate + ICP) -> poseEstimation ->
+ * updateMap (whatever the gate says: the reference's check is commented out) -> the frame becomes the reference frame.
+ * The result is bit for bit that of bshot_extract_scan, bshot_match_mutual / bshot_match_frame_to_map, bshot_ransac,
+ * bshot_evaluate_estimation, bshot_gmap_update_from_frame and bshot_frame_commit called in that order, except h_diff_rad
+ * (device acosf).  The context keeps the pose of the last step on the device and the INITIAL / RUN status.
+ * After the preprocessor's two count read-backs nothing goes back to the host until one copy of the report at the end.
+ * Needs bshot_gmap_create first (BSHOT_E_STATE).  A target set larger than max_targets returns BSHOT_E_CAPACITY; any
+ * error leaves pose, status, map and reference frame as they were before the step. */
+typedef struct bshot_odom_params {
+    bshot_params front;          /* bshot_params_default(): the reference's extraction literals */
+    double vert_init_rad;        /* -0.6    test/odometry_test.cpp:32 */
+    double lowpt_th;             /* -1950   test/odometry_test.cpp:33 */
+    float map_range;             /* 100000  src/lidar_odometry.cpp:198 */
+    int ransac_iterations;       /* 2000    src/lidar_odometry.cpp:255 */
+    float inlier_threshold;      /* 1500    src/lidar_odometry.cpp:258 */
+    int run_icp;                 /* 1       src/lidar_odometry.cpp:6 */
+} bshot_odom_params;
+void bshot_odom_params_default(bshot_odom_params* p);
+
+typedef struct bshot_odom_report {
+    float pose[16];              /* T_best, row-major: what poseEstimation sets */
+    float T_ransac[16];          /* RANSAC's transformation (identity when it kept everything) */
+    size_t n_points, n_targets;  /* preprocessed points; size of the target set */
+    int n_keypoints, n_pairs, n_inliers, ransac_iterations, icp_iterations, should_update_map, was_initial;
+    float h_diff_rad, t_diff_mm; /* the gate's heading and translation change */
+} bshot_odom_report;
+
+/* raw returns (as bshot_extract_scan) -> pose; out may be NULL */
+int bshot_odometry_step(bshot_ctx* ctx, const bshot_odom_params* p, const double* azimuth_deg, const double* vertical_deg,
+                        const unsigned short* distance, size_t n, const double* ring_deg, size_t nv, bshot_odom_report* out);
+/* an already-preprocessed host cloud (stride 12 or 16 bytes, as bshot_extract_frame): skips the preprocessor */
+int bshot_odometry_step_cloud(bshot_ctx* ctx, const bshot_odom_params* p, const float* xyz, size_t n, size_t stride_bytes,
+                              bshot_odom_report* out);
+/* INITIAL status, identity pose, empty map, no reference frame, fresh persistent normals: the next step replays the
+ * sequence as a new context would */
+int bshot_odometry_reset(bshot_ctx* ctx);
+/* bshot_ransac on device buffers, asynchronous on the context stream: d_src4 / d_tgt4 float4 points (x, y, z, any),
+ * d_pairs n_pairs_cap x 2 ints (index into src, index into tgt; every valid one must be in range), *d_n_pairs (int) of
+ * them valid.  Outputs (device): d_inlier_pairs_out (n_pairs_cap x 2 ints), *d_n_inliers_out (int), d_transform_out
+ * (16 floats, row-major), *d_iterations_out (int).  Bit for bit bshot_ransac's results, adaptive stop included
+ * (device log / pow may move its count when k lies within a few ulps of an integer). */
+int bshot_ransac_dev(bshot_ctx* ctx, const void* d_src4, const void* d_tgt4, const void* d_pairs, const void* d_n_pairs, size_t n_pairs_cap,
+                     int max_iterations, float inlier_threshold, void* d_inlier_pairs_out, void* d_n_inliers_out, void* d_transform_out,
+                     void* d_iterations_out);
+
 /* ---- ISS keypoints and keypoint repeatability (the reference's kp_test evaluation) ------------ */
 /* issKpDetection (src/lidar_odometry.cpp:447-461): pcl::ISSKeypoint3D (PCL 1.8, border radius 0) on the cloud the context
  * holds (after bshot_set_cloud / bshot_extract_frame / bshot_process_frame[_dev] / bshot_extract_scan), on its voxel table.
