@@ -845,20 +845,16 @@ int bshot_match_frame_to_map(bshot_ctx* ctx, const float ref_pos[3], float range
     if (!ref_pos) { set_error("bshot_match_frame_to_map: null position"); return BSHOT_E_INVALID; }
     if (!ctx->gmap.d_tab || ctx->last_top_k == 0) { set_error("bshot_match_frame_to_map: needs a map and an extracted frame"); return BSHOT_E_STATE; }
     const size_t k = ctx->last_top_k;
-    unsigned* d_total = ctx->gmap.d_ctl + 6;
-    // target set = map keypoints in range ++ reference (previous) frame, assembled on the device (src/lidar_odometry.cpp:197-206)
-    BSHOT_TRY(gmap_gather(ctx, ref_pos, range, ctx->d_prev_kp, ctx->d_prev_bits, ctx->d_prev_count, ctx->n_prev, ref_pose3x4, ctx->d_t, ctx->max_targets, d_total));
-    const size_t nt_cap = std::min(ctx->max_targets, ctx->gmap.entries_upper + ctx->n_prev);
+    size_t nt_cap;
+    BSHOT_TRY(frame_match_map(ctx, k, ref_pos, range, ref_pose3x4, /*pose_on_device=*/false, &nt_cap));
     if (nt_cap == 0) { if (n_pairs_out) *n_pairs_out = 0; if (n_targets_out) *n_targets_out = 0; return sync(ctx); }
-    const unsigned* d_nq = reinterpret_cast<const unsigned*>(ctx->d_kp_count);
-    BSHOT_TRY(hamming_match_rq(ctx, ctx->d_bits, k, ctx->d_t, nt_cap, 0, ctx->d_cand, d_nq, d_total));
-    BSHOT_TRY(hamming_mutual_pairs(ctx, ctx->d_cand, k, ctx->d_pairs, ctx->d_pair_count, d_nq));
     BSHOT_TRY(d2h(ctx, &ctx->h_scratch[1], ctx->d_pair_count, sizeof(int)));
     BSHOT_TRY(d2h(ctx, &ctx->h_scratch[40], ctx->gmap.d_ctl, 8 * sizeof(unsigned)));
     if (pairs_out) BSHOT_CUDA_TRY(cudaMemcpyAsync(ctx->h_pairs, ctx->d_pairs, sizeof(int) * 3 * k, cudaMemcpyDeviceToHost, ctx->stream));
     BSHOT_TRY(sync(ctx));
-    const size_t gathered = (size_t)(unsigned)ctx->h_scratch[44] + 0, total = (size_t)(unsigned)ctx->h_scratch[46];
-    if (gathered + ctx->n_prev > ctx->max_targets && total == ctx->max_targets) { set_error("bshot_match_frame_to_map: target set exceeds max_targets %zu", ctx->max_targets); return BSHOT_E_CAPACITY; }
+    const unsigned* ctl = reinterpret_cast<const unsigned*>(&ctx->h_scratch[40]);
+    const size_t total = ctl[6];
+    if (target_set_overflow(ctl, ctx->n_prev, ctx->max_targets)) { set_error("bshot_match_frame_to_map: target set exceeds max_targets %zu", ctx->max_targets); return BSHOT_E_CAPACITY; }
     const int np = std::min(ctx->h_scratch[1], (int)k);
     if (n_pairs_out) *n_pairs_out = np;
     if (n_targets_out) *n_targets_out = total;

@@ -1,12 +1,15 @@
 // frame.cu -- the reference's per-frame call order on the resident cloud, fully asynchronous:
 // extractKeypoints -> computeDescriptors -> featureMatching (test/odometry_test.cpp:174-194,
 // src/lidar_odometry.cpp:51-265 up to the RANSAC call).
+#include <algorithm>
+
 #include "stages.h"
 
 namespace bshot {
 
 __global__ void copy_prev_kernel(const uint64_t* __restrict__ bits, const float4* __restrict__ kp, const int* __restrict__ count, unsigned cap,
-                                 uint64_t* __restrict__ prev, float4* __restrict__ prev_kp, int* __restrict__ prev_count) {
+                                 const int* __restrict__ skip, uint64_t* __restrict__ prev, float4* __restrict__ prev_kp, int* __restrict__ prev_count) {
+    if (skip && *skip) return;
     const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
     const int k = *count;
     if (i < cap * 6 && (int)(i / 6) < k) prev[i] = bits[i];
@@ -14,13 +17,27 @@ __global__ void copy_prev_kernel(const uint64_t* __restrict__ bits, const float4
     if (i == 0) *prev_count = k;
 }
 
-// the current frame becomes the reference frame (descriptors + keypoint positions + count stay on the device)
-int frame_commit(Ctx* c, size_t k) {
-    copy_prev_kernel<<<(unsigned)((k * 6 + 255) / 256), 256, 0, c->stream>>>(c->d_bits, c->d_kp, c->d_kp_count, (unsigned)k, c->d_prev_bits, c->d_prev_kp,
-                                                                            c->d_prev_count);
+int frame_commit(Ctx* c, size_t k, const int* d_skip) {
+    copy_prev_kernel<<<(unsigned)((k * 6 + 255) / 256), 256, 0, c->stream>>>(c->d_bits, c->d_kp, c->d_kp_count, (unsigned)k, d_skip, c->d_prev_bits,
+                                                                            c->d_prev_kp, c->d_prev_count);
     count_launch(c);
-    c->n_prev = k;
+    if (!d_skip) c->n_prev = k;
     return check_launch("copy_prev_kernel");
+}
+
+int frame_match_map(Ctx* c, size_t k, const float pos[3], float range, const float* ref_pose12, bool pose_on_device, size_t* nt_cap_out) {
+    unsigned* d_total = c->gmap.d_ctl + 6;
+    BSHOT_TRY(gmap_gather(c, pos, range, c->d_prev_kp, c->d_prev_bits, c->d_prev_count, c->n_prev, ref_pose12, c->d_t, c->max_targets, d_total,
+                          pose_on_device));
+    const size_t nt_cap = std::min(c->max_targets, c->gmap.entries_upper + c->n_prev);
+    *nt_cap_out = nt_cap;
+    if (nt_cap == 0) {
+        BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_pair_count, 0, sizeof(int), c->stream));
+        return BSHOT_OK;
+    }
+    const unsigned* d_nq = reinterpret_cast<const unsigned*>(c->d_kp_count);
+    BSHOT_TRY(hamming_match_rq(c, c->d_bits, k, c->d_t, nt_cap, 0, c->d_cand, d_nq, d_total));
+    return hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq);
 }
 
 // extractKeypoints + computeDescriptors (src/lidar_odometry.cpp:51-184) on a cloud in device memory, asynchronous

@@ -173,35 +173,14 @@ icp_fit_kernel(float4* __restrict__ cur, unsigned ns, const float4* __restrict__
     if (t == 0 && s_stop) st->done = 1;
 }
 
-// pcl::transformPointCloud(cb.cloud1_keypoints, icp_cloud, T_est) (src/lidar_odometry.cpp:284) + key reset
-__global__ void icp_init_kernel(const float* __restrict__ src, unsigned ns, const float* __restrict__ pre, float4* __restrict__ cur, unsigned long long* __restrict__ keys) {
-    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= ns) return;
-    const float x = src[3 * i], y = src[3 * i + 1], z = src[3 * i + 2];
-    float4 o;
-    o.x = ((pre[0] * x + pre[1] * y) + pre[2] * z) + pre[3];
-    o.y = ((pre[4] * x + pre[5] * y) + pre[6] * z) + pre[7];
-    o.z = ((pre[8] * x + pre[9] * y) + pre[10] * z) + pre[11];
-    o.w = 0.f;
-    cur[i] = o;
-    keys[i] = ~0ull;
-}
-
-__global__ void icp_pad_kernel(const float* __restrict__ xyz, unsigned n, float4* __restrict__ out) {
-    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = make_float4(xyz[3 * i], xyz[3 * i + 1], xyz[3 * i + 2], 0.f);
-}
-
-// host points in, host results out; one synchronisation at the end
+// host points in, host results out: the points, the pre-transform and both counts are uploaded and icp_run_dev runs on the
+// true counts (no padding); one synchronisation at the end
 int icp_run(Ctx* c, const float* src_xyz, size_t n_src, const float* tgt_xyz, size_t n_tgt, const float* pre4x4, int max_iterations,
             float* final4x4_out, int* iterations_out, int* state_out, double* mse_out) {
     const float ident[16] = {1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1, 0, 0, 0, 0, 1};
-    IcpState h;
-    for (int e = 0; e < 16; ++e) h.final_T[e] = ident[e];
-    h.prev_mse = 1.7976931348623157e308;   // correspondences_prev_mse_ starts at numeric_limits<double>::max()
-    h.mse = 0.0; h.iterations = 0; h.state = ICP_NOT_CONVERGED; h.done = 0; h.pad = 0;
+    IcpState h = {};
     if (n_src && n_tgt && max_iterations > 0) {
-        const size_t bytes = 12 * (n_src + n_tgt) + 16 * (n_src + n_tgt) + 8 * n_src + sizeof(IcpState) + 64 + 256 * 8;
+        const size_t bytes = 12 * (n_src + n_tgt) + 16 * (n_src + n_tgt) + 8 * n_src + sizeof(IcpState) + 64 + 8 + 256 * 8;
         BSHOT_TRY(scratch_reserve(c, 2, bytes));
         char* base = (char*)c->d_pre[2];
         size_t off = 0;
@@ -210,23 +189,18 @@ int icp_run(Ctx* c, const float* src_xyz, size_t n_src, const float* tgt_xyz, si
         float4* d_cur = (float4*)take(16 * n_src); float4* d_tgt = (float4*)take(16 * n_tgt);
         unsigned long long* d_keys = (unsigned long long*)take(8 * n_src);
         IcpState* d_st = (IcpState*)take(sizeof(IcpState)); float* d_pre = (float*)take(64);
+        unsigned* d_counts = (unsigned*)take(8);
+        const unsigned counts[2] = {(unsigned)n_src, (unsigned)n_tgt};
         BSHOT_CUDA_TRY(cudaMemcpyAsync(d_src, src_xyz, 12 * n_src, cudaMemcpyHostToDevice, c->stream));
         BSHOT_CUDA_TRY(cudaMemcpyAsync(d_tgt3, tgt_xyz, 12 * n_tgt, cudaMemcpyHostToDevice, c->stream));
         BSHOT_CUDA_TRY(cudaMemcpyAsync(d_pre, pre4x4 ? pre4x4 : ident, 64, cudaMemcpyHostToDevice, c->stream));
-        BSHOT_CUDA_TRY(cudaMemcpyAsync(d_st, &h, sizeof(IcpState), cudaMemcpyHostToDevice, c->stream));
-        const unsigned ns = (unsigned)n_src, nt = (unsigned)n_tgt;
-        icp_init_kernel<<<(ns + 255) / 256, 256, 0, c->stream>>>(d_src, ns, d_pre, d_cur, d_keys);
-        icp_pad_kernel<<<(nt + 255) / 256, 256, 0, c->stream>>>(d_tgt3, nt, d_tgt);
-        const dim3 grid((ns + ICP_SRC - 1) / ICP_SRC, (nt + ICP_TGT - 1) / ICP_TGT);
-        for (int it = 0; it < max_iterations; ++it) {
-            icp_nn_kernel<<<grid, ICP_SRC, 0, c->stream>>>(d_cur, ns, d_tgt, nt, d_keys, d_st);
-            icp_fit_kernel<<<1, ICP_T, 0, c->stream>>>(d_cur, ns, d_tgt, d_keys, d_st, max_iterations);
-        }
-        count_launch(c, 2 + 2 * max_iterations);
-        BSHOT_TRY(check_launch("icp kernels"));
+        BSHOT_CUDA_TRY(cudaMemcpyAsync(d_counts, counts, sizeof(counts), cudaMemcpyHostToDevice, c->stream));
+        BSHOT_TRY(icp_run_dev(c, d_src, 3, reinterpret_cast<const int*>(d_counts), n_src, d_tgt3, 3, d_counts + 1, n_tgt, d_pre, max_iterations, nullptr, d_cur,
+                              d_tgt, d_keys, d_st));
         BSHOT_CUDA_TRY(cudaMemcpyAsync(&h, d_st, sizeof(IcpState), cudaMemcpyDeviceToHost, c->stream));
         BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
     } else {
+        for (int e = 0; e < 16; ++e) h.final_T[e] = ident[e];
         h.state = ICP_NO_CORRESPONDENCES;
     }
     if (final4x4_out) for (int e = 0; e < 16; ++e) final4x4_out[e] = h.final_T[e];
@@ -236,13 +210,14 @@ int icp_run(Ctx* c, const float* src_xyz, size_t n_src, const float* tgt_xyz, si
     return BSHOT_OK;
 }
 
-// ---- device inputs (the odometry step) -----------------------------------------------------------------------------------
-// Sources: the frame's keypoints (float4) moved by the device-side pre-transform; targets: any float4 array.  Both counts
-// stay on the device: the kernels above run on the host-known capacities, and the slots past the true counts hold NaN,
-// which never becomes a correspondence (icp_nn_kernel tests d == d), so icp_fit_kernel's 256 strided partial sums -- and
-// hence every bit of the result -- depend only on the true points.  A set *d_skip makes every launch a no-op.
-__global__ void icp_init_dev_kernel(const float4* __restrict__ src, const int* __restrict__ d_ns, unsigned ns_cap, const float4* __restrict__ tgt,
-                                    const unsigned* __restrict__ d_nt, unsigned nt_cap, const float* __restrict__ pre, const int* __restrict__ skip,
+// ---- device inputs (the odometry step; icp_run on its uploads) -----------------------------------------------------------------
+// Sources moved by the device-side pre-transform (pcl::transformPointCloud(cb.cloud1_keypoints, icp_cloud, T_est),
+// src/lidar_odometry.cpp:284) and targets are point arrays of src_stride / tgt_stride floats (3: packed xyz, 4: float4).
+// Both counts stay on the device: the kernels above run on the host-known capacities, and the slots past the true counts
+// hold NaN, which never becomes a correspondence (icp_nn_kernel tests d == d), so icp_fit_kernel's 256 strided partial sums
+// -- and hence every bit of the result -- depend only on the true points.  A set *d_skip makes every launch a no-op.
+__global__ void icp_init_dev_kernel(const float* __restrict__ src, int src_stride, const int* __restrict__ d_ns, unsigned ns_cap, const float* __restrict__ tgt,
+                                    int tgt_stride, const unsigned* __restrict__ d_nt, unsigned nt_cap, const float* __restrict__ pre, const int* __restrict__ skip,
                                     float4* __restrict__ cur, float4* __restrict__ tgt_out, unsigned long long* __restrict__ keys, IcpState* __restrict__ st) {
     const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
     const unsigned ns = min((unsigned)max(*d_ns, 0), ns_cap), nt = min(*d_nt, nt_cap);
@@ -250,8 +225,8 @@ __global__ void icp_init_dev_kernel(const float4* __restrict__ src, const int* _
     if (i < ns_cap) {
         float4 o = make_float4(nan, nan, nan, 0.f);
         if (i < ns) {
-            const float4 p = src[i];
-            const float x = p.x, y = p.y, z = p.z;
+            const float* p = src + (size_t)src_stride * i;
+            const float x = p[0], y = p[1], z = p[2];
             o.x = ((pre[0] * x + pre[1] * y) + pre[2] * z) + pre[3];
             o.y = ((pre[4] * x + pre[5] * y) + pre[6] * z) + pre[7];
             o.z = ((pre[8] * x + pre[9] * y) + pre[10] * z) + pre[11];
@@ -260,8 +235,8 @@ __global__ void icp_init_dev_kernel(const float4* __restrict__ src, const int* _
         keys[i] = ~0ull;
     }
     if (i < nt_cap) {
-        const float4 q = (i < nt) ? tgt[i] : make_float4(nan, nan, nan, 0.f);
-        tgt_out[i] = make_float4(q.x, q.y, q.z, 0.f);
+        const float* q = tgt + (size_t)tgt_stride * i;
+        tgt_out[i] = (i < nt) ? make_float4(q[0], q[1], q[2], 0.f) : make_float4(nan, nan, nan, 0.f);
     }
     if (i == 0) {
         for (int e = 0; e < 16; ++e) st->final_T[e] = (e % 5 == 0) ? 1.0f : 0.0f;
@@ -272,10 +247,12 @@ __global__ void icp_init_dev_kernel(const float4* __restrict__ src, const int* _
     }
 }
 
-int icp_run_dev(Ctx* c, const float4* d_src, const int* d_ns, size_t ns_cap, const float4* d_tgt, const unsigned* d_nt, size_t nt_cap, const float* d_pre,
-                int max_iterations, const int* d_skip, float4* d_cur, float4* d_tgt_buf, unsigned long long* d_keys, IcpState* d_st) {
+int icp_run_dev(Ctx* c, const float* d_src, int src_stride, const int* d_ns, size_t ns_cap, const float* d_tgt, int tgt_stride, const unsigned* d_nt,
+                size_t nt_cap, const float* d_pre, int max_iterations, const int* d_skip, float4* d_cur, float4* d_tgt_buf, unsigned long long* d_keys,
+                IcpState* d_st) {
     const unsigned ns = (unsigned)ns_cap, nt = (unsigned)nt_cap, nmax = std::max(std::max(ns, nt), 1u);
-    icp_init_dev_kernel<<<(nmax + 255) / 256, 256, 0, c->stream>>>(d_src, d_ns, ns, d_tgt, d_nt, nt, d_pre, d_skip, d_cur, d_tgt_buf, d_keys, d_st);
+    icp_init_dev_kernel<<<(nmax + 255) / 256, 256, 0, c->stream>>>(d_src, src_stride, d_ns, ns, d_tgt, tgt_stride, d_nt, nt, d_pre, d_skip, d_cur, d_tgt_buf,
+                                                                   d_keys, d_st);
     count_launch(c);
     if (ns && nt) {
         const dim3 grid((ns + ICP_SRC - 1) / ICP_SRC, (nt + ICP_TGT - 1) / ICP_TGT);

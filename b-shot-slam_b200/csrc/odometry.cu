@@ -33,9 +33,9 @@ __global__ void odom_reset_kernel(OdomDev* d) {
     if (threadIdx.x == 0) d->err = 0;
 }
 
-// bshot_match_frame_to_map's capacity test on device counts: ctl[4] map entries in range, ctl[6] targets assembled
-__global__ void odom_check_kernel(const unsigned* __restrict__ ctl, unsigned long long n_prev, unsigned long long max_targets, OdomDev* d) {
-    if ((unsigned long long)ctl[4] + n_prev > max_targets && (unsigned long long)ctl[6] == max_targets) d->err = BSHOT_E_CAPACITY;
+// bshot_match_frame_to_map's capacity test on the device counts
+__global__ void odom_check_kernel(const unsigned* __restrict__ ctl, size_t n_prev, size_t max_targets, OdomDev* d) {
+    if (target_set_overflow(ctl, n_prev, max_targets)) d->err = BSHOT_E_CAPACITY;
 }
 
 // evaluateEstimation's gate (src/lidar_odometry.cpp:267-281): T_est = T_ref when rejected, else T_ransac
@@ -72,17 +72,6 @@ __global__ void odom_final_kernel(OdomDev* d, const IcpState* __restrict__ icp, 
     } else {
         d->eff_count = 0;
     }
-}
-
-// frame_commit's copy, skipped after an error (the reference frame stays)
-__global__ void odom_commit_kernel(const uint64_t* __restrict__ bits, const float4* __restrict__ kp, const int* __restrict__ count, unsigned cap,
-                                   const OdomDev* __restrict__ d, uint64_t* __restrict__ prev, float4* __restrict__ prev_kp, int* __restrict__ prev_count) {
-    if (d->err) return;
-    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
-    const int k = *count;
-    if (i < cap * 6 && (int)(i / 6) < k) prev[i] = bits[i];
-    if (i < cap && (int)i < k) prev_kp[i] = kp[i];
-    if (i == 0) *prev_count = k;
 }
 
 int odom_ensure(Ctx* c) {
@@ -150,20 +139,11 @@ int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_
         d_nt = d_nq;
         nt_cap = k;
     } else {         // :197-206: map keypoints in range of the last pose ++ the reference frame moved by that pose
-        unsigned* d_total = g.d_ctl + 6;
-        BSHOT_TRY(gmap_gather(c, nullptr, p->map_range, c->d_prev_kp, c->d_prev_bits, c->d_prev_count, c->n_prev, d->pose, c->d_t, c->max_targets, d_total,
-                              /*pose_on_device=*/true));
-        odom_check_kernel<<<1, 1, 0, c->stream>>>(g.d_ctl, (unsigned long long)c->n_prev, (unsigned long long)c->max_targets, d);
+        BSHOT_TRY(frame_match_map(c, k, nullptr, p->map_range, d->pose, /*pose_on_device=*/true, &nt_cap));
+        odom_check_kernel<<<1, 1, 0, c->stream>>>(g.d_ctl, c->n_prev, c->max_targets, d);
         count_launch(c);
-        nt_cap = std::min(c->max_targets, g.entries_upper + c->n_prev);
-        if (nt_cap == 0) {
-            BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_pair_count, 0, sizeof(int), c->stream));
-        } else {
-            BSHOT_TRY(hamming_match_rq(c, c->d_bits, k, c->d_t, nt_cap, 0, c->d_cand, d_nq, d_total));
-            BSHOT_TRY(hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq));
-        }
         tgt_pos = g.d_tpos;
-        d_nt = d_total;
+        d_nt = g.d_ctl + 6;
     }
     // featureMatching's RANSAC (:251-261) on the pairs (query, match, distance) the matcher left on the device
     BSHOT_TRY(ransac_run_dev(c, c->d_kp, tgt_pos, c->d_pairs, 3, c->d_pair_count, k, p->ransac_iterations, (double)p->inlier_threshold, o.d_inlier_pairs,
@@ -171,8 +151,8 @@ int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_
     odom_gate_kernel<<<1, 1, 0, c->stream>>>(d);
     count_launch(c);
     if (p->run_icp) {   // :283-293 on the frame's keypoints and the target set
-        BSHOT_TRY(icp_run_dev(c, c->d_kp, c->d_kp_count, k, tgt_pos, d_nt, nt_cap, d->T_est, 10, &d->err, o.d_icp_cur, o.d_icp_tgt, o.d_icp_keys,
-                              o.d_icp_state));
+        BSHOT_TRY(icp_run_dev(c, reinterpret_cast<const float*>(c->d_kp), 4, c->d_kp_count, k, reinterpret_cast<const float*>(tgt_pos), 4, d_nt, nt_cap,
+                              d->T_est, 10, &d->err, o.d_icp_cur, o.d_icp_tgt, o.d_icp_keys, o.d_icp_state));
     }
     odom_final_kernel<<<1, 1, 0, c->stream>>>(d, o.d_icp_state, p->run_icp ? 1 : 0, c->d_kp_count, c->d_pair_count, initial ? nullptr : g.d_ctl + 6, (int)k,
                                               (unsigned long long)n, initial ? 1 : 0);
@@ -180,10 +160,7 @@ int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_
     BSHOT_TRY(check_launch("odometry step kernels"));
     // updateMap (:343-358) with T_best, whatever the gate said; after an error the count is 0 and the map stays
     BSHOT_TRY(gmap_update(c, c->d_kp, c->d_kp_ratio, c->d_bits, &d->eff_count, c->last_top_k, d->pose, /*pose_on_device=*/true));
-    odom_commit_kernel<<<(unsigned)((k * 6 + 255) / 256), 256, 0, c->stream>>>(c->d_bits, c->d_kp, c->d_kp_count, (unsigned)k, d, c->d_prev_bits,
-                                                                                c->d_prev_kp, c->d_prev_count);
-    count_launch(c);
-    BSHOT_TRY(check_launch("odom_commit_kernel"));
+    BSHOT_TRY(frame_commit(c, k, &d->err));   // skipped after an error: the reference frame stays
     OdomDev* h = reinterpret_cast<OdomDev*>(o.h_out);
     BSHOT_CUDA_TRY(cudaMemcpyAsync(h, d, offsetof(OdomDev, err) + sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));

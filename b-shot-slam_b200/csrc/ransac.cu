@@ -11,9 +11,10 @@
 //   * score: number of correspondences with |T * src - tgt|^2 < threshold^2 (float transform, float norm);
 //   * adaptive stop: k = log(1 - 0.99) / log(1 - w^3) re-evaluated at every new best, first best wins ties;
 //   * result: the correspondences within the threshold of the best model, in their original order, and that model.
-// The sample sequence does not depend on the scores, so it is generated up front (host, a few microseconds), ALL
-// max_iterations + 1 hypotheses are scored in parallel (one warp each), and the adaptive loop is replayed over the
-// scores on the host exactly as PCL runs it.  This file is compiled with -fmad=false: the double-precision Jacobi SVD
+// The sample sequence does not depend on the scores, so it is generated up front (on the host for host inputs, a few
+// microseconds; on the device for device inputs), ALL hypotheses are scored in parallel (one warp each), and the adaptive
+// loop is replayed over the scores exactly as PCL runs it.  Both entry points then share one tail: scoring, the adaptive
+// stop (ransac_adaptive_stop, on the host for host inputs), the inlier flags and the in-order compaction.  This file is compiled with -fmad=false: the double-precision Jacobi SVD
 // then uses only IEEE +, -, *, /, sqrt and is bit-identical to the oracle's restatement (orc_ransac).
 #include <math.h>
 
@@ -63,9 +64,46 @@ __host__ __device__ inline float transfer_sqd(const float T[16], float sx, float
     return (dx * dx + dy * dy) + dz * dz;
 }
 
+// ---- the tail both entry points run after their sampler -----------------------------------------------------------------
+// score every hypothesis -> adaptive stop -> inlier flags of the best model -> in-order compaction.  The state lives on the
+// device: n correspondences, n_valid hypotheses drawn, and the adaptive stop's best hypothesis (-1: none) and iterations.
+struct RansacDevState {
+    double sdt;
+    int n, n_valid, best, iterations;
+};
+
+// RandomSampleConsensus::computeModel replayed over the scores: the host call runs it on the host after reading the counts
+// back, the device call on one device thread
+__host__ __device__ inline void ransac_adaptive_stop(RansacDevState* st, const int* counts, int max_iterations) {
+    int iterations = 0, best = -1, n_best = -2147483647;
+    double k = 1.0;
+    const double log_probability = log(1.0 - 0.99), one_over_indices = 1.0 / (double)st->n;
+    while ((double)iterations < k) {
+        if (iterations >= st->n_valid) break;  // no sample could be drawn: PCL breaks out
+        const int cnt = counts[iterations];
+        if (cnt > n_best) {
+            n_best = cnt;
+            best = iterations;
+            const double w = (double)n_best * one_over_indices;
+            double p_no_outliers = 1.0 - pow(w, 3.0);
+            p_no_outliers = fmax(2.220446049250313e-16, p_no_outliers);
+            p_no_outliers = fmin(1.0 - 2.220446049250313e-16, p_no_outliers);
+            k = log_probability / log(p_no_outliers);
+        }
+        ++iterations;
+        if (iterations > max_iterations) break;
+    }
+    st->best = best;
+    st->iterations = iterations;
+}
+
 // one warp per hypothesis: model from its three pairs, inlier count over all correspondences
-__device__ __forceinline__ void ransac_score_one(const float4* __restrict__ src, const float4* __restrict__ tgt, unsigned n, const int* __restrict__ samples,
-                                                 unsigned h, unsigned lane, double thresh2, float* __restrict__ models, int* __restrict__ counts) {
+__global__ void __launch_bounds__(128)
+ransac_score_dev_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const RansacDevState* __restrict__ st, const int* __restrict__ samples,
+                        double thresh2, float* __restrict__ models, int* __restrict__ counts) {
+    const unsigned lane = threadIdx.x & 31, h = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (st->n < 3 || h >= (unsigned)st->n_valid) return;
+    const unsigned n = (unsigned)st->n;
     float T[16];
     {
         double s[3][3], d[3][3];
@@ -87,26 +125,100 @@ __device__ __forceinline__ void ransac_score_one(const float4* __restrict__ src,
     if (lane < 16) models[16 * h + lane] = T[lane];
 }
 
-__global__ void __launch_bounds__(128)
-ransac_score_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, unsigned n, const int* __restrict__ samples, unsigned n_hyp,
-                    double thresh2, float* __restrict__ models, int* __restrict__ counts) {
-    const unsigned lane = threadIdx.x & 31, h = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (h >= n_hyp) return;
-    ransac_score_one(src, tgt, n, samples, h, lane, thresh2, models, counts);
-}
-
-__device__ __forceinline__ unsigned char ransac_is_inlier(const float* __restrict__ model, const float4 a, const float4 b, double thresh2) {
+__global__ void ransac_select_dev_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const RansacDevState* __restrict__ st,
+                                         const float* __restrict__ models, double thresh2, unsigned char* __restrict__ inlier) {
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (st->best < 0 || i >= (unsigned)st->n) return;
+    const float* model = models + 16 * (size_t)st->best;
     float T[16];
 #pragma unroll
     for (int k = 0; k < 16; ++k) T[k] = model[k];
-    return ((double)transfer_sqd(T, a.x, a.y, a.z, b.x, b.y, b.z) < thresh2) ? 1 : 0;
+    const float4 a = src[i], b = tgt[i];
+    inlier[i] = ((double)transfer_sqd(T, a.x, a.y, a.z, b.x, b.y, b.z) < thresh2) ? 1 : 0;
 }
 
-__global__ void ransac_select_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, unsigned n, const float* __restrict__ model,
-                                     double thresh2, unsigned char* __restrict__ inlier) {
-    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= n) return;
-    inlier[i] = ransac_is_inlier(model, src[i], tgt[i], thresh2);
+// one CTA: the inliers of the best model in their original order, or (fewer than 3 correspondences / no hypothesis / fewer
+// than 3 inliers) every correspondence with the identity -- PCL's behaviour
+__global__ void __launch_bounds__(1024)
+ransac_finish_kernel(const RansacDevState* __restrict__ st, const int* __restrict__ pairs, int stride, const unsigned char* __restrict__ inlier,
+                     const float* __restrict__ models, int* __restrict__ pairs_out, int* __restrict__ n_out, float* __restrict__ T_out,
+                     int* __restrict__ iterations_out) {
+    __shared__ unsigned ws[32];
+    __shared__ unsigned carry;
+    const unsigned tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const unsigned n = (unsigned)max(st->n, 0);
+    const int best = st->best;
+    bool keep_all = n < 3 || best < 0;
+    if (tid == 0) carry = 0;
+    __syncthreads();
+    if (!keep_all) {
+        unsigned c = 0;
+        for (unsigned i = tid; i < n; i += 1024) c += inlier[i];
+        for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
+        if (lane == 0) atomicAdd(&carry, c);
+        __syncthreads();
+        keep_all = carry < 3;
+        __syncthreads();
+        if (tid == 0) carry = 0;
+        __syncthreads();
+    }
+    for (unsigned base = 0; base < n; base += 1024) {
+        const unsigned i = base + tid;
+        const unsigned f = (i < n) ? (keep_all ? 1u : (unsigned)inlier[i]) : 0u;
+        unsigned inc = f;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned up = __shfl_up_sync(0xffffffffu, inc, o);
+            if (lane >= (unsigned)o) inc += up;
+        }
+        if (lane == 31) ws[wid] = inc;
+        __syncthreads();
+        if (wid == 0) {
+            const unsigned v = ws[lane];
+            unsigned winc = v;
+#pragma unroll
+            for (int o = 1; o < 32; o <<= 1) {
+                const unsigned up = __shfl_up_sync(0xffffffffu, winc, o);
+                if (lane >= (unsigned)o) winc += up;
+            }
+            ws[lane] = winc - v;
+        }
+        __syncthreads();
+        const unsigned excl = carry + ws[wid] + inc - f;
+        if (f) { pairs_out[2 * excl] = pairs[(size_t)stride * i]; pairs_out[2 * excl + 1] = pairs[(size_t)stride * i + 1]; }
+        __syncthreads();
+        if (tid == 1023) carry = excl + f;
+        __syncthreads();
+    }
+    if (tid < 16) T_out[tid] = keep_all ? ((tid % 5 == 0) ? 1.0f : 0.0f) : models[16 * (size_t)best + tid];
+    if (tid == 0) { *n_out = (int)carry; *iterations_out = keep_all ? 0 : st->iterations; }
+}
+
+// scratch of both entry points: correspondence sources | targets (cap each) in d_gather; the state, samples, models, counts
+// and inlier flags in d_partial, then (16-byte aligned) `extra` bytes of the entry point's own
+struct RansacScratch {
+    float4 *s4, *t4;
+    RansacDevState* st;
+    int* samples;
+    float* models;
+    int* counts;
+    unsigned char* inlier;
+    char* extra;
+};
+
+static int ransac_scratch(Ctx* c, const char* who, int max_iterations, size_t cap, size_t extra, RansacScratch* r) {
+    const size_t n_hyp = (size_t)max_iterations + 1;
+    char* base = reinterpret_cast<char*>(c->d_partial);
+    r->s4 = reinterpret_cast<float4*>(c->d_gather);
+    r->t4 = r->s4 + cap;
+    r->st = reinterpret_cast<RansacDevState*>(base);
+    r->samples = reinterpret_cast<int*>(base + 64);
+    r->models = reinterpret_cast<float*>(r->samples + 3 * n_hyp);
+    r->counts = reinterpret_cast<int*>(r->models + 16 * n_hyp);
+    r->inlier = reinterpret_cast<unsigned char*>(r->counts + n_hyp);
+    r->extra = base + ((64 + (3 + 16 + 1) * n_hyp * 4 + cap + 15) & ~(size_t)15);
+    if ((size_t)(r->extra - base) + extra > c->partial_cap * 8) { set_error("%s: scratch too small for %d iterations", who, max_iterations); return BSHOT_E_CAPACITY; }
+    return BSHOT_OK;
 }
 
 // ---- host: PCL's sample sequence ------------------------------------------------------------------------------------------
@@ -163,7 +275,7 @@ static double sample_dist_threshold(const float* src4, size_t n) {
 int ransac_run(Ctx* c, const float* src_xyz, const float* tgt_xyz, const int* pairs, size_t n_pairs, int max_iterations, double threshold,
                int* inlier_pairs_out, int* n_inliers_out, float* transform_out, int* iterations_out) {
     if (n_inliers_out) *n_inliers_out = 0;
-    auto keep_all = [&]() {  // PCL: computeModel failed / fewer than 3 inliers -> all correspondences stay, identity
+    auto keep_all = [&]() {  // PCL: computeModel failed -> all correspondences stay, identity
         if (inlier_pairs_out) memcpy(inlier_pairs_out, pairs, sizeof(int) * 2 * n_pairs);
         if (n_inliers_out) *n_inliers_out = (int)n_pairs;
         if (transform_out) for (int k = 0; k < 16; ++k) transform_out[k] = (k % 5 == 0) ? 1.0f : 0.0f;
@@ -201,66 +313,41 @@ int ransac_run(Ctx* c, const float* src_xyz, const float* tgt_xyz, const int* pa
         samples[3 * h] = shuffled[0]; samples[3 * h + 1] = shuffled[1]; samples[3 * h + 2] = shuffled[2];
     }
     if (n_valid == 0) return keep_all();
-    // ---- score every hypothesis on the device -----------------------------------------------------------------------------
-    float4* d_src = reinterpret_cast<float4*>(c->d_gather);          // max_kp x 48 B scratch: sources | targets
-    float4* d_tgt = d_src + n;
-    int* d_samples = reinterpret_cast<int*>(c->d_partial);            // >= 2 x 256 x max_kp u64
-    float* d_models = reinterpret_cast<float*>(d_samples + 3 * n_hyp);
-    int* d_counts = reinterpret_cast<int*>(d_models + 16 * n_hyp);
-    unsigned char* d_inlier = reinterpret_cast<unsigned char*>(d_counts + n_hyp);
-    if ((3 + 16 + 1) * n_hyp * 4 + n > c->partial_cap * 8) { set_error("bshot_ransac: scratch too small for %d iterations", max_iterations); return BSHOT_E_CAPACITY; }
-    BSHOT_CUDA_TRY(cudaMemcpyAsync(d_src, s4.data(), 16 * n, cudaMemcpyHostToDevice, c->stream));
-    BSHOT_CUDA_TRY(cudaMemcpyAsync(d_tgt, t4.data(), 16 * n, cudaMemcpyHostToDevice, c->stream));
-    BSHOT_CUDA_TRY(cudaMemcpyAsync(d_samples, samples.data(), sizeof(int) * 3 * n_valid, cudaMemcpyHostToDevice, c->stream));
+    // ---- the shared tail on the uploaded correspondences and samples -----------------------------------------------------------
+    // own scratch: results {n_inliers, iterations, T[16]} | input pairs (2n ints) | output pairs (2n ints)
+    RansacScratch r;
+    BSHOT_TRY(ransac_scratch(c, "bshot_ransac", max_iterations, n, 4 * (18 + 4 * n), &r));
+    int* d_res = reinterpret_cast<int*>(r.extra);
+    int* d_pairs_in = d_res + 18;
+    int* d_pairs_out = d_pairs_in + 2 * n;
+    RansacDevState st = {sdt, (int)n, (int)n_valid, -1, 0};
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(r.s4, s4.data(), 16 * n, cudaMemcpyHostToDevice, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(r.t4, t4.data(), 16 * n, cudaMemcpyHostToDevice, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(d_pairs_in, pairs, sizeof(int) * 2 * n, cudaMemcpyHostToDevice, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(r.samples, samples.data(), sizeof(int) * 3 * n_valid, cudaMemcpyHostToDevice, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(r.st, &st, sizeof(st), cudaMemcpyHostToDevice, c->stream));
     const double thresh2 = threshold * threshold;
-    ransac_score_kernel<<<(unsigned)((n_valid * 32 + 127) / 128), 128, 0, c->stream>>>(d_src, d_tgt, (unsigned)n, d_samples, (unsigned)n_valid, thresh2, d_models,
-                                                                                     d_counts);
+    ransac_score_dev_kernel<<<(unsigned)((n_valid * 32 + 127) / 128), 128, 0, c->stream>>>(r.s4, r.t4, r.st, r.samples, thresh2, r.models, r.counts);
     count_launch(c);
-    BSHOT_TRY(check_launch("ransac_score_kernel"));
+    BSHOT_TRY(check_launch("ransac_score_dev_kernel"));
     std::vector<int> counts(n_valid);
-    BSHOT_CUDA_TRY(cudaMemcpyAsync(counts.data(), d_counts, sizeof(int) * n_valid, cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(counts.data(), r.counts, sizeof(int) * n_valid, cudaMemcpyDeviceToHost, c->stream));
     BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
-    // ---- RandomSampleConsensus::computeModel replayed over the scores --------------------------------------------------------
-    int iterations = 0, best = -1, n_best = -2147483647;
-    double k = 1.0;
-    const double log_probability = log(1.0 - 0.99), one_over_indices = 1.0 / (double)n;
-    while ((double)iterations < k) {
-        if ((size_t)iterations >= n_valid) break;  // no sample could be drawn: PCL breaks out
-        const int cnt = counts[iterations];
-        if (cnt > n_best) {
-            n_best = cnt;
-            best = iterations;
-            const double w = (double)n_best * one_over_indices;
-            double p_no_outliers = 1.0 - pow(w, 3.0);
-            p_no_outliers = std::max(2.220446049250313e-16, p_no_outliers);
-            p_no_outliers = std::min(1.0 - 2.220446049250313e-16, p_no_outliers);
-            k = log_probability / log(p_no_outliers);
-        }
-        ++iterations;
-        if (iterations > max_iterations) break;
-    }
-    if (best < 0) return keep_all();
-    // ---- inliers of the best model, original order ---------------------------------------------------------------------------
-    ransac_select_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(d_src, d_tgt, (unsigned)n, d_models + 16 * (size_t)best, thresh2, d_inlier);
-    count_launch(c);
-    BSHOT_TRY(check_launch("ransac_select_kernel"));
-    std::vector<unsigned char> inl(n);
-    float model[16];
-    BSHOT_CUDA_TRY(cudaMemcpyAsync(inl.data(), d_inlier, n, cudaMemcpyDeviceToHost, c->stream));
-    BSHOT_CUDA_TRY(cudaMemcpyAsync(model, d_models + 16 * (size_t)best, sizeof(model), cudaMemcpyDeviceToHost, c->stream));
+    ransac_adaptive_stop(&st, counts.data(), max_iterations);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(r.st, &st, sizeof(st), cudaMemcpyHostToDevice, c->stream));
+    ransac_select_dev_kernel<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(r.s4, r.t4, r.st, r.models, thresh2, r.inlier);
+    ransac_finish_kernel<<<1, 1024, 0, c->stream>>>(r.st, d_pairs_in, 2, r.inlier, r.models, d_pairs_out, d_res, reinterpret_cast<float*>(d_res + 2), d_res + 1);
+    count_launch(c, 2);
+    BSHOT_TRY(check_launch("ransac_select_dev_kernel / ransac_finish_kernel"));
+    int res[18];
+    std::vector<int> kept(2 * n);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(res, d_res, sizeof(res), cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(kept.data(), d_pairs_out, sizeof(int) * 2 * n, cudaMemcpyDeviceToHost, c->stream));
     BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
-    size_t m = 0;
-    for (size_t i = 0; i < n; ++i) m += inl[i];
-    if (m < 3) return keep_all();
-    m = 0;
-    for (size_t i = 0; i < n; ++i)
-        if (inl[i]) {
-            if (inlier_pairs_out) { inlier_pairs_out[2 * m] = pairs[2 * i]; inlier_pairs_out[2 * m + 1] = pairs[2 * i + 1]; }
-            ++m;
-        }
-    if (n_inliers_out) *n_inliers_out = (int)m;
-    if (transform_out) memcpy(transform_out, model, sizeof(model));
-    if (iterations_out) *iterations_out = iterations;
+    if (inlier_pairs_out) memcpy(inlier_pairs_out, kept.data(), sizeof(int) * 2 * (size_t)res[0]);
+    if (n_inliers_out) *n_inliers_out = res[0];
+    if (transform_out) memcpy(transform_out, res + 2, sizeof(float) * 16);
+    if (iterations_out) *iterations_out = res[1];
     return BSHOT_OK;
 }
 
@@ -270,11 +357,7 @@ int ransac_run(Ctx* c, const float* src_xyz, const float* tgt_xyz, const int* pa
 // swap chain (the only sequential part: draw j always swaps position j % 3) runs on one thread with positions 0..2 in
 // registers, the distance tests of the 208 triples run in parallel, and one thread walks the test results in order, which
 // makes a try a hypothesis, counts the tries of the current hypothesis and gives up after 1000 -- exactly the host loop, for
-// any number of tries.  Scores, selection and the adaptive-stop replay are the host's, fed by device-side counts.
-struct RansacDevState {
-    double sdt;
-    int n, n_valid, best, iterations;
-};
+// any number of tries.  The tail after the sampler is the host call's.
 
 constexpr int RS_TRIES = 208;           // tries per batch: 3 x 208 = 624 draws = one twist
 constexpr int RS_THREADS = 256;
@@ -401,103 +484,8 @@ ransac_sample_kernel(const float4* __restrict__ s4, RansacDevState* __restrict__
     }
 }
 
-__global__ void __launch_bounds__(128)
-ransac_score_dev_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const RansacDevState* __restrict__ st, const int* __restrict__ samples,
-                        double thresh2, float* __restrict__ models, int* __restrict__ counts) {
-    const unsigned lane = threadIdx.x & 31, h = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    if (st->n < 3 || h >= (unsigned)st->n_valid) return;
-    ransac_score_one(src, tgt, (unsigned)st->n, samples, h, lane, thresh2, models, counts);
-}
-
-// RandomSampleConsensus::computeModel replayed over the scores (one thread; the host loop verbatim)
 __global__ void ransac_replay_kernel(RansacDevState* __restrict__ st, const int* __restrict__ counts, int max_iterations) {
-    if (threadIdx.x != 0 || blockIdx.x != 0) return;
-    const int n = st->n, n_valid = st->n_valid;
-    if (n < 3) return;
-    int iterations = 0, best = -1, n_best = -2147483647;
-    double k = 1.0;
-    const double log_probability = log(1.0 - 0.99), one_over_indices = 1.0 / (double)n;
-    while ((double)iterations < k) {
-        if (iterations >= n_valid) break;
-        const int cnt = counts[iterations];
-        if (cnt > n_best) {
-            n_best = cnt;
-            best = iterations;
-            const double w = (double)n_best * one_over_indices;
-            double p_no_outliers = 1.0 - pow(w, 3.0);
-            p_no_outliers = fmax(2.220446049250313e-16, p_no_outliers);
-            p_no_outliers = fmin(1.0 - 2.220446049250313e-16, p_no_outliers);
-            k = log_probability / log(p_no_outliers);
-        }
-        ++iterations;
-        if (iterations > max_iterations) break;
-    }
-    st->best = best;
-    st->iterations = iterations;
-}
-
-__global__ void ransac_select_dev_kernel(const float4* __restrict__ src, const float4* __restrict__ tgt, const RansacDevState* __restrict__ st,
-                                         const float* __restrict__ models, double thresh2, unsigned char* __restrict__ inlier) {
-    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (st->best < 0 || i >= (unsigned)st->n) return;
-    inlier[i] = ransac_is_inlier(models + 16 * (size_t)st->best, src[i], tgt[i], thresh2);
-}
-
-// one CTA: the inliers of the best model in their original order, or (fewer than 3 correspondences / no hypothesis / fewer
-// than 3 inliers) every correspondence with the identity -- PCL's behaviour, as ransac_run's keep_all
-__global__ void __launch_bounds__(1024)
-ransac_finish_kernel(const RansacDevState* __restrict__ st, const int* __restrict__ pairs, int stride, const unsigned char* __restrict__ inlier,
-                     const float* __restrict__ models, int* __restrict__ pairs_out, int* __restrict__ n_out, float* __restrict__ T_out,
-                     int* __restrict__ iterations_out) {
-    __shared__ unsigned ws[32];
-    __shared__ unsigned carry;
-    const unsigned tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    const unsigned n = (unsigned)max(st->n, 0);
-    const int best = st->best;
-    bool keep_all = n < 3 || best < 0;
-    if (tid == 0) carry = 0;
-    __syncthreads();
-    if (!keep_all) {
-        unsigned c = 0;
-        for (unsigned i = tid; i < n; i += 1024) c += inlier[i];
-        for (int o = 16; o > 0; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-        if (lane == 0) atomicAdd(&carry, c);
-        __syncthreads();
-        keep_all = carry < 3;
-        __syncthreads();
-        if (tid == 0) carry = 0;
-        __syncthreads();
-    }
-    for (unsigned base = 0; base < n; base += 1024) {
-        const unsigned i = base + tid;
-        const unsigned f = (i < n) ? (keep_all ? 1u : (unsigned)inlier[i]) : 0u;
-        unsigned inc = f;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned up = __shfl_up_sync(0xffffffffu, inc, o);
-            if (lane >= (unsigned)o) inc += up;
-        }
-        if (lane == 31) ws[wid] = inc;
-        __syncthreads();
-        if (wid == 0) {
-            const unsigned v = ws[lane];
-            unsigned winc = v;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const unsigned up = __shfl_up_sync(0xffffffffu, winc, o);
-                if (lane >= (unsigned)o) winc += up;
-            }
-            ws[lane] = winc - v;
-        }
-        __syncthreads();
-        const unsigned excl = carry + ws[wid] + inc - f;
-        if (f) { pairs_out[2 * excl] = pairs[(size_t)stride * i]; pairs_out[2 * excl + 1] = pairs[(size_t)stride * i + 1]; }
-        __syncthreads();
-        if (tid == 1023) carry = excl + f;
-        __syncthreads();
-    }
-    if (tid < 16) T_out[tid] = keep_all ? ((tid % 5 == 0) ? 1.0f : 0.0f) : models[16 * (size_t)best + tid];
-    if (tid == 0) { *n_out = (int)carry; *iterations_out = keep_all ? 0 : st->iterations; }
+    if (threadIdx.x == 0 && blockIdx.x == 0) ransac_adaptive_stop(st, counts, max_iterations);
 }
 
 int ransac_run_dev(Ctx* c, const float4* d_src, const float4* d_tgt, const int* d_pairs, int pair_stride, const int* d_n_pairs, size_t n_cap,
@@ -505,29 +493,20 @@ int ransac_run_dev(Ctx* c, const float4* d_src, const float4* d_tgt, const int* 
     if (n_cap > c->max_kp) { set_error("bshot_ransac_dev: %zu correspondences > max_keypoints %zu", n_cap, c->max_kp); return BSHOT_E_CAPACITY; }
     if (max_iterations < 1 || max_iterations > 100000) { set_error("bshot_ransac_dev: bad max_iterations"); return BSHOT_E_INVALID; }
     const size_t n_hyp = (size_t)max_iterations + 1, cap = std::max<size_t>(n_cap, 1);
-    // scratch: correspondence sources | targets in d_gather; state, samples, models, counts, inlier flags (+ the shuffled
-    // list when it does not fit in shared memory) in d_partial
-    float4* s4 = reinterpret_cast<float4*>(c->d_gather);
-    float4* t4 = s4 + cap;
-    char* base = reinterpret_cast<char*>(c->d_partial);
-    RansacDevState* st = reinterpret_cast<RansacDevState*>(base);
-    int* samples = reinterpret_cast<int*>(base + 64);
-    float* models = reinterpret_cast<float*>(samples + 3 * n_hyp);
-    int* counts = reinterpret_cast<int*>(models + 16 * n_hyp);
-    unsigned char* inlier = reinterpret_cast<unsigned char*>(counts + n_hyp);
-    int* g_shuffled = reinterpret_cast<int*>(base + ((64 + (3 + 16 + 1) * n_hyp * 4 + cap + 15) & ~(size_t)15));
+    // the shuffled list: n ints in shared memory when they fit, else in the scratch
     const size_t smem = 4 * cap;
     const bool in_smem = smem <= 160 * 1024;
-    const size_t need = (size_t)(reinterpret_cast<char*>(g_shuffled) - base) + (in_smem ? 0 : 4 * cap);
-    if (need > c->partial_cap * 8) { set_error("bshot_ransac_dev: scratch too small for %d iterations", max_iterations); return BSHOT_E_CAPACITY; }
+    RansacScratch r;
+    BSHOT_TRY(ransac_scratch(c, "bshot_ransac_dev", max_iterations, cap, in_smem ? 0 : 4 * cap, &r));
     const double thresh2 = threshold * threshold;
-    ransac_gather_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, c->stream>>>(d_src, d_tgt, d_pairs, pair_stride, d_n_pairs, (unsigned)n_cap, d_skip, s4, t4, st);
+    ransac_gather_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, c->stream>>>(d_src, d_tgt, d_pairs, pair_stride, d_n_pairs, (unsigned)n_cap, d_skip, r.s4, r.t4,
+                                                                              r.st);
     if (in_smem && smem > 48 * 1024) BSHOT_CUDA_TRY(cudaFuncSetAttribute(ransac_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    ransac_sample_kernel<<<1, RS_THREADS, in_smem ? smem : 0, c->stream>>>(s4, st, (unsigned)n_hyp, samples, in_smem ? nullptr : g_shuffled);
-    ransac_score_dev_kernel<<<(unsigned)((n_hyp * 32 + 127) / 128), 128, 0, c->stream>>>(s4, t4, st, samples, thresh2, models, counts);
-    ransac_replay_kernel<<<1, 32, 0, c->stream>>>(st, counts, max_iterations);
-    ransac_select_dev_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, c->stream>>>(s4, t4, st, models, thresh2, inlier);
-    ransac_finish_kernel<<<1, 1024, 0, c->stream>>>(st, d_pairs, pair_stride, inlier, models, d_pairs_out, d_n_out, d_T_out, d_iterations_out);
+    ransac_sample_kernel<<<1, RS_THREADS, in_smem ? smem : 0, c->stream>>>(r.s4, r.st, (unsigned)n_hyp, r.samples, in_smem ? nullptr : reinterpret_cast<int*>(r.extra));
+    ransac_score_dev_kernel<<<(unsigned)((n_hyp * 32 + 127) / 128), 128, 0, c->stream>>>(r.s4, r.t4, r.st, r.samples, thresh2, r.models, r.counts);
+    ransac_replay_kernel<<<1, 32, 0, c->stream>>>(r.st, r.counts, max_iterations);
+    ransac_select_dev_kernel<<<(unsigned)((cap + 255) / 256), 256, 0, c->stream>>>(r.s4, r.t4, r.st, r.models, thresh2, r.inlier);
+    ransac_finish_kernel<<<1, 1024, 0, c->stream>>>(r.st, d_pairs, pair_stride, r.inlier, r.models, d_pairs_out, d_n_out, d_T_out, d_iterations_out);
     count_launch(c, 6);
     return check_launch("device RANSAC kernels");
 }

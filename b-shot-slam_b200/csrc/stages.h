@@ -69,10 +69,12 @@ int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t
 int gmap_gather(Ctx* c, const float pos[3], float range, const float4* d_ref_kp, const uint64_t* d_ref_bits, const int* d_ref_count,
                 size_t ref_cap, const float* ref_pose12, uint64_t* d_t_out, size_t out_cap, unsigned* d_total, bool pose_on_device = false);
 
-// RANSAC correspondence rejection (ransac.cu)
+// RANSAC correspondence rejection (ransac.cu).  ransac_run draws PCL's sample sequence on the host, ransac_run_dev on the
+// device; after the sampler both run the same device tail (scoring, adaptive stop, inlier flags, ordered compaction).
+// ransac_run is synchronous
 int ransac_run(Ctx* c, const float* src_xyz, const float* tgt_xyz, const int* pairs, size_t n_pairs, int max_iterations, double threshold,
                int* inlier_pairs_out, int* n_inliers_out, float* transform_out, int* iterations_out);
-// the same on device inputs: d_pairs = n_cap records of pair_stride ints (query, match, ...), *d_n_pairs of them valid;
+// device inputs: d_pairs = n_cap records of pair_stride ints (query, match, ...), *d_n_pairs of them valid;
 // outputs in device memory.  A set *d_skip (may be null) treats the input as empty.  Asynchronous
 int ransac_run_dev(Ctx* c, const float4* d_src, const float4* d_tgt, const int* d_pairs, int pair_stride, const int* d_n_pairs, size_t n_cap,
                    int max_iterations, double threshold, int* d_pairs_out, int* d_n_out, float* d_T_out, int* d_iterations_out, const int* d_skip);
@@ -85,9 +87,11 @@ struct IcpState {
 };
 int icp_run(Ctx* c, const float* src_xyz, size_t n_src, const float* tgt_xyz, size_t n_tgt, const float* pre4x4, int max_iterations,
             float* final4x4_out, int* iterations_out, int* state_out, double* mse_out);
-// the same on device inputs with device-side counts (see icp.cu); the result stays in *d_st
-int icp_run_dev(Ctx* c, const float4* d_src, const int* d_ns, size_t ns_cap, const float4* d_tgt, const unsigned* d_nt, size_t nt_cap, const float* d_pre,
-                int max_iterations, const int* d_skip, float4* d_cur, float4* d_tgt_buf, unsigned long long* d_keys, IcpState* d_st);
+// icp_run uploads its inputs and runs icp_run_dev.  Points are src_stride / tgt_stride floats apart (3 or 4), the counts are
+// device-side with host-known capacities (see icp.cu); the result stays in *d_st.  Asynchronous
+int icp_run_dev(Ctx* c, const float* d_src, int src_stride, const int* d_ns, size_t ns_cap, const float* d_tgt, int tgt_stride, const unsigned* d_nt,
+                size_t nt_cap, const float* d_pre, int max_iterations, const int* d_skip, float4* d_cur, float4* d_tgt_buf, unsigned long long* d_keys,
+                IcpState* d_st);
 
 // scan preprocessor (preprocess.cu); scratch_reserve grows one of the context's on-demand scratch buffers
 int scratch_reserve(Ctx* c, int which, size_t bytes);
@@ -116,7 +120,19 @@ int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_
 
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);
-int frame_commit(Ctx* c, size_t k);
+// the current frame becomes the reference frame (descriptors, keypoint positions and count stay on the device).  A set
+// *d_skip (may be null) leaves the reference frame as it is; with a flag the caller sets c->n_prev once it has read it
+int frame_commit(Ctx* c, size_t k, const int* d_skip = nullptr);
+// featureMatching against the map (src/lidar_odometry.cpp:197-206), used by bshot_match_frame_to_map and the odometry step:
+// target set = map keypoints in range ++ the reference frame moved by ref_pose12 (gmap_gather into d_t / gmap.d_tpos, the
+// count in gmap.d_ctl[6]), then the mutual nearest neighbours of the frame's k descriptors -> d_pairs / d_pair_count (0 when
+// the target set is empty by its host-side bound *nt_cap_out)
+int frame_match_map(Ctx* c, size_t k, const float pos[3], float range, const float* ref_pose12, bool pose_on_device, size_t* nt_cap_out);
+// the target set overflowed max_targets: more candidates than max_targets, and the gather stopped at max_targets.  ctl is
+// gmap.d_ctl after frame_match_map ([4] map keypoints in range, [6] targets assembled)
+__host__ __device__ inline bool target_set_overflow(const unsigned* ctl, size_t n_prev, size_t max_targets) {
+    return (size_t)ctl[4] + n_prev > max_targets && (size_t)ctl[6] == max_targets;
+}
 int frame_run(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);
 
 }  // namespace bshot
