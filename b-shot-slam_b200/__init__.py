@@ -38,6 +38,7 @@ EXPORTS = [
     "bshot_preprocess", "bshot_preprocess_select", "bshot_extract_scan", "bshot_icp", "bshot_evaluate_estimation", "bshot_set_matcher",
     "bshot_iss_params_default", "bshot_detect_iss", "bshot_kp_repeatability", "bshot_voxel_grid",
     "bshot_odom_params_default", "bshot_odometry_step", "bshot_odometry_step_cloud", "bshot_odometry_reset", "bshot_ransac_dev",
+    "bshot_gmap_export", "bshot_gmap_import", "bshot_relocalize", "bshot_relocalize_cloud",
 ]
 
 
@@ -62,6 +63,12 @@ class OdomReport(C.Structure):
                 ("n_keypoints", C.c_int), ("n_pairs", C.c_int), ("n_inliers", C.c_int), ("ransac_iterations", C.c_int),
                 ("icp_iterations", C.c_int), ("should_update_map", C.c_int), ("was_initial", C.c_int),
                 ("h_diff_rad", C.c_float), ("t_diff_mm", C.c_float)]
+
+
+class RelocReport(C.Structure):
+    _fields_ = [("pose", C.c_float * 16), ("T_ransac", C.c_float * 16), ("n_points", C.c_size_t), ("n_map", C.c_size_t),
+                ("n_icp_targets", C.c_size_t), ("n_keypoints", C.c_int), ("n_pairs", C.c_int), ("n_inliers", C.c_int),
+                ("ransac_iterations", C.c_int), ("icp_iterations", C.c_int), ("accepted", C.c_int)]
 
 
 E_INVALID, E_CAPACITY, E_CUDA, E_STATE = -1, -2, -3, -4
@@ -175,6 +182,10 @@ def lib():
         L.bshot_odometry_step_cloud.argtypes = [vp, C.POINTER(OdomParams), vp, sz, sz, C.POINTER(OdomReport)]
         L.bshot_odometry_reset.argtypes = [vp]
         L.bshot_ransac_dev.argtypes = [vp, vp, vp, vp, vp, sz, ci, cf, vp, vp, vp, vp]
+        L.bshot_gmap_export.argtypes = [vp, vp, vp, sz, C.POINTER(sz)]
+        L.bshot_gmap_import.argtypes = [vp, vp, vp, sz]
+        L.bshot_relocalize.argtypes = [vp, C.POINTER(OdomParams), ci, vp, vp, vp, sz, vp, sz, C.POINTER(RelocReport)]
+        L.bshot_relocalize_cloud.argtypes = [vp, C.POINTER(OdomParams), ci, vp, sz, sz, C.POINTER(RelocReport)]
         _LIB = L
     return _LIB
 
@@ -225,7 +236,7 @@ def odom_default_params(**kw):
 
 
 def _report(r):
-    out = {name: getattr(r, name) for name, _ in OdomReport._fields_ if name not in ("pose", "T_ransac")}
+    out = {name: getattr(r, name) for name, _ in type(r)._fields_ if name not in ("pose", "T_ransac")}
     out["pose"] = np.ctypeslib.as_array(r.pose).reshape(4, 4).copy()
     out["T_ransac"] = np.ctypeslib.as_array(r.T_ransac).reshape(4, 4).copy()
     return out
@@ -500,6 +511,26 @@ class Context:
         _chk(lib().bshot_gmap_get_keypoints(self.h, _p(pos), rng, _p(xyz), _p(desc), n.value, C.byref(n)))
         return xyz, desc
 
+    def gmap_export(self):
+        """every map entry in map order (blocks in ascending lattice coordinates, x outermost; entries of a block in
+        insertion order) -> (xyzr (n, 4) float32 {x, y, z, seg_ratio}, desc (n, 6) uint64)"""
+        n = C.c_size_t()
+        rc = lib().bshot_gmap_export(self.h, None, None, 0, C.byref(n))
+        if rc not in (0, E_CAPACITY):
+            _chk(rc)
+        xyzr = np.empty((n.value, 4), np.float32)
+        desc = np.empty((n.value, 6), np.uint64)
+        _chk(lib().bshot_gmap_export(self.h, _p(xyzr), _p(desc), n.value, C.byref(n)))
+        return xyzr, desc
+
+    def gmap_import(self, xyzr, desc):
+        """replace the map by these entries (a gmap_export result restores its map); on an error the map is empty"""
+        xyzr = np.ascontiguousarray(xyzr, dtype=np.float32).reshape(-1, 4)
+        desc = np.ascontiguousarray(desc, dtype=np.uint64).reshape(-1, 6)
+        if xyzr.shape[0] != desc.shape[0]:
+            raise BshotError("gmap_import: xyzr and desc differ in length", E_INVALID)
+        _chk(lib().bshot_gmap_import(self.h, _p(xyzr), _p(desc), xyzr.shape[0]))
+
     def extract_frame(self, xyz, params):
         xyz = np.ascontiguousarray(xyz, dtype=np.float32)
         k = params.top_k
@@ -610,6 +641,31 @@ class Context:
         assert xyz.ndim == 2 and xyz.shape[1] in (3, 4)
         r = OdomReport()
         _chk(lib().bshot_odometry_step_cloud(self.h, C.byref(params), _p(xyz), xyz.shape[0], xyz.shape[1] * 4, C.byref(r)))
+        self.n_points, self.n_kp = r.n_points, r.n_keypoints
+        return _report(r)
+
+    def relocalize(self, azimuth_deg, vertical_deg, distance, ring_deg, params=None, min_inliers=15):
+        """one rotation against the whole map without a prior pose: extraction -> matching against every map entry ->
+        RANSAC -> ICP around T_ransac.  With n_inliers >= min_inliers the pose becomes "pose" (T_best), the status RUN, and
+        the map and reference frame move on as after a step; otherwise nothing changes.  Returns the report as a dict."""
+        params = odom_default_params() if params is None else params
+        az = np.ascontiguousarray(azimuth_deg, dtype=np.float64)
+        ve = np.ascontiguousarray(vertical_deg, dtype=np.float64)
+        di = np.ascontiguousarray(distance, dtype=np.uint16)
+        ring = np.ascontiguousarray(ring_deg, dtype=np.float64)
+        assert az.shape == ve.shape == di.shape
+        r = RelocReport()
+        _chk(lib().bshot_relocalize(self.h, C.byref(params), min_inliers, _p(az), _p(ve), _p(di), az.size, _p(ring), ring.size, C.byref(r)))
+        self.n_points, self.n_kp = r.n_points, r.n_keypoints
+        return _report(r)
+
+    def relocalize_cloud(self, xyz, params=None, min_inliers=15):
+        """the same on an already-preprocessed (N, 3) or (N, 4) float32 cloud"""
+        params = odom_default_params() if params is None else params
+        xyz = np.ascontiguousarray(xyz, dtype=np.float32)
+        assert xyz.ndim == 2 and xyz.shape[1] in (3, 4)
+        r = RelocReport()
+        _chk(lib().bshot_relocalize_cloud(self.h, C.byref(params), min_inliers, _p(xyz), xyz.shape[0], xyz.shape[1] * 4, C.byref(r)))
         self.n_points, self.n_kp = r.n_points, r.n_keypoints
         return _report(r)
 

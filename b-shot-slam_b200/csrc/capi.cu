@@ -782,6 +782,19 @@ int bshot_gmap_get_keypoints(bshot_ctx* ctx, const float pos[3], float range, fl
     return sync(ctx);
 }
 
+int bshot_gmap_export(bshot_ctx* ctx, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t* n_out) {
+    CHECK_CTX(ctx);
+    if (!ctx->gmap.d_tab) { set_error("bshot_gmap_export: no map (bshot_gmap_create)"); return BSHOT_E_STATE; }
+    return gmap_export(ctx, xyzr_out, desc_out, cap, n_out);
+}
+
+int bshot_gmap_import(bshot_ctx* ctx, const float* xyzr, const uint64_t* desc, size_t n) {
+    CHECK_CTX(ctx);
+    if (!ctx->gmap.d_tab) { set_error("bshot_gmap_import: no map (bshot_gmap_create)"); return BSHOT_E_STATE; }
+    if (n && (!xyzr || !desc)) { set_error("bshot_gmap_import: null input"); return BSHOT_E_INVALID; }
+    return gmap_import(ctx, xyzr, desc, n);
+}
+
 int bshot_extract_frame(bshot_ctx* ctx, const bshot_params* p, const float* xyz, size_t n, size_t stride_bytes, int* kp_idx_out, float* kp_xyz_out,
                         float* seg_ratio_out, uint64_t* bits_out, int* n_kp_out) {
     CHECK_CTX(ctx);
@@ -990,6 +1003,40 @@ int bshot_odometry_step_cloud(bshot_ctx* ctx, const bshot_odom_params* p, const 
     BSHOT_TRY(frame_args_ok(ctx, &p->front, n, stride_bytes, "bshot_odometry_step_cloud"));
     BSHOT_TRY(h2d(ctx, ctx->d_raw, xyz, n * stride_bytes));
     return odometry_run(ctx, p, ctx->d_raw, n, (int)(stride_bytes / 4), out);
+}
+
+static int reloc_args_ok(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const char* who) {
+    if (min_inliers < 3) { set_error("%s: min_inliers %d < 3", who, min_inliers); return BSHOT_E_INVALID; }
+    return odom_args_ok(ctx, p, who);
+}
+
+int bshot_relocalize(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const double* azimuth_deg, const double* vertical_deg,
+                     const unsigned short* distance, size_t n, const double* ring_deg, size_t nv, bshot_reloc_report* out) {
+    CHECK_CTX(ctx);
+    bshot_odom_params dp;
+    if (!p) { bshot_odom_params_default(&dp); p = &dp; }
+    if (n && (!azimuth_deg || !vertical_deg || !distance)) { set_error("bshot_relocalize: null input"); return BSHOT_E_INVALID; }
+    if (nv && !ring_deg) { set_error("bshot_relocalize: null ring table"); return BSHOT_E_INVALID; }
+    if (n > 0xFFFFFFFFull) { set_error("bshot_relocalize: too many returns"); return BSHOT_E_CAPACITY; }
+    BSHOT_TRY(reloc_args_ok(ctx, p, min_inliers, "bshot_relocalize"));
+    size_t kept = 0;
+    const float* d_cloud = nullptr;
+    BSHOT_TRY(preprocess_run(ctx, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, p->vert_init_rad, p->lowpt_th, nullptr, 1, nullptr, std::max<size_t>(n, 1),
+                             &kept, &d_cloud));
+    BSHOT_TRY(frame_args_ok(ctx, &p->front, kept, 12, "bshot_relocalize"));
+    return relocalize_run(ctx, p, min_inliers, d_cloud, kept, 3, out);
+}
+
+int bshot_relocalize_cloud(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const float* xyz, size_t n, size_t stride_bytes,
+                           bshot_reloc_report* out) {
+    CHECK_CTX(ctx);
+    bshot_odom_params dp;
+    if (!p) { bshot_odom_params_default(&dp); p = &dp; }
+    if (!xyz && n) { set_error("bshot_relocalize_cloud: null cloud"); return BSHOT_E_INVALID; }
+    BSHOT_TRY(reloc_args_ok(ctx, p, min_inliers, "bshot_relocalize_cloud"));
+    BSHOT_TRY(frame_args_ok(ctx, &p->front, n, stride_bytes, "bshot_relocalize_cloud"));
+    BSHOT_TRY(h2d(ctx, ctx->d_raw, xyz, n * stride_bytes));
+    return relocalize_run(ctx, p, min_inliers, ctx->d_raw, n, (int)(stride_bytes / 4), out);
 }
 
 int bshot_odometry_reset(bshot_ctx* ctx) {

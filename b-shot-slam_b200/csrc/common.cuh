@@ -96,6 +96,15 @@ struct Gmap {
     unsigned tab_cap = 0, max_entries = 0, max_chunks = 0, max_probe = 0, epoch = 0;
     size_t n_gathered = 0;
     size_t entries_upper = 0;           // host-side upper bound of the number of entries (sizes the match grid without a sync)
+    // the whole map in map order (gmap_gather_all, export, relocalisation) and the import's rebuild: allocated by the first
+    // call that needs them
+    float4* d_apos = nullptr;           // max_entries: positions + seg-ratio in map order
+    uint64_t* d_adesc = nullptr;        // max_entries: descriptors in map order
+    unsigned long long* d_skeys[2] = {nullptr, nullptr};  // max(tab_cap, max_entries): radix ping-pong (block order keys / slots)
+    unsigned* d_svals[2] = {nullptr, nullptr};            // max(tab_cap, max_entries): slots / entry indices
+    unsigned* d_shist = nullptr;        // radix histograms
+    unsigned* d_boff = nullptr;         // tab_cap: entry offset of each listed block / first sorted entry of each slot (import)
+    unsigned* d_actl = nullptr;         // [0] listed blocks [1] entries gathered [2] import error bits [3] import entries
 };
 
 // ISS keypoints (iss.cu): max_points-sized buffers, allocated by the first bshot_detect_iss of the context

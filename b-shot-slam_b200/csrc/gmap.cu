@@ -16,6 +16,7 @@
 // table slot {key, count, first chunk, last chunk} plus a chain of 32-index chunks, so a warp reads a block 32 entries
 // at a time.  Admission is sequential per block (the rule is order dependent) and parallel across blocks: one warp per
 // block touched by the frame walks the frame's keypoints in order.
+#include <algorithm>
 #include <cmath>
 
 #include "common.cuh"
@@ -171,13 +172,43 @@ __host__ __device__ inline GmapCube gm_cube(float px, float py, float pz, float 
     return c;
 }
 
+// one step of a running exclusive scan over a CTA of 1024 threads: *carry (shared, 0 before the first step) + the exclusive
+// prefix of v over this step's threads; *carry then holds the running total.  Every thread must call it
+__device__ __forceinline__ unsigned cta_scan_1024(unsigned v, unsigned* ws, unsigned* carry) {
+    const unsigned tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    unsigned inc = v;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const unsigned up = __shfl_up_sync(0xffffffffu, inc, o);
+        if (lane >= (unsigned)o) inc += up;
+    }
+    if (lane == 31) ws[wid] = inc;
+    __syncthreads();
+    if (wid == 0) {
+        const unsigned u = ws[lane];
+        unsigned winc = u;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const unsigned up = __shfl_up_sync(0xffffffffu, winc, o);
+            if (lane >= (unsigned)o) winc += up;
+        }
+        ws[lane] = winc - u;
+    }
+    __syncthreads();
+    const unsigned excl = *carry + ws[wid] + inc - v;
+    __syncthreads();
+    if (tid == 1023) *carry = excl + v;
+    __syncthreads();
+    return excl;
+}
+
 // one CTA: counts of the probed blocks in loop order (x outermost, z innermost), exclusive scan -> offsets
 __global__ void __launch_bounds__(1024)
 gm_probe_kernel(const GmapBlock* __restrict__ tab, unsigned mask, GmapCube cube, const float* __restrict__ dev_pose, float range,
                 unsigned* __restrict__ probe_slot, unsigned* __restrict__ probe_off, unsigned* __restrict__ ctl, unsigned max_probe) {
     __shared__ unsigned ws[32];
     __shared__ unsigned carry;
-    const unsigned tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
+    const unsigned tid = threadIdx.x;
     if (dev_pose) {   // position = translation of the row-major [R|T]; a non-finite pose probes nothing
         cube = gm_cube(dev_pose[3], dev_pose[7], dev_pose[11], range);
         if (cube.nx <= 0 || cube.ny <= 0 || cube.nz <= 0) cube.nx = cube.ny = cube.nz = 0;
@@ -195,41 +226,19 @@ gm_probe_kernel(const GmapBlock* __restrict__ tab, unsigned mask, GmapCube cube,
             if (slot != 0xFFFFFFFFu) cnt = tab[slot].count;
             probe_slot[p] = slot;
         }
-        unsigned inc = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const unsigned up = __shfl_up_sync(0xffffffffu, inc, o);
-            if (lane >= (unsigned)o) inc += up;
-        }
-        if (lane == 31) ws[wid] = inc;
-        __syncthreads();
-        if (wid == 0) {
-            const unsigned v = ws[lane];
-            unsigned winc = v;
-#pragma unroll
-            for (int o = 1; o < 32; o <<= 1) {
-                const unsigned up = __shfl_up_sync(0xffffffffu, winc, o);
-                if (lane >= (unsigned)o) winc += up;
-            }
-            ws[lane] = winc - v;
-        }
-        __syncthreads();
-        const unsigned excl = carry + ws[wid] + inc - cnt;
+        const unsigned excl = cta_scan_1024(cnt, ws, &carry);
         if (p < np) probe_off[p] = excl;
-        __syncthreads();
-        if (tid == 1023) carry = excl + cnt;
-        __syncthreads();
     }
     if (tid == 0) { ctl[4] = carry; ctl[5] = np; }
 }
 
-// one warp per probed block: entries in insertion order -> out[offset + j]
+// one warp per listed block (*d_np of them): entries in insertion order -> out[offset + j]
 __global__ void __launch_bounds__(128)
 gm_collect_kernel(const GmapBlock* __restrict__ tab, const unsigned* __restrict__ probe_slot, const unsigned* __restrict__ probe_off,
-                  const unsigned* __restrict__ ctl, const unsigned* __restrict__ chunks, const float4* __restrict__ e_pos,
+                  const unsigned* __restrict__ d_np, const unsigned* __restrict__ chunks, const float4* __restrict__ e_pos,
                   const uint64_t* __restrict__ e_desc, float4* __restrict__ out_pos, uint64_t* __restrict__ out_desc, unsigned out_cap) {
     const unsigned lane = threadIdx.x & 31;
-    const unsigned np = ctl[5];
+    const unsigned np = *d_np;
     for (unsigned p = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; p < np; p += (gridDim.x * blockDim.x) >> 5) {
         const unsigned slot = probe_slot[p];
         if (slot == 0xFFFFFFFFu) continue;
@@ -268,6 +277,104 @@ __global__ void gm_append_ref_kernel(const float4* __restrict__ ref_kp, const ui
     for (int k = 0; k < 6; ++k) out_desc[(size_t)(base + i) * 6 + k] = ref_bits[(size_t)i * 6 + k];
 }
 
+// ---- the whole map in map order (gmap_gather_all), and the import's rebuild ---------------------------------------------
+// Map order: occupied blocks in ascending lattice coordinates (x outermost, z innermost: the order gm_probe_kernel visits
+// them), entries of a block in insertion order.  A block's coordinates are roundf(p / 10 m) of any of its entries (the
+// block id was computed from that same stored position).  actl: [0] listed blocks, [1] entries gathered, [2] import
+// error bits (1 non-finite position, 2 table / chunks full), [3] import entries.
+constexpr unsigned GM_AXIS_BIAS = 1u << 20;
+
+__device__ __forceinline__ unsigned long long gm_order_key(float4 p) {
+    const unsigned kx = ((unsigned)(int)roundf(p.x / (float)GM_PREC) + GM_AXIS_BIAS) & 0x1FFFFFu;
+    const unsigned ky = ((unsigned)(int)roundf(p.y / (float)GM_PREC) + GM_AXIS_BIAS) & 0x1FFFFFu;
+    const unsigned kz = ((unsigned)(int)roundf(p.z / (float)GM_PREC) + GM_AXIS_BIAS) & 0x1FFFFFu;
+    return ((unsigned long long)kx << 42) | ((unsigned long long)ky << 21) | (unsigned long long)kz;
+}
+
+// occupied, non-empty slots -> (order key, slot); the list's order is irrelevant (the keys are distinct and get sorted)
+__global__ void gm_list_blocks_kernel(const GmapBlock* __restrict__ tab, unsigned tab_cap, const unsigned* __restrict__ chunks,
+                                      const float4* __restrict__ e_pos, unsigned long long* __restrict__ keys, unsigned* __restrict__ slots,
+                                      unsigned* __restrict__ actl) {
+    const unsigned s = blockIdx.x * blockDim.x + threadIdx.x;
+    if (s >= tab_cap || tab[s].key == 0ull || tab[s].count == 0u) return;
+    const unsigned long long k = gm_order_key(e_pos[chunks[tab[s].first * 33u]]);
+    const unsigned i = atomicAdd(&actl[0], 1u);
+    keys[i] = k;
+    slots[i] = s;
+}
+
+// one CTA: entry offsets of the listed blocks in their sorted order; actl[1] = entries
+__global__ void __launch_bounds__(1024)
+gm_block_offsets_kernel(const GmapBlock* __restrict__ tab, const unsigned* __restrict__ slots, unsigned* __restrict__ off, unsigned* __restrict__ actl) {
+    __shared__ unsigned ws[32];
+    __shared__ unsigned carry;
+    if (threadIdx.x == 0) carry = 0;
+    __syncthreads();
+    const unsigned nb = actl[0];
+    for (unsigned base = 0; base < nb; base += 1024) {
+        const unsigned i = base + threadIdx.x;
+        const unsigned cnt = i < nb ? tab[slots[i]].count : 0u;
+        const unsigned excl = cta_scan_1024(cnt, ws, &carry);
+        if (i < nb) off[i] = excl;
+    }
+    if (threadIdx.x == 0) actl[1] = carry;
+}
+
+// import: the entries already sit at pool index = input index.  Block slot of every entry (created when new), its count,
+// and (slot, input index) for the stable sort by slot
+__global__ void gm_import_find_kernel(const float4* __restrict__ e_pos, unsigned n, GmapBlock* tab, unsigned mask, unsigned long long* __restrict__ keys,
+                                      unsigned* __restrict__ idx, unsigned* __restrict__ actl) {
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i == 0) actl[3] = n;
+    if (i >= n) return;
+    const float4 p = e_pos[i];
+    unsigned slot = 0xFFFFFFFFu;
+    if (!(isfinite(p.x) && isfinite(p.y) && isfinite(p.z))) atomicOr(&actl[2], 1u);
+    else if ((slot = gm_find(tab, mask, gm_block_id(p.x, p.y, p.z), true)) == 0xFFFFFFFFu) atomicOr(&actl[2], 2u);
+    else atomicAdd(&tab[slot].count, 1u);
+    keys[i] = slot;
+    idx[i] = i;
+}
+
+// import, one CTA over every table slot in slot order: first entry of the slot in the slot-sorted list (start) and
+// ceil(count / 32) consecutive chunks, first / last of the block; then the control words
+__global__ void __launch_bounds__(1024)
+gm_import_blocks_kernel(GmapBlock* tab, unsigned tab_cap, unsigned* __restrict__ start, unsigned* __restrict__ ctl, unsigned* __restrict__ actl,
+                        unsigned max_chunks) {
+    __shared__ unsigned ws[32];
+    __shared__ unsigned carry_e, carry_c;
+    if (threadIdx.x == 0) carry_e = carry_c = 0;
+    __syncthreads();
+    for (unsigned base = 0; base < tab_cap; base += 1024) {
+        const unsigned s = base + threadIdx.x;
+        const unsigned cnt = (s < tab_cap && tab[s].key != 0ull) ? tab[s].count : 0u, nch = (cnt + 31u) / 32u;
+        const unsigned e0 = cta_scan_1024(cnt, ws, &carry_e);
+        const unsigned c0 = cta_scan_1024(nch, ws, &carry_c);
+        if (s < tab_cap) start[s] = e0;
+        if (cnt) { tab[s].first = c0; tab[s].last = c0 + nch - 1u; }
+    }
+    if (threadIdx.x == 0) {
+        if (carry_c > max_chunks) actl[2] |= 2u;
+        ctl[0] = carry_e;
+        ctl[2] = carry_c;
+        ctl[3] = 0u;
+    }
+}
+
+// import: sorted position j -> rank r in its block -> chunk first + r / 32, lane r % 32; a chunk's first entry links it
+__global__ void gm_import_chain_kernel(const unsigned long long* __restrict__ slot_of, const unsigned* __restrict__ idx, unsigned n,
+                                       const GmapBlock* __restrict__ tab, unsigned tab_cap, const unsigned* __restrict__ start,
+                                       unsigned* __restrict__ chunks, unsigned max_chunks) {
+    const unsigned j = blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= n) return;
+    const unsigned long long s = slot_of[j];
+    if (s >= tab_cap) return;   // an entry without a block: the import fails
+    const unsigned r = j - start[s], cnt = tab[s].count, ch = tab[s].first + r / 32u;
+    if (ch >= max_chunks) return;
+    chunks[ch * 33u + (r & 31u)] = idx[j];
+    if ((r & 31u) == 0u) chunks[ch * 33u + 32u] = r + 32u < cnt ? ch + 1u : 0xFFFFFFFFu;
+}
+
 // ---- host side -----------------------------------------------------------------------------------------------------------
 int gmap_create(Ctx* c, size_t max_entries, size_t max_blocks) {
     Gmap& g = c->gmap;
@@ -295,7 +402,8 @@ int gmap_create(Ctx* c, size_t max_entries, size_t max_blocks) {
 
 void gmap_free(Ctx* c) {
     Gmap& g = c->gmap;
-    void* ptrs[] = {g.d_tab, g.d_epos, g.d_edesc, g.d_chunks, g.d_world, g.d_blk_of, g.d_touched, g.d_probe_slot, g.d_probe_off, g.d_ctl, g.d_pose, g.d_tpos};
+    void* ptrs[] = {g.d_tab, g.d_epos, g.d_edesc, g.d_chunks, g.d_world, g.d_blk_of, g.d_touched, g.d_probe_slot, g.d_probe_off, g.d_ctl, g.d_pose, g.d_tpos,
+                    g.d_apos, g.d_adesc, g.d_skeys[0], g.d_skeys[1], g.d_svals[0], g.d_svals[1], g.d_shist, g.d_boff, g.d_actl};
     for (void* p : ptrs) if (p) cudaFree(p);
     g = Gmap();
 }
@@ -349,13 +457,112 @@ int gmap_gather(Ctx* c, const float pos[3], float range, const float4* d_ref_kp,
         BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_pose + 12, ref_pose12, sizeof(float) * 12, pose_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, c->stream));
     gm_probe_kernel<<<1, 1024, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.tab_cap - 1, cube, pose_on_device ? g.d_pose + 12 : nullptr, range,
                                                g.d_probe_slot, g.d_probe_off, g.d_ctl, g.max_probe);
-    gm_collect_kernel<<<(unsigned)c->sm_count * 2u, 128, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.d_probe_slot, g.d_probe_off, g.d_ctl, g.d_chunks,
+    gm_collect_kernel<<<(unsigned)c->sm_count * 2u, 128, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.d_probe_slot, g.d_probe_off, g.d_ctl + 5, g.d_chunks,
                                                                         g.d_epos, g.d_edesc, g.d_tpos, d_t_out, (unsigned)out_cap);
     const unsigned nref = d_ref_bits ? (unsigned)ref_cap : 0u;
     gm_append_ref_kernel<<<(std::max(nref, 1u) + 255) / 256, 256, 0, c->stream>>>(d_ref_kp, d_ref_bits, d_ref_count, nref, g.d_pose + 12, ref_pose12 ? 1 : 0, g.d_ctl,
                                                                                 g.d_tpos, d_t_out, (unsigned)out_cap, d_total);
     count_launch(c, 3);
     return check_launch("map gather kernels");
+}
+
+// buffers of the whole-map gather and the import (entry-sized), allocated by the first call that needs them
+static int gmap_all_alloc(Ctx* c) {
+    Gmap& g = c->gmap;
+    if (g.d_apos) return BSHOT_OK;
+    const size_t m = std::max<size_t>(g.tab_cap, g.max_entries);
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_apos, sizeof(float4) * g.max_entries));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_adesc, 48 * (size_t)g.max_entries));
+    for (int k = 0; k < 2; ++k) {
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_skeys[k], sizeof(unsigned long long) * m));
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_svals[k], sizeof(unsigned) * m));
+    }
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_shist, sizeof(unsigned) * radix_hist_words(m)));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_boff, sizeof(unsigned) * g.tab_cap));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_actl, sizeof(unsigned) * 8));
+    return BSHOT_OK;
+}
+
+int gmap_gather_all(Ctx* c, size_t* nt_cap_out) {
+    Gmap& g = c->gmap;
+    if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
+    BSHOT_TRY(gmap_all_alloc(c));
+    const size_t nt_cap = std::min<size_t>(g.entries_upper, g.max_entries);
+    *nt_cap_out = nt_cap;
+    BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_actl, 0, sizeof(unsigned) * 8, c->stream));
+    if (nt_cap == 0) return BSHOT_OK;
+    GmapBlock* tab = reinterpret_cast<GmapBlock*>(g.d_tab);
+    gm_list_blocks_kernel<<<(g.tab_cap + 255) / 256, 256, 0, c->stream>>>(tab, g.tab_cap, g.d_chunks, g.d_epos, g.d_skeys[0], g.d_svals[0], g.d_actl);
+    count_launch(c);
+    BSHOT_TRY(check_launch("gm_list_blocks_kernel"));
+    // 63-bit keys: 8 passes, the result is back in buffer 0
+    BSHOT_TRY(radix_sort_pairs(c, g.d_skeys, g.d_svals, g.d_shist, g.d_actl, std::min<size_t>(g.tab_cap, nt_cap), 8));
+    gm_block_offsets_kernel<<<1, 1024, 0, c->stream>>>(tab, g.d_svals[0], g.d_boff, g.d_actl);
+    gm_collect_kernel<<<(unsigned)c->sm_count * 2u, 128, 0, c->stream>>>(tab, g.d_svals[0], g.d_boff, g.d_actl, g.d_chunks, g.d_epos, g.d_edesc, g.d_apos,
+                                                                        g.d_adesc, g.max_entries);
+    count_launch(c, 2);
+    return check_launch("map gather-all kernels");
+}
+
+int gmap_export(Ctx* c, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t* n_out) {
+    Gmap& g = c->gmap;
+    size_t nt_cap;
+    BSHOT_TRY(gmap_gather_all(c, &nt_cap));
+    unsigned* h = reinterpret_cast<unsigned*>(&c->h_scratch[48]);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(h, g.d_actl, sizeof(unsigned) * 4, cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    const size_t n = h[1], m = std::min(n, cap);
+    if (n_out) *n_out = n;
+    if (xyzr_out && m) BSHOT_CUDA_TRY(cudaMemcpyAsync(xyzr_out, g.d_apos, sizeof(float4) * m, cudaMemcpyDeviceToHost, c->stream));
+    if (desc_out && m) BSHOT_CUDA_TRY(cudaMemcpyAsync(desc_out, g.d_adesc, 48 * m, cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    if (n > cap) { set_error("bshot_gmap_export: %zu entries > capacity %zu", n, cap); return BSHOT_E_CAPACITY; }
+    return BSHOT_OK;
+}
+
+int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n) {
+    Gmap& g = c->gmap;
+    if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
+    BSHOT_TRY(gmap_reset(c));
+    g.entries_upper = 0;
+    if (n > g.max_entries) {
+        BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+        set_error("bshot_gmap_import: %zu entries > max_entries %u", n, g.max_entries);
+        return BSHOT_E_CAPACITY;
+    }
+    if (n == 0) { BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream)); return BSHOT_OK; }
+    BSHOT_TRY(gmap_all_alloc(c));
+    const unsigned nn = (unsigned)n;
+    GmapBlock* tab = reinterpret_cast<GmapBlock*>(g.d_tab);
+    BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_actl, 0, sizeof(unsigned) * 8, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_epos, xyzr, sizeof(float4) * n, cudaMemcpyHostToDevice, c->stream));
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_edesc, desc, 48 * n, cudaMemcpyHostToDevice, c->stream));
+    gm_import_find_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_epos, nn, tab, g.tab_cap - 1, g.d_skeys[0], g.d_svals[0], g.d_actl);
+    count_launch(c);
+    BSHOT_TRY(check_launch("gm_import_find_kernel"));
+    // stable by slot: the input order survives inside a block.  Slots are < tab_cap (a power of two)
+    unsigned bits = 0;
+    while ((1u << bits) < g.tab_cap) ++bits;
+    const unsigned passes = (bits + 7) / 8;
+    BSHOT_TRY(radix_sort_pairs(c, g.d_skeys, g.d_svals, g.d_shist, g.d_actl + 3, n, passes));
+    gm_import_blocks_kernel<<<1, 1024, 0, c->stream>>>(tab, g.tab_cap, g.d_boff, g.d_ctl, g.d_actl, g.max_chunks);
+    gm_import_chain_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_skeys[passes & 1], g.d_svals[passes & 1], nn, tab, g.tab_cap, g.d_boff, g.d_chunks,
+                                                                    g.max_chunks);
+    count_launch(c, 2);
+    BSHOT_TRY(check_launch("map import kernels"));
+    unsigned* h = reinterpret_cast<unsigned*>(&c->h_scratch[48]);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(h, g.d_actl, sizeof(unsigned) * 4, cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    if (h[2]) {
+        const int rc = (h[2] & 1u) ? BSHOT_E_INVALID : BSHOT_E_CAPACITY;
+        BSHOT_TRY(gmap_reset(c));
+        BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+        if (rc == BSHOT_E_INVALID) set_error("bshot_gmap_import: non-finite position");
+        else set_error("bshot_gmap_import: more blocks or chunks than the map holds (%u slots, %u chunks)", g.tab_cap, g.max_chunks);
+        return rc;
+    }
+    g.entries_upper = n;
+    return BSHOT_OK;
 }
 
 }  // namespace bshot

@@ -10,7 +10,13 @@
 // max_targets is detected on the device (the host call's test, on device counts): the flag makes RANSAC and ICP no-ops and
 // keeps the pose, the map and the reference frame as they were.  Compiled with -fmad=false: the gate and the composition
 // T_best = F * T_est give the host's bits.
+//
+// Relocalisation (relocalize_run) reuses the same stages without a prior pose: the whole map in map order is the target
+// set (gmap_gather_all), RANSAC and ICP (around T_ransac) run as in the step, and the step's tail -- pose, status, map
+// update, reference frame -- runs only when enough inliers survived; one device flag skips it otherwise.
+#include <algorithm>
 #include <cmath>
+#include <cstddef>
 
 #include "common.cuh"
 #include "odom_math.cuh"
@@ -22,6 +28,9 @@ struct OdomDev {
     bshot_odom_report rep;   // copied to the host at the end of a step, together with err
     int err;                 // BSHOT_E_* raised on the device during the step (0 = none)
     int eff_count;           // keypoints the map update takes: the frame's count, 0 after an error
+    int reject;              // relocalisation: not accepted (or an error), skips the tail like err skips the step's
+    int pad;
+    bshot_reloc_report rrep; // copied to the host at the end of a relocalisation, together with err and reject
     float pose[16];          // pose of the last successful step, row-major (identity after a reset)
     float T_est[16];
     float T_ransac[16];
@@ -30,7 +39,7 @@ struct OdomDev {
 
 __global__ void odom_reset_kernel(OdomDev* d) {
     if (threadIdx.x < 16) d->pose[threadIdx.x] = (threadIdx.x % 5 == 0) ? 1.0f : 0.0f;
-    if (threadIdx.x == 0) d->err = 0;
+    if (threadIdx.x == 0) { d->err = 0; d->reject = 0; }
 }
 
 // bshot_match_frame_to_map's capacity test on the device counts
@@ -67,6 +76,35 @@ __global__ void odom_final_kernel(OdomDev* d, const IcpState* __restrict__ icp, 
     r.icp_iterations = run_icp ? icp->iterations : 0;
     r.was_initial = was_initial;
     if (d->err == 0) {
+        for (int e = 0; e < 16; ++e) d->pose[e] = T_best[e];
+        d->eff_count = *kp_count;
+    } else {
+        d->eff_count = 0;
+    }
+}
+
+// relocalisation: T_best, the report, accepted; when accepted the new pose, the status flag and the map update's count
+__global__ void reloc_final_kernel(OdomDev* d, const IcpState* __restrict__ icp, int run_icp, int min_inliers, const int* __restrict__ kp_count,
+                                   const int* __restrict__ pair_count, const unsigned* __restrict__ n_map, const unsigned* __restrict__ n_icp, int k,
+                                   unsigned long long n_points) {
+    float T_best[16];
+    if (run_icp) mul4x4(icp->final_T, d->T_ransac, T_best);
+    else for (int e = 0; e < 16; ++e) T_best[e] = d->T_ransac[e];
+    bshot_reloc_report& r = d->rrep;
+    for (int e = 0; e < 16; ++e) { r.pose[e] = T_best[e]; r.T_ransac[e] = d->T_ransac[e]; }
+    const int nk = min(max(*kp_count, 0), k);
+    r.n_points = (size_t)n_points;
+    r.n_map = (size_t)*n_map;
+    r.n_icp_targets = run_icp ? (size_t)*n_icp : 0;
+    r.n_keypoints = nk;
+    r.n_pairs = min(max(*pair_count, 0), k);
+    r.n_inliers = d->n_inliers;
+    r.ransac_iterations = d->ransac_iterations;
+    r.icp_iterations = run_icp ? icp->iterations : 0;
+    const bool accepted = d->err == 0 && d->n_inliers >= min_inliers;
+    r.accepted = accepted ? 1 : 0;
+    d->reject = accepted ? 0 : 1;
+    if (accepted) {
         for (int e = 0; e < 16; ++e) d->pose[e] = T_best[e];
         d->eff_count = *kp_count;
     } else {
@@ -173,6 +211,64 @@ int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_
     c->n_prev = k;
     o.run = true;
     if (out) *out = h->rep;
+    return BSHOT_OK;
+}
+
+// relocalisation: the step's extraction, the whole map as the target set, RANSAC, ICP against the map around T_ransac,
+// acceptance by inlier count, and -- when accepted -- the step's tail.  One copy back (report + flags) at the end
+int relocalize_run(Ctx* c, const bshot_odom_params* p, int min_inliers, const float* d_cloud, size_t n, int stride_floats, bshot_reloc_report* out) {
+    BSHOT_TRY(odom_ensure(c));
+    Odom& o = c->odom;
+    Gmap& g = c->gmap;
+    OdomDev* d = o.d;
+    BSHOT_TRY(frame_extract(c, &p->front, d_cloud, n, stride_floats));
+    const size_t k = (size_t)p->front.top_k;
+    BSHOT_CUDA_TRY(cudaMemsetAsync(&d->err, 0, sizeof(int), c->stream));
+    const unsigned* d_nq = reinterpret_cast<const unsigned*>(c->d_kp_count);
+    // targets: every map entry in map order (no reference frame)
+    size_t nm_cap;
+    BSHOT_TRY(gmap_gather_all(c, &nm_cap));
+    const unsigned* d_nm = g.d_actl + 1;
+    if (nm_cap == 0) {
+        BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_pair_count, 0, sizeof(int), c->stream));
+    } else {
+        BSHOT_TRY(hamming_match_rq(c, c->d_bits, k, g.d_adesc, nm_cap, 0, c->d_cand, d_nq, d_nm));
+        BSHOT_TRY(hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq));
+    }
+    BSHOT_TRY(ransac_run_dev(c, c->d_kp, g.d_apos, c->d_pairs, 3, c->d_pair_count, k, p->ransac_iterations, (double)p->inlier_threshold, o.d_inlier_pairs,
+                             &d->n_inliers, d->T_ransac, &d->ransac_iterations, nullptr));
+    if (p->run_icp) {   // map keypoints within map_range of T_ransac's translation ([R|T] = its first 12 floats)
+        BSHOT_TRY(gmap_gather(c, nullptr, p->map_range, nullptr, nullptr, nullptr, 0, d->T_ransac, c->d_t, c->max_targets, g.d_ctl + 6,
+                              /*pose_on_device=*/true));
+        odom_check_kernel<<<1, 1, 0, c->stream>>>(g.d_ctl, 0, c->max_targets, d);
+        count_launch(c);
+        const size_t nt_cap = std::min(c->max_targets, g.entries_upper);
+        BSHOT_TRY(icp_run_dev(c, reinterpret_cast<const float*>(c->d_kp), 4, c->d_kp_count, k, reinterpret_cast<const float*>(g.d_tpos), 4, g.d_ctl + 6, nt_cap,
+                              d->T_ransac, 10, &d->err, o.d_icp_cur, o.d_icp_tgt, o.d_icp_keys, o.d_icp_state));
+    }
+    reloc_final_kernel<<<1, 1, 0, c->stream>>>(d, o.d_icp_state, p->run_icp ? 1 : 0, min_inliers, c->d_kp_count, c->d_pair_count, d_nm, g.d_ctl + 6, (int)k,
+                                               (unsigned long long)n);
+    count_launch(c);
+    BSHOT_TRY(check_launch("relocalisation kernels"));
+    // the step's tail; not accepted: the count is 0 and the reference frame is skipped
+    BSHOT_TRY(gmap_update(c, c->d_kp, c->d_kp_ratio, c->d_bits, &d->eff_count, c->last_top_k, d->pose, /*pose_on_device=*/true));
+    BSHOT_TRY(frame_commit(c, k, &d->reject));
+    OdomDev* h = reinterpret_cast<OdomDev*>(o.h_out);
+    const size_t first = offsetof(OdomDev, err), last = offsetof(OdomDev, rrep) + sizeof(bshot_reloc_report);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(reinterpret_cast<char*>(h) + first, reinterpret_cast<const char*>(d) + first, last - first, cudaMemcpyDeviceToHost,
+                                   c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    c->n_kp = (size_t)h->rrep.n_keypoints;
+    if (h->err) {
+        set_error("bshot_relocalize: ICP target set exceeds max_targets %zu", c->max_targets);
+        return h->err;
+    }
+    if (h->rrep.accepted) {
+        g.entries_upper += c->last_top_k;
+        c->n_prev = k;
+        o.run = true;
+    }
+    if (out) *out = h->rrep;
     return BSHOT_OK;
 }
 

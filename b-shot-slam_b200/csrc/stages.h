@@ -68,6 +68,19 @@ int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t
                 bool pose_on_device = false);
 int gmap_gather(Ctx* c, const float pos[3], float range, const float4* d_ref_kp, const uint64_t* d_ref_bits, const int* d_ref_count,
                 size_t ref_cap, const float* ref_pose12, uint64_t* d_t_out, size_t out_cap, unsigned* d_total, bool pose_on_device = false);
+// the whole map in map order (occupied blocks in ascending lattice coordinates, x outermost, entries in insertion order) ->
+// gmap.d_apos / d_adesc, the count in gmap.d_actl[1]; *nt_cap_out = its host-side bound.  Asynchronous
+int gmap_gather_all(Ctx* c, size_t* nt_cap_out);
+// synchronous: export copies min(count, cap) records (float4 position + seg-ratio, 48-byte descriptor); import replaces
+// the map by n entries without the admission rule, keeping the input order inside each block (an empty map on any error)
+int gmap_export(Ctx* c, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t* n_out);
+int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n);
+
+// stable LSD radix sort of (u64 key, u32 value) pairs, 8 bits a pass (voxel_grid.cu): *d_m pairs (at most m_cap) in
+// keys[0] / vals[0], `passes` passes from the low byte up; the result is in keys[passes & 1] / vals[passes & 1].  hist
+// holds radix_hist_words(m_cap) words
+size_t radix_hist_words(size_t m_cap);
+int radix_sort_pairs(Ctx* c, unsigned long long* keys[2], unsigned* vals[2], unsigned* hist, const unsigned* d_m, size_t m_cap, unsigned passes);
 
 // RANSAC correspondence rejection (ransac.cu).  ransac_run draws PCL's sample sequence on the host, ransac_run_dev on the
 // device; after the sampler both run the same device tail (scoring, adaptive stop, inlier flags, ordered compaction).
@@ -117,6 +130,8 @@ int odom_ensure(Ctx* c);
 void odom_free(Ctx* c);
 int odometry_reset(Ctx* c);
 int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_t n, int stride_floats, bshot_odom_report* out);
+// relocalisation against the whole map (odometry.cu); the same shape as odometry_run
+int relocalize_run(Ctx* c, const bshot_odom_params* p, int min_inliers, const float* d_cloud, size_t n, int stride_floats, bshot_reloc_report* out);
 
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);

@@ -7,7 +7,7 @@
 //   bbox      tiles of 1024 points: bbox of the finite points + finite count per tile; the last CTA derives inv-leaf
 //             bins, multipliers, PCL's overflow test and the number of significant key bits (-> radix passes)
 //   key       finite points -> (voxel index, point index), compacted in index order
-//   4 x (hist, scatter)  stable LSD radix sort of the voxel indices, 8 bits a pass; passes beyond the significant bits
+//   4 x (rx_hist, rx_scatter)  stable LSD radix sort of the voxel indices, 8 bits a pass; passes beyond the significant bits
 //             return at once, so the pass count costs no host round trip
 //   heads, seg  first sorted position of every voxel (voxel count on the device)
 //   centroid  one warp per voxel: the warp gathers 256 points at a time in parallel, then replays the fp32 sums in
@@ -230,13 +230,18 @@ vg_key_kernel(const float* __restrict__ in, unsigned n, int stride, float3 inv, 
     }
 }
 
+// ---- stable LSD radix sort of (key, value) pairs, 8 bits a pass (also the map's sorts, gmap.cu) -----------------------
+// *d_m pairs; a pass at or past *d_npasses (null: never) returns at once, so a pass count decided on the device costs no
+// host round trip.  Pass p reads buffer p & 1 and writes the other.
+
 // radix pass `pass`: 256 digit counts of each RX_TILE tile, hist[tile * 256 + digit]
+template <typename K>
 __global__ void __launch_bounds__(VG_THREADS)
-vg_hist_kernel(const VgParams* __restrict__ P, unsigned pass, const unsigned* __restrict__ keys0, const unsigned* __restrict__ keys1,
-               unsigned* __restrict__ hist) {
-    if (pass >= P->npasses) return;
-    const unsigned m = P->m, sh = 8u * pass;
-    const unsigned* __restrict__ keys = (pass & 1) ? keys1 : keys0;
+rx_hist_kernel(const unsigned* __restrict__ d_m, const unsigned* __restrict__ d_npasses, unsigned pass, const K* __restrict__ keys0,
+               const K* __restrict__ keys1, unsigned* __restrict__ hist) {
+    if (d_npasses && pass >= *d_npasses) return;
+    const unsigned m = *d_m, sh = 8u * pass;
+    const K* __restrict__ keys = (pass & 1) ? keys1 : keys0;
     __shared__ unsigned s[256];
     s[threadIdx.x] = 0;
     __syncthreads();
@@ -244,7 +249,7 @@ vg_hist_kernel(const VgParams* __restrict__ P, unsigned pass, const unsigned* __
 #pragma unroll
     for (int k = 0; k < RX_ITEMS; ++k) {
         const unsigned i = t0 + k * VG_THREADS + threadIdx.x;
-        if (i < m) atomicAdd(&s[(keys[i] >> sh) & 255u], 1u);
+        if (i < m) atomicAdd(&s[(unsigned)(keys[i] >> sh) & 255u], 1u);
     }
     __syncthreads();
     hist[blockIdx.x * 256 + threadIdx.x] = s[threadIdx.x];
@@ -253,14 +258,15 @@ vg_hist_kernel(const VgParams* __restrict__ P, unsigned pass, const unsigned* __
 // radix pass `pass`: stable scatter.  Warp w of a tile owns its items [w * 256, (w + 1) * 256) and takes them 32 at a
 // time in index order; within 32, lanes with the same digit are ranked by lane.  Position = digits before + this
 // digit in earlier tiles + in earlier warps of this tile + earlier in this warp.
+template <typename K>
 __global__ void __launch_bounds__(VG_THREADS)
-vg_scatter_kernel(const VgParams* __restrict__ P, unsigned pass, unsigned* __restrict__ keys0, unsigned* __restrict__ vals0,
-                  unsigned* __restrict__ keys1, unsigned* __restrict__ vals1, const unsigned* __restrict__ hist) {
-    if (pass >= P->npasses) return;
-    const unsigned m = P->m, sh = 8u * pass;
-    const unsigned* __restrict__ kin = (pass & 1) ? keys1 : keys0;
+rx_scatter_kernel(const unsigned* __restrict__ d_m, const unsigned* __restrict__ d_npasses, unsigned pass, K* __restrict__ keys0,
+                  unsigned* __restrict__ vals0, K* __restrict__ keys1, unsigned* __restrict__ vals1, const unsigned* __restrict__ hist) {
+    if (d_npasses && pass >= *d_npasses) return;
+    const unsigned m = *d_m, sh = 8u * pass;
+    const K* __restrict__ kin = (pass & 1) ? keys1 : keys0;
     const unsigned* __restrict__ vin = (pass & 1) ? vals1 : vals0;
-    unsigned* __restrict__ kout = (pass & 1) ? keys0 : keys1;
+    K* __restrict__ kout = (pass & 1) ? keys0 : keys1;
     unsigned* __restrict__ vout = (pass & 1) ? vals0 : vals1;
     __shared__ unsigned s_cnt[RX_WARPS][256];
     __shared__ unsigned s_base[256], s_warp[VG_THREADS / 32];
@@ -275,14 +281,15 @@ vg_scatter_kernel(const VgParams* __restrict__ P, unsigned pass, unsigned* __res
     }
     s_base[d0] = block_excl_scan(tot, s_warp, nullptr) + pre;  // its __syncthreads also orders the zeroing above
     const unsigned lt = (1u << lane) - 1u;
-    unsigned key[RX_ITEMS], val[RX_ITEMS], dig[RX_ITEMS], loc[RX_ITEMS];
+    K key[RX_ITEMS];
+    unsigned val[RX_ITEMS], dig[RX_ITEMS], loc[RX_ITEMS];
     const unsigned w0 = blockIdx.x * RX_TILE + wid * (32 * RX_ITEMS);
 #pragma unroll
     for (int r = 0; r < RX_ITEMS; ++r) {
         const unsigned i = w0 + r * 32 + lane;
-        key[r] = i < m ? kin[i] : 0u;
+        key[r] = i < m ? kin[i] : (K)0;
         val[r] = i < m ? vin[i] : 0u;
-        dig[r] = i < m ? (key[r] >> sh) & 255u : 256u;
+        dig[r] = i < m ? (unsigned)(key[r] >> sh) & 255u : 256u;
         const unsigned peers = __match_any_sync(0xffffffffu, dig[r]);
         const unsigned old = dig[r] < 256u ? s_cnt[wid][dig[r]] : 0u;
         __syncwarp();
@@ -306,6 +313,24 @@ vg_scatter_kernel(const VgParams* __restrict__ P, unsigned pass, unsigned* __res
         kout[pos] = key[r];
         vout[pos] = val[r];
     }
+}
+
+template <typename K>
+static int radix_sort_launch(Ctx* c, K* keys[2], unsigned* vals[2], unsigned* hist, const unsigned* d_m, const unsigned* d_npasses, size_t m_cap,
+                             unsigned passes) {
+    const unsigned rtiles = (unsigned)std::max<size_t>((m_cap + RX_TILE - 1) / RX_TILE, 1);
+    for (unsigned pass = 0; pass < passes; ++pass) {
+        rx_hist_kernel<K><<<rtiles, VG_THREADS, 0, c->stream>>>(d_m, d_npasses, pass, keys[0], keys[1], hist);
+        rx_scatter_kernel<K><<<rtiles, VG_THREADS, 0, c->stream>>>(d_m, d_npasses, pass, keys[0], vals[0], keys[1], vals[1], hist);
+    }
+    count_launch(c, 2 * passes);
+    return check_launch("radix sort");
+}
+
+size_t radix_hist_words(size_t m_cap) { return 256 * std::max<size_t>((m_cap + RX_TILE - 1) / RX_TILE, 1); }
+
+int radix_sort_pairs(Ctx* c, unsigned long long* keys[2], unsigned* vals[2], unsigned* hist, const unsigned* d_m, size_t m_cap, unsigned passes) {
+    return radix_sort_launch<unsigned long long>(c, keys, vals, hist, d_m, nullptr, m_cap, passes);
 }
 
 __device__ __forceinline__ unsigned vg_heads(const unsigned* __restrict__ K, unsigned m, unsigned i0, bool h[4]) {
@@ -458,21 +483,18 @@ int voxel_grid(Ctx* c, const float* xyz, size_t n, int stride_floats, const floa
     if (n == 0) { *count_out = 0; return BSHOT_OK; }
     const unsigned nn = (unsigned)n;
     const float3 iv = make_float3(inv[0], inv[1], inv[2]);
-    const unsigned tiles = (nn + VG_TILE - 1) / VG_TILE, rtiles = (nn + RX_TILE - 1) / RX_TILE;
+    const unsigned tiles = (nn + VG_TILE - 1) / VG_TILE;
     const unsigned cblocks = std::min<unsigned>((nn + RX_WARPS - 1) / RX_WARPS, (unsigned)c->sm_count * 16u);
     VgParams* P = reinterpret_cast<VgParams*>(g.d_ctl);
     cudaStream_t s = c->stream;
     BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_in, xyz, sizeof(float) * stride_floats * n, cudaMemcpyHostToDevice, s));
     vg_bbox_kernel<<<tiles, VG_THREADS, 0, s>>>(g.d_in, nn, stride_floats, iv, P, g.d_tile);
     vg_key_kernel<<<tiles, VG_THREADS, 0, s>>>(g.d_in, nn, stride_floats, iv, P, g.d_tile, g.d_keys[0], g.d_vals[0]);
-    for (unsigned pass = 0; pass < RX_PASSES; ++pass) {
-        vg_hist_kernel<<<rtiles, VG_THREADS, 0, s>>>(P, pass, g.d_keys[0], g.d_keys[1], g.d_hist);
-        vg_scatter_kernel<<<rtiles, VG_THREADS, 0, s>>>(P, pass, g.d_keys[0], g.d_vals[0], g.d_keys[1], g.d_vals[1], g.d_hist);
-    }
+    BSHOT_TRY(radix_sort_launch<unsigned>(c, g.d_keys, g.d_vals, g.d_hist, &P->m, &P->npasses, n, RX_PASSES));
     vg_head_count_kernel<<<tiles, VG_THREADS, 0, s>>>(P, g.d_keys[0], g.d_keys[1], g.d_tile);
     vg_seg_kernel<<<tiles, VG_THREADS, 0, s>>>(P, g.d_keys[0], g.d_keys[1], g.d_tile, g.d_seg);
     vg_centroid_kernel<<<cblocks, VG_THREADS, 0, s>>>(P, g.d_vals[0], g.d_vals[1], g.d_seg, g.d_in, nn, stride_floats, g.d_out);
-    count_launch(c, 5 + 2 * RX_PASSES);
+    count_launch(c, 5);
     BSHOT_TRY(check_launch("voxel_grid"));
     BSHOT_CUDA_TRY(cudaMemcpyAsync(g.h_out, g.d_out, sizeof(float) * (4 + 3 * std::min(cap, n)), cudaMemcpyDeviceToHost, s));
     BSHOT_CUDA_TRY(cudaStreamSynchronize(s));

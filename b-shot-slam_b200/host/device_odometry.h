@@ -2,12 +2,14 @@
 // rotation's velodyne::Laser records go to bshot_odometry_step, which runs the preprocessor, extraction, matching against
 // the map, RANSAC, the gate + ICP, the map update and the reference-frame hand-over on the device and returns the pose.
 // LidarOdometry and its reference-named stage methods stay available for callers that want the stages one by one.
+// relocalize() finds a rotation in the whole map without a prior pose; exportMap / importMap save and restore the map.
 #ifndef BSHOT_B200_HOST_DEVICE_ODOMETRY_H
 #define BSHOT_B200_HOST_DEVICE_ODOMETRY_H
 
 #include <vector>
 
 #include "../../include/bshot_b200.h"
+#include "bshot_bits.h"
 #include "bshot_headers_bits.h"
 #include "preprocess.h"
 
@@ -47,6 +49,44 @@ public:
 
     const bshot_odom_report& report() const { return report_; }
 
+    // relocalisation of one rotation against the whole map (no prior pose): true when at least min_inliers() RANSAC inliers
+    // survived; then pose_ is the new pose and the next step() continues in the map frame.  Otherwise nothing changes.
+    // reloc_report() holds the last report; last_status() / bshot_last_error() say why a call failed
+    bool relocalize(const std::vector<velodyne::Laser>& lasers, const std::vector<double>& ring_deg) {
+        const size_t n = lasers.size();
+        az_.resize(n); vert_.resize(n); dist_.resize(n);
+        for (size_t i = 0; i < n; ++i) { az_[i] = lasers[i].azimuth; vert_[i] = lasers[i].vertical; dist_[i] = lasers[i].distance; }
+        if (!ctx_) return false;
+        bshot_reloc_report r;
+        status_ = bshot_relocalize(ctx_, &params_, min_inliers_, az_.data(), vert_.data(), dist_.data(), n, ring_deg.data(), ring_deg.size(), &r);
+        if (status_ != BSHOT_OK) return false;
+        reloc_report_ = r;
+        if (!r.accepted) return false;
+        for (int row = 0; row < 4; ++row) for (int col = 0; col < 4; ++col) pose_(row, col) = r.pose[4 * row + col];
+        return true;
+    }
+    const bshot_reloc_report& reloc_report() const { return reloc_report_; }
+    int& min_inliers() { return min_inliers_; }
+
+    // the map as arrays: xyzr 4 floats {x, y, z, seg_ratio} per entry, in map order (bshot_gmap_export); importMap puts
+    // such arrays back as they were (bshot_gmap_import).  Both return a BSHOT_* status
+    int exportMap(std::vector<float>& xyzr, std::vector<bshot_descriptor>& desc) {
+        if (!ctx_) return status_;
+        size_t n = 0;
+        status_ = bshot_gmap_export(ctx_, nullptr, nullptr, 0, &n);
+        if (status_ != BSHOT_OK && status_ != BSHOT_E_CAPACITY) return status_;
+        xyzr.resize(4 * n);
+        desc.resize(n);
+        status_ = bshot_gmap_export(ctx_, xyzr.data(), reinterpret_cast<uint64_t*>(desc.data()), n, &n);
+        return status_;
+    }
+    int importMap(const std::vector<float>& xyzr, const std::vector<bshot_descriptor>& desc) {
+        if (!ctx_) return status_;
+        if (xyzr.size() != 4 * desc.size()) return status_ = BSHOT_E_INVALID;
+        status_ = bshot_gmap_import(ctx_, xyzr.data(), reinterpret_cast<const uint64_t*>(desc.data()), desc.size());
+        return status_;
+    }
+
     // INITIAL status, identity pose, empty map, no reference frame
     int reset() {
         if (ctx_) status_ = bshot_odometry_reset(ctx_);
@@ -62,6 +102,8 @@ private:
     bshot_ctx* ctx_ = nullptr;
     bshot_odom_params params_;
     bshot_odom_report report_ = bshot_odom_report();
+    bshot_reloc_report reloc_report_ = bshot_reloc_report();
+    int min_inliers_ = 15;   // the gate's own constant (src/lidar_odometry.cpp:269-281)
     Matrix4f pose_ = Matrix4f::Identity();
     int status_ = BSHOT_OK;
     std::vector<double> az_, vert_;

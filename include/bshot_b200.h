@@ -190,6 +190,18 @@ int bshot_match_frame_to_map(bshot_ctx* ctx, const float ref_pos[3], float range
                              int* n_pairs_out, size_t* n_targets_out, float* target_xyz_out, size_t target_cap);
 /* the frame extracted last becomes the reference frame (passSrc2Ref, src/lidar_odometry.cpp:43-47); asynchronous */
 int bshot_frame_commit(bshot_ctx* ctx);
+/* every map entry in map order: occupied blocks in ascending lattice coordinates (x outermost, z innermost, as
+ * bshot_gmap_get_keypoints visits them), entries of a block in insertion order.  Unlike bshot_gmap_get_keypoints it is
+ * not limited by a probe budget.  xyzr_out cap x 4 floats {x, y, z, seg_ratio}, desc_out cap x 6 u64 (either may be NULL);
+ * *n_out = entries.  count > cap: the first cap are written and BSHOT_E_CAPACITY is returned.  Needs bshot_gmap_create
+ * (BSHOT_E_STATE). */
+int bshot_gmap_export(bshot_ctx* ctx, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t* n_out);
+/* replaces the map by these n entries (layout of bshot_gmap_export), without the admission rule: entries of one block keep
+ * their relative order in the input, so a bshot_gmap_export result restores the map it came from and every later call
+ * behaves as on the exporting context.  Positions are stored as given.  Non-finite x, y or z: BSHOT_E_INVALID;
+ * n > max_entries, or more blocks / chunks than the table holds: BSHOT_E_CAPACITY.  On any error the map is empty.
+ * The pose, the status and the reference frame of the odometry step are not touched. */
+int bshot_gmap_import(bshot_ctx* ctx, const float* xyzr, const uint64_t* desc, size_t n);
 
 /* ---- RANSAC correspondence rejection (the consumer of the path's output) ----------------------------------------------------
  * Replaces Ransac_based_Rejection.setMaximumIterations(2000) / setInputSource / setInputTarget / setInlierThreshold(1500) /
@@ -294,6 +306,32 @@ int bshot_odometry_step_cloud(bshot_ctx* ctx, const bshot_odom_params* p, const 
 /* INITIAL status, identity pose, empty map, no reference frame, fresh persistent normals: the next step replays the
  * sequence as a new context would */
 int bshot_odometry_reset(bshot_ctx* ctx);
+
+/* ---- relocalisation: a scan against the whole map, without a prior pose ----------------------------------------------
+ * The scan is extracted as by the step (p->front), then its descriptors are matched against EVERY map entry in map order
+ * (bshot_gmap_export's order; the reference frame is not a target): mutual nearest neighbours, the matcher chosen by size
+ * (the tensor-core pipeline above 2^21 pairs) -> RANSAC (p->ransac_iterations, p->inlier_threshold; sources the keypoints
+ * in the sensor frame, targets the entries' positions) -> T_ransac, sensor to map.  p->run_icp: ICP (10 iterations,
+ * pre = T_ransac) against the map keypoints within p->map_range of T_ransac's translation, T_best = ICP * T_ransac.
+ * accepted = n_inliers >= min_inliers (no heading / translation gate: there is no prior pose; 15 is the gate's own
+ * constant).  When accepted, the step's tail runs unchanged: the stored pose becomes T_best, the status RUN, the map is
+ * updated with the frame at T_best and the frame becomes the reference frame, so the next bshot_odometry_step continues
+ * in the map frame.  When not, pose, status, map and reference frame stay as they were (the extraction's cross-frame
+ * front-end state, the persistent normals, moves on as after any extraction).
+ * Errors: no map BSHOT_E_STATE; min_inliers < 3 BSHOT_E_INVALID; an ICP target set larger than max_targets
+ * BSHOT_E_CAPACITY, with the state unchanged.  An empty map is no error: accepted = 0.  After the preprocessor's count
+ * read-backs nothing goes back to the host but the report. */
+typedef struct bshot_reloc_report {
+    float pose[16];             /* T_best = ICP * T_ransac (T_ransac without ICP), row-major; adopted when accepted */
+    float T_ransac[16];
+    size_t n_points, n_map, n_icp_targets;   /* preprocessed points; map entries searched; ICP targets */
+    int n_keypoints, n_pairs, n_inliers, ransac_iterations, icp_iterations, accepted;
+} bshot_reloc_report;
+/* raw returns (as bshot_odometry_step) / a preprocessed host cloud (as bshot_odometry_step_cloud); out may be NULL */
+int bshot_relocalize(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const double* azimuth_deg, const double* vertical_deg,
+                     const unsigned short* distance, size_t n, const double* ring_deg, size_t nv, bshot_reloc_report* out);
+int bshot_relocalize_cloud(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const float* xyz, size_t n, size_t stride_bytes,
+                           bshot_reloc_report* out);
 /* bshot_ransac on device buffers, asynchronous on the context stream: d_src4 / d_tgt4 float4 points (x, y, z, any),
  * d_pairs n_pairs_cap x 2 ints (index into src, index into tgt; every valid one must be in range), *d_n_pairs (int) of
  * them valid.  Outputs (device): d_inlier_pairs_out (n_pairs_cap x 2 ints), *d_n_inliers_out (int), d_transform_out
