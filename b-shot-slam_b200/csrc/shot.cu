@@ -10,6 +10,7 @@
 //            per neighbour), fp64 intermediates like PCL
 //   phase D  L2 normalisation, optional float output, 88 nibbles -> packed 352-bit record
 // The float histogram never has to touch HBM when only the bits are wanted.
+#include <math.h>
 #include <stdlib.h>
 
 #include "eigh3.cuh"
@@ -116,7 +117,7 @@ template <int SH_THREADS>
 __global__ void __launch_bounds__(SH_THREADS, (SH_THREADS == 128) ? BSHOT_SH_MINBLOCKS : 1)
 shot_kernel(const GridParams* __restrict__ gp, const unsigned* __restrict__ cell_start,
             const float4* __restrict__ sorted, const float4* __restrict__ kp, const int* __restrict__ kp_count,
-            const float4* __restrict__ normals, unsigned normals_limit, float radius, int lrf_only,
+            const float4* __restrict__ normals, unsigned normals_limit, float radius, float r2_4, int lrf_only,
             float* __restrict__ rf_out, int* __restrict__ nn_out, float* __restrict__ shot_out,
             uint64_t* __restrict__ bits_out, unsigned long long* __restrict__ sum_nn, const unsigned* __restrict__ order) {
     __shared__ ShotSmem sm;
@@ -454,7 +455,7 @@ shot_kernel(const GridParams* __restrict__ gp, const unsigned* __restrict__ cell
         // error 1e-7 against a grid of ~4e-6).  Saves the fp64 sqrt and five fp64 divisions per neighbour.
         const float r12 = (float)radius1_2, r34 = (float)radius3_4, r14 = (float)radius1_4;
         const float inv_r12 = 1.0f / r12;
-        const float R2_4 = (float)(((double)R * (double)R) / 4.0);  // distance > R/2  <=>  sqd > R^2/4 (exact for fp32 sqd)
+        // distance > R/2  <=>  sqd > r2_4, exact for an fp32 sqd: r2_4 is R^2/4 rounded DOWN (shell_threshold)
         const float F_45 = (float)RAD_45, F_135 = (float)RAD_135, F_78 = (float)RAD_PI_7_8;
         const float INV_90 = (float)(1.0 / RAD_90), INV_45 = (float)(1.0 / RAD_45);
         for_each([&](const float4 p) {
@@ -484,7 +485,7 @@ shot_kernel(const GridParams* __restrict__ gp, const unsigned* __restrict__ cell
             if (same_sign || (xr == 0.0f)) desc_index += (fabsf(xr) >= fabsf(yr)) ? 0 : 4;
             else desc_index += (fabsf(xr) > fabsf(yr)) ? 4 : 0;
             desc_index += zr > 0.0f ? 1 : 0;
-            const bool outer = sqd > R2_4;
+            const bool outer = sqd > r2_4;
             desc_index += outer ? 2 : 0;
             const int step_index = (int)floor(bin + 0.5);
             const int volume_index = desc_index * 11;
@@ -665,6 +666,17 @@ shot_order_kernel(const float4* __restrict__ kp, const int* __restrict__ kp_coun
     }
 }
 
+// The half-radius shell test, distance > R/2, as a test on the fp32 squared distance: sqd > R^2/4.  R^2/4 is exact in
+// double; the largest float not above it makes `sqd > threshold` exact for every fp32 sqd.  Rounding to nearest instead
+// can round up, and a neighbour with sqd equal to that value would land in the inner shell where PCL puts it in the outer.
+// Passed as a kernel parameter: the comparison reads it from the constant bank and holds no register in the vote loop.
+static float shell_threshold(float radius) {
+    const double q = ((double)radius * (double)radius) / 4.0;
+    float t = (float)q;
+    if ((double)t > q) t = nextafterf(t, 0.0f);
+    return t;
+}
+
 int shot_compute(Ctx* c, float radius, bool lrf_only, bool write_shot) {
     const size_t k = c->n_kp;
     if (k == 0) return BSHOT_OK;
@@ -678,10 +690,11 @@ int shot_compute(Ctx* c, float radius, bool lrf_only, bool write_shot) {
         count_launch(c);
         order = c->d_shot_order;
     }
+    const float r2_4 = shell_threshold(radius);
     static const int nthreads = [] { const char* e = getenv("BSHOT_SHOT_THREADS"); const int v = e ? atoi(e) : 128; return (v == 64 || v == 128 || v == 256) ? v : 128; }();
 #define BSHOT_LAUNCH_SHOT(NT)                                                                                              \
     shot_kernel<NT><<<(unsigned)k, NT, 0, c->stream>>>(c->d_grid, c->d_cell_start, c->d_sorted, c->d_kp, c->d_kp_count,   \
-                                                      c->d_normals, limit, radius, lrf_only ? 1 : 0, c->d_rf, c->d_nn,   \
+                                                      c->d_normals, limit, radius, r2_4, lrf_only ? 1 : 0, c->d_rf, c->d_nn, \
                                                       write_shot ? c->d_shot : nullptr, c->d_bits, c->d_sum_nn, order)
     if (nthreads == 64) BSHOT_LAUNCH_SHOT(64);
     else if (nthreads == 256) BSHOT_LAUNCH_SHOT(256);
