@@ -5,7 +5,12 @@
 // assembled target keypoints with PCL's defaults, i.e. PCL 1.8's loop
 //   * correspondences: the nearest target of every (moved) source point, exact, squared distance in float (FLANN L2_Simple:
 //     ((dx*dx) + dy*dy) + dz*dz), no distance cap (sqrt(DBL_MAX)), no rejectors; ties -> lowest target index;
-//   * transformation: TransformationEstimationSVD<.., float> = Umeyama without scaling on all pairs, float sums;
+//   * transformation: TransformationEstimationSVD<.., float> = Umeyama without scaling on all pairs, float sums; pcl::umeyama's
+//     rank rule (float precision): rank 3 -> S(2) = sign(det Sigma), rank 2 -> right-handed completion.  Rank <= 1 (all
+//     pairs on one target, sources on a line, ...) -> a deterministic proper rotation with R v0 = u0, the identity at rank 0
+//     (rigid_rotation_rank01; rank 0 when sv[0] is within the fp32 rounding noise of Sigma, rigid_noise_floor).  At exact
+//     rank <= 1 PCL's choice depends on Eigen's SVD internals and may be improper; for 0 < sv[1] <= 1e-5 sv[0] PCL keeps
+//     the roll about the line, which this rule drops (DESIGN 3.5);
 //   * the source is moved by it (float 4x4 * point, left to right), final = T * final;
 //   * DefaultConvergenceCriteria as ICP configures it: 10 iterations; rotation threshold 1.0 and translation threshold 0
 //     (transformation_epsilon = 0) -> only an exact identity stops it; |mse - previous mse| < 1e-12; relative mse never
@@ -69,12 +74,27 @@ __device__ __forceinline__ T block_sum(T v, T* sh) {
     return sh[0];
 }
 
+// N sums in one pass of the halving tree: each value is reduced exactly as block_sum reduces it.  sh: N * ICP_T floats
+template <int N>
+__device__ __forceinline__ void block_sum_n(float (&v)[N], float* sh) {
+    const int t = threadIdx.x;
+    __syncthreads();
+    for (int e = 0; e < N; ++e) sh[e * ICP_T + t] = v[e];
+    __syncthreads();
+    for (int s = ICP_T / 2; s > 0; s >>= 1) {
+        if (t < s)
+            for (int e = 0; e < N; ++e) sh[e * ICP_T + t] = sh[e * ICP_T + t] + sh[e * ICP_T + t + s];
+        __syncthreads();
+    }
+    for (int e = 0; e < N; ++e) v[e] = sh[e * ICP_T];
+}
+
 // one CTA: Umeyama over the correspondences, move the source, compose, test convergence, re-arm the keys
 __global__ void __launch_bounds__(ICP_T)
 icp_fit_kernel(float4* __restrict__ cur, unsigned ns, const float4* __restrict__ tgt, unsigned long long* __restrict__ keys, IcpState* __restrict__ st,
                int max_iterations) {
     if (st->done) return;
-    __shared__ float shf[ICP_T];
+    __shared__ float shf[11 * ICP_T];
     __shared__ double shd[ICP_T];
     __shared__ float Rt[16];
     __shared__ int s_stop;
@@ -88,20 +108,25 @@ icp_fit_kernel(float4* __restrict__ cur, unsigned ns, const float4* __restrict__
         return;
     }
     const float one_over_n = 1.0f / (float)n;
-    float sm[3], dm[3];
+    // the centroids, and sum |p|_1, sum |q|_1 for the rank-0 noise floor
+    float sm[3], dm[3], abs_pq[2];
     {
-        float a[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        float a[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
         for (unsigned i = t; i < ns; i += ICP_T) {
             const unsigned long long k = keys[i];
             if (k == ~0ull) continue;
             const float4 p = cur[i], q = tgt[(unsigned)k];
             a[0] += p.x; a[1] += p.y; a[2] += p.z; a[3] += q.x; a[4] += q.y; a[5] += q.z;
+            a[6] += (fabsf(p.x) + fabsf(p.y)) + fabsf(p.z); a[7] += (fabsf(q.x) + fabsf(q.y)) + fabsf(q.z);
         }
-        for (int c = 0; c < 3; ++c) { sm[c] = block_sum(a[c], shf) * one_over_n; dm[c] = block_sum(a[3 + c], shf) * one_over_n; }
+        block_sum_n(a, shf);
+        for (int c = 0; c < 3; ++c) { sm[c] = a[c] * one_over_n; dm[c] = a[3 + c] * one_over_n; }
+        abs_pq[0] = a[6]; abs_pq[1] = a[7];
     }
-    float sigma[9];
+    // the cross-covariance, and sum |s|_1, sum |d|_1 of the centred points
+    float sigma[9], abs_sd[2];
     {
-        float a[9] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+        float a[11] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
         for (unsigned i = t; i < ns; i += ICP_T) {
             const unsigned long long k = keys[i];
             if (k == ~0ull) continue;
@@ -109,8 +134,11 @@ icp_fit_kernel(float4* __restrict__ cur, unsigned ns, const float4* __restrict__
             const float s[3] = {p.x - sm[0], p.y - sm[1], p.z - sm[2]}, d[3] = {q.x - dm[0], q.y - dm[1], q.z - dm[2]};
             for (int r = 0; r < 3; ++r)
                 for (int c = 0; c < 3; ++c) a[3 * r + c] += d[r] * s[c];
+            a[9] += (fabsf(s[0]) + fabsf(s[1])) + fabsf(s[2]); a[10] += (fabsf(d[0]) + fabsf(d[1])) + fabsf(d[2]);
         }
-        for (int e = 0; e < 9; ++e) sigma[e] = one_over_n * block_sum(a[e], shf);
+        block_sum_n(a, shf);
+        for (int e = 0; e < 9; ++e) sigma[e] = one_over_n * a[e];
+        abs_sd[0] = a[9]; abs_sd[1] = a[10];
     }
     double mse_sum = 0.0;
     for (unsigned i = t; i < ns; i += ICP_T) {
@@ -123,14 +151,24 @@ icp_fit_kernel(float4* __restrict__ cur, unsigned ns, const float4* __restrict__
         for (int e = 0; e < 9; ++e) sg[e] = (double)sigma[e];
         svd3_hestenes(sg, U, sv, V);
         const double det = sg[0] * (sg[4] * sg[8] - sg[5] * sg[7]) - sg[1] * (sg[3] * sg[8] - sg[5] * sg[6]) + sg[2] * (sg[3] * sg[7] - sg[4] * sg[6]);
-        double sgn = 1.0;
-        if (sv[2] <= sv[0] * 1e-5) {  // rank <= 2 (isMuchSmallerThan, float precision): right-handed completion, R = U V^T
-            U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
-            V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
-        } else if (det < 0) sgn = -1.0;   // S(2) = -1
+        // rank = number of singular values not much smaller than sv[0] (isMuchSmallerThan, float precision 1e-5); rank 0
+        // when sv[0] is within the fp32 rounding noise of Sigma (rigid_noise_floor)
+        const double floor0 = rigid_noise_floor((double)abs_pq[0], (double)abs_pq[1], (double)abs_sd[0], (double)abs_sd[1], (double)n,
+                                                (double)((n + ICP_T - 1) / ICP_T + 8), 5.9604644775390625e-08);
+        double Rd[9];
+        const bool rank0 = sv[0] <= floor0;
+        if (rank0 || sv[1] <= sv[0] * 1e-5) rigid_rotation_rank01(U, V, rank0, Rd);   // rank <= 1: see rigid_math.cuh (DESIGN 3.5)
+        else {
+            double sgn = 1.0;
+            if (sv[2] <= sv[0] * 1e-5) {  // rank 2: right-handed completion, R = U V^T
+                U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
+                V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
+            } else if (det < 0) sgn = -1.0;   // rank 3: S(2) = -1
+            for (int r = 0; r < 3; ++r)
+                for (int c = 0; c < 3; ++c) Rd[3 * r + c] = (U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + sgn * (U[3 * r + 2] * V[3 * c + 2]);
+        }
         float R[9];
-        for (int r = 0; r < 3; ++r)
-            for (int c = 0; c < 3; ++c) R[3 * r + c] = (float)((U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + sgn * (U[3 * r + 2] * V[3 * c + 2]));
+        for (int e = 0; e < 9; ++e) R[e] = (float)Rd[e];
         for (int r = 0; r < 3; ++r) {
             Rt[4 * r] = R[3 * r]; Rt[4 * r + 1] = R[3 * r + 1]; Rt[4 * r + 2] = R[3 * r + 2];
             Rt[4 * r + 3] = dm[r] - ((R[3 * r] * sm[0] + R[3 * r + 1] * sm[1]) + R[3 * r + 2] * sm[2]);

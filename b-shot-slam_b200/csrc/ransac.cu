@@ -28,8 +28,11 @@
 namespace bshot {
 
 // Umeyama without scaling for three point pairs (pcl::umeyama / Eigen::umeyama, with_scaling = false), double in, float
-// 4x4 row-major out.  rank 2 (three non-collinear points): the third columns of U and V are completed as cross products,
-// so both bases are right handed and R = U V^T is the proper rotation that Eq. (40)-(43) select.
+// 4x4 row-major out.  Three pairs give rank <= 2 (pcl::umeyama counts it at double precision, 1e-12).  Rank 2: the third
+// columns of U and V are completed as cross products, so both bases are right handed and R = U V^T is the proper rotation
+// that Eq. (40)-(43) select.  Rank <= 1 (collinear source or target triples, coincident targets): a deterministic proper
+// rotation with R v0 = u0, the identity at rank 0 (rigid_rotation_rank01); PCL's choice there depends on Eigen's SVD
+// internals and may be improper (DESIGN 3.5).
 __host__ __device__ inline void umeyama3(const double src[3][3], const double dst[3][3], float T[16]) {
     double sm[3], dm[3];
     for (int c = 0; c < 3; ++c) { sm[c] = (src[0][c] + src[1][c] + src[2][c]) / 3.0; dm[c] = (dst[0][c] + dst[1][c] + dst[2][c]) / 3.0; }
@@ -42,12 +45,22 @@ __host__ __device__ inline void umeyama3(const double src[3][3], const double ds
         }
     double U[9], s[3], V[9];
     svd3_hestenes(sigma, U, s, V);
-    // complete the last columns to right-handed bases (rank <= 2 for three points)
-    U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
-    V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
+    // rank 0: s0 within the double rounding noise of Sigma (coincident targets whose mean does not round back to them)
+    double abs_s = 0.0, abs_d = 0.0, abs_p = 0.0, abs_q = 0.0;
+    for (int i = 0; i < 3; ++i)
+        for (int c = 0; c < 3; ++c) {
+            abs_p += fabs(src[i][c]); abs_q += fabs(dst[i][c]); abs_s += fabs(src[i][c] - sm[c]); abs_d += fabs(dst[i][c] - dm[c]);
+        }
+    const bool rank0 = s[0] <= rigid_noise_floor(abs_p, abs_q, abs_s, abs_d, 3.0, 3.0, 1.1102230246251565e-16);
     double R[9];
-    for (int r = 0; r < 3; ++r)
-        for (int c = 0; c < 3; ++c) R[3 * r + c] = (U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + U[3 * r + 2] * V[3 * c + 2];
+    if (rank0 || s[1] <= s[0] * 1e-12) rigid_rotation_rank01(U, V, rank0, R);
+    else {
+        // complete the last columns to right-handed bases (rank 2)
+        U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
+        V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
+        for (int r = 0; r < 3; ++r)
+            for (int c = 0; c < 3; ++c) R[3 * r + c] = (U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + U[3 * r + 2] * V[3 * c + 2];
+    }
     for (int r = 0; r < 3; ++r) {
         const double t = dm[r] - ((R[3 * r] * sm[0] + R[3 * r + 1] * sm[1]) + R[3 * r + 2] * sm[2]);
         T[4 * r] = (float)R[3 * r]; T[4 * r + 1] = (float)R[3 * r + 1]; T[4 * r + 2] = (float)R[3 * r + 2]; T[4 * r + 3] = (float)t;

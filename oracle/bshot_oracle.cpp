@@ -909,7 +909,8 @@ struct OrcMt19937 {
     }
 };
 
-// Eigen::JacobiSVD stand-in: one-sided Jacobi (Hestenes) in double, singular values descending
+// Eigen::JacobiSVD stand-in: one-sided Jacobi (Hestenes) in double, singular values descending; a column of U whose
+// singular value is exactly zero is left zero (the callers complete the bases)
 void orc_svd3(const double a_in[9], double U[9], double sv[3], double V[9]) {
     double a[3][3], v[3][3] = {{1, 0, 0}, {0, 1, 0}, {0, 0, 1}};
     for (int r = 0; r < 3; ++r) for (int c = 0; c < 3; ++c) a[r][c] = a_in[3 * r + c];
@@ -945,6 +946,51 @@ void orc_svd3(const double a_in[9], double U[9], double sv[3], double V[9]) {
     }
 }
 
+// R for a cross-covariance of rank 0 or 1, Sigma = s0 u0 v0^T: a deterministic proper rotation with R v0 = u0 (any such R
+// is optimal).  u0.v0 >= 0: the minimal rotation; u0.v0 < 0: a half-turn about a = v0 x e_j (e_j: the axis of v0's smallest
+// component), then the minimal rotation from -v0 to u0.  Rank 0: the identity, as pcl::umeyama gives for Sigma = 0.
+// pcl::umeyama's own rank <= 1 result depends on Eigen's SVD internals (and can be improper): a deliberate difference.
+// Rank 0 is s0 at or below orc_noise_floor: the rounding noise of Sigma when one side is a single point (the rounded
+// centroid does not return that point, so Sigma is tiny but not zero), twice gamma_{k+3} (Ad (Ap + 2 As) + As (Aq + 2 Ad))
+// with A* the means of the 1-norms of the sources, targets, centred sources and centred targets.
+double orc_noise_floor(double P, double Q, double S, double D, double n, double k, double u) {
+    const double ap = P / n, aq = Q / n, as = S / n, ad = D / n;
+    return 2.0 * ((k + 3.0) * u) * (ad * (ap + 2.0 * as) + as * (aq + 2.0 * ad));
+}
+
+void orc_rotation_min(const double v[3], const double u[3], double R[9]) {
+    const double c = (v[0] * u[0] + v[1] * u[1]) + v[2] * u[2];
+    const double k[3] = {v[1] * u[2] - v[2] * u[1], v[2] * u[0] - v[0] * u[2], v[0] * u[1] - v[1] * u[0]};
+    const double f = 1.0 / (1.0 + c);
+    R[0] = c + k[0] * k[0] * f; R[1] = k[0] * k[1] * f - k[2]; R[2] = k[0] * k[2] * f + k[1];
+    R[3] = k[1] * k[0] * f + k[2]; R[4] = c + k[1] * k[1] * f; R[5] = k[1] * k[2] * f - k[0];
+    R[6] = k[2] * k[0] * f - k[1]; R[7] = k[2] * k[1] * f + k[0]; R[8] = c + k[2] * k[2] * f;
+}
+
+void orc_rotation_rank01(const double U[9], const double V[9], bool rank0, double R[9]) {
+    if (rank0) {
+        for (int e = 0; e < 9; ++e) R[e] = (e % 4 == 0) ? 1.0 : 0.0;
+        return;
+    }
+    const double u[3] = {U[0], U[3], U[6]}, v[3] = {V[0], V[3], V[6]};
+    if ((v[0] * u[0] + v[1] * u[1]) + v[2] * u[2] >= 0.0) { orc_rotation_min(v, u, R); return; }
+    const double ax[3] = {std::fabs(v[0]), std::fabs(v[1]), std::fabs(v[2])};
+    const int j = (ax[0] <= ax[1] && ax[0] <= ax[2]) ? 0 : (ax[1] <= ax[2] ? 1 : 2);
+    double a[3] = {0.0, 0.0, 0.0};
+    if (j == 0) { a[1] = v[2]; a[2] = -v[1]; }
+    else if (j == 1) { a[0] = -v[2]; a[2] = v[0]; }
+    else { a[0] = v[1]; a[1] = -v[0]; }
+    const double na = std::sqrt((a[0] * a[0] + a[1] * a[1]) + a[2] * a[2]);
+    for (int r = 0; r < 3; ++r) a[r] = a[r] / na;
+    double H[9], M[9];
+    for (int r = 0; r < 3; ++r)
+        for (int q = 0; q < 3; ++q) H[3 * r + q] = 2.0 * a[r] * a[q] - (r == q ? 1.0 : 0.0);
+    const double w[3] = {-v[0], -v[1], -v[2]};
+    orc_rotation_min(w, u, M);
+    for (int r = 0; r < 3; ++r)
+        for (int q = 0; q < 3; ++q) R[3 * r + q] = (M[3 * r] * H[q] + M[3 * r + 1] * H[3 + q]) + M[3 * r + 2] * H[6 + q];
+}
+
 // pcl::umeyama (with_scaling = false) on three pairs; float row-major 4x4 (estimateRigidTransformationSVD's cast)
 void orc_umeyama3(const double src[3][3], const double dst[3][3], float T[16]) {
     double sm[3], dm[3];
@@ -958,12 +1004,21 @@ void orc_umeyama3(const double src[3][3], const double dst[3][3], float T[16]) {
         }
     double U[9], sv[3], V[9];
     orc_svd3(sigma, U, sv, V);
-    // rank 2: right-handed completion of both bases -> R = U V^T is the proper rotation of Eq. (40)-(43)
-    U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
-    V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
     double R[9];
-    for (int r = 0; r < 3; ++r)
-        for (int c = 0; c < 3; ++c) R[3 * r + c] = (U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + U[3 * r + 2] * V[3 * c + 2];
+    double abs_s = 0.0, abs_d = 0.0, abs_p = 0.0, abs_q = 0.0;
+    for (int i = 0; i < 3; ++i)
+        for (int c = 0; c < 3; ++c) {
+            abs_p += std::fabs(src[i][c]); abs_q += std::fabs(dst[i][c]); abs_s += std::fabs(src[i][c] - sm[c]); abs_d += std::fabs(dst[i][c] - dm[c]);
+        }
+    const bool rank0 = sv[0] <= orc_noise_floor(abs_p, abs_q, abs_s, abs_d, 3.0, 3.0, 1.1102230246251565e-16);
+    if (rank0 || sv[1] <= sv[0] * 1e-12) orc_rotation_rank01(U, V, rank0, R);   // rank <= 1 (double precision)
+    else {
+        // rank 2: right-handed completion of both bases -> R = U V^T is the proper rotation of Eq. (40)-(43)
+        U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
+        V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
+        for (int r = 0; r < 3; ++r)
+            for (int c = 0; c < 3; ++c) R[3 * r + c] = (U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + U[3 * r + 2] * V[3 * c + 2];
+    }
     for (int r = 0; r < 3; ++r) {
         const double t = dm[r] - ((R[3 * r] * sm[0] + R[3 * r + 1] * sm[1]) + R[3 * r + 2] * sm[2]);
         T[4 * r] = (float)R[3 * r]; T[4 * r + 1] = (float)R[3 * r + 1]; T[4 * r + 2] = (float)R[3 * r + 2]; T[4 * r + 3] = (float)t;
@@ -1142,14 +1197,35 @@ int orc_icp(const float* src_xyz, size_t n_src, const float* tgt_xyz, size_t n_t
         double U[9], sv[3], V[9];
         orc_svd3(sg, U, sv, V);
         const double det = sg[0] * (sg[4] * sg[8] - sg[5] * sg[7]) - sg[1] * (sg[3] * sg[8] - sg[5] * sg[6]) + sg[2] * (sg[3] * sg[7] - sg[4] * sg[6]);
-        double sgn = 1.0;
-        if (sv[2] <= sv[0] * 1e-5) {
-            U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
-            V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
-        } else if (det < 0) sgn = -1.0;
+        double Rd[9];
+        // sums of the 1-norms of the sources, targets, centred sources and centred targets: the rank-0 noise floor
+        const float abs_p = orc_strided_sum<float>(n_src, [&](size_t i) {
+            return nn[i] >= 0 ? (std::fabs(cur[3 * i]) + std::fabs(cur[3 * i + 1])) + std::fabs(cur[3 * i + 2]) : 0.f; });
+        const float abs_q = orc_strided_sum<float>(n_src, [&](size_t i) {
+            if (nn[i] < 0) return 0.f;
+            const float* q = &tgt_xyz[3 * nn[i]];
+            return (std::fabs(q[0]) + std::fabs(q[1])) + std::fabs(q[2]); });
+        const float abs_s = orc_strided_sum<float>(n_src, [&](size_t i) {
+            return nn[i] >= 0 ? (std::fabs(cur[3 * i] - sm[0]) + std::fabs(cur[3 * i + 1] - sm[1])) + std::fabs(cur[3 * i + 2] - sm[2]) : 0.f; });
+        const float abs_d = orc_strided_sum<float>(n_src, [&](size_t i) {
+            if (nn[i] < 0) return 0.f;
+            const float* q = &tgt_xyz[3 * nn[i]];
+            return (std::fabs(q[0] - dm[0]) + std::fabs(q[1] - dm[1])) + std::fabs(q[2] - dm[2]); });
+        const bool rank0 = sv[0] <= orc_noise_floor((double)abs_p, (double)abs_q, (double)abs_s, (double)abs_d, (double)n,
+                                                    (double)((n + 255) / 256 + 8), 5.9604644775390625e-08);
+        if (rank0 || sv[1] <= sv[0] * 1e-5) orc_rotation_rank01(U, V, rank0, Rd);   // rank <= 1 (float precision)
+        else {
+            double sgn = 1.0;
+            if (sv[2] <= sv[0] * 1e-5) {   // rank 2
+                U[2] = U[3] * U[7] - U[6] * U[4]; U[5] = U[6] * U[1] - U[0] * U[7]; U[8] = U[0] * U[4] - U[3] * U[1];
+                V[2] = V[3] * V[7] - V[6] * V[4]; V[5] = V[6] * V[1] - V[0] * V[7]; V[8] = V[0] * V[4] - V[3] * V[1];
+            } else if (det < 0) sgn = -1.0;
+            for (int r = 0; r < 3; ++r)
+                for (int c = 0; c < 3; ++c) Rd[3 * r + c] = (U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + sgn * (U[3 * r + 2] * V[3 * c + 2]);
+        }
         float Rt[16];
         for (int r = 0; r < 3; ++r) {
-            for (int c = 0; c < 3; ++c) Rt[4 * r + c] = (float)((U[3 * r] * V[3 * c] + U[3 * r + 1] * V[3 * c + 1]) + sgn * (U[3 * r + 2] * V[3 * c + 2]));
+            for (int c = 0; c < 3; ++c) Rt[4 * r + c] = (float)Rd[3 * r + c];
             Rt[4 * r + 3] = dm[r] - ((Rt[4 * r] * sm[0] + Rt[4 * r + 1] * sm[1]) + Rt[4 * r + 2] * sm[2]);
         }
         Rt[12] = Rt[13] = Rt[14] = 0.f; Rt[15] = 1.f;
