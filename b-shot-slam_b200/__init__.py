@@ -39,6 +39,7 @@ EXPORTS = [
     "bshot_iss_params_default", "bshot_detect_iss", "bshot_kp_repeatability", "bshot_voxel_grid",
     "bshot_odom_params_default", "bshot_odometry_step", "bshot_odometry_step_cloud", "bshot_odometry_reset", "bshot_ransac_dev",
     "bshot_gmap_export", "bshot_gmap_import", "bshot_relocalize", "bshot_relocalize_cloud",
+    "bshot_gmap_scans", "bshot_loop_params_default", "bshot_detect_loop",
 ]
 
 
@@ -69,6 +70,18 @@ class RelocReport(C.Structure):
     _fields_ = [("pose", C.c_float * 16), ("T_ransac", C.c_float * 16), ("n_points", C.c_size_t), ("n_map", C.c_size_t),
                 ("n_icp_targets", C.c_size_t), ("n_keypoints", C.c_int), ("n_pairs", C.c_int), ("n_inliers", C.c_int),
                 ("ransac_iterations", C.c_int), ("icp_iterations", C.c_int), ("accepted", C.c_int)]
+
+
+class LoopParams(C.Structure):
+    _fields_ = [("min_gap", C.c_int), ("min_inliers", C.c_int), ("ransac_iterations", C.c_int), ("inlier_threshold", C.c_float),
+                ("map_range", C.c_float), ("run_icp", C.c_int)]
+
+
+class LoopReport(C.Structure):
+    _fields_ = [("T_loop", C.c_float * 16), ("T_ransac", C.c_float * 16), ("T_rel", C.c_float * 16), ("pose", C.c_float * 16),
+                ("n_candidates", C.c_size_t), ("n_icp_targets", C.c_size_t), ("scan", C.c_int), ("match_scan", C.c_int), ("votes", C.c_int),
+                ("n_keypoints", C.c_int), ("n_pairs", C.c_int), ("n_inliers", C.c_int), ("ransac_iterations", C.c_int),
+                ("icp_iterations", C.c_int), ("accepted", C.c_int)]
 
 
 E_INVALID, E_CAPACITY, E_CUDA, E_STATE = -1, -2, -3, -4
@@ -186,6 +199,10 @@ def lib():
         L.bshot_gmap_import.argtypes = [vp, vp, vp, sz]
         L.bshot_relocalize.argtypes = [vp, C.POINTER(OdomParams), ci, vp, vp, vp, sz, vp, sz, C.POINTER(RelocReport)]
         L.bshot_relocalize_cloud.argtypes = [vp, C.POINTER(OdomParams), ci, vp, sz, sz, C.POINTER(RelocReport)]
+        L.bshot_gmap_scans.argtypes = [vp, vp, sz, vp, sz, C.POINTER(sz), C.POINTER(sz)]
+        L.bshot_loop_params_default.argtypes = [C.POINTER(LoopParams)]
+        L.bshot_loop_params_default.restype = None
+        L.bshot_detect_loop.argtypes = [vp, C.POINTER(LoopParams), C.POINTER(LoopReport)]
         _LIB = L
     return _LIB
 
@@ -235,10 +252,22 @@ def odom_default_params(**kw):
     return p
 
 
+def loop_params_default(**kw):
+    """parameters of bshot_detect_loop; keyword arguments override fields"""
+    p = LoopParams()
+    lib().bshot_loop_params_default(C.byref(p))
+    for k, v in kw.items():
+        if not hasattr(p, k):
+            raise AttributeError(k)
+        setattr(p, k, v)
+    return p
+
+
 def _report(r):
-    out = {name: getattr(r, name) for name, _ in type(r)._fields_ if name not in ("pose", "T_ransac")}
-    out["pose"] = np.ctypeslib.as_array(r.pose).reshape(4, 4).copy()
-    out["T_ransac"] = np.ctypeslib.as_array(r.T_ransac).reshape(4, 4).copy()
+    mats = [name for name, _ in type(r)._fields_ if name in ("pose", "T_ransac", "T_loop", "T_rel")]
+    out = {name: getattr(r, name) for name, _ in type(r)._fields_ if name not in mats}
+    for name in mats:
+        out[name] = np.ctypeslib.as_array(getattr(r, name)).reshape(4, 4).copy()
     return out
 
 
@@ -531,6 +560,21 @@ class Context:
             raise BshotError("gmap_import: xyzr and desc differ in length", E_INVALID)
         _chk(lib().bshot_gmap_import(self.h, _p(xyzr), _p(desc), xyzr.shape[0]))
 
+    def gmap_scans(self):
+        """the update that wrote each entry, in gmap_export's order, and the pose each update used ->
+        (entry_scans (n,) uint32, poses (m, 4, 4) float32 row-major)"""
+        n, m = C.c_size_t(), C.c_size_t()
+        rc = lib().bshot_gmap_scans(self.h, None, 0, None, 0, C.byref(n), C.byref(m))
+        if rc not in (0, E_CAPACITY):
+            _chk(rc)
+        tags = np.empty(n.value, np.uint32)
+        p12 = np.empty((m.value, 3, 4), np.float32)
+        _chk(lib().bshot_gmap_scans(self.h, _p(tags), n.value, _p(p12), m.value, C.byref(n), C.byref(m)))
+        poses = np.zeros((m.value, 4, 4), np.float32)
+        poses[:, :3] = p12
+        poses[:, 3, 3] = 1.0
+        return tags, poses
+
     def extract_frame(self, xyz, params):
         xyz = np.ascontiguousarray(xyz, dtype=np.float32)
         k = params.top_k
@@ -667,6 +711,14 @@ class Context:
         r = RelocReport()
         _chk(lib().bshot_relocalize_cloud(self.h, C.byref(params), min_inliers, _p(xyz), xyz.shape[0], xyz.shape[1] * 4, C.byref(r)))
         self.n_points, self.n_kp = r.n_points, r.n_keypoints
+        return _report(r)
+
+    def detect_loop(self, params=None):
+        """is the last scan the odometry took a revisit of a scan at least params.min_gap updates older?  Read only.
+        Returns the report as a dict: T_loop / T_ransac / T_rel / pose (4 x 4 float32), match_scan, votes, accepted, ..."""
+        params = loop_params_default() if params is None else params
+        r = LoopReport()
+        _chk(lib().bshot_detect_loop(self.h, C.byref(params), C.byref(r)))
         return _report(r)
 
     def odometry_reset(self):

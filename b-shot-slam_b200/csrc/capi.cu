@@ -269,6 +269,7 @@ int bshot_ctx_reset(bshot_ctx* ctx) {
     ctx->normals_valid = 0;
     ctx->have_normals = false;
     ctx->n_prev = 0;
+    ctx->gmap.last_by_scan = false;   // no reference frame: nothing for bshot_detect_loop to query
     ctx->n_map = 0;
     ctx->gate_top_k = 0;
     return sync(ctx);
@@ -755,6 +756,8 @@ int bshot_gmap_add(bshot_ctx* ctx, const float* xyz, const float* seg_ratio, con
     BSHOT_TRY(h2d(ctx, ctx->d_q, desc, 48 * n));
     BSHOT_TRY(gmap_update(ctx, d_pos, d_ratio, ctx->d_q, nullptr, n, pose3x4));
     ctx->gmap.entries_upper += n;
+    ++ctx->gmap.n_updates;
+    ctx->gmap.last_by_scan = false;
     return sync(ctx);
 }
 
@@ -763,6 +766,8 @@ int bshot_gmap_update_from_frame(bshot_ctx* ctx, const float* pose3x4) {
     if (!ctx->have_kp || ctx->last_top_k == 0) { set_error("bshot_gmap_update_from_frame: no extracted frame"); return BSHOT_E_STATE; }
     BSHOT_TRY(gmap_update(ctx, ctx->d_kp, ctx->d_kp_ratio, ctx->d_bits, ctx->d_kp_count, ctx->last_top_k, pose3x4));
     ctx->gmap.entries_upper += ctx->last_top_k;
+    ++ctx->gmap.n_updates;
+    ctx->gmap.last_by_scan = false;
     return BSHOT_OK;  // asynchronous
 }
 
@@ -793,6 +798,13 @@ int bshot_gmap_import(bshot_ctx* ctx, const float* xyzr, const uint64_t* desc, s
     if (!ctx->gmap.d_tab) { set_error("bshot_gmap_import: no map (bshot_gmap_create)"); return BSHOT_E_STATE; }
     if (n && (!xyzr || !desc)) { set_error("bshot_gmap_import: null input"); return BSHOT_E_INVALID; }
     return gmap_import(ctx, xyzr, desc, n);
+}
+
+int bshot_gmap_scans(bshot_ctx* ctx, uint32_t* entry_scan_out, size_t entry_cap, float* poses3x4_out, size_t pose_cap, size_t* n_entries_out,
+                     size_t* n_scans_out) {
+    CHECK_CTX(ctx);
+    if (!ctx->gmap.d_tab) { set_error("bshot_gmap_scans: no map (bshot_gmap_create)"); return BSHOT_E_STATE; }
+    return gmap_scans(ctx, entry_scan_out, entry_cap, poses3x4_out, pose_cap, n_entries_out, n_scans_out);
 }
 
 int bshot_extract_frame(bshot_ctx* ctx, const bshot_params* p, const float* xyz, size_t n, size_t stride_bytes, int* kp_idx_out, float* kp_xyz_out,
@@ -1037,6 +1049,29 @@ int bshot_relocalize_cloud(bshot_ctx* ctx, const bshot_odom_params* p, int min_i
     BSHOT_TRY(frame_args_ok(ctx, &p->front, n, stride_bytes, "bshot_relocalize_cloud"));
     BSHOT_TRY(h2d(ctx, ctx->d_raw, xyz, n * stride_bytes));
     return relocalize_run(ctx, p, min_inliers, ctx->d_raw, n, (int)(stride_bytes / 4), out);
+}
+
+void bshot_loop_params_default(bshot_loop_params* p) {
+    if (!p) return;
+    p->min_gap = 100;
+    p->min_inliers = 15;
+    p->ransac_iterations = 2000;
+    p->inlier_threshold = 1500.0f;
+    p->map_range = 100000.0f;
+    p->run_icp = 1;
+}
+
+int bshot_detect_loop(bshot_ctx* ctx, const bshot_loop_params* p, bshot_loop_report* out) {
+    CHECK_CTX(ctx);
+    bshot_loop_params dp;
+    if (!p) { bshot_loop_params_default(&dp); p = &dp; }
+    if (p->min_gap < 1) { set_error("bshot_detect_loop: min_gap %d < 1", p->min_gap); return BSHOT_E_INVALID; }
+    if (p->min_inliers < 3) { set_error("bshot_detect_loop: min_inliers %d < 3", p->min_inliers); return BSHOT_E_INVALID; }
+    if (p->ransac_iterations < 1 || p->ransac_iterations > 100000) { set_error("bshot_detect_loop: ransac_iterations %d outside [1, 100000]", p->ransac_iterations); return BSHOT_E_INVALID; }
+    if (!(p->inlier_threshold > 0.0f) || !std::isfinite(p->inlier_threshold)) { set_error("bshot_detect_loop: inlier_threshold must be finite and > 0"); return BSHOT_E_INVALID; }
+    if (!(p->map_range >= 0.0f) || !std::isfinite(p->map_range)) { set_error("bshot_detect_loop: map_range must be finite and >= 0"); return BSHOT_E_INVALID; }
+    if (!ctx->gmap.d_tab) { set_error("bshot_detect_loop: needs a map (bshot_gmap_create)"); return BSHOT_E_STATE; }
+    return loop_run(ctx, p, out);
 }
 
 int bshot_odometry_reset(bshot_ctx* ctx) {

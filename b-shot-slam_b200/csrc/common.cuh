@@ -105,6 +105,21 @@ struct Gmap {
     unsigned* d_shist = nullptr;        // radix histograms
     unsigned* d_boff = nullptr;         // tab_cap: entry offset of each listed block / first sorted entry of each slot (import)
     unsigned* d_actl = nullptr;         // [0] listed blocks [1] entries gathered [2] import error bits [3] import entries
+    unsigned* d_atag = nullptr;         // max_entries: tags in map order (gmap_gather_all with tags)
+    // loop closure (gmap_scans, bshot_detect_loop).  Updates are numbered 0, 1, ... since create / reset / import (update
+    // 0) / odometry reset; n_updates advances where entries_upper does, once the update has succeeded
+    unsigned* d_etag = nullptr;         // max_entries: index of the update that wrote each entry
+    float* d_traj = nullptr;            // traj_cap x 12: row-major [R|T] each update used (identity without a pose)
+    size_t traj_cap = 0;
+    unsigned n_updates = 0;
+    bool last_by_scan = false;          // the last update was a step or an accepted relocalisation, and its scan is still the reference frame
+    // loop-closure selections, allocated by the first detection: candidates in map order, tile counts / offsets, counts
+    float4* d_lpos = nullptr;           // max_entries
+    uint64_t* d_ldesc = nullptr;        // max_entries x 6
+    unsigned* d_ltag = nullptr;         // max_entries
+    unsigned* d_ltile = nullptr;        // 2 x ltile_cap
+    size_t ltile_cap = 0;
+    unsigned* d_lctl = nullptr;         // [0] candidates [1] candidates (uncapped) [2] ICP targets (<= max_targets) [3] ICP targets (uncapped)
 };
 
 // ISS keypoints (iss.cu): max_points-sized buffers, allocated by the first bshot_detect_iss of the context
@@ -140,6 +155,8 @@ struct Odom {
     float4* d_icp_tgt = nullptr;        // max_targets: ICP targets, NaN past the true count
     IcpState* d_icp_state = nullptr;
     void* h_out = nullptr;              // pinned staging of the report
+    void* d_loop = nullptr;             // loop detection's report, error flag and RANSAC outputs (LoopDev, odometry.cu)
+    void* h_loop = nullptr;             // pinned staging of its report
     bool run = false;                   // RUN status: a step has succeeded since creation / bshot_odometry_reset
 };
 

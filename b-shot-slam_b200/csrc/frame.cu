@@ -21,7 +21,10 @@ int frame_commit(Ctx* c, size_t k, const int* d_skip) {
     copy_prev_kernel<<<(unsigned)((k * 6 + 255) / 256), 256, 0, c->stream>>>(c->d_bits, c->d_kp, c->d_kp_count, (unsigned)k, d_skip, c->d_prev_bits,
                                                                             c->d_prev_kp, c->d_prev_count);
     count_launch(c);
-    if (!d_skip) c->n_prev = k;
+    if (!d_skip) {
+        c->n_prev = k;
+        c->gmap.last_by_scan = false;   // the reference frame is no longer the scan of the last map update
+    }
     return check_launch("copy_prev_kernel");
 }
 

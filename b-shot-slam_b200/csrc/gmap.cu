@@ -68,8 +68,9 @@ __device__ __forceinline__ unsigned gm_find(GmapBlock* tab, unsigned mask, unsig
 __global__ void gm_prepare_kernel(const float4* __restrict__ kp, const float* __restrict__ ratio, const int* __restrict__ count_dev,
                                   unsigned n_cap, const float* __restrict__ pose, int have_pose, GmapBlock* tab, unsigned mask,
                                   float4* __restrict__ world, unsigned* __restrict__ blk_of, unsigned* __restrict__ touched_list,
-                                  unsigned* __restrict__ ctl, unsigned epoch) {
+                                  unsigned* __restrict__ ctl, unsigned epoch, unsigned update, float* __restrict__ traj) {
     const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < 12) traj[(size_t)update * 12 + i] = have_pose ? pose[i] : (i % 5 == 0 ? 1.0f : 0.0f);   // the pose this update uses
     const unsigned n = count_dev ? min(n_cap, (unsigned)max(*count_dev, 0)) : n_cap;
     if (i >= n) return;
     const float4 p = kp[i];
@@ -96,8 +97,8 @@ __global__ void gm_prepare_kernel(const float4* __restrict__ kp, const float* __
 __global__ void __launch_bounds__(128)
 gm_admit_kernel(const float4* __restrict__ world, const unsigned* __restrict__ blk_of, const uint64_t* __restrict__ bits,
                 const int* __restrict__ count_dev, unsigned n_cap, GmapBlock* tab, const unsigned* __restrict__ touched_list,
-                unsigned* __restrict__ ctl, float4* __restrict__ e_pos, uint64_t* __restrict__ e_desc, unsigned* __restrict__ chunks,
-                unsigned max_entries, unsigned max_chunks) {
+                unsigned* __restrict__ ctl, float4* __restrict__ e_pos, uint64_t* __restrict__ e_desc, unsigned* __restrict__ e_tag,
+                unsigned* __restrict__ chunks, unsigned max_entries, unsigned max_chunks, unsigned update) {
     const unsigned lane = threadIdx.x & 31, w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
     if (w >= ctl[1]) return;
     const unsigned slot = touched_list[w];
@@ -151,7 +152,7 @@ gm_admit_kernel(const float4* __restrict__ world, const unsigned* __restrict__ b
                 if (lane == 0) chunks[last * 33u + (cnt & 31u)] = e;
                 ++cnt;
             }
-            if (lane == 0) e_pos[e] = p;
+            if (lane == 0) { e_pos[e] = p; e_tag[e] = update; }   // an overwrite takes this update's tag: its descriptor is this scan's
             if (lane < 6) e_desc[(size_t)e * 6 + lane] = bits[(size_t)k * 6 + lane];
             __syncwarp();
             __threadfence_block();
@@ -236,7 +237,8 @@ gm_probe_kernel(const GmapBlock* __restrict__ tab, unsigned mask, GmapCube cube,
 __global__ void __launch_bounds__(128)
 gm_collect_kernel(const GmapBlock* __restrict__ tab, const unsigned* __restrict__ probe_slot, const unsigned* __restrict__ probe_off,
                   const unsigned* __restrict__ d_np, const unsigned* __restrict__ chunks, const float4* __restrict__ e_pos,
-                  const uint64_t* __restrict__ e_desc, float4* __restrict__ out_pos, uint64_t* __restrict__ out_desc, unsigned out_cap) {
+                  const uint64_t* __restrict__ e_desc, float4* __restrict__ out_pos, uint64_t* __restrict__ out_desc, unsigned out_cap,
+                  const unsigned* __restrict__ e_tag, unsigned* __restrict__ out_tag) {
     const unsigned lane = threadIdx.x & 31;
     const unsigned np = *d_np;
     for (unsigned p = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; p < np; p += (gridDim.x * blockDim.x) >> 5) {
@@ -249,6 +251,7 @@ gm_collect_kernel(const GmapBlock* __restrict__ tab, const unsigned* __restrict_
             if (j < cnt && off + j < out_cap) {
                 const unsigned e = chunks[c * 33u + lane];
                 out_pos[off + j] = e_pos[e];
+                if (out_tag) out_tag[off + j] = e_tag[e];
 #pragma unroll
                 for (int k = 0; k < 6; ++k) out_desc[(size_t)(off + j) * 6 + k] = e_desc[(size_t)e * 6 + k];
             }
@@ -323,10 +326,12 @@ gm_block_offsets_kernel(const GmapBlock* __restrict__ tab, const unsigned* __res
 // import: the entries already sit at pool index = input index.  Block slot of every entry (created when new), its count,
 // and (slot, input index) for the stable sort by slot
 __global__ void gm_import_find_kernel(const float4* __restrict__ e_pos, unsigned n, GmapBlock* tab, unsigned mask, unsigned long long* __restrict__ keys,
-                                      unsigned* __restrict__ idx, unsigned* __restrict__ actl) {
+                                      unsigned* __restrict__ idx, unsigned* __restrict__ actl, unsigned* __restrict__ e_tag, float* __restrict__ traj) {
     const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i == 0) actl[3] = n;
+    if (i < 12) traj[i] = (i % 5 == 0) ? 1.0f : 0.0f;   // the import is update 0, in the map frame
     if (i >= n) return;
+    e_tag[i] = 0u;
     const float4 p = e_pos[i];
     unsigned slot = 0xFFFFFFFFu;
     if (!(isfinite(p.x) && isfinite(p.y) && isfinite(p.z))) atomicOr(&actl[2], 1u);
@@ -397,13 +402,17 @@ int gmap_create(Ctx* c, size_t max_entries, size_t max_blocks) {
     BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_ctl, sizeof(unsigned) * 8));
     BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_pose, sizeof(float) * 24));
     BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_tpos, sizeof(float4) * c->max_targets));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_etag, sizeof(unsigned) * max_entries));
+    g.traj_cap = 1024;
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_traj, sizeof(float) * 12 * g.traj_cap));
     return gmap_reset(c);
 }
 
 void gmap_free(Ctx* c) {
     Gmap& g = c->gmap;
     void* ptrs[] = {g.d_tab, g.d_epos, g.d_edesc, g.d_chunks, g.d_world, g.d_blk_of, g.d_touched, g.d_probe_slot, g.d_probe_off, g.d_ctl, g.d_pose, g.d_tpos,
-                    g.d_apos, g.d_adesc, g.d_skeys[0], g.d_skeys[1], g.d_svals[0], g.d_svals[1], g.d_shist, g.d_boff, g.d_actl};
+                    g.d_apos, g.d_adesc, g.d_skeys[0], g.d_skeys[1], g.d_svals[0], g.d_svals[1], g.d_shist, g.d_boff, g.d_actl,
+                    g.d_etag, g.d_traj, g.d_atag, g.d_lpos, g.d_ldesc, g.d_ltag, g.d_ltile, g.d_lctl};
     for (void* p : ptrs) if (p) cudaFree(p);
     g = Gmap();
 }
@@ -415,6 +424,8 @@ int gmap_reset(Ctx* c) {
     BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_ctl, 0, sizeof(unsigned) * 8, c->stream));
     g.epoch = 0;
     g.n_gathered = 0;
+    g.n_updates = 0;
+    g.last_by_scan = false;
     return BSHOT_OK;
 }
 
@@ -424,15 +435,25 @@ int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t
     if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
     if (n_cap == 0) return BSHOT_OK;
     if (n_cap > c->max_kp) { set_error("map update: %zu keypoints > capacity %zu", n_cap, c->max_kp); return BSHOT_E_CAPACITY; }
+    if (g.n_updates >= g.traj_cap) {   // the trajectory doubles; the caller advances n_updates once the update succeeded
+        float* grown = nullptr;
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&grown, sizeof(float) * 24 * g.traj_cap));
+        BSHOT_CUDA_TRY(cudaMemcpyAsync(grown, g.d_traj, sizeof(float) * 12 * g.traj_cap, cudaMemcpyDeviceToDevice, c->stream));
+        BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+        BSHOT_CUDA_TRY(cudaFree(g.d_traj));
+        g.d_traj = grown;
+        g.traj_cap *= 2;
+    }
     if (pose12) BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_pose, pose12, sizeof(float) * 12, pose_on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyHostToDevice, c->stream));
     BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_ctl + 1, 0, sizeof(unsigned), c->stream));
     ++g.epoch;
     const unsigned n = (unsigned)n_cap;
     gm_prepare_kernel<<<(n + 255) / 256, 256, 0, c->stream>>>(d_kp, d_ratio, d_count, n, g.d_pose, pose12 ? 1 : 0, reinterpret_cast<GmapBlock*>(g.d_tab),
-                                                             g.tab_cap - 1, g.d_world, g.d_blk_of, g.d_touched, g.d_ctl, g.epoch);
+                                                             g.tab_cap - 1, g.d_world, g.d_blk_of, g.d_touched, g.d_ctl, g.epoch, g.n_updates, g.d_traj);
     // at most n blocks are touched: one warp each (warps beyond the device-side count exit)
     gm_admit_kernel<<<(n * 32 + 127) / 128, 128, 0, c->stream>>>(g.d_world, g.d_blk_of, d_bits, d_count, n, reinterpret_cast<GmapBlock*>(g.d_tab), g.d_touched,
-                                                                g.d_ctl, g.d_epos, g.d_edesc, g.d_chunks, g.max_entries, g.max_chunks);
+                                                                g.d_ctl, g.d_epos, g.d_edesc, g.d_etag, g.d_chunks, g.max_entries, g.max_chunks,
+                                                                g.n_updates);
     count_launch(c, 2);
     return check_launch("map update kernels");
 }
@@ -458,7 +479,7 @@ int gmap_gather(Ctx* c, const float pos[3], float range, const float4* d_ref_kp,
     gm_probe_kernel<<<1, 1024, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.tab_cap - 1, cube, pose_on_device ? g.d_pose + 12 : nullptr, range,
                                                g.d_probe_slot, g.d_probe_off, g.d_ctl, g.max_probe);
     gm_collect_kernel<<<(unsigned)c->sm_count * 2u, 128, 0, c->stream>>>(reinterpret_cast<const GmapBlock*>(g.d_tab), g.d_probe_slot, g.d_probe_off, g.d_ctl + 5, g.d_chunks,
-                                                                        g.d_epos, g.d_edesc, g.d_tpos, d_t_out, (unsigned)out_cap);
+                                                                        g.d_epos, g.d_edesc, g.d_tpos, d_t_out, (unsigned)out_cap, nullptr, nullptr);
     const unsigned nref = d_ref_bits ? (unsigned)ref_cap : 0u;
     gm_append_ref_kernel<<<(std::max(nref, 1u) + 255) / 256, 256, 0, c->stream>>>(d_ref_kp, d_ref_bits, d_ref_count, nref, g.d_pose + 12, ref_pose12 ? 1 : 0, g.d_ctl,
                                                                                 g.d_tpos, d_t_out, (unsigned)out_cap, d_total);
@@ -480,10 +501,11 @@ static int gmap_all_alloc(Ctx* c) {
     BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_shist, sizeof(unsigned) * radix_hist_words(m)));
     BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_boff, sizeof(unsigned) * g.tab_cap));
     BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_actl, sizeof(unsigned) * 8));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_atag, sizeof(unsigned) * g.max_entries));
     return BSHOT_OK;
 }
 
-int gmap_gather_all(Ctx* c, size_t* nt_cap_out) {
+int gmap_gather_all(Ctx* c, size_t* nt_cap_out, bool with_tags) {
     Gmap& g = c->gmap;
     if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
     BSHOT_TRY(gmap_all_alloc(c));
@@ -499,7 +521,7 @@ int gmap_gather_all(Ctx* c, size_t* nt_cap_out) {
     BSHOT_TRY(radix_sort_pairs(c, g.d_skeys, g.d_svals, g.d_shist, g.d_actl, std::min<size_t>(g.tab_cap, nt_cap), 8));
     gm_block_offsets_kernel<<<1, 1024, 0, c->stream>>>(tab, g.d_svals[0], g.d_boff, g.d_actl);
     gm_collect_kernel<<<(unsigned)c->sm_count * 2u, 128, 0, c->stream>>>(tab, g.d_svals[0], g.d_boff, g.d_actl, g.d_chunks, g.d_epos, g.d_edesc, g.d_apos,
-                                                                        g.d_adesc, g.max_entries);
+                                                                        g.d_adesc, g.max_entries, g.d_etag, with_tags ? g.d_atag : nullptr);
     count_launch(c, 2);
     return check_launch("map gather-all kernels");
 }
@@ -537,7 +559,8 @@ int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n) {
     BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_actl, 0, sizeof(unsigned) * 8, c->stream));
     BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_epos, xyzr, sizeof(float4) * n, cudaMemcpyHostToDevice, c->stream));
     BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_edesc, desc, 48 * n, cudaMemcpyHostToDevice, c->stream));
-    gm_import_find_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_epos, nn, tab, g.tab_cap - 1, g.d_skeys[0], g.d_svals[0], g.d_actl);
+    gm_import_find_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_epos, nn, tab, g.tab_cap - 1, g.d_skeys[0], g.d_svals[0], g.d_actl, g.d_etag,
+                                                                    g.d_traj);
     count_launch(c);
     BSHOT_TRY(check_launch("gm_import_find_kernel"));
     // stable by slot: the input order survives inside a block.  Slots are < tab_cap (a power of two)
@@ -562,7 +585,140 @@ int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n) {
         return rc;
     }
     g.entries_upper = n;
+    g.n_updates = 1;
     return BSHOT_OK;
+}
+
+// ---- loop closure: entry tags, trajectory, candidate selection (loop_run, odometry.cu) ----------------------------------
+int gmap_scans(Ctx* c, uint32_t* entry_scan_out, size_t entry_cap, float* poses3x4_out, size_t pose_cap, size_t* n_entries_out, size_t* n_scans_out) {
+    Gmap& g = c->gmap;
+    size_t n = 0;
+    if (entry_scan_out || n_entries_out) {   // the tags need the whole-map gather; the trajectory alone does not
+        size_t nt_cap;
+        BSHOT_TRY(gmap_gather_all(c, &nt_cap, /*with_tags=*/true));
+        unsigned* h = reinterpret_cast<unsigned*>(&c->h_scratch[48]);
+        BSHOT_CUDA_TRY(cudaMemcpyAsync(h, g.d_actl, sizeof(unsigned) * 4, cudaMemcpyDeviceToHost, c->stream));
+        BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+        n = h[1];
+    }
+    const size_t m = std::min(n, entry_cap), ns = g.n_updates, ms = std::min(ns, pose_cap);
+    if (n_entries_out) *n_entries_out = n;
+    if (n_scans_out) *n_scans_out = ns;
+    if (entry_scan_out && m) BSHOT_CUDA_TRY(cudaMemcpyAsync(entry_scan_out, g.d_atag, sizeof(unsigned) * m, cudaMemcpyDeviceToHost, c->stream));
+    if (poses3x4_out && ms) BSHOT_CUDA_TRY(cudaMemcpyAsync(poses3x4_out, g.d_traj, sizeof(float) * 12 * ms, cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    if ((entry_scan_out && n > entry_cap) || (poses3x4_out && ns > pose_cap)) {
+        set_error("bshot_gmap_scans: %zu entries / %zu scans > capacities %zu / %zu", n, ns, entry_cap, pose_cap);
+        return BSHOT_E_CAPACITY;
+    }
+    return BSHOT_OK;
+}
+
+// A stable selection of *d_n entries in three launches: count per 1024-entry tile, one CTA scans the tile counts, each tile
+// writes its selected entries at its offset in their order.  mode 0 keeps the loop candidates (tag + min_gap <= scan),
+// mode 1 the entries whose block lattice coordinates lie in the +-range cube around the translation of the device pose T
+// (gmap_gather's block test).  ctl_out[0] = min(selected, out_cap), ctl_out[1] = selected; with err, more than out_cap
+// selected sets *err = BSHOT_E_CAPACITY
+struct GmSelect { int mode; unsigned scan, min_gap; const float* T; float range; };
+
+__device__ __forceinline__ bool gm_selected(const GmSelect& s, const float4* __restrict__ pos, const unsigned* __restrict__ tag, unsigned e) {
+    if (s.mode == 0) return (unsigned long long)tag[e] + s.min_gap <= s.scan;
+    const GmapCube cube = gm_cube(s.T[3], s.T[7], s.T[11], s.range);
+    if (cube.nx <= 0 || cube.ny <= 0 || cube.nz <= 0) return false;   // a non-finite pose selects nothing
+    const float4 p = pos[e];
+    const int bx = (int)roundf(p.x / (float)GM_PREC), by = (int)roundf(p.y / (float)GM_PREC), bz = (int)roundf(p.z / (float)GM_PREC);
+    return bx >= cube.x0 && bx < cube.x0 + cube.nx && by >= cube.y0 && by < cube.y0 + cube.ny && bz >= cube.z0 && bz < cube.z0 + cube.nz;
+}
+
+__global__ void __launch_bounds__(1024)
+gm_select_count_kernel(GmSelect s, const float4* __restrict__ pos, const unsigned* __restrict__ tag, const unsigned* __restrict__ d_n, unsigned* __restrict__ tile_cnt) {
+    const unsigned e = blockIdx.x * 1024u + threadIdx.x;
+    const unsigned n = *d_n;
+    if (blockIdx.x * 1024u >= n) return;   // the whole tile is past the count
+    const int cnt = __syncthreads_count(e < n && gm_selected(s, pos, tag, e));
+    if (threadIdx.x == 0) tile_cnt[blockIdx.x] = (unsigned)cnt;
+}
+
+__global__ void __launch_bounds__(1024)
+gm_select_scan_kernel(const unsigned* __restrict__ d_n, const unsigned* __restrict__ tile_cnt, unsigned* __restrict__ tile_off, unsigned* __restrict__ ctl_out,
+                      unsigned out_cap, int* err) {
+    __shared__ unsigned ws[32];
+    __shared__ unsigned carry;
+    if (threadIdx.x == 0) carry = 0;
+    __syncthreads();
+    const unsigned nt = (*d_n + 1023u) / 1024u;
+    for (unsigned base = 0; base < nt; base += 1024) {
+        const unsigned t = base + threadIdx.x;
+        const unsigned excl = cta_scan_1024(t < nt ? tile_cnt[t] : 0u, ws, &carry);
+        if (t < nt) tile_off[t] = excl;
+    }
+    if (threadIdx.x == 0) {
+        ctl_out[0] = min(carry, out_cap);
+        ctl_out[1] = carry;
+        if (err && carry > out_cap) *err = BSHOT_E_CAPACITY;
+    }
+}
+
+__global__ void __launch_bounds__(1024)
+gm_select_scatter_kernel(GmSelect s, const float4* __restrict__ pos, const uint64_t* __restrict__ desc, const unsigned* __restrict__ tag,
+                         const unsigned* __restrict__ d_n, const unsigned* __restrict__ tile_off, float4* __restrict__ out_pos, uint64_t* __restrict__ out_desc,
+                         unsigned* __restrict__ out_tag, unsigned out_cap) {
+    __shared__ unsigned wcnt[32];
+    const unsigned e = blockIdx.x * 1024u + threadIdx.x, lane = threadIdx.x & 31u, wid = threadIdx.x >> 5;
+    const unsigned n = *d_n;
+    if (blockIdx.x * 1024u >= n) return;
+    const bool sel = e < n && gm_selected(s, pos, tag, e);
+    const unsigned m = __ballot_sync(0xffffffffu, sel);
+    if (lane == 0) wcnt[wid] = __popc(m);
+    __syncthreads();
+    if (!sel) return;
+    unsigned o = tile_off[blockIdx.x] + __popc(m & ((1u << lane) - 1u));
+    for (unsigned w = 0; w < wid; ++w) o += wcnt[w];
+    if (o >= out_cap) return;
+    out_pos[o] = pos[e];
+    if (out_tag) out_tag[o] = tag[e];
+    if (out_desc)
+#pragma unroll
+        for (int k = 0; k < 6; ++k) out_desc[(size_t)o * 6 + k] = desc[(size_t)e * 6 + k];
+}
+
+static int gm_select(Ctx* c, const GmSelect& s, const float4* pos, const uint64_t* desc, const unsigned* tag, const unsigned* d_n, size_t n_cap, float4* out_pos,
+                     uint64_t* out_desc, unsigned* out_tag, unsigned out_cap, unsigned* ctl_out, int* err) {
+    Gmap& g = c->gmap;
+    if (n_cap == 0) {
+        BSHOT_CUDA_TRY(cudaMemsetAsync(ctl_out, 0, sizeof(unsigned) * 2, c->stream));
+        return BSHOT_OK;
+    }
+    const unsigned tiles = (unsigned)((n_cap + 1023) / 1024);
+    gm_select_count_kernel<<<tiles, 1024, 0, c->stream>>>(s, pos, tag, d_n, g.d_ltile);
+    gm_select_scan_kernel<<<1, 1024, 0, c->stream>>>(d_n, g.d_ltile, g.d_ltile + g.ltile_cap, ctl_out, out_cap, err);
+    gm_select_scatter_kernel<<<tiles, 1024, 0, c->stream>>>(s, pos, desc, tag, d_n, g.d_ltile + g.ltile_cap, out_pos, out_desc, out_tag, out_cap);
+    count_launch(c, 3);
+    return check_launch("map selection kernels");
+}
+
+int gmap_loop_candidates(Ctx* c, unsigned scan, unsigned min_gap, size_t* nc_cap_out) {
+    Gmap& g = c->gmap;
+    if (!g.d_lpos) {
+        g.ltile_cap = (g.max_entries + 1023) / 1024;
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_lpos, sizeof(float4) * g.max_entries));
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_ldesc, 48 * (size_t)g.max_entries));
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_ltag, sizeof(unsigned) * g.max_entries));
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_ltile, sizeof(unsigned) * 2 * g.ltile_cap));
+        BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_lctl, sizeof(unsigned) * 4));
+    }
+    size_t nm_cap = 0;
+    // no entry can be min_gap updates older than the scan: nothing to gather
+    if ((unsigned long long)scan >= min_gap) BSHOT_TRY(gmap_gather_all(c, &nm_cap, /*with_tags=*/true));
+    *nc_cap_out = nm_cap;
+    const GmSelect s = {0, scan, min_gap, nullptr, 0.0f};
+    return gm_select(c, s, g.d_apos, g.d_adesc, g.d_atag, g.d_actl + 1, nm_cap, g.d_lpos, g.d_ldesc, g.d_ltag, g.max_entries, g.d_lctl, nullptr);
+}
+
+int gmap_loop_icp_targets(Ctx* c, const float* d_T, float range, size_t nc_cap, int* d_err) {
+    Gmap& g = c->gmap;
+    const GmSelect s = {1, 0u, 0u, d_T, range};
+    return gm_select(c, s, g.d_lpos, nullptr, nullptr, g.d_lctl, nc_cap, g.d_tpos, nullptr, nullptr, (unsigned)c->max_targets, g.d_lctl + 2, d_err);
 }
 
 }  // namespace bshot

@@ -38,6 +38,18 @@ __host__ __device__ inline void mul4x4(const float* a, const float* b, float* o)
     for (int e = 0; e < 16; ++e) o[e] = r[e];
 }
 
+// rigid inverse [R^T | -R^T t] of a row-major [R|t; 0 0 0 1]: -(((r0i t0 + r1i t1) + r2i t2)) per row i (loop closure's T_rel)
+__host__ __device__ inline void rigid_inverse4x4(const float* m, float* o) {
+    float r[16];
+    for (int i = 0; i < 3; ++i) {
+        for (int j = 0; j < 3; ++j) r[4 * i + j] = m[4 * j + i];
+        r[4 * i + 3] = -((m[i] * m[3] + m[4 + i] * m[7]) + m[8 + i] * m[11]);
+        r[12 + i] = 0.0f;
+    }
+    r[15] = 1.0f;
+    for (int e = 0; e < 16; ++e) o[e] = r[e];
+}
+
 // T_ij = T_ref^-1 * T_ransac; heading change acos(T_ij(1,1)), translation |t_ij|; returns true when the estimate is rejected
 // (more than 10 degrees, more than 1200 mm or fewer than 15 correspondences, :281)
 __host__ __device__ inline bool estimation_gate(const float* T_ransac, const float* T_ref, int n_correspondences, float* h_diff, float* t_diff) {

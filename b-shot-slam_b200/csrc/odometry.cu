@@ -14,6 +14,11 @@
 // Relocalisation (relocalize_run) reuses the same stages without a prior pose: the whole map in map order is the target
 // set (gmap_gather_all), RANSAC and ICP (around T_ransac) run as in the step, and the step's tail -- pose, status, map
 // update, reference frame -- runs only when enough inliers survived; one device flag skips it otherwise.
+//
+// Loop detection (loop_run) reuses them once more on the reference frame, read only: the map's entries of updates at least
+// min_gap older than the scan are the target set (gmap_loop_candidates), RANSAC, ICP against the candidates around
+// T_ransac, then the candidates RANSAC kept vote for the scan they came from.  Its own device report (LoopDev); the only
+// scratch it writes is the matcher's, RANSAC's and ICP's, which every step rewrites before reading.
 #include <algorithm>
 #include <cmath>
 #include <cstddef>
@@ -112,6 +117,61 @@ __global__ void reloc_final_kernel(OdomDev* d, const IcpState* __restrict__ icp,
     }
 }
 
+// loop detection's device report
+struct LoopDev {
+    bshot_loop_report rep;   // copied to the host at the end, together with err
+    int err;                 // BSHOT_E_CAPACITY: more ICP targets than max_targets (ICP is skipped)
+    int n_inliers, ransac_iterations, pad;
+    float T_ransac[16];
+};
+
+// the vote over the candidates RANSAC kept (update index -> count; the most frequent, the lowest on ties), then T_loop,
+// T_rel = T_j^-1 * T_loop and the report.  n^2 tag comparisons for n inliers (n <= the reference frame's keypoints)
+__global__ void __launch_bounds__(256)
+loop_final_kernel(LoopDev* d, const IcpState* __restrict__ icp, int run_icp, int min_inliers, const int* __restrict__ inl, const unsigned* __restrict__ cand_tag,
+                  const float* __restrict__ traj, unsigned scan, const int* __restrict__ kp_count, const int* __restrict__ pair_count,
+                  const unsigned* __restrict__ lctl, int k) {
+    __shared__ unsigned long long best;   // (count << 32) | ~tag
+    if (threadIdx.x == 0) best = 0ull;
+    __syncthreads();
+    const int n = min(max(d->n_inliers, 0), k);
+    for (int t = threadIdx.x; t < n; t += blockDim.x) {
+        const unsigned tag = cand_tag[inl[2 * t + 1]];
+        unsigned cnt = 0;
+        for (int u = 0; u < n; ++u) cnt += cand_tag[inl[2 * u + 1]] == tag ? 1u : 0u;
+        atomicMax(&best, ((unsigned long long)cnt << 32) | (unsigned long long)(0xFFFFFFFFu - tag));
+    }
+    __syncthreads();
+    if (threadIdx.x != 0) return;
+    bshot_loop_report& r = d->rep;
+    float T_loop[16], Tj[16], Tj_inv[16];
+    if (run_icp) mul4x4(icp->final_T, d->T_ransac, T_loop);
+    else for (int e = 0; e < 16; ++e) T_loop[e] = d->T_ransac[e];
+    const int match = best ? (int)(0xFFFFFFFFu - (unsigned)(best & 0xFFFFFFFFull)) : -1;
+    for (int e = 0; e < 16; ++e) {
+        r.T_loop[e] = T_loop[e];
+        r.T_ransac[e] = d->T_ransac[e];
+        r.pose[e] = e < 12 ? traj[(size_t)scan * 12 + e] : (e == 15 ? 1.0f : 0.0f);
+        r.T_rel[e] = (e % 5 == 0) ? 1.0f : 0.0f;
+        Tj[e] = match >= 0 && e < 12 ? traj[(size_t)match * 12 + e] : (e == 15 ? 1.0f : 0.0f);
+    }
+    if (match >= 0) {
+        rigid_inverse4x4(Tj, Tj_inv);
+        mul4x4(Tj_inv, T_loop, r.T_rel);
+    }
+    r.n_candidates = lctl[0];
+    r.n_icp_targets = run_icp ? lctl[2] : 0;
+    r.scan = (int)scan;
+    r.match_scan = match;
+    r.votes = best ? (int)(best >> 32) : 0;
+    r.n_keypoints = min(max(*kp_count, 0), k);
+    r.n_pairs = min(max(*pair_count, 0), k);
+    r.n_inliers = d->n_inliers;
+    r.ransac_iterations = d->ransac_iterations;
+    r.icp_iterations = run_icp ? icp->iterations : 0;
+    r.accepted = (d->err == 0 && d->n_inliers >= min_inliers) ? 1 : 0;
+}
+
 int odom_ensure(Ctx* c) {
     Odom& o = c->odom;
     if (o.d) return BSHOT_OK;
@@ -122,6 +182,8 @@ int odom_ensure(Ctx* c) {
     BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_icp_tgt, sizeof(float4) * c->max_targets));
     BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_icp_state, sizeof(IcpState)));
     BSHOT_CUDA_TRY(cudaMallocHost(&o.h_out, sizeof(OdomDev)));
+    BSHOT_CUDA_TRY(cudaMalloc((void**)&o.d_loop, sizeof(LoopDev)));
+    BSHOT_CUDA_TRY(cudaMallocHost(&o.h_loop, sizeof(LoopDev)));
     BSHOT_CUDA_TRY(cudaMemsetAsync(o.d, 0, sizeof(OdomDev), c->stream));
     odom_reset_kernel<<<1, 32, 0, c->stream>>>(o.d);
     count_launch(c);
@@ -131,9 +193,10 @@ int odom_ensure(Ctx* c) {
 
 void odom_free(Ctx* c) {
     Odom& o = c->odom;
-    void* ptrs[] = {o.d, o.d_inlier_pairs, o.d_icp_cur, o.d_icp_keys, o.d_icp_tgt, o.d_icp_state};
+    void* ptrs[] = {o.d, o.d_inlier_pairs, o.d_icp_cur, o.d_icp_keys, o.d_icp_tgt, o.d_icp_state, o.d_loop};
     for (void* p : ptrs) if (p) cudaFree(p);
     if (o.h_out) cudaFreeHost(o.h_out);
+    if (o.h_loop) cudaFreeHost(o.h_loop);
     o = Odom();
 }
 
@@ -208,6 +271,8 @@ int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_
         return h->err;
     }
     g.entries_upper += c->last_top_k;
+    ++g.n_updates;
+    g.last_by_scan = true;
     c->n_prev = k;
     o.run = true;
     if (out) *out = h->rep;
@@ -265,10 +330,59 @@ int relocalize_run(Ctx* c, const bshot_odom_params* p, int min_inliers, const fl
     }
     if (h->rrep.accepted) {
         g.entries_upper += c->last_top_k;
+        ++g.n_updates;
+        g.last_by_scan = true;
         c->n_prev = k;
         o.run = true;
     }
     if (out) *out = h->rrep;
+    return BSHOT_OK;
+}
+
+// loop detection on the reference frame (scan i = the last update): candidates, mutual nearest neighbours, RANSAC, ICP
+// around T_ransac, vote and T_rel.  Asynchronous up to one copy back (report + error) at the end
+int loop_run(Ctx* c, const bshot_loop_params* p, bshot_loop_report* out) {
+    Gmap& g = c->gmap;
+    Odom& o = c->odom;
+    if (!g.d_tab || !o.d || !g.last_by_scan || g.n_updates == 0) {
+        set_error("bshot_detect_loop: the last map update was not an odometry step or an accepted relocalisation");
+        return BSHOT_E_STATE;
+    }
+    LoopDev* d = reinterpret_cast<LoopDev*>(o.d_loop);
+    const unsigned scan = g.n_updates - 1;
+    const size_t k = c->n_prev;
+    BSHOT_CUDA_TRY(cudaMemsetAsync(d, 0, sizeof(LoopDev), c->stream));
+    size_t nc_cap;
+    BSHOT_TRY(gmap_loop_candidates(c, scan, (unsigned)p->min_gap, &nc_cap));
+    const unsigned* d_nq = reinterpret_cast<const unsigned*>(c->d_prev_count);
+    if (nc_cap == 0) {
+        BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_pair_count, 0, sizeof(int), c->stream));
+    } else {
+        BSHOT_TRY(hamming_match_rq(c, c->d_prev_bits, k, g.d_ldesc, nc_cap, 0, c->d_cand, d_nq, g.d_lctl));
+        BSHOT_TRY(hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq));
+    }
+    BSHOT_TRY(ransac_run_dev(c, c->d_prev_kp, g.d_lpos, c->d_pairs, 3, c->d_pair_count, k, p->ransac_iterations, (double)p->inlier_threshold, o.d_inlier_pairs,
+                             &d->n_inliers, d->T_ransac, &d->ransac_iterations, nullptr));
+    if (p->run_icp) {
+        BSHOT_TRY(gmap_loop_icp_targets(c, d->T_ransac, p->map_range, nc_cap, &d->err));
+        const size_t nt_cap = std::min(c->max_targets, nc_cap);
+        BSHOT_TRY(icp_run_dev(c, reinterpret_cast<const float*>(c->d_prev_kp), 4, c->d_prev_count, k, reinterpret_cast<const float*>(g.d_tpos), 4, g.d_lctl + 2,
+                              nt_cap, d->T_ransac, 10, &d->err, o.d_icp_cur, o.d_icp_tgt, o.d_icp_keys, o.d_icp_state));
+    } else {
+        BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_lctl + 2, 0, sizeof(unsigned) * 2, c->stream));
+    }
+    loop_final_kernel<<<1, 256, 0, c->stream>>>(d, o.d_icp_state, p->run_icp ? 1 : 0, p->min_inliers, o.d_inlier_pairs, g.d_ltag, g.d_traj, scan, c->d_prev_count,
+                                                c->d_pair_count, g.d_lctl, (int)k);
+    count_launch(c);
+    BSHOT_TRY(check_launch("loop detection kernels"));
+    LoopDev* h = reinterpret_cast<LoopDev*>(o.h_loop);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(h, d, offsetof(LoopDev, err) + sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    if (h->err) {
+        set_error("bshot_detect_loop: ICP target set exceeds max_targets %zu", c->max_targets);
+        return h->err;
+    }
+    if (out) *out = h->rep;
     return BSHOT_OK;
 }
 

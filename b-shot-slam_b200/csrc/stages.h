@@ -70,11 +70,19 @@ int gmap_gather(Ctx* c, const float pos[3], float range, const float4* d_ref_kp,
                 size_t ref_cap, const float* ref_pose12, uint64_t* d_t_out, size_t out_cap, unsigned* d_total, bool pose_on_device = false);
 // the whole map in map order (occupied blocks in ascending lattice coordinates, x outermost, entries in insertion order) ->
 // gmap.d_apos / d_adesc, the count in gmap.d_actl[1]; *nt_cap_out = its host-side bound.  Asynchronous
-int gmap_gather_all(Ctx* c, size_t* nt_cap_out);
+int gmap_gather_all(Ctx* c, size_t* nt_cap_out, bool with_tags = false);
 // synchronous: export copies min(count, cap) records (float4 position + seg-ratio, 48-byte descriptor); import replaces
 // the map by n entries without the admission rule, keeping the input order inside each block (an empty map on any error)
 int gmap_export(Ctx* c, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t* n_out);
 int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n);
+// synchronous: the entries' tags in export order and the trajectory (bshot_gmap_scans)
+int gmap_scans(Ctx* c, uint32_t* entry_scan_out, size_t entry_cap, float* poses3x4_out, size_t pose_cap, size_t* n_entries_out, size_t* n_scans_out);
+// loop closure, asynchronous: the whole map in map order with tags, then the entries with tag + min_gap <= scan, in map order
+// -> gmap.d_lpos / d_ldesc / d_ltag, count in gmap.d_lctl[0] (*nc_cap_out = its host-side bound).  Then the candidates whose
+// block lies in the +-range cube around the translation of the device pose d_T -> gmap.d_tpos, count in gmap.d_lctl[2];
+// more than max_targets sets *d_err = BSHOT_E_CAPACITY
+int gmap_loop_candidates(Ctx* c, unsigned scan, unsigned min_gap, size_t* nc_cap_out);
+int gmap_loop_icp_targets(Ctx* c, const float* d_T, float range, size_t nc_cap, int* d_err);
 
 // stable LSD radix sort of (u64 key, u32 value) pairs, 8 bits a pass (voxel_grid.cu): *d_m pairs (at most m_cap) in
 // keys[0] / vals[0], `passes` passes from the low byte up; the result is in keys[passes & 1] / vals[passes & 1].  hist
@@ -132,6 +140,8 @@ int odometry_reset(Ctx* c);
 int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_t n, int stride_floats, bshot_odom_report* out);
 // relocalisation against the whole map (odometry.cu); the same shape as odometry_run
 int relocalize_run(Ctx* c, const bshot_odom_params* p, int min_inliers, const float* d_cloud, size_t n, int stride_floats, bshot_reloc_report* out);
+// loop detection on the reference frame against the map's older entries (odometry.cu); reads, never changes, the odometry's state
+int loop_run(Ctx* c, const bshot_loop_params* p, bshot_loop_report* out);
 
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);

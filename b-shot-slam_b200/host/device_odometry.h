@@ -3,6 +3,8 @@
 // the map, RANSAC, the gate + ICP, the map update and the reference-frame hand-over on the device and returns the pose.
 // LidarOdometry and its reference-named stage methods stay available for callers that want the stages one by one.
 // relocalize() finds a rotation in the whole map without a prior pose; exportMap / importMap save and restore the map.
+// detectLoop() asks whether the last rotation revisits an older one; trajectory() and the loop report's T_rel are the nodes
+// and edges a pose-graph back end takes.
 #ifndef BSHOT_B200_HOST_DEVICE_ODOMETRY_H
 #define BSHOT_B200_HOST_DEVICE_ODOMETRY_H
 
@@ -21,6 +23,7 @@ public:
     explicit DeviceOdometry(int device = 0, size_t max_points = 131072, size_t max_keypoints = 1024, size_t max_targets = 1u << 16,
                             size_t max_map = 1u << 16, size_t max_blocks = 4096) {
         bshot_odom_params_default(&params_);
+        bshot_loop_params_default(&loop_params_);
         status_ = bshot_ctx_create(&ctx_, device, max_points, max_keypoints, max_targets);
         if (status_ == BSHOT_OK) status_ = bshot_gmap_create(ctx_, max_map, max_blocks);
     }
@@ -87,6 +90,34 @@ public:
         return status_;
     }
 
+    // is the last rotation step() took a revisit of a rotation at least loopParams().min_gap map updates older?  true when
+    // accepted; *r (may be null) receives the report either way.  Read only: the pose, the map and the next step() are
+    // unaffected.  last_status() / bshot_last_error() say why a call failed
+    bool detectLoop(bshot_loop_report* r = nullptr) {
+        if (!ctx_) return false;
+        bshot_loop_report rep;
+        status_ = bshot_detect_loop(ctx_, &loop_params_, &rep);
+        if (status_ != BSHOT_OK) return false;
+        if (r) *r = rep;
+        return rep.accepted != 0;
+    }
+    bshot_loop_params& loopParams() { return loop_params_; }
+
+    // the pose each map update used, in update order (bshot_gmap_scans); empty after an error
+    void trajectory(std::vector<Matrix4f>& poses) {
+        poses.clear();
+        if (!ctx_) return;
+        size_t m = 0;   // no entry output: the map is not gathered, only the trajectory is read
+        status_ = bshot_gmap_scans(ctx_, nullptr, 0, nullptr, 0, nullptr, &m);
+        if (status_ != BSHOT_OK) return;
+        std::vector<float> p12(12 * m);
+        status_ = bshot_gmap_scans(ctx_, nullptr, 0, p12.data(), m, nullptr, &m);
+        if (status_ != BSHOT_OK) return;
+        poses.assign(m, Matrix4f::Identity());
+        for (size_t u = 0; u < m; ++u)
+            for (int row = 0; row < 3; ++row) for (int col = 0; col < 4; ++col) poses[u](row, col) = p12[12 * u + 4 * row + col];
+    }
+
     // INITIAL status, identity pose, empty map, no reference frame
     int reset() {
         if (ctx_) status_ = bshot_odometry_reset(ctx_);
@@ -101,6 +132,7 @@ public:
 private:
     bshot_ctx* ctx_ = nullptr;
     bshot_odom_params params_;
+    bshot_loop_params loop_params_;
     bshot_odom_report report_ = bshot_odom_report();
     bshot_reloc_report reloc_report_ = bshot_reloc_report();
     int min_inliers_ = 15;   // the gate's own constant (src/lidar_odometry.cpp:269-281)

@@ -156,7 +156,8 @@ int bshot_process_frame(bshot_ctx* ctx, const bshot_params* p, const float* xyz,
  * the context stream, no host copies -- the HBM-resident timing leg of bench.py. */
 int bshot_process_frame_dev(bshot_ctx* ctx, const bshot_params* p, const void* d_xyz, size_t n,
                             size_t stride_bytes);
-/* download the results of the last bshot_process_frame_dev (synchronous) */
+/* download the results of the last bshot_process_frame_dev (synchronous).  The pairs are those of the context's last
+ * matching run: a later match, step, relocalisation or loop detection replaces them */
 int bshot_fetch_frame(bshot_ctx* ctx, int top_k, int* kp_idx_out, uint64_t* bits_out, int* n_kp_out,
                       int* pairs_out, int* n_pairs_out);
 
@@ -332,6 +333,56 @@ int bshot_relocalize(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers
                      const unsigned short* distance, size_t n, const double* ring_deg, size_t nv, bshot_reloc_report* out);
 int bshot_relocalize_cloud(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const float* xyz, size_t n, size_t stride_bytes,
                            bshot_reloc_report* out);
+/* ---- loop closure: revisits of older scans in the map, as constraints for a pose-graph back end ------------------------
+ * Map updates are numbered 0, 1, 2, ... since bshot_gmap_create, bshot_gmap_reset or bshot_odometry_reset.  One update is
+ * each: odometry step that returns BSHOT_OK, accepted relocalisation, successful bshot_gmap_update_from_frame, successful
+ * bshot_gmap_add with n > 0, and successful bshot_gmap_import with n > 0 -- the imported map is update 0, with the
+ * identity pose (its entries are in the map frame), and later updates count on from 1.  Failed calls and relocalisations
+ * that are not accepted take no number.  Every map entry carries the number of the update that wrote it (an overwrite at
+ * an equal position takes the new number: its descriptor is that scan's), and the map keeps the pose each update used
+ * (the identity where it had none): the trajectory.  Neither changes what the map stores or returns.
+ * bshot_gmap_scans: entry_scan_out[e] is the update of entry e of bshot_gmap_export's order, poses3x4_out (pose_cap x 12
+ * floats, row-major [R|T]) the trajectory; *n_entries_out / *n_scans_out their lengths.  Either output may be NULL; an
+ * output whose count is above its capacity gets the first cap records and BSHOT_E_CAPACITY is returned.  With
+ * entry_scan_out and n_entries_out both NULL the map is not gathered: only the trajectory is read.  No map: BSHOT_E_STATE.  Synchronous. */
+int bshot_gmap_scans(bshot_ctx* ctx, uint32_t* entry_scan_out, size_t entry_cap, float* poses3x4_out, size_t pose_cap,
+                     size_t* n_entries_out, size_t* n_scans_out);
+
+/* bshot_detect_loop: is the last scan the odometry took (scan i, the reference frame the context holds, update i) a
+ * revisit of an older scan?  A read-only query; no extraction.  Candidates: the map entries written by updates
+ * j <= i - min_gap, in map order.  The reference frame's descriptors are matched against them (mutual nearest neighbours,
+ * the matcher chosen by size or bshot_set_matcher) -> RANSAC (sources the scan's keypoints in its sensor frame) -> T_ransac;
+ * run_icp: ICP (10 iterations, pre = T_ransac) against the candidates whose block lies in the +-map_range cube around
+ * T_ransac's translation, T_loop = ICP * T_ransac.  The candidates RANSAC's inliers point to vote with their update index:
+ * match_scan = the most frequent (the lowest on ties), votes = its count, -1 without inliers.  T_rel = T_j^-1 * T_loop
+ * (rigid inverse, T_j the trajectory's pose of match_scan; the identity when match_scan = -1) is the loop edge (j, i):
+ * scan i in scan j's frame.  accepted = n_inliers >= min_inliers.  No candidates is no error: n_candidates = 0, not
+ * accepted.  Pose, status, map, tags, trajectory, reference frame and the front end's state stay as they were.  The
+ * matcher's pair buffer is shared with every matching call: after a detection, bshot_fetch_frame's pairs are the
+ * detection's (reference frame -> candidates), as after any later matching call; the next step rewrites them.
+ * Errors: BSHOT_E_STATE without a map, or when the last update was not a step or an accepted relocalisation (no step
+ * yet, or an import / add / update_from_frame / reset / bshot_ctx_reset / bshot_frame_commit since); BSHOT_E_INVALID for min_gap < 1,
+ * min_inliers < 3 or the bounds of bshot_odom_params; BSHOT_E_CAPACITY when the ICP targets exceed max_targets. */
+typedef struct bshot_loop_params {
+    int min_gap;            /* 100: entries of updates j <= i - min_gap are candidates */
+    int min_inliers;        /* 15: accepted when at least this many correspondences survive RANSAC (>= 3) */
+    int ransac_iterations;  /* 2000 */
+    float inlier_threshold; /* 1500 mm */
+    float map_range;        /* 100000 mm: ICP targets = candidates whose block lies in this cube around T_ransac */
+    int run_icp;            /* 1 */
+} bshot_loop_params;
+void bshot_loop_params_default(bshot_loop_params* p);
+
+typedef struct bshot_loop_report {
+    float T_loop[16];       /* scan i's pose as the candidates place it: ICP * T_ransac (T_ransac without ICP), row-major */
+    float T_ransac[16];
+    float T_rel[16];        /* T_j^-1 * T_loop: scan i in scan j's frame, the loop edge (j, i) */
+    float pose[16];         /* the odometry's own pose of scan i (T_i); T_i^-1 * T_loop is the drift */
+    size_t n_candidates, n_icp_targets;
+    int scan, match_scan, votes, n_keypoints, n_pairs, n_inliers, ransac_iterations, icp_iterations, accepted;
+} bshot_loop_report;
+int bshot_detect_loop(bshot_ctx* ctx, const bshot_loop_params* p, bshot_loop_report* out);
+
 /* bshot_ransac on device buffers, asynchronous on the context stream: d_src4 / d_tgt4 float4 points (x, y, z, any),
  * d_pairs n_pairs_cap x 2 ints (index into src, index into tgt; every valid one must be in range), *d_n_pairs (int) of
  * them valid.  Outputs (device): d_inlier_pairs_out (n_pairs_cap x 2 ints), *d_n_inliers_out (int), d_transform_out
