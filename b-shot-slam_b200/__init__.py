@@ -39,7 +39,8 @@ EXPORTS = [
     "bshot_iss_params_default", "bshot_detect_iss", "bshot_kp_repeatability", "bshot_voxel_grid",
     "bshot_odom_params_default", "bshot_odometry_step", "bshot_odometry_step_cloud", "bshot_odometry_reset", "bshot_ransac_dev",
     "bshot_gmap_export", "bshot_gmap_import", "bshot_relocalize", "bshot_relocalize_cloud",
-    "bshot_gmap_scans", "bshot_loop_params_default", "bshot_detect_loop",
+    "bshot_gmap_scans", "bshot_loop_params_default", "bshot_detect_loop", "bshot_gmap_reanchor",
+    "bshot_graph_params_default", "bshot_optimize_trajectory",
 ]
 
 
@@ -75,6 +76,21 @@ class RelocReport(C.Structure):
 class LoopParams(C.Structure):
     _fields_ = [("min_gap", C.c_int), ("min_inliers", C.c_int), ("ransac_iterations", C.c_int), ("inlier_threshold", C.c_float),
                 ("map_range", C.c_float), ("run_icp", C.c_int)]
+
+
+class GraphEdge(C.Structure):
+    _fields_ = [("from_", C.c_int32), ("to", C.c_int32), ("T", C.c_float * 16)]
+
+
+class GraphParams(C.Structure):
+    _fields_ = [("odom_sigma_mm", C.c_float), ("odom_sigma_deg", C.c_float), ("loop_sigma_mm", C.c_float), ("loop_sigma_deg", C.c_float),
+                ("max_iterations", C.c_int), ("max_cg_iterations", C.c_int), ("grad_tolerance", C.c_double), ("step_tolerance", C.c_double),
+                ("cg_tolerance", C.c_double)]
+
+
+class GraphReport(C.Structure):
+    _fields_ = [("n_nodes", C.c_int), ("n_edges", C.c_int), ("iterations", C.c_int), ("cg_iterations", C.c_int), ("status", C.c_int),
+                ("cost_initial", C.c_double), ("cost_final", C.c_double), ("grad_inf_final", C.c_double)]
 
 
 class LoopReport(C.Structure):
@@ -203,6 +219,10 @@ def lib():
         L.bshot_loop_params_default.argtypes = [C.POINTER(LoopParams)]
         L.bshot_loop_params_default.restype = None
         L.bshot_detect_loop.argtypes = [vp, C.POINTER(LoopParams), C.POINTER(LoopReport)]
+        L.bshot_gmap_reanchor.argtypes = [vp, vp, sz, vp]
+        L.bshot_graph_params_default.argtypes = [C.POINTER(GraphParams)]
+        L.bshot_graph_params_default.restype = None
+        L.bshot_optimize_trajectory.argtypes = [vp, vp, sz, C.POINTER(GraphParams), vp, sz, vp, C.POINTER(GraphReport)]
         _LIB = L
     return _LIB
 
@@ -249,6 +269,17 @@ def odom_default_params(**kw):
             setattr(p.front, k, v)
         else:
             raise AttributeError(k)
+    return p
+
+
+def graph_params_default(**kw):
+    """parameters of bshot_optimize_trajectory; keyword arguments override fields"""
+    p = GraphParams()
+    lib().bshot_graph_params_default(C.byref(p))
+    for k, v in kw.items():
+        if not hasattr(p, k):
+            raise AttributeError(k)
+        setattr(p, k, v)
     return p
 
 
@@ -720,6 +751,54 @@ class Context:
         r = LoopReport()
         _chk(lib().bshot_detect_loop(self.h, C.byref(params), C.byref(r)))
         return _report(r)
+
+    def gmap_reanchor(self, poses):
+        """move the map to a corrected trajectory: poses (n, 4, 4) or (n, 3, 4), the corrected pose of every map update
+        (n = len(gmap_scans()[1])).  Each entry moves by T'_u * T_u^-1 of the update u that wrote it; the trajectory
+        becomes poses.  Returns the odometry's new pose (4 x 4 float32)"""
+        p = np.asarray(poses, dtype=np.float32)
+        if p.ndim != 3 or p.shape[1:] not in ((4, 4), (3, 4)):
+            raise BshotError("gmap_reanchor: poses of shape (n, 4, 4) or (n, 3, 4) expected", E_INVALID)
+        p12 = np.ascontiguousarray(p[:, :3, :])
+        pose = np.empty((4, 4), np.float32)
+        _chk(lib().bshot_gmap_reanchor(self.h, _p(p12), p12.shape[0], _p(pose)))
+        return pose
+
+    def optimize_trajectory(self, loops, params=None):
+        """the trajectory's pose graph with these loop edges, optimised on the device (read only).  loops: detect_loop
+        report dicts (edge (match_scan, scan), measurement T_rel) or (from, to, T 4 x 4) tuples.  Returns a dict: poses
+        (n, 4, 4) float32, loop_cost (L,) float64 and the report fields"""
+        params = graph_params_default() if params is None else params
+        edges = (GraphEdge * max(len(loops), 1))()
+        for k, e in enumerate(loops):
+            if isinstance(e, dict):
+                f, t, T = e["match_scan"], e["scan"], e["T_rel"]
+            else:
+                f, t, T = e
+            edges[k].from_, edges[k].to = int(f), int(t)
+            edges[k].T[:] = [float(v) for v in np.asarray(T, np.float32).reshape(16)]
+        n = len(self.gmap_scans_poses())
+        p12 = np.empty((max(n, 1), 3, 4), np.float32)
+        cost = np.empty(max(len(loops), 1), np.float64)
+        r = GraphReport()
+        _chk(lib().bshot_optimize_trajectory(self.h, C.cast(edges, C.c_void_p), len(loops), C.byref(params), _p(p12), n, _p(cost), C.byref(r)))
+        poses = np.zeros((n, 4, 4), np.float32)
+        poses[:, :3] = p12[:n]
+        poses[:, 3, 3] = 1.0
+        out = {name: getattr(r, name) for name, _ in GraphReport._fields_}
+        out.update(poses=poses, loop_cost=cost[:len(loops)].copy())
+        return out
+
+    def gmap_scans_poses(self):
+        """the trajectory alone (no map gather) -> (m, 4, 4) float32"""
+        m = C.c_size_t()
+        _chk(lib().bshot_gmap_scans(self.h, None, 0, None, 0, None, C.byref(m)))
+        p12 = np.empty((m.value, 3, 4), np.float32)
+        _chk(lib().bshot_gmap_scans(self.h, None, 0, _p(p12), m.value, None, C.byref(m)))
+        poses = np.zeros((m.value, 4, 4), np.float32)
+        poses[:, :3] = p12
+        poses[:, 3, 3] = 1.0
+        return poses
 
     def odometry_reset(self):
         """INITIAL status, identity pose, empty map, no reference frame"""

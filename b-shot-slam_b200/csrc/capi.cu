@@ -807,6 +807,73 @@ int bshot_gmap_scans(bshot_ctx* ctx, uint32_t* entry_scan_out, size_t entry_cap,
     return gmap_scans(ctx, entry_scan_out, entry_cap, poses3x4_out, pose_cap, n_entries_out, n_scans_out);
 }
 
+// a finite rigid [R|T] (row-major, rows 4 floats apart): max |R^T R - I| <= 1e-3 and det R > 0
+static bool rigid_ok(const float* T, const char* who, const char* what, size_t index) {
+    for (int r = 0; r < 3; ++r)
+        for (int e = 0; e < 4; ++e)
+            if (!std::isfinite(T[4 * r + e])) { set_error("%s: %s %zu is not finite", who, what, index); return false; }
+    double R[3][3], dev = 0.0;
+    for (int i = 0; i < 3; ++i) for (int j = 0; j < 3; ++j) R[i][j] = T[4 * i + j];
+    for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) {
+            const double d = R[0][i] * R[0][j] + R[1][i] * R[1][j] + R[2][i] * R[2][j] - (i == j ? 1.0 : 0.0);
+            dev = std::max(dev, std::fabs(d));
+        }
+    const double det = R[0][0] * (R[1][1] * R[2][2] - R[1][2] * R[2][1]) - R[0][1] * (R[1][0] * R[2][2] - R[1][2] * R[2][0]) +
+                       R[0][2] * (R[1][0] * R[2][1] - R[1][1] * R[2][0]);
+    if (dev > 1e-3 || !(det > 0.0)) { set_error("%s: %s %zu is not a rotation (|R^T R - I| %.3g, det %.3g)", who, what, index, dev, det); return false; }
+    return true;
+}
+
+int bshot_gmap_reanchor(bshot_ctx* ctx, const float* poses3x4, size_t n, float* pose_out) {
+    CHECK_CTX(ctx);
+    if (!ctx->gmap.d_tab) { set_error("bshot_gmap_reanchor: no map (bshot_gmap_create)"); return BSHOT_E_STATE; }
+    if (n != ctx->gmap.n_updates) { set_error("bshot_gmap_reanchor: %zu poses for %u map updates", n, ctx->gmap.n_updates); return BSHOT_E_INVALID; }
+    if (n && !poses3x4) { set_error("bshot_gmap_reanchor: null poses"); return BSHOT_E_INVALID; }
+    for (size_t u = 0; u < n; ++u)
+        if (!rigid_ok(poses3x4 + 12 * u, "bshot_gmap_reanchor", "pose", u)) return BSHOT_E_INVALID;
+    return reanchor_run(ctx, poses3x4, n, pose_out);
+}
+
+void bshot_graph_params_default(bshot_graph_params* p) {
+    if (!p) return;
+    p->odom_sigma_mm = 20.0f;
+    p->odom_sigma_deg = 0.1f;
+    p->loop_sigma_mm = 100.0f;
+    p->loop_sigma_deg = 1.0f;
+    p->max_iterations = 50;
+    p->max_cg_iterations = 2000;
+    p->grad_tolerance = 1e-6;
+    p->step_tolerance = 1e-9;
+    p->cg_tolerance = 1e-10;
+}
+
+int bshot_optimize_trajectory(bshot_ctx* ctx, const bshot_graph_edge* loops, size_t n_loops, const bshot_graph_params* p, float* poses3x4_out,
+                              size_t pose_cap, double* loop_cost_out, bshot_graph_report* out) {
+    CHECK_CTX(ctx);
+    const char* who = "bshot_optimize_trajectory";
+    bshot_graph_params dp;
+    if (!p) { bshot_graph_params_default(&dp); p = &dp; }
+    if (!ctx->gmap.d_tab) { set_error("%s: no map (bshot_gmap_create)", who); return BSHOT_E_STATE; }
+    const float sig[4] = {p->odom_sigma_mm, p->odom_sigma_deg, p->loop_sigma_mm, p->loop_sigma_deg};
+    for (float s : sig) if (!(s > 0.0f) || !std::isfinite(s)) { set_error("%s: every sigma must be finite and > 0", who); return BSHOT_E_INVALID; }
+    if (p->max_iterations < 0 || p->max_cg_iterations < 0) { set_error("%s: negative iteration count", who); return BSHOT_E_INVALID; }
+    if (!(p->grad_tolerance >= 0.0) || !(p->step_tolerance >= 0.0) || !(p->cg_tolerance >= 0.0)) { set_error("%s: negative tolerance", who); return BSHOT_E_INVALID; }
+    if (n_loops && !loops) { set_error("%s: null loop edges", who); return BSHOT_E_INVALID; }
+    if (n_loops > 0x7FFFFFFFull) { set_error("%s: too many loop edges", who); return BSHOT_E_INVALID; }
+    const size_t n = ctx->gmap.n_updates;
+    for (size_t k = 0; k < n_loops; ++k) {
+        const bshot_graph_edge& e = loops[k];
+        if (e.from < 0 || e.to < 0 || (size_t)e.from >= n || (size_t)e.to >= n || e.from == e.to) {
+            set_error("%s: loop edge %zu (%d, %d) outside [0, %zu) or a self-loop", who, k, e.from, e.to, n);
+            return BSHOT_E_INVALID;
+        }
+        if (!rigid_ok(e.T, who, "loop edge", k)) return BSHOT_E_INVALID;
+    }
+    if (pose_cap < n || (n && !poses3x4_out)) { set_error("%s: %zu nodes > pose capacity %zu", who, n, pose_cap); return BSHOT_E_CAPACITY; }
+    return pose_graph_run(ctx, loops, n_loops, p, poses3x4_out, loop_cost_out, out);
+}
+
 int bshot_extract_frame(bshot_ctx* ctx, const bshot_params* p, const float* xyz, size_t n, size_t stride_bytes, int* kp_idx_out, float* kp_xyz_out,
                         float* seg_ratio_out, uint64_t* bits_out, int* n_kp_out) {
     CHECK_CTX(ctx);

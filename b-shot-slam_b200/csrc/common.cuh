@@ -120,6 +120,11 @@ struct Gmap {
     unsigned* d_ltile = nullptr;        // 2 x ltile_cap
     size_t ltile_cap = 0;
     unsigned* d_lctl = nullptr;         // [0] candidates [1] candidates (uncapped) [2] ICP targets (<= max_targets) [3] ICP targets (uncapped)
+    // re-anchoring (bshot_gmap_reanchor), allocated by the first call
+    float* d_rtraj = nullptr;           // rcap x 12: the new trajectory
+    float* d_rcorr = nullptr;           // rcap x 12 corrections C_u, then the odometry's new pose (16)
+    unsigned* d_rchg = nullptr;         // rcap flags: update u changed; then the count of entries to rebuild
+    size_t rcap = 0;
 };
 
 // ISS keypoints (iss.cu): max_points-sized buffers, allocated by the first bshot_detect_iss of the context

@@ -323,15 +323,18 @@ gm_block_offsets_kernel(const GmapBlock* __restrict__ tab, const unsigned* __res
     if (threadIdx.x == 0) actl[1] = carry;
 }
 
-// import: the entries already sit at pool index = input index.  Block slot of every entry (created when new), its count,
-// and (slot, input index) for the stable sort by slot
-__global__ void gm_import_find_kernel(const float4* __restrict__ e_pos, unsigned n, GmapBlock* tab, unsigned mask, unsigned long long* __restrict__ keys,
-                                      unsigned* __restrict__ idx, unsigned* __restrict__ actl, unsigned* __restrict__ e_tag, float* __restrict__ traj) {
+// import: the entries already sit at pool index = input index (*d_n of them, n_cap without a device count).  Block slot
+// of every entry (created when new), its count, and (slot, input index) for the stable sort by slot.  Tags from tag_src
+// (null: 0); with traj the trajectory's update 0 becomes the identity
+__global__ void gm_import_find_kernel(const float4* __restrict__ e_pos, unsigned n_cap, const unsigned* __restrict__ d_n, GmapBlock* tab, unsigned mask,
+                                      unsigned long long* __restrict__ keys, unsigned* __restrict__ idx, unsigned* __restrict__ actl,
+                                      const unsigned* __restrict__ tag_src, unsigned* __restrict__ e_tag, float* __restrict__ traj) {
     const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned n = d_n ? min(*d_n, n_cap) : n_cap;
     if (i == 0) actl[3] = n;
-    if (i < 12) traj[i] = (i % 5 == 0) ? 1.0f : 0.0f;   // the import is update 0, in the map frame
+    if (traj && i < 12) traj[i] = (i % 5 == 0) ? 1.0f : 0.0f;   // the import is update 0, in the map frame
     if (i >= n) return;
-    e_tag[i] = 0u;
+    e_tag[i] = tag_src ? tag_src[i] : 0u;
     const float4 p = e_pos[i];
     unsigned slot = 0xFFFFFFFFu;
     if (!(isfinite(p.x) && isfinite(p.y) && isfinite(p.z))) atomicOr(&actl[2], 1u);
@@ -342,7 +345,8 @@ __global__ void gm_import_find_kernel(const float4* __restrict__ e_pos, unsigned
 }
 
 // import, one CTA over every table slot in slot order: first entry of the slot in the slot-sorted list (start) and
-// ceil(count / 32) consecutive chunks, first / last of the block; then the control words
+// ceil(count / 32) consecutive chunks, first / last of the block; then the entry and chunk counts (the dropped count
+// ctl[3] stays: a re-anchor keeps it, an import starts from a reset map)
 __global__ void __launch_bounds__(1024)
 gm_import_blocks_kernel(GmapBlock* tab, unsigned tab_cap, unsigned* __restrict__ start, unsigned* __restrict__ ctl, unsigned* __restrict__ actl,
                         unsigned max_chunks) {
@@ -362,22 +366,48 @@ gm_import_blocks_kernel(GmapBlock* tab, unsigned tab_cap, unsigned* __restrict__
         if (carry_c > max_chunks) actl[2] |= 2u;
         ctl[0] = carry_e;
         ctl[2] = carry_c;
-        ctl[3] = 0u;
     }
 }
 
-// import: sorted position j -> rank r in its block -> chunk first + r / 32, lane r % 32; a chunk's first entry links it
-__global__ void gm_import_chain_kernel(const unsigned long long* __restrict__ slot_of, const unsigned* __restrict__ idx, unsigned n,
+// import: sorted position j -> rank r in its block -> chunk first + r / 32, lane r % 32; a chunk's first entry links it.
+// *d_n entries (gm_import_find_kernel's count)
+__global__ void gm_import_chain_kernel(const unsigned long long* __restrict__ slot_of, const unsigned* __restrict__ idx, const unsigned* __restrict__ d_n,
                                        const GmapBlock* __restrict__ tab, unsigned tab_cap, const unsigned* __restrict__ start,
                                        unsigned* __restrict__ chunks, unsigned max_chunks) {
     const unsigned j = blockIdx.x * blockDim.x + threadIdx.x;
-    if (j >= n) return;
+    if (j >= *d_n) return;
     const unsigned long long s = slot_of[j];
     if (s >= tab_cap) return;   // an entry without a block: the import fails
     const unsigned r = j - start[s], cnt = tab[s].count, ch = tab[s].first + r / 32u;
     if (ch >= max_chunks) return;
     chunks[ch * 33u + (r & 31u)] = idx[j];
     if ((r & 31u) == 0u) chunks[ch * 33u + 32u] = r + 32u < cnt ? ch + 1u : 0xFFFFFFFFu;
+}
+
+// re-anchor: the whole map in map order (*d_n entries), each entry of a changed update u moved by that update's correction
+// C_u (row-major 3x4) with gm_prepare_kernel's arithmetic and snapped to the lattice as createKeypoint does; the entries of
+// unchanged updates are copied as they are.  Written straight into the entry pool at pool index = map-order index, with
+// their descriptors, where the rebuild reads them; *n_out = the count, for the rebuild
+__global__ void gm_reanchor_move_kernel(const float4* __restrict__ apos, const uint64_t* __restrict__ adesc, const unsigned* __restrict__ atag,
+                                        const unsigned* __restrict__ d_n, unsigned n_cap, const float* __restrict__ corr, const unsigned* __restrict__ changed,
+                                        unsigned n_upd, float4* __restrict__ e_pos, uint64_t* __restrict__ e_desc, unsigned* __restrict__ n_out) {
+    const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
+    const unsigned n = min(*d_n, n_cap);
+    if (i == 0) *n_out = n;
+    if (i >= n) return;
+#pragma unroll
+    for (int k = 0; k < 6; ++k) e_desc[(size_t)i * 6 + k] = adesc[(size_t)i * 6 + k];
+    const float4 p = apos[i];
+    const unsigned u = atag[i];
+    if (u >= n_upd || !changed[u]) { e_pos[i] = p; return; }
+    const float* C = corr + (size_t)u * 12;
+    float x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[0], p.x), __fmul_rn(C[1], p.y)), __fmul_rn(C[2], p.z)), C[3]);
+    float y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[4], p.x), __fmul_rn(C[5], p.y)), __fmul_rn(C[6], p.z)), C[7]);
+    float z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[8], p.x), __fmul_rn(C[9], p.y)), __fmul_rn(C[10], p.z)), C[11]);
+    x = (float)((int)truncf(x / GM_LATTICE) * (int)GM_LATTICE);
+    y = (float)((int)truncf(y / GM_LATTICE) * (int)GM_LATTICE);
+    z = (float)((int)truncf(z / GM_LATTICE) * (int)GM_LATTICE);
+    e_pos[i] = make_float4(x, y, z, p.w);
 }
 
 // ---- host side -----------------------------------------------------------------------------------------------------------
@@ -412,7 +442,7 @@ void gmap_free(Ctx* c) {
     Gmap& g = c->gmap;
     void* ptrs[] = {g.d_tab, g.d_epos, g.d_edesc, g.d_chunks, g.d_world, g.d_blk_of, g.d_touched, g.d_probe_slot, g.d_probe_off, g.d_ctl, g.d_pose, g.d_tpos,
                     g.d_apos, g.d_adesc, g.d_skeys[0], g.d_skeys[1], g.d_svals[0], g.d_svals[1], g.d_shist, g.d_boff, g.d_actl,
-                    g.d_etag, g.d_traj, g.d_atag, g.d_lpos, g.d_ldesc, g.d_ltag, g.d_ltile, g.d_lctl};
+                    g.d_etag, g.d_traj, g.d_atag, g.d_lpos, g.d_ldesc, g.d_ltag, g.d_ltile, g.d_lctl, g.d_rtraj, g.d_rcorr, g.d_rchg};
     for (void* p : ptrs) if (p) cudaFree(p);
     g = Gmap();
 }
@@ -542,6 +572,37 @@ int gmap_export(Ctx* c, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t*
     return BSHOT_OK;
 }
 
+int gmap_import_dev(Ctx* c, const float4* d_pos, const uint64_t* d_desc, const unsigned* d_tag, size_t n_cap, const unsigned* d_n, const char* who) {
+    Gmap& g = c->gmap;
+    BSHOT_TRY(gmap_all_alloc(c));
+    const unsigned nn = (unsigned)n_cap;
+    GmapBlock* tab = reinterpret_cast<GmapBlock*>(g.d_tab);
+    BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_tab, 0, sizeof(GmapBlock) * g.tab_cap, c->stream));
+    BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_actl, 0, sizeof(unsigned) * 8, c->stream));
+    if (d_pos != g.d_epos) BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_epos, d_pos, sizeof(float4) * n_cap, cudaMemcpyDeviceToDevice, c->stream));
+    if (d_desc != g.d_edesc) BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_edesc, d_desc, 48 * n_cap, cudaMemcpyDeviceToDevice, c->stream));
+    gm_import_find_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_epos, nn, d_n, tab, g.tab_cap - 1, g.d_skeys[0], g.d_svals[0], g.d_actl, d_tag, g.d_etag,
+                                                                    d_tag ? nullptr : g.d_traj);
+    count_launch(c);
+    BSHOT_TRY(check_launch("gm_import_find_kernel"));
+    // stable by slot: the input order survives inside a block.  Slots are < tab_cap (a power of two)
+    unsigned bits = 0;
+    while ((1u << bits) < g.tab_cap) ++bits;
+    const unsigned passes = (bits + 7) / 8;
+    BSHOT_TRY(radix_sort_pairs(c, g.d_skeys, g.d_svals, g.d_shist, g.d_actl + 3, n_cap, passes));
+    gm_import_blocks_kernel<<<1, 1024, 0, c->stream>>>(tab, g.tab_cap, g.d_boff, g.d_ctl, g.d_actl, g.max_chunks);
+    gm_import_chain_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_skeys[passes & 1], g.d_svals[passes & 1], g.d_actl + 3, tab, g.tab_cap, g.d_boff,
+                                                                    g.d_chunks, g.max_chunks);
+    count_launch(c, 2);
+    BSHOT_TRY(check_launch("map import kernels"));
+    unsigned* h = reinterpret_cast<unsigned*>(&c->h_scratch[48]);
+    BSHOT_CUDA_TRY(cudaMemcpyAsync(h, g.d_actl, sizeof(unsigned) * 4, cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
+    if (h[2] & 1u) { set_error("%s: non-finite position", who); return BSHOT_E_INVALID; }
+    if (h[2]) { set_error("%s: more blocks or chunks than the map holds (%u slots, %u chunks)", who, g.tab_cap, g.max_chunks); return BSHOT_E_CAPACITY; }
+    return BSHOT_OK;
+}
+
 int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n) {
     Gmap& g = c->gmap;
     if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
@@ -553,39 +614,66 @@ int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n) {
         return BSHOT_E_CAPACITY;
     }
     if (n == 0) { BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream)); return BSHOT_OK; }
-    BSHOT_TRY(gmap_all_alloc(c));
-    const unsigned nn = (unsigned)n;
-    GmapBlock* tab = reinterpret_cast<GmapBlock*>(g.d_tab);
-    BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_actl, 0, sizeof(unsigned) * 8, c->stream));
     BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_epos, xyzr, sizeof(float4) * n, cudaMemcpyHostToDevice, c->stream));
     BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_edesc, desc, 48 * n, cudaMemcpyHostToDevice, c->stream));
-    gm_import_find_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_epos, nn, tab, g.tab_cap - 1, g.d_skeys[0], g.d_svals[0], g.d_actl, g.d_etag,
-                                                                    g.d_traj);
-    count_launch(c);
-    BSHOT_TRY(check_launch("gm_import_find_kernel"));
-    // stable by slot: the input order survives inside a block.  Slots are < tab_cap (a power of two)
-    unsigned bits = 0;
-    while ((1u << bits) < g.tab_cap) ++bits;
-    const unsigned passes = (bits + 7) / 8;
-    BSHOT_TRY(radix_sort_pairs(c, g.d_skeys, g.d_svals, g.d_shist, g.d_actl + 3, n, passes));
-    gm_import_blocks_kernel<<<1, 1024, 0, c->stream>>>(tab, g.tab_cap, g.d_boff, g.d_ctl, g.d_actl, g.max_chunks);
-    gm_import_chain_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_skeys[passes & 1], g.d_svals[passes & 1], nn, tab, g.tab_cap, g.d_boff, g.d_chunks,
-                                                                    g.max_chunks);
-    count_launch(c, 2);
-    BSHOT_TRY(check_launch("map import kernels"));
-    unsigned* h = reinterpret_cast<unsigned*>(&c->h_scratch[48]);
-    BSHOT_CUDA_TRY(cudaMemcpyAsync(h, g.d_actl, sizeof(unsigned) * 4, cudaMemcpyDeviceToHost, c->stream));
-    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
-    if (h[2]) {
-        const int rc = (h[2] & 1u) ? BSHOT_E_INVALID : BSHOT_E_CAPACITY;
+    const int rc = gmap_import_dev(c, g.d_epos, g.d_edesc, nullptr, n, nullptr, "bshot_gmap_import");
+    if (rc == BSHOT_E_INVALID || rc == BSHOT_E_CAPACITY) {   // an empty map
         BSHOT_TRY(gmap_reset(c));
         BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
-        if (rc == BSHOT_E_INVALID) set_error("bshot_gmap_import: non-finite position");
-        else set_error("bshot_gmap_import: more blocks or chunks than the map holds (%u slots, %u chunks)", g.tab_cap, g.max_chunks);
         return rc;
     }
+    BSHOT_TRY(rc);
     g.entries_upper = n;
     g.n_updates = 1;
+    return BSHOT_OK;
+}
+
+// re-anchor (bshot_gmap_reanchor): the whole map in map order with its tags, every entry moved by the correction of the
+// update that wrote it into the entry pool, and the table rebuilt from there in that order.  When the moved map does not
+// fit, the table is rebuilt from the untouched gather buffers: export order makes that the map as it was.  Then the trajectory
+// becomes poses3x4 and the pose d_pose (16 floats) the one reanchor_corrections derived
+int gmap_reanchor(Ctx* c, const float* poses3x4, size_t n, float* d_pose, float* pose_out) {
+    Gmap& g = c->gmap;
+    if (n) {
+        if (g.rcap < n) {   // sized like the trajectory, which grows by doubling
+            const size_t cap = std::max<size_t>(g.traj_cap, n);
+            void* old[] = {g.d_rtraj, g.d_rcorr, g.d_rchg};
+            for (void* p : old) if (p) cudaFree(p);
+            g.d_rtraj = g.d_rcorr = nullptr;
+            g.d_rchg = nullptr;
+            g.rcap = 0;
+            BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_rtraj, sizeof(float) * 12 * cap));
+            BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_rcorr, sizeof(float) * (12 * cap + 16)));
+            BSHOT_CUDA_TRY(cudaMalloc((void**)&g.d_rchg, sizeof(unsigned) * (cap + 1)));
+            g.rcap = cap;
+        }
+        float* d_pose_new = g.d_rcorr + 12 * g.rcap;
+        unsigned* d_count = g.d_rchg + g.rcap;
+        BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_rtraj, poses3x4, sizeof(float) * 12 * n, cudaMemcpyHostToDevice, c->stream));
+        BSHOT_TRY(reanchor_corrections(c, g.d_traj, g.d_rtraj, (unsigned)n, g.d_rcorr, g.d_rchg, d_pose, d_pose_new));
+        size_t nt_cap;
+        BSHOT_TRY(gmap_gather_all(c, &nt_cap, /*with_tags=*/true));
+        if (nt_cap) {
+            const unsigned nn = (unsigned)nt_cap;
+            gm_reanchor_move_kernel<<<(nn + 255) / 256, 256, 0, c->stream>>>(g.d_apos, g.d_adesc, g.d_atag, g.d_actl + 1, nn, g.d_rcorr, g.d_rchg, (unsigned)n,
+                                                                              g.d_epos, g.d_edesc, d_count);
+            count_launch(c);
+            BSHOT_TRY(check_launch("gm_reanchor_move_kernel"));
+            const int rc = gmap_import_dev(c, g.d_epos, g.d_edesc, g.d_atag, nt_cap, d_count, "bshot_gmap_reanchor");
+            if (rc == BSHOT_E_INVALID || rc == BSHOT_E_CAPACITY) {
+                BSHOT_TRY(gmap_import_dev(c, g.d_apos, g.d_adesc, g.d_atag, nt_cap, d_count, "bshot_gmap_reanchor (restoring the map)"));
+                if (rc == BSHOT_E_INVALID) set_error("bshot_gmap_reanchor: a moved entry is not finite; nothing changed");
+                else set_error("bshot_gmap_reanchor: the moved map needs more blocks or chunks than the map holds (%u slots, %u chunks); nothing changed",
+                               g.tab_cap, g.max_chunks);
+                return rc;
+            }
+            BSHOT_TRY(rc);
+        }
+        BSHOT_CUDA_TRY(cudaMemcpyAsync(g.d_traj, g.d_rtraj, sizeof(float) * 12 * n, cudaMemcpyDeviceToDevice, c->stream));
+        BSHOT_CUDA_TRY(cudaMemcpyAsync(d_pose, d_pose_new, sizeof(float) * 16, cudaMemcpyDeviceToDevice, c->stream));
+    }
+    if (pose_out) BSHOT_CUDA_TRY(cudaMemcpyAsync(pose_out, d_pose, sizeof(float) * 16, cudaMemcpyDeviceToHost, c->stream));
+    BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
     return BSHOT_OK;
 }
 

@@ -172,6 +172,46 @@ loop_final_kernel(LoopDev* d, const IcpState* __restrict__ icp, int run_icp, int
     r.accepted = (d->err == 0 && d->n_inliers >= min_inliers) ? 1 : 0;
 }
 
+// re-anchoring: one thread per update.  An update whose new pose equals its old one bit for bit is unchanged (its entries
+// and, for the last update, the odometry's pose stay); otherwise C_u = T'_u * T_u^-1 in fp32 (odom_math.cuh, no FMA)
+__global__ void reanchor_corr_kernel(const float* __restrict__ traj, const float* __restrict__ traj_new, unsigned n, float* __restrict__ corr,
+                                     unsigned* __restrict__ changed, const float* __restrict__ pose, float* __restrict__ pose_new) {
+    const unsigned u = blockIdx.x * blockDim.x + threadIdx.x;
+    if (u >= n) return;
+    float T[16], Tn[16], T_inv[16], C[16];
+    bool chg = false;
+    for (int e = 0; e < 16; ++e) {
+        T[e] = e < 12 ? traj[(size_t)u * 12 + e] : (e == 15 ? 1.0f : 0.0f);
+        Tn[e] = e < 12 ? traj_new[(size_t)u * 12 + e] : T[e];
+        chg = chg || __float_as_uint(T[e]) != __float_as_uint(Tn[e]);
+    }
+    changed[u] = chg ? 1u : 0u;
+    if (chg) {
+        rigid_inverse4x4(T, T_inv);
+        mul4x4(Tn, T_inv, C);
+        for (int e = 0; e < 12; ++e) corr[(size_t)u * 12 + e] = C[e];
+    }
+    if (u != n - 1) return;
+    bool at_last = true;   // the pose is the last update's (the case after a step)
+    for (int e = 0; e < 12; ++e) at_last = at_last && __float_as_uint(pose[e]) == __float_as_uint(T[e]);
+    float P[16];
+    if (!chg) for (int e = 0; e < 16; ++e) P[e] = pose[e];
+    else if (at_last) for (int e = 0; e < 16; ++e) P[e] = Tn[e];
+    else mul4x4(C, pose, P);
+    for (int e = 0; e < 16; ++e) pose_new[e] = P[e];
+}
+
+int reanchor_corrections(Ctx* c, const float* d_traj, const float* d_new, unsigned n, float* d_corr, unsigned* d_changed, const float* d_pose, float* d_pose_new) {
+    reanchor_corr_kernel<<<(n + 127) / 128, 128, 0, c->stream>>>(d_traj, d_new, n, d_corr, d_changed, d_pose, d_pose_new);
+    count_launch(c);
+    return check_launch("reanchor_corr_kernel");
+}
+
+int reanchor_run(Ctx* c, const float* poses3x4, size_t n, float* pose_out) {
+    BSHOT_TRY(odom_ensure(c));
+    return gmap_reanchor(c, poses3x4, n, c->odom.d->pose, pose_out);
+}
+
 int odom_ensure(Ctx* c) {
     Odom& o = c->odom;
     if (o.d) return BSHOT_OK;

@@ -75,6 +75,13 @@ int gmap_gather_all(Ctx* c, size_t* nt_cap_out, bool with_tags = false);
 // the map by n entries without the admission rule, keeping the input order inside each block (an empty map on any error)
 int gmap_export(Ctx* c, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t* n_out);
 int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n);
+// the import's device core, synchronous: rebuilds the table from d_pos / d_desc (*d_n entries, n_cap without a device
+// count) in their order, without the admission rule.  d_tag null: every tag 0 and the trajectory's update 0 the identity
+// (an import); otherwise the tags from d_tag and the trajectory untouched.  Host state (update count, bounds) is the
+// caller's; on BSHOT_E_INVALID / BSHOT_E_CAPACITY (messages prefixed by who) the table is unusable until rebuilt or reset
+int gmap_import_dev(Ctx* c, const float4* d_pos, const uint64_t* d_desc, const unsigned* d_tag, size_t n_cap, const unsigned* d_n, const char* who);
+// bshot_gmap_reanchor's work (synchronous), n == the update count, checked by the caller; d_pose: the odometry's pose
+int gmap_reanchor(Ctx* c, const float* poses3x4, size_t n, float* d_pose, float* pose_out);
 // synchronous: the entries' tags in export order and the trajectory (bshot_gmap_scans)
 int gmap_scans(Ctx* c, uint32_t* entry_scan_out, size_t entry_cap, float* poses3x4_out, size_t pose_cap, size_t* n_entries_out, size_t* n_scans_out);
 // loop closure, asynchronous: the whole map in map order with tags, then the entries with tag + min_gap <= scan, in map order
@@ -142,6 +149,15 @@ int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_
 int relocalize_run(Ctx* c, const bshot_odom_params* p, int min_inliers, const float* d_cloud, size_t n, int stride_floats, bshot_reloc_report* out);
 // loop detection on the reference frame against the map's older entries (odometry.cu); reads, never changes, the odometry's state
 int loop_run(Ctx* c, const bshot_loop_params* p, bshot_loop_report* out);
+// re-anchoring (odometry.cu, without FMA): per update u of n, changed[u] = d_new's pose differs from d_traj's in any bit,
+// and then corr[u] = T'_u * T_u^-1 (row-major 3x4); pose_new = the odometry's pose d_pose moved by update n - 1's
+// correction (T'_{n-1} itself when d_pose is T_{n-1}).  Asynchronous
+int reanchor_corrections(Ctx* c, const float* d_traj, const float* d_new, unsigned n, float* d_corr, unsigned* d_changed, const float* d_pose, float* d_pose_new);
+// bshot_optimize_trajectory on the map's trajectory (posegraph.cu), inputs checked by the caller; synchronous
+int pose_graph_run(Ctx* c, const bshot_graph_edge* loops, size_t n_loops, const bshot_graph_params* p, float* poses_out, double* loop_cost_out,
+                   bshot_graph_report* out);
+// bshot_gmap_reanchor on the odometry's pose (gmap_reanchor)
+int reanchor_run(Ctx* c, const float* poses3x4, size_t n, float* pose_out);
 
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);

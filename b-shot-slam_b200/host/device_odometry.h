@@ -4,7 +4,7 @@
 // LidarOdometry and its reference-named stage methods stay available for callers that want the stages one by one.
 // relocalize() finds a rotation in the whole map without a prior pose; exportMap / importMap save and restore the map.
 // detectLoop() asks whether the last rotation revisits an older one; trajectory() and the loop report's T_rel are the nodes
-// and edges a pose-graph back end takes.
+// and edges a pose-graph back end takes; reanchor() moves the map and the pose to the trajectory the back end returns.
 #ifndef BSHOT_B200_HOST_DEVICE_ODOMETRY_H
 #define BSHOT_B200_HOST_DEVICE_ODOMETRY_H
 
@@ -24,6 +24,7 @@ public:
                             size_t max_map = 1u << 16, size_t max_blocks = 4096) {
         bshot_odom_params_default(&params_);
         bshot_loop_params_default(&loop_params_);
+        bshot_graph_params_default(&graph_params_);
         status_ = bshot_ctx_create(&ctx_, device, max_points, max_keypoints, max_targets);
         if (status_ == BSHOT_OK) status_ = bshot_gmap_create(ctx_, max_map, max_blocks);
     }
@@ -51,6 +52,8 @@ public:
     }
 
     const bshot_odom_report& report() const { return report_; }
+    // the pose the last step(), accepted relocalize() or reanchor() set
+    const Matrix4f& pose() const { return pose_; }
 
     // relocalisation of one rotation against the whole map (no prior pose): true when at least min_inliers() RANSAC inliers
     // survived; then pose_ is the new pose and the next step() continues in the map frame.  Otherwise nothing changes.
@@ -118,6 +121,48 @@ public:
             for (int row = 0; row < 3; ++row) for (int col = 0; col < 4; ++col) poses[u](row, col) = p12[12 * u + 4 * row + col];
     }
 
+    // move the map, the trajectory and the pose to a corrected trajectory (one pose per map update, in update order, as a
+    // pose-graph back end returns it from trajectory() and the loop edges; bshot_gmap_reanchor).  On success pose_ is the
+    // odometry's new pose and the next step() continues from it.  Returns a BSHOT_* status; on an error nothing changes
+    int reanchor(const std::vector<Matrix4f>& poses) {
+        if (!ctx_) return status_;
+        std::vector<float> p12(12 * poses.size());
+        for (size_t u = 0; u < poses.size(); ++u)
+            for (int row = 0; row < 3; ++row) for (int col = 0; col < 4; ++col) p12[12 * u + 4 * row + col] = poses[u](row, col);
+        float T[16];
+        status_ = bshot_gmap_reanchor(ctx_, p12.data(), poses.size(), T);
+        if (status_ == BSHOT_OK)
+            for (int row = 0; row < 4; ++row) for (int col = 0; col < 4; ++col) pose_(row, col) = T[4 * row + col];
+        return status_;
+    }
+
+    // the trajectory's pose graph with the accepted detections as loop edges (match_scan, scan, T_rel), optimised on the
+    // device (bshot_optimize_trajectory, read only): poses gets one optimised pose per map update, *rep (may be null) the
+    // report.  Returns a BSHOT_* status; reanchor(poses) applies the result
+    int optimizeTrajectory(const std::vector<bshot_loop_report>& loops, std::vector<Matrix4f>& poses, bshot_graph_report* rep = nullptr) {
+        poses.clear();
+        if (!ctx_) return status_;
+        std::vector<bshot_graph_edge> edges(loops.size());
+        for (size_t k = 0; k < loops.size(); ++k) {
+            edges[k].from = loops[k].match_scan;
+            edges[k].to = loops[k].scan;
+            for (int e = 0; e < 16; ++e) edges[k].T[e] = loops[k].T_rel[e];
+        }
+        size_t m = 0;
+        status_ = bshot_gmap_scans(ctx_, nullptr, 0, nullptr, 0, nullptr, &m);
+        if (status_ != BSHOT_OK) return status_;
+        std::vector<float> p12(12 * (m ? m : 1));
+        bshot_graph_report r;
+        status_ = bshot_optimize_trajectory(ctx_, edges.data(), edges.size(), &graph_params_, p12.data(), m, nullptr, &r);
+        if (status_ != BSHOT_OK) return status_;
+        if (rep) *rep = r;
+        poses.assign(m, Matrix4f::Identity());
+        for (size_t u = 0; u < m; ++u)
+            for (int row = 0; row < 3; ++row) for (int col = 0; col < 4; ++col) poses[u](row, col) = p12[12 * u + 4 * row + col];
+        return status_;
+    }
+    bshot_graph_params& graphParams() { return graph_params_; }
+
     // INITIAL status, identity pose, empty map, no reference frame
     int reset() {
         if (ctx_) status_ = bshot_odometry_reset(ctx_);
@@ -133,6 +178,7 @@ private:
     bshot_ctx* ctx_ = nullptr;
     bshot_odom_params params_;
     bshot_loop_params loop_params_;
+    bshot_graph_params graph_params_;
     bshot_odom_report report_ = bshot_odom_report();
     bshot_reloc_report reloc_report_ = bshot_reloc_report();
     int min_inliers_ = 15;   // the gate's own constant (src/lidar_odometry.cpp:269-281)

@@ -383,6 +383,58 @@ typedef struct bshot_loop_report {
 } bshot_loop_report;
 int bshot_detect_loop(bshot_ctx* ctx, const bshot_loop_params* p, bshot_loop_report* out);
 
+/* bshot_gmap_reanchor: move the map to a corrected trajectory, as a pose-graph back end computes it from the loop edges.
+ * poses3x4 (n x 12 floats, row-major [R|T]) is the corrected pose of every map update, n = bshot_gmap_scans' *n_scans_out.
+ * Update u's correction is C_u = T'_u * T_u^-1 (fp32, rigid inverse, as T_rel); an update whose pose equals its trajectory
+ * pose bit for bit is unchanged.  Every entry of a changed update moves by its update's correction (R p + T, rounded as an
+ * update transforms keypoints) and is snapped to the 10 mm lattice; its seg-ratio, descriptor and tag stay, and the entries
+ * of unchanged updates stay bit for bit.  The map is then rebuilt from the entries in export order, without the admission
+ * rule: two entries moved onto one position both stay, as after bshot_gmap_import.  The trajectory becomes poses3x4 bit
+ * for bit.  The odometry's pose becomes T'_{n-1} when it equals T_{n-1} (as after a step), else C_{n-1} * pose; the
+ * reference frame is kept in its sensor frame and moves with the pose; before the first odometry step the pose is the
+ * identity, and it moves by the same rule.  pose_out (16 floats, may be NULL) gets the new pose.
+ * Re-anchoring is not an update: the update count, the status and the reference frame stay, so bshot_detect_loop can run
+ * again on the same scan.  Re-anchoring with the current trajectory changes nothing.  Errors (nothing changes):
+ * BSHOT_E_STATE without a map; BSHOT_E_INVALID when n is not the update count, or a pose is not finite, has
+ * max |R^T R - I| > 1e-3 or det R <= 0; BSHOT_E_CAPACITY when the moved map needs more blocks or chunks than the map
+ * holds.  Synchronous. */
+int bshot_gmap_reanchor(bshot_ctx* ctx, const float* poses3x4, size_t n, float* pose_out);
+
+/* bshot_optimize_trajectory: the pose graph of the map's trajectory, optimised on the device in float64.  Nodes: the n
+ * trajectory poses (bshot_gmap_scans); node 0 is fixed (it defines the map frame).  Odometry edges (u, u + 1) with
+ * measurement Z = T_u^-1 T_{u+1} (float64, from the fp32 trajectory); loop edges: the caller's list, e.g. {match_scan, scan,
+ * T_rel} of accepted bshot_detect_loop reports.  Edge (a, b) with measurement Z = [R_z | t_z]: residuals
+ * r_t = R_a^T (t_b - t_a) - t_z (mm) and r_phi = Log(R_z^T R_a^T R_b) (rad); cost F = 1/2 sum |r_t|^2 / s_t^2 + |r_phi|^2 / s_phi^2
+ * with the sigmas of the edge's class.  Levenberg-Marquardt on t <- t + rho, R <- R Exp(phi): (H + lambda diag H) d = -g
+ * (lambda starts at 1e-4), solved by conjugate gradients preconditioned with the block-tridiagonal part of the damped
+ * matrix (block cyclic reduction along the chain).  A step that lowers F is accepted (lambda / 10), otherwise lambda * 10;
+ * every solve counts as an iteration.  Stops when |g|_inf <= grad_tolerance (tested before each solve: a graph without
+ * loop edges takes 0 iterations), when max |d| <= step_tolerance (that step is not taken), or after max_iterations.
+ * Read only: map, tags, trajectory, pose and reference frame are unchanged; bshot_gmap_reanchor applies the result.
+ * poses3x4_out (pose_cap x 12 floats): the optimised poses; node 0, and every node when no step was accepted, keep their
+ * input bits.  loop_cost_out[k] (may be NULL): loop edge k's final 1/2 r^T W r.  out (may be NULL): the report.
+ * Deterministic: identical inputs give identical bits.  Errors: BSHOT_E_STATE without a map; BSHOT_E_INVALID for an edge
+ * index outside [0, n), from == to, a non-finite or non-rigid T (as bshot_gmap_reanchor checks), a sigma <= 0 or a negative
+ * iteration count or tolerance; BSHOT_E_CAPACITY when pose_cap < n (nothing is written).  n = 1 returns the trajectory
+ * after 0 iterations.  Synchronous; one copy back at the end. */
+typedef struct bshot_graph_edge {
+    int32_t from, to;       /* `to`'s pose in `from`'s frame is T */
+    float T[16];            /* row-major */
+} bshot_graph_edge;
+typedef struct bshot_graph_params {
+    float odom_sigma_mm, odom_sigma_deg;   /* 20 mm, 0.1 deg */
+    float loop_sigma_mm, loop_sigma_deg;   /* 100 mm, 1 deg */
+    int max_iterations, max_cg_iterations; /* 50, 2000 */
+    double grad_tolerance, step_tolerance, cg_tolerance;   /* 1e-6, 1e-9, 1e-10 (relative residual) */
+} bshot_graph_params;
+void bshot_graph_params_default(bshot_graph_params* p);
+typedef struct bshot_graph_report {
+    int n_nodes, n_edges, iterations, cg_iterations, status;   /* status: 1 gradient, 2 step, 3 max_iterations */
+    double cost_initial, cost_final, grad_inf_final;
+} bshot_graph_report;
+int bshot_optimize_trajectory(bshot_ctx* ctx, const bshot_graph_edge* loops, size_t n_loops, const bshot_graph_params* p, float* poses3x4_out,
+                              size_t pose_cap, double* loop_cost_out, bshot_graph_report* out);
+
 /* bshot_ransac on device buffers, asynchronous on the context stream: d_src4 / d_tgt4 float4 points (x, y, z, any),
  * d_pairs n_pairs_cap x 2 ints (index into src, index into tgt; every valid one must be in range), *d_n_pairs (int) of
  * them valid.  Outputs (device): d_inlier_pairs_out (n_pairs_cap x 2 ints), *d_n_inliers_out (int), d_transform_out
