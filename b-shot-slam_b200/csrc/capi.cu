@@ -742,8 +742,18 @@ int bshot_gmap_size(bshot_ctx* ctx, size_t* entries_out, size_t* dropped_out) {
     return BSHOT_OK;
 }
 
+// a map update's pose (NULL = identity) must be finite: a NaN or an infinity would make every keypoint unstorable, and the
+// update would still count and write its pose into the trajectory
+static bool pose_finite(const float* pose3x4, const char* who) {
+    if (pose3x4)
+        for (int k = 0; k < 12; ++k)
+            if (!std::isfinite(pose3x4[k])) { set_error("%s: the pose is not finite", who); return false; }
+    return true;
+}
+
 int bshot_gmap_add(bshot_ctx* ctx, const float* xyz, const float* seg_ratio, const uint64_t* desc, size_t n, const float* pose3x4) {
     CHECK_CTX(ctx);
+    if (!pose_finite(pose3x4, "bshot_gmap_add")) return BSHOT_E_INVALID;
     if (n == 0) return BSHOT_OK;
     if (!xyz || !seg_ratio || !desc) { set_error("bshot_gmap_add: null input"); return BSHOT_E_INVALID; }
     if (n > ctx->max_kp) { set_error("bshot_gmap_add: %zu keypoints > max_keypoints %zu per call", n, ctx->max_kp); return BSHOT_E_CAPACITY; }
@@ -764,6 +774,7 @@ int bshot_gmap_add(bshot_ctx* ctx, const float* xyz, const float* seg_ratio, con
 int bshot_gmap_update_from_frame(bshot_ctx* ctx, const float* pose3x4) {
     CHECK_CTX(ctx);
     if (!ctx->have_kp || ctx->last_top_k == 0) { set_error("bshot_gmap_update_from_frame: no extracted frame"); return BSHOT_E_STATE; }
+    if (!pose_finite(pose3x4, "bshot_gmap_update_from_frame")) return BSHOT_E_INVALID;
     BSHOT_TRY(gmap_update(ctx, ctx->d_kp, ctx->d_kp_ratio, ctx->d_bits, ctx->d_kp_count, ctx->last_top_k, pose3x4));
     ctx->gmap.entries_upper += ctx->last_top_k;
     ++ctx->gmap.n_updates;

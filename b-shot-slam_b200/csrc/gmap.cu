@@ -28,6 +28,15 @@ constexpr unsigned GM_PREC = 10000;          // block edge (mm), src/mymap.h:49
 constexpr float GM_LATTICE = 10.0f;          // position lattice (mm), src/keypoint.cpp:25
 constexpr float GM_REJECT_MM = 800.0f;       // src/mymap.cpp:17
 constexpr unsigned long long GM_OCC = 1ull << 63;
+// A storable position: every coordinate finite and within +-2.1e9 mm (2100 km), so the lattice snap
+// (|int(trunc(v / 10))| * 10 <= 2^31 - 1) and the block id (|roundf(v / 10 m)| * 10 m <= 2^31 - 1, up to 2.147485e9 mm)
+// stay inside int32.  Tested on the unsnapped coordinates: a float made from an int is always finite, and a
+// saturated int32 times 10 wraps near the origin
+constexpr float GM_MAX_MM = 2.1e9f;
+
+__host__ __device__ __forceinline__ bool gm_storable(float x, float y, float z) {
+    return fabsf(x) <= GM_MAX_MM && fabsf(y) <= GM_MAX_MM && fabsf(z) <= GM_MAX_MM;   // false for NaN
+}
 
 struct GmapBlock {
     unsigned long long key;   // GM_OCC | block id (21 bits per axis), 0 = free
@@ -80,16 +89,16 @@ __global__ void gm_prepare_kernel(const float4* __restrict__ kp, const float* __
         y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[4], p.x), __fmul_rn(pose[5], p.y)), __fmul_rn(pose[6], p.z)), pose[7]);
         z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[8], p.x), __fmul_rn(pose[9], p.y)), __fmul_rn(pose[10], p.z)), pose[11]);
     }
+    // a keypoint that is not storable (a non-finite position or pose, or beyond GM_MAX_MM) is skipped; it is not a drop
+    if (!gm_storable(x, y, z)) { blk_of[i] = 0xFFFFFFFFu; return; }
     // Keypoint::createKeypoint: int(trunc(pos / prec)) * prec
     x = (float)((int)truncf(x / GM_LATTICE) * (int)GM_LATTICE);
     y = (float)((int)truncf(y / GM_LATTICE) * (int)GM_LATTICE);
     z = (float)((int)truncf(z / GM_LATTICE) * (int)GM_LATTICE);
     world[i] = make_float4(x, y, z, ratio[i]);
-    const bool ok = isfinite(x) && isfinite(y) && isfinite(z);
-    unsigned slot = 0xFFFFFFFFu;
-    if (ok) slot = gm_find(tab, mask, gm_block_id(x, y, z), true);
+    const unsigned slot = gm_find(tab, mask, gm_block_id(x, y, z), true);
     blk_of[i] = slot;
-    if (slot == 0xFFFFFFFFu) { if (ok) atomicAdd(&ctl[3], 1u); return; }  // table full: counted, reported by the host
+    if (slot == 0xFFFFFFFFu) { atomicAdd(&ctl[3], 1u); return; }  // table full: counted, reported by the host
     if (atomicExch(&tab[slot].touched, epoch) != epoch) touched_list[atomicAdd(&ctl[1], 1u)] = slot;
 }
 
@@ -134,14 +143,18 @@ gm_admit_kernel(const float4* __restrict__ world, const unsigned* __restrict__ b
             if (reject) continue;
             unsigned e = same;  // keypoints_[block][position] = keypoint: overwrite at an equal position, else insert
             if (e == 0xFFFFFFFFu) {
-                if (lane == 0) e = atomicAdd(&ctl[0], 1u);
-                e = __shfl_sync(0xffffffffu, e, 0);
-                if (e >= max_entries) { if (lane == 0) { atomicAdd(&ctl[3], 1u); atomicSub(&ctl[0], 1u); } continue; }
+                // the chunk first, then the entry: an entry index below max_entries cannot be given back (another warp
+                // may already hold the next one), a chunk that is not linked is only unused
+                unsigned nc = 0xFFFFFFFFu;
                 if ((cnt & 31u) == 0u) {  // new chunk
-                    unsigned nc = 0;
                     if (lane == 0) nc = atomicAdd(&ctl[2], 1u);
                     nc = __shfl_sync(0xffffffffu, nc, 0);
                     if (nc >= max_chunks) { if (lane == 0) atomicAdd(&ctl[3], 1u); continue; }
+                }
+                if (lane == 0) e = atomicAdd(&ctl[0], 1u);
+                e = __shfl_sync(0xffffffffu, e, 0);
+                if (e >= max_entries) { if (lane == 0) { atomicAdd(&ctl[3], 1u); atomicSub(&ctl[0], 1u); } continue; }
+                if (nc != 0xFFFFFFFFu) {
                     if (lane == 0) {
                         chunks[nc * 33u + 32u] = 0xFFFFFFFFu;
                         if (cnt == 0u) first = nc; else chunks[last * 33u + 32u] = nc;
@@ -284,7 +297,7 @@ __global__ void gm_append_ref_kernel(const float4* __restrict__ ref_kp, const ui
 // Map order: occupied blocks in ascending lattice coordinates (x outermost, z innermost: the order gm_probe_kernel visits
 // them), entries of a block in insertion order.  A block's coordinates are roundf(p / 10 m) of any of its entries (the
 // block id was computed from that same stored position).  actl: [0] listed blocks, [1] entries gathered, [2] import
-// error bits (1 non-finite position, 2 table / chunks full), [3] import entries.
+// error bits (1 position not storable, 2 table / chunks full), [3] import entries.
 constexpr unsigned GM_AXIS_BIAS = 1u << 20;
 
 __device__ __forceinline__ unsigned long long gm_order_key(float4 p) {
@@ -337,7 +350,7 @@ __global__ void gm_import_find_kernel(const float4* __restrict__ e_pos, unsigned
     e_tag[i] = tag_src ? tag_src[i] : 0u;
     const float4 p = e_pos[i];
     unsigned slot = 0xFFFFFFFFu;
-    if (!(isfinite(p.x) && isfinite(p.y) && isfinite(p.z))) atomicOr(&actl[2], 1u);
+    if (!gm_storable(p.x, p.y, p.z)) atomicOr(&actl[2], 1u);
     else if ((slot = gm_find(tab, mask, gm_block_id(p.x, p.y, p.z), true)) == 0xFFFFFFFFu) atomicOr(&actl[2], 2u);
     else atomicAdd(&tab[slot].count, 1u);
     keys[i] = slot;
@@ -404,6 +417,8 @@ __global__ void gm_reanchor_move_kernel(const float4* __restrict__ apos, const u
     float x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[0], p.x), __fmul_rn(C[1], p.y)), __fmul_rn(C[2], p.z)), C[3]);
     float y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[4], p.x), __fmul_rn(C[5], p.y)), __fmul_rn(C[6], p.z)), C[7]);
     float z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[8], p.x), __fmul_rn(C[9], p.y)), __fmul_rn(C[10], p.z)), C[11]);
+    // an entry moved out of the storable range stays unsnapped: the rebuild rejects it and the map is restored
+    if (!gm_storable(x, y, z)) { e_pos[i] = make_float4(x, y, z, p.w); return; }
     x = (float)((int)truncf(x / GM_LATTICE) * (int)GM_LATTICE);
     y = (float)((int)truncf(y / GM_LATTICE) * (int)GM_LATTICE);
     z = (float)((int)truncf(z / GM_LATTICE) * (int)GM_LATTICE);
@@ -598,7 +613,7 @@ int gmap_import_dev(Ctx* c, const float4* d_pos, const uint64_t* d_desc, const u
     unsigned* h = reinterpret_cast<unsigned*>(&c->h_scratch[48]);
     BSHOT_CUDA_TRY(cudaMemcpyAsync(h, g.d_actl, sizeof(unsigned) * 4, cudaMemcpyDeviceToHost, c->stream));
     BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
-    if (h[2] & 1u) { set_error("%s: non-finite position", who); return BSHOT_E_INVALID; }
+    if (h[2] & 1u) { set_error("%s: a position is not finite or beyond +-2.1e9 mm", who); return BSHOT_E_INVALID; }
     if (h[2]) { set_error("%s: more blocks or chunks than the map holds (%u slots, %u chunks)", who, g.tab_cap, g.max_chunks); return BSHOT_E_CAPACITY; }
     return BSHOT_OK;
 }
@@ -662,7 +677,7 @@ int gmap_reanchor(Ctx* c, const float* poses3x4, size_t n, float* d_pose, float*
             const int rc = gmap_import_dev(c, g.d_epos, g.d_edesc, g.d_atag, nt_cap, d_count, "bshot_gmap_reanchor");
             if (rc == BSHOT_E_INVALID || rc == BSHOT_E_CAPACITY) {
                 BSHOT_TRY(gmap_import_dev(c, g.d_apos, g.d_adesc, g.d_atag, nt_cap, d_count, "bshot_gmap_reanchor (restoring the map)"));
-                if (rc == BSHOT_E_INVALID) set_error("bshot_gmap_reanchor: a moved entry is not finite; nothing changed");
+                if (rc == BSHOT_E_INVALID) set_error("bshot_gmap_reanchor: a moved entry is not finite or beyond +-2.1e9 mm; nothing changed");
                 else set_error("bshot_gmap_reanchor: the moved map needs more blocks or chunks than the map holds (%u slots, %u chunks); nothing changed",
                                g.tab_cap, g.max_chunks);
                 return rc;

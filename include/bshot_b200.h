@@ -173,9 +173,14 @@ int bshot_fetch_frame(bshot_ctx* ctx, int top_k, int* kp_idx_out, uint64_t* bits
  *   bshot_extract_frame -> bshot_match_frame_to_map -> (host: pose) -> bshot_gmap_update_from_frame(pose) -> bshot_frame_commit */
 int bshot_gmap_create(bshot_ctx* ctx, size_t max_entries, size_t max_blocks);
 int bshot_gmap_reset(bshot_ctx* ctx);
-/* entries stored so far; dropped = keypoints lost to a full table / pool (0 unless the capacities are too small) */
+/* entries stored so far (bshot_gmap_export returns exactly these); dropped = keypoints lost to a full block table, chunk
+ * pool or entry pool (0 unless the capacities are too small).  Keypoints skipped as not storable are not dropped. */
 int bshot_gmap_size(bshot_ctx* ctx, size_t* entries_out, size_t* dropped_out);
-/* Map::addKeypoint for n keypoints given on the host (xyz n x 3 floats, in keypoint order), n <= max_keypoints per call */
+/* Map::addKeypoint for n keypoints given on the host (xyz n x 3 floats, in keypoint order), n <= max_keypoints per call.
+ * A keypoint is stored only when its transformed position is storable: x, y and z finite and within +-2.1e9 mm (2100 km;
+ * the 10 mm snap and the 10 m block id must fit int32).  Other keypoints (NaN, +-Inf, farther) are skipped, uncounted.
+ * A pose with a non-finite element returns BSHOT_E_INVALID and changes nothing (no update is counted, the trajectory is
+ * not written); so does bshot_gmap_update_from_frame. */
 int bshot_gmap_add(bshot_ctx* ctx, const float* xyz, const float* seg_ratio, const uint64_t* desc, size_t n, const float* pose3x4);
 /* updateMap for the frame extracted last (keypoints, seg-ratios and descriptors are still on the device); asynchronous */
 int bshot_gmap_update_from_frame(bshot_ctx* ctx, const float* pose3x4);
@@ -199,7 +204,8 @@ int bshot_frame_commit(bshot_ctx* ctx);
 int bshot_gmap_export(bshot_ctx* ctx, float* xyzr_out, uint64_t* desc_out, size_t cap, size_t* n_out);
 /* replaces the map by these n entries (layout of bshot_gmap_export), without the admission rule: entries of one block keep
  * their relative order in the input, so a bshot_gmap_export result restores the map it came from and every later call
- * behaves as on the exporting context.  Positions are stored as given.  Non-finite x, y or z: BSHOT_E_INVALID;
+ * behaves as on the exporting context.  Positions are stored as given.  A position that is not storable (as
+ * bshot_gmap_add defines it: non-finite, or beyond +-2.1e9 mm): BSHOT_E_INVALID;
  * n > max_entries, or more blocks / chunks than the table holds: BSHOT_E_CAPACITY.  On any error the map is empty.
  * The pose, the status and the reference frame of the odometry step are not touched. */
 int bshot_gmap_import(bshot_ctx* ctx, const float* xyzr, const uint64_t* desc, size_t n);
@@ -396,7 +402,7 @@ int bshot_detect_loop(bshot_ctx* ctx, const bshot_loop_params* p, bshot_loop_rep
  * Re-anchoring is not an update: the update count, the status and the reference frame stay, so bshot_detect_loop can run
  * again on the same scan.  Re-anchoring with the current trajectory changes nothing.  Errors (nothing changes):
  * BSHOT_E_STATE without a map; BSHOT_E_INVALID when n is not the update count, or a pose is not finite, has
- * max |R^T R - I| > 1e-3 or det R <= 0; BSHOT_E_CAPACITY when the moved map needs more blocks or chunks than the map
+ * max |R^T R - I| > 1e-3 or det R <= 0, or a moved entry is not storable (bshot_gmap_add); BSHOT_E_CAPACITY when the moved map needs more blocks or chunks than the map
  * holds.  Synchronous. */
 int bshot_gmap_reanchor(bshot_ctx* ctx, const float* poses3x4, size_t n, float* pose_out);
 
