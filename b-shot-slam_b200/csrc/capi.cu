@@ -485,8 +485,7 @@ int bshot_match_mutual(bshot_ctx* ctx, const uint64_t* q, size_t nq, const uint6
     BSHOT_TRY(upload_qt(ctx, q, nq, t, nt, "bshot_match_mutual"));
     if (count_out) *count_out = 0;
     if (nq == 0 || nt == 0) return sync(ctx);
-    BSHOT_TRY(hamming_match_rq(ctx, ctx->d_q, nq, ctx->d_t, nt, 0, ctx->d_cand));
-    BSHOT_TRY(hamming_mutual_pairs(ctx, ctx->d_cand, nq, ctx->d_pairs, ctx->d_pair_count));
+    BSHOT_TRY(match_mutual(ctx, ctx->d_q, nq, ctx->d_t, nt));
     BSHOT_TRY(d2h(ctx, ctx->h_scratch, ctx->d_pair_count, sizeof(int)));
     BSHOT_TRY(sync(ctx));
     const int n = ctx->h_scratch[0];
@@ -728,7 +727,6 @@ int bshot_gmap_create(bshot_ctx* ctx, size_t max_entries, size_t max_blocks) {
 int bshot_gmap_reset(bshot_ctx* ctx) {
     CHECK_CTX(ctx);
     BSHOT_TRY(gmap_reset(ctx));
-    ctx->gmap.entries_upper = 0;
     return sync(ctx);
 }
 
@@ -765,9 +763,7 @@ int bshot_gmap_add(bshot_ctx* ctx, const float* xyz, const float* seg_ratio, con
     BSHOT_TRY(h2d(ctx, d_ratio, seg_ratio, sizeof(float) * n));
     BSHOT_TRY(h2d(ctx, ctx->d_q, desc, 48 * n));
     BSHOT_TRY(gmap_update(ctx, d_pos, d_ratio, ctx->d_q, nullptr, n, pose3x4));
-    ctx->gmap.entries_upper += n;
-    ++ctx->gmap.n_updates;
-    ctx->gmap.last_by_scan = false;
+    gmap_record_update(ctx, n, /*by_scan=*/false);
     return sync(ctx);
 }
 
@@ -776,9 +772,7 @@ int bshot_gmap_update_from_frame(bshot_ctx* ctx, const float* pose3x4) {
     if (!ctx->have_kp || ctx->last_top_k == 0) { set_error("bshot_gmap_update_from_frame: no extracted frame"); return BSHOT_E_STATE; }
     if (!pose_finite(pose3x4, "bshot_gmap_update_from_frame")) return BSHOT_E_INVALID;
     BSHOT_TRY(gmap_update(ctx, ctx->d_kp, ctx->d_kp_ratio, ctx->d_bits, ctx->d_kp_count, ctx->last_top_k, pose3x4));
-    ctx->gmap.entries_upper += ctx->last_top_k;
-    ++ctx->gmap.n_updates;
-    ctx->gmap.last_by_scan = false;
+    gmap_record_update(ctx, ctx->last_top_k, /*by_scan=*/false);
     return BSHOT_OK;  // asynchronous
 }
 
@@ -1058,12 +1052,35 @@ void bshot_odom_params_default(bshot_odom_params* p) {
     p->run_icp = 1;
 }
 
-static int odom_args_ok(bshot_ctx* ctx, const bshot_odom_params* p, const char* who) {
-    if (p->ransac_iterations < 1 || p->ransac_iterations > 100000) { set_error("%s: ransac_iterations %d outside [1, 100000]", who, p->ransac_iterations); return BSHOT_E_INVALID; }
-    if (!(p->inlier_threshold > 0.0f) || !std::isfinite(p->inlier_threshold)) { set_error("%s: inlier_threshold must be finite and > 0", who); return BSHOT_E_INVALID; }
-    if (!(p->map_range >= 0.0f) || !std::isfinite(p->map_range)) { set_error("%s: map_range must be finite and >= 0", who); return BSHOT_E_INVALID; }
+// the registration parameters of the step, relocalisation (min_inliers) and loop detection (min_inliers), and the map
+static int reg_args_ok(bshot_ctx* ctx, const int* min_inliers, int ransac_iterations, float inlier_threshold, float map_range, const char* who) {
+    if (min_inliers && *min_inliers < 3) { set_error("%s: min_inliers %d < 3", who, *min_inliers); return BSHOT_E_INVALID; }
+    if (ransac_iterations < 1 || ransac_iterations > 100000) { set_error("%s: ransac_iterations %d outside [1, 100000]", who, ransac_iterations); return BSHOT_E_INVALID; }
+    if (!(inlier_threshold > 0.0f) || !std::isfinite(inlier_threshold)) { set_error("%s: inlier_threshold must be finite and > 0", who); return BSHOT_E_INVALID; }
+    if (!(map_range >= 0.0f) || !std::isfinite(map_range)) { set_error("%s: map_range must be finite and >= 0", who); return BSHOT_E_INVALID; }
     if (!ctx->gmap.d_tab) { set_error("%s: needs a map (bshot_gmap_create)", who); return BSHOT_E_STATE; }
     return BSHOT_OK;
+}
+
+// raw returns of the step or a relocalisation: the returns' and the parameters' checks, then Preprocessor::run, whose two
+// count read-backs size the front end's grids; the cloud (*kept points, 3 floats each) stays on the device in *d_cloud
+static int scan_to_device(bshot_ctx* ctx, const bshot_odom_params* p, const int* min_inliers, const double* azimuth_deg, const double* vertical_deg,
+                          const unsigned short* distance, size_t n, const double* ring_deg, size_t nv, const char* who, const float** d_cloud, size_t* kept) {
+    if (n && (!azimuth_deg || !vertical_deg || !distance)) { set_error("%s: null input", who); return BSHOT_E_INVALID; }
+    if (nv && !ring_deg) { set_error("%s: null ring table", who); return BSHOT_E_INVALID; }
+    if (n > 0xFFFFFFFFull) { set_error("%s: too many returns", who); return BSHOT_E_CAPACITY; }
+    BSHOT_TRY(reg_args_ok(ctx, min_inliers, p->ransac_iterations, p->inlier_threshold, p->map_range, who));
+    BSHOT_TRY(preprocess_run(ctx, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, p->vert_init_rad, p->lowpt_th, nullptr, 1, nullptr, std::max<size_t>(n, 1),
+                             kept, d_cloud));
+    return frame_args_ok(ctx, &p->front, *kept, 12, who);
+}
+
+// a preprocessed host cloud of the step or a relocalisation: the checks, then the upload into ctx->d_raw
+static int cloud_to_device(bshot_ctx* ctx, const bshot_odom_params* p, const int* min_inliers, const float* xyz, size_t n, size_t stride_bytes, const char* who) {
+    if (!xyz && n) { set_error("%s: null cloud", who); return BSHOT_E_INVALID; }
+    BSHOT_TRY(reg_args_ok(ctx, min_inliers, p->ransac_iterations, p->inlier_threshold, p->map_range, who));
+    BSHOT_TRY(frame_args_ok(ctx, &p->front, n, stride_bytes, who));
+    return h2d(ctx, ctx->d_raw, xyz, n * stride_bytes);
 }
 
 int bshot_odometry_step(bshot_ctx* ctx, const bshot_odom_params* p, const double* azimuth_deg, const double* vertical_deg, const unsigned short* distance,
@@ -1071,16 +1088,9 @@ int bshot_odometry_step(bshot_ctx* ctx, const bshot_odom_params* p, const double
     CHECK_CTX(ctx);
     bshot_odom_params dp;
     if (!p) { bshot_odom_params_default(&dp); p = &dp; }
-    if (n && (!azimuth_deg || !vertical_deg || !distance)) { set_error("bshot_odometry_step: null input"); return BSHOT_E_INVALID; }
-    if (nv && !ring_deg) { set_error("bshot_odometry_step: null ring table"); return BSHOT_E_INVALID; }
-    if (n > 0xFFFFFFFFull) { set_error("bshot_odometry_step: too many returns"); return BSHOT_E_CAPACITY; }
-    BSHOT_TRY(odom_args_ok(ctx, p, "bshot_odometry_step"));
-    // Preprocessor::run; its two count read-backs size the front end's grids, the cloud stays on the device
     size_t kept = 0;
     const float* d_cloud = nullptr;
-    BSHOT_TRY(preprocess_run(ctx, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, p->vert_init_rad, p->lowpt_th, nullptr, 1, nullptr, std::max<size_t>(n, 1),
-                             &kept, &d_cloud));
-    BSHOT_TRY(frame_args_ok(ctx, &p->front, kept, 12, "bshot_odometry_step"));
+    BSHOT_TRY(scan_to_device(ctx, p, nullptr, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, "bshot_odometry_step", &d_cloud, &kept));
     return odometry_run(ctx, p, d_cloud, kept, 3, out);
 }
 
@@ -1088,16 +1098,8 @@ int bshot_odometry_step_cloud(bshot_ctx* ctx, const bshot_odom_params* p, const 
     CHECK_CTX(ctx);
     bshot_odom_params dp;
     if (!p) { bshot_odom_params_default(&dp); p = &dp; }
-    if (!xyz && n) { set_error("bshot_odometry_step_cloud: null cloud"); return BSHOT_E_INVALID; }
-    BSHOT_TRY(odom_args_ok(ctx, p, "bshot_odometry_step_cloud"));
-    BSHOT_TRY(frame_args_ok(ctx, &p->front, n, stride_bytes, "bshot_odometry_step_cloud"));
-    BSHOT_TRY(h2d(ctx, ctx->d_raw, xyz, n * stride_bytes));
+    BSHOT_TRY(cloud_to_device(ctx, p, nullptr, xyz, n, stride_bytes, "bshot_odometry_step_cloud"));
     return odometry_run(ctx, p, ctx->d_raw, n, (int)(stride_bytes / 4), out);
-}
-
-static int reloc_args_ok(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const char* who) {
-    if (min_inliers < 3) { set_error("%s: min_inliers %d < 3", who, min_inliers); return BSHOT_E_INVALID; }
-    return odom_args_ok(ctx, p, who);
 }
 
 int bshot_relocalize(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers, const double* azimuth_deg, const double* vertical_deg,
@@ -1105,15 +1107,9 @@ int bshot_relocalize(bshot_ctx* ctx, const bshot_odom_params* p, int min_inliers
     CHECK_CTX(ctx);
     bshot_odom_params dp;
     if (!p) { bshot_odom_params_default(&dp); p = &dp; }
-    if (n && (!azimuth_deg || !vertical_deg || !distance)) { set_error("bshot_relocalize: null input"); return BSHOT_E_INVALID; }
-    if (nv && !ring_deg) { set_error("bshot_relocalize: null ring table"); return BSHOT_E_INVALID; }
-    if (n > 0xFFFFFFFFull) { set_error("bshot_relocalize: too many returns"); return BSHOT_E_CAPACITY; }
-    BSHOT_TRY(reloc_args_ok(ctx, p, min_inliers, "bshot_relocalize"));
     size_t kept = 0;
     const float* d_cloud = nullptr;
-    BSHOT_TRY(preprocess_run(ctx, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, p->vert_init_rad, p->lowpt_th, nullptr, 1, nullptr, std::max<size_t>(n, 1),
-                             &kept, &d_cloud));
-    BSHOT_TRY(frame_args_ok(ctx, &p->front, kept, 12, "bshot_relocalize"));
+    BSHOT_TRY(scan_to_device(ctx, p, &min_inliers, azimuth_deg, vertical_deg, distance, n, ring_deg, nv, "bshot_relocalize", &d_cloud, &kept));
     return relocalize_run(ctx, p, min_inliers, d_cloud, kept, 3, out);
 }
 
@@ -1122,10 +1118,7 @@ int bshot_relocalize_cloud(bshot_ctx* ctx, const bshot_odom_params* p, int min_i
     CHECK_CTX(ctx);
     bshot_odom_params dp;
     if (!p) { bshot_odom_params_default(&dp); p = &dp; }
-    if (!xyz && n) { set_error("bshot_relocalize_cloud: null cloud"); return BSHOT_E_INVALID; }
-    BSHOT_TRY(reloc_args_ok(ctx, p, min_inliers, "bshot_relocalize_cloud"));
-    BSHOT_TRY(frame_args_ok(ctx, &p->front, n, stride_bytes, "bshot_relocalize_cloud"));
-    BSHOT_TRY(h2d(ctx, ctx->d_raw, xyz, n * stride_bytes));
+    BSHOT_TRY(cloud_to_device(ctx, p, &min_inliers, xyz, n, stride_bytes, "bshot_relocalize_cloud"));
     return relocalize_run(ctx, p, min_inliers, ctx->d_raw, n, (int)(stride_bytes / 4), out);
 }
 
@@ -1144,11 +1137,7 @@ int bshot_detect_loop(bshot_ctx* ctx, const bshot_loop_params* p, bshot_loop_rep
     bshot_loop_params dp;
     if (!p) { bshot_loop_params_default(&dp); p = &dp; }
     if (p->min_gap < 1) { set_error("bshot_detect_loop: min_gap %d < 1", p->min_gap); return BSHOT_E_INVALID; }
-    if (p->min_inliers < 3) { set_error("bshot_detect_loop: min_inliers %d < 3", p->min_inliers); return BSHOT_E_INVALID; }
-    if (p->ransac_iterations < 1 || p->ransac_iterations > 100000) { set_error("bshot_detect_loop: ransac_iterations %d outside [1, 100000]", p->ransac_iterations); return BSHOT_E_INVALID; }
-    if (!(p->inlier_threshold > 0.0f) || !std::isfinite(p->inlier_threshold)) { set_error("bshot_detect_loop: inlier_threshold must be finite and > 0"); return BSHOT_E_INVALID; }
-    if (!(p->map_range >= 0.0f) || !std::isfinite(p->map_range)) { set_error("bshot_detect_loop: map_range must be finite and >= 0"); return BSHOT_E_INVALID; }
-    if (!ctx->gmap.d_tab) { set_error("bshot_detect_loop: needs a map (bshot_gmap_create)"); return BSHOT_E_STATE; }
+    BSHOT_TRY(reg_args_ok(ctx, &p->min_inliers, p->ransac_iterations, p->inlier_threshold, p->map_range, "bshot_detect_loop"));
     return loop_run(ctx, p, out);
 }
 

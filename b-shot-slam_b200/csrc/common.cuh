@@ -95,7 +95,8 @@ struct Gmap {
     float4* d_tpos = nullptr;           // positions of the assembled target set (max_targets)
     unsigned tab_cap = 0, max_entries = 0, max_chunks = 0, max_probe = 0, epoch = 0;
     size_t n_gathered = 0;
-    size_t entries_upper = 0;           // host-side upper bound of the number of entries (sizes the match grid without a sync)
+    size_t entries_upper = 0;           // host-side upper bound of the number of entries (sizes the match grid without a sync);
+                                        // it and n_updates are written only by gmap_reset and gmap_record_update
     // the whole map in map order (gmap_gather_all, export, relocalisation) and the import's rebuild: allocated by the first
     // call that needs them
     float4* d_apos = nullptr;           // max_entries: positions + seg-ratio in map order
@@ -107,7 +108,7 @@ struct Gmap {
     unsigned* d_actl = nullptr;         // [0] listed blocks [1] entries gathered [2] import error bits [3] import entries
     unsigned* d_atag = nullptr;         // max_entries: tags in map order (gmap_gather_all with tags)
     // loop closure (gmap_scans, bshot_detect_loop).  Updates are numbered 0, 1, ... since create / reset / import (update
-    // 0) / odometry reset; n_updates advances where entries_upper does, once the update has succeeded
+    // 0) / odometry reset; gmap_record_update advances n_updates with entries_upper, once the update has succeeded
     unsigned* d_etag = nullptr;         // max_entries: index of the update that wrote each entry
     float* d_traj = nullptr;            // traj_cap x 12: row-major [R|T] each update used (identity without a pose)
     size_t traj_cap = 0;
@@ -352,6 +353,15 @@ __device__ __forceinline__ float sqdist_rn(float ax, float ay, float az, float b
 // (a0*b0 + a1*b1) + a2*b2 in fp32 without contraction
 __device__ __forceinline__ float dot3_rn(float ax, float ay, float az, float bx, float by, float bz) {
     return __fadd_rn(__fadd_rn(__fmul_rn(ax, bx), __fmul_rn(ay, by)), __fmul_rn(az, bz));
+}
+
+// R * p + T on a row-major 3x4 [R|T] in fp32 without contraction: the products summed left to right, then the translation
+// (updateMap's kp_pos = R * kp_pos + T, src/lidar_odometry.cpp:351).  The map and the keypoint repeatability move points
+// with it, so the same pose puts a point at the same bits in both
+__device__ __forceinline__ float3 pose_apply_rn(const float* m, float x, float y, float z) {
+    return make_float3(__fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], x), __fmul_rn(m[1], y)), __fmul_rn(m[2], z)), m[3]),
+                       __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[4], x), __fmul_rn(m[5], y)), __fmul_rn(m[6], z)), m[7]),
+                       __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[8], x), __fmul_rn(m[9], y)), __fmul_rn(m[10], z)), m[11]));
 }
 
 }  // namespace bshot

@@ -28,19 +28,21 @@ int frame_commit(Ctx* c, size_t k, const int* d_skip) {
     return check_launch("copy_prev_kernel");
 }
 
-int frame_match_map(Ctx* c, size_t k, const float pos[3], float range, const float* ref_pose12, bool pose_on_device, size_t* nt_cap_out) {
-    unsigned* d_total = c->gmap.d_ctl + 6;
-    BSHOT_TRY(gmap_gather(c, pos, range, c->d_prev_kp, c->d_prev_bits, c->d_prev_count, c->n_prev, ref_pose12, c->d_t, c->max_targets, d_total,
-                          pose_on_device));
-    const size_t nt_cap = std::min(c->max_targets, c->gmap.entries_upper + c->n_prev);
-    *nt_cap_out = nt_cap;
+int match_mutual(Ctx* c, const uint64_t* d_q, size_t k, const uint64_t* d_t, size_t nt_cap, const unsigned* d_nq, const unsigned* d_nt) {
     if (nt_cap == 0) {
         BSHOT_CUDA_TRY(cudaMemsetAsync(c->d_pair_count, 0, sizeof(int), c->stream));
         return BSHOT_OK;
     }
-    const unsigned* d_nq = reinterpret_cast<const unsigned*>(c->d_kp_count);
-    BSHOT_TRY(hamming_match_rq(c, c->d_bits, k, c->d_t, nt_cap, 0, c->d_cand, d_nq, d_total));
+    BSHOT_TRY(hamming_match_rq(c, d_q, k, d_t, nt_cap, 0, c->d_cand, d_nq, d_nt));
     return hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq);
+}
+
+int frame_match_map(Ctx* c, size_t k, const float pos[3], float range, const float* ref_pose12, bool pose_on_device, size_t* nt_cap_out) {
+    unsigned* d_total = c->gmap.d_ctl + 6;
+    BSHOT_TRY(gmap_gather(c, pos, range, c->d_prev_kp, c->d_prev_bits, c->d_prev_count, c->n_prev, ref_pose12, c->d_t, c->max_targets, d_total,
+                          pose_on_device));
+    *nt_cap_out = std::min(c->max_targets, c->gmap.entries_upper + c->n_prev);
+    return match_mutual(c, c->d_bits, k, c->d_t, *nt_cap_out, reinterpret_cast<const unsigned*>(c->d_kp_count), d_total);
 }
 
 // extractKeypoints + computeDescriptors (src/lidar_odometry.cpp:51-184) on a cloud in device memory, asynchronous
@@ -86,8 +88,7 @@ int frame_run(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int s
     const size_t nt = initial ? k : c->n_prev;
     const unsigned* d_nq = reinterpret_cast<const unsigned*>(c->d_kp_count);
     const unsigned* d_nt = reinterpret_cast<const unsigned*>(initial ? c->d_kp_count : c->d_prev_count);
-    BSHOT_TRY(hamming_match_rq(c, c->d_bits, k, tgt, nt, 0, c->d_cand, d_nq, d_nt));
-    BSHOT_TRY(hamming_mutual_pairs(c, c->d_cand, k, c->d_pairs, c->d_pair_count, d_nq));
+    BSHOT_TRY(match_mutual(c, c->d_bits, k, tgt, nt, d_nq, d_nt));
     BSHOT_TRY(frame_commit(c, k));
     mark(6);
     c->ev_valid = c->timing;

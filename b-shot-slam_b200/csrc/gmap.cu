@@ -72,6 +72,12 @@ __device__ __forceinline__ unsigned gm_find(GmapBlock* tab, unsigned mask, unsig
     return 0xFFFFFFFFu;
 }
 
+// Keypoint::createKeypoint: int(trunc(pos / prec)) * prec on every axis, for a storable position
+__device__ __forceinline__ float3 gm_snap(float3 p) {
+    return make_float3((float)((int)truncf(p.x / GM_LATTICE) * (int)GM_LATTICE), (float)((int)truncf(p.y / GM_LATTICE) * (int)GM_LATTICE),
+                       (float)((int)truncf(p.z / GM_LATTICE) * (int)GM_LATTICE));
+}
+
 // ---- update (addKeypoint for a whole frame) --------------------------------------------------------------------------
 // world position, lattice snap, block slot of every keypoint; first toucher of a block lists it
 __global__ void gm_prepare_kernel(const float4* __restrict__ kp, const float* __restrict__ ratio, const int* __restrict__ count_dev,
@@ -83,20 +89,12 @@ __global__ void gm_prepare_kernel(const float4* __restrict__ kp, const float* __
     const unsigned n = count_dev ? min(n_cap, (unsigned)max(*count_dev, 0)) : n_cap;
     if (i >= n) return;
     const float4 p = kp[i];
-    float x = p.x, y = p.y, z = p.z;
-    if (have_pose) {  // kp_pos = R * kp_pos + T (src/lidar_odometry.cpp:351), row-major 3x4 [R|T]
-        x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[0], p.x), __fmul_rn(pose[1], p.y)), __fmul_rn(pose[2], p.z)), pose[3]);
-        y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[4], p.x), __fmul_rn(pose[5], p.y)), __fmul_rn(pose[6], p.z)), pose[7]);
-        z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[8], p.x), __fmul_rn(pose[9], p.y)), __fmul_rn(pose[10], p.z)), pose[11]);
-    }
+    float3 w = have_pose ? pose_apply_rn(pose, p.x, p.y, p.z) : make_float3(p.x, p.y, p.z);
     // a keypoint that is not storable (a non-finite position or pose, or beyond GM_MAX_MM) is skipped; it is not a drop
-    if (!gm_storable(x, y, z)) { blk_of[i] = 0xFFFFFFFFu; return; }
-    // Keypoint::createKeypoint: int(trunc(pos / prec)) * prec
-    x = (float)((int)truncf(x / GM_LATTICE) * (int)GM_LATTICE);
-    y = (float)((int)truncf(y / GM_LATTICE) * (int)GM_LATTICE);
-    z = (float)((int)truncf(z / GM_LATTICE) * (int)GM_LATTICE);
-    world[i] = make_float4(x, y, z, ratio[i]);
-    const unsigned slot = gm_find(tab, mask, gm_block_id(x, y, z), true);
+    if (!gm_storable(w.x, w.y, w.z)) { blk_of[i] = 0xFFFFFFFFu; return; }
+    w = gm_snap(w);
+    world[i] = make_float4(w.x, w.y, w.z, ratio[i]);
+    const unsigned slot = gm_find(tab, mask, gm_block_id(w.x, w.y, w.z), true);
     blk_of[i] = slot;
     if (slot == 0xFFFFFFFFu) { atomicAdd(&ctl[3], 1u); return; }  // table full: counted, reported by the host
     if (atomicExch(&tab[slot].touched, epoch) != epoch) touched_list[atomicAdd(&ctl[1], 1u)] = slot;
@@ -282,13 +280,8 @@ __global__ void gm_append_ref_kernel(const float4* __restrict__ ref_kp, const ui
     if (i == 0) *total_out = min(base + n, out_cap);
     if (i >= n || base + i >= out_cap) return;
     const float4 p = ref_kp[i];
-    float x = p.x, y = p.y, z = p.z;
-    if (have_pose) {
-        x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[0], p.x), __fmul_rn(pose[1], p.y)), __fmul_rn(pose[2], p.z)), pose[3]);
-        y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[4], p.x), __fmul_rn(pose[5], p.y)), __fmul_rn(pose[6], p.z)), pose[7]);
-        z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(pose[8], p.x), __fmul_rn(pose[9], p.y)), __fmul_rn(pose[10], p.z)), pose[11]);
-    }
-    out_pos[base + i] = make_float4(x, y, z, 0.0f);
+    const float3 w = have_pose ? pose_apply_rn(pose, p.x, p.y, p.z) : make_float3(p.x, p.y, p.z);
+    out_pos[base + i] = make_float4(w.x, w.y, w.z, 0.0f);
 #pragma unroll
     for (int k = 0; k < 6; ++k) out_desc[(size_t)(base + i) * 6 + k] = ref_bits[(size_t)i * 6 + k];
 }
@@ -398,7 +391,7 @@ __global__ void gm_import_chain_kernel(const unsigned long long* __restrict__ sl
 }
 
 // re-anchor: the whole map in map order (*d_n entries), each entry of a changed update u moved by that update's correction
-// C_u (row-major 3x4) with gm_prepare_kernel's arithmetic and snapped to the lattice as createKeypoint does; the entries of
+// C_u (row-major 3x4) and snapped to the lattice as gm_prepare_kernel moves and snaps a keypoint; the entries of
 // unchanged updates are copied as they are.  Written straight into the entry pool at pool index = map-order index, with
 // their descriptors, where the rebuild reads them; *n_out = the count, for the rebuild
 __global__ void gm_reanchor_move_kernel(const float4* __restrict__ apos, const uint64_t* __restrict__ adesc, const unsigned* __restrict__ atag,
@@ -413,16 +406,10 @@ __global__ void gm_reanchor_move_kernel(const float4* __restrict__ apos, const u
     const float4 p = apos[i];
     const unsigned u = atag[i];
     if (u >= n_upd || !changed[u]) { e_pos[i] = p; return; }
-    const float* C = corr + (size_t)u * 12;
-    float x = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[0], p.x), __fmul_rn(C[1], p.y)), __fmul_rn(C[2], p.z)), C[3]);
-    float y = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[4], p.x), __fmul_rn(C[5], p.y)), __fmul_rn(C[6], p.z)), C[7]);
-    float z = __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(C[8], p.x), __fmul_rn(C[9], p.y)), __fmul_rn(C[10], p.z)), C[11]);
+    float3 w = pose_apply_rn(corr + (size_t)u * 12, p.x, p.y, p.z);
     // an entry moved out of the storable range stays unsnapped: the rebuild rejects it and the map is restored
-    if (!gm_storable(x, y, z)) { e_pos[i] = make_float4(x, y, z, p.w); return; }
-    x = (float)((int)truncf(x / GM_LATTICE) * (int)GM_LATTICE);
-    y = (float)((int)truncf(y / GM_LATTICE) * (int)GM_LATTICE);
-    z = (float)((int)truncf(z / GM_LATTICE) * (int)GM_LATTICE);
-    e_pos[i] = make_float4(x, y, z, p.w);
+    if (gm_storable(w.x, w.y, w.z)) w = gm_snap(w);
+    e_pos[i] = make_float4(w.x, w.y, w.z, p.w);
 }
 
 // ---- host side -----------------------------------------------------------------------------------------------------------
@@ -469,9 +456,17 @@ int gmap_reset(Ctx* c) {
     BSHOT_CUDA_TRY(cudaMemsetAsync(g.d_ctl, 0, sizeof(unsigned) * 8, c->stream));
     g.epoch = 0;
     g.n_gathered = 0;
+    g.entries_upper = 0;
     g.n_updates = 0;
     g.last_by_scan = false;
     return BSHOT_OK;
+}
+
+void gmap_record_update(Ctx* c, size_t n_cap, bool by_scan) {
+    Gmap& g = c->gmap;
+    g.entries_upper += n_cap;
+    ++g.n_updates;
+    g.last_by_scan = by_scan;
 }
 
 // ctl: [0] entries, [1] touched blocks of the current update, [2] chunks, [3] dropped (capacity), [4] gathered map entries, [5] probes
@@ -480,7 +475,7 @@ int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t
     if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
     if (n_cap == 0) return BSHOT_OK;
     if (n_cap > c->max_kp) { set_error("map update: %zu keypoints > capacity %zu", n_cap, c->max_kp); return BSHOT_E_CAPACITY; }
-    if (g.n_updates >= g.traj_cap) {   // the trajectory doubles; the caller advances n_updates once the update succeeded
+    if (g.n_updates >= g.traj_cap) {   // the trajectory doubles; gmap_record_update advances n_updates once the update succeeded
         float* grown = nullptr;
         BSHOT_CUDA_TRY(cudaMalloc((void**)&grown, sizeof(float) * 24 * g.traj_cap));
         BSHOT_CUDA_TRY(cudaMemcpyAsync(grown, g.d_traj, sizeof(float) * 12 * g.traj_cap, cudaMemcpyDeviceToDevice, c->stream));
@@ -622,7 +617,6 @@ int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n) {
     Gmap& g = c->gmap;
     if (!g.d_tab) { set_error("map: bshot_gmap_create first"); return BSHOT_E_STATE; }
     BSHOT_TRY(gmap_reset(c));
-    g.entries_upper = 0;
     if (n > g.max_entries) {
         BSHOT_CUDA_TRY(cudaStreamSynchronize(c->stream));
         set_error("bshot_gmap_import: %zu entries > max_entries %u", n, g.max_entries);
@@ -638,8 +632,7 @@ int gmap_import(Ctx* c, const float* xyzr, const uint64_t* desc, size_t n) {
         return rc;
     }
     BSHOT_TRY(rc);
-    g.entries_upper = n;
-    g.n_updates = 1;
+    gmap_record_update(c, n, /*by_scan=*/false);   // update 0
     return BSHOT_OK;
 }
 

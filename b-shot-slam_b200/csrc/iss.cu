@@ -227,18 +227,13 @@ struct Pose12 {
     float m[12];
 };
 
-// R * p + T in fp32, products summed left to right, then the translation (as updateMap, src/lidar_odometry.cpp:351)
-__device__ __forceinline__ float4 apply_pose(const Pose12& P, bool has, float x, float y, float z) {
-    if (!has) return make_float4(x, y, z, 0.0f);
-    const float* m = P.m;
-    return make_float4(__fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[0], x), __fmul_rn(m[1], y)), __fmul_rn(m[2], z)), m[3]),
-                       __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[4], x), __fmul_rn(m[5], y)), __fmul_rn(m[6], z)), m[7]),
-                       __fadd_rn(__fadd_rn(__fadd_rn(__fmul_rn(m[8], x), __fmul_rn(m[9], y)), __fmul_rn(m[10], z)), m[11]), 0.0f);
-}
-
+// the points moved by the pose as updateMap moves keypoints (pose_apply_rn), w = 0
 __global__ void rep_pose_kernel(const float* __restrict__ xyz, unsigned n, Pose12 P, int has, float4* __restrict__ out) {
     const unsigned i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = apply_pose(P, has != 0, xyz[3 * (size_t)i], xyz[3 * (size_t)i + 1], xyz[3 * (size_t)i + 2]);
+    if (i >= n) return;
+    const float x = xyz[3 * (size_t)i], y = xyz[3 * (size_t)i + 1], z = xyz[3 * (size_t)i + 2];
+    const float3 q = has ? pose_apply_rn(P.m, x, y, z) : make_float3(x, y, z);
+    out[i] = make_float4(q.x, q.y, q.z, 0.0f);
 }
 
 // one warp per point of A: nearest point of B by fp32 squared distance, lowest index on ties

@@ -62,6 +62,9 @@ int hamming_tc2_partials(Ctx* c, const void* d_q, size_t nq, const void* d_t, si
 int gmap_create(Ctx* c, size_t max_entries, size_t max_blocks);
 void gmap_free(Ctx* c);
 int gmap_reset(Ctx* c);
+// a map update has succeeded: at most n_cap more entries, the next update number, and whether the update was a scan that is
+// now the reference frame (a step or an accepted relocalisation).  Every kind of update records itself here, once
+void gmap_record_update(Ctx* c, size_t n_cap, bool by_scan);
 // pose_on_device: pose12 / ref_pose12 are device pointers (the odometry step); gmap_gather then takes the position from the
 // translation of ref_pose12 on the device (pos unused)
 int gmap_update(Ctx* c, const float4* d_kp, const float* d_ratio, const uint64_t* d_bits, const int* d_count, size_t n_cap, const float* pose12,
@@ -139,15 +142,17 @@ int kp_repeatability(Ctx* c, const float* a_xyz, size_t na, const float* a_pose,
 int voxel_grid(Ctx* c, const float* xyz, size_t n, int stride_floats, const float inv[3], size_t cap, size_t* count_out);
 void vg_free(Ctx* c);
 
-// per-scan odometry step (odometry.cu): odometry_run takes the cloud already on the device and ends with one
-// synchronisation (the report); odometry_reset is synchronous
+// registration against the map (odometry.cu): the odometry step, relocalisation and loop detection run the same
+// registration (match_mutual, RANSAC, optional ICP, one final kernel, one copy of the report back) on different target
+// sets.  odometry_run takes the cloud already on the device and ends with one synchronisation (the report);
+// odometry_reset is synchronous
 int odom_ensure(Ctx* c);
 void odom_free(Ctx* c);
 int odometry_reset(Ctx* c);
 int odometry_run(Ctx* c, const bshot_odom_params* p, const float* d_cloud, size_t n, int stride_floats, bshot_odom_report* out);
-// relocalisation against the whole map (odometry.cu); the same shape as odometry_run
+// relocalisation against the whole map; the same shape as odometry_run, and the same end when accepted
 int relocalize_run(Ctx* c, const bshot_odom_params* p, int min_inliers, const float* d_cloud, size_t n, int stride_floats, bshot_reloc_report* out);
-// loop detection on the reference frame against the map's older entries (odometry.cu); reads, never changes, the odometry's state
+// loop detection on the reference frame against the map's older entries; reads, never changes, the odometry's state
 int loop_run(Ctx* c, const bshot_loop_params* p, bshot_loop_report* out);
 // re-anchoring (odometry.cu, without FMA): per update u of n, changed[u] = d_new's pose differs from d_traj's in any bit,
 // and then corr[u] = T'_u * T_u^-1 (row-major 3x4); pose_new = the odometry's pose d_pose moved by update n - 1's
@@ -161,13 +166,16 @@ int reanchor_run(Ctx* c, const float* poses3x4, size_t n, float* pose_out);
 
 // whole frame on the resident cloud (frame.cu)
 int frame_extract(Ctx* c, const bshot_params* p, const float* d_raw, size_t n, int stride_floats);
+// mutual nearest neighbours of k query descriptors against nt_cap targets -> c->d_pairs / c->d_pair_count.  d_nq / d_nt
+// (may be null) are the device-side counts within those bounds; nt_cap == 0 only sets the pair count to 0
+int match_mutual(Ctx* c, const uint64_t* d_q, size_t k, const uint64_t* d_t, size_t nt_cap, const unsigned* d_nq = nullptr,
+                 const unsigned* d_nt = nullptr);
 // the current frame becomes the reference frame (descriptors, keypoint positions and count stay on the device).  A set
 // *d_skip (may be null) leaves the reference frame as it is; with a flag the caller sets c->n_prev once it has read it
 int frame_commit(Ctx* c, size_t k, const int* d_skip = nullptr);
 // featureMatching against the map (src/lidar_odometry.cpp:197-206), used by bshot_match_frame_to_map and the odometry step:
 // target set = map keypoints in range ++ the reference frame moved by ref_pose12 (gmap_gather into d_t / gmap.d_tpos, the
-// count in gmap.d_ctl[6]), then the mutual nearest neighbours of the frame's k descriptors -> d_pairs / d_pair_count (0 when
-// the target set is empty by its host-side bound *nt_cap_out)
+// count in gmap.d_ctl[6]), then match_mutual of the frame's k descriptors against it (its bound *nt_cap_out)
 int frame_match_map(Ctx* c, size_t k, const float pos[3], float range, const float* ref_pose12, bool pose_on_device, size_t* nt_cap_out);
 // the target set overflowed max_targets: more candidates than max_targets, and the gather stopped at max_targets.  ctl is
 // gmap.d_ctl after frame_match_map ([4] map keypoints in range, [6] targets assembled)
